@@ -7,7 +7,7 @@ One bench "step" = one RK3 step of integrate! = CFL reduction + 3 fused stage ke
 N > 1: the same workload weak-scaled — every rank owns a 512 x 512 x 512 slab of a 512 x 512 x (512 N)
 grid of cubic cells, 3-plane halos exchanged over NCCL each stage ("scaling": "weak").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--n 512] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--n 512] [--impl reference] [--dump-outputs DIR]
     torchrun --nproc-per-node N ... bench.py --gpus N ...
 
 Prints ONE JSON line (rank 0).  `value` = device-timed (CUDA events on the library's compute stream,
@@ -39,6 +39,8 @@ PERIOD = 3.0
 B_ALG = 136.0          # bytes per cell-update, 3-D f64 RK3 advection with a stored velocity: (8 + 3N) * s (SURVEY.md §8d)
 CPU_SAMPLE_N = 128     # cpu_baseline leg of the main line: the same configuration on a 128^3 grid (~0.12 s per RK3 step on 16 cores)
 REF_SAMPLE_N = 256     # --impl reference: a 256^3 grid (~1 s per RK3 step on 16 cores; 512^3 would take ~8 s per step)
+DUMP_NODES = 1 << 20   # --dump-outputs: nodes of the final level set written (8 MB of values + 8 MB of indices in float64)
+DUMP_SEED = 0
 
 
 def enright_tables(n, nz_glob, lz):
@@ -219,12 +221,25 @@ def timed_steps(m, ctx, eq, steps, warmup, dist, barrier, time_stages=True):
     barrier()
     cnt = ctx.counters()
     ctx.set_option(L.OPT_TIME_STAGES, 0)
+    eq.t = t                                  # lsm_integrate was called directly: record the time integrate! would have left
     if dist is not None:
         import torch
         tt = torch.tensor([ms], dtype=torch.float64, device=f"cuda:{ctx.device}")
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
         ms = float(tt.item())
     return ms, cnt, low
+
+
+def dump_outputs(out_dir, eq):
+    """--dump-outputs: what a caller of the timed path receives after its last step, i.e. the level set and the final time.
+    The level set is written at DUMP_NODES nodes drawn with a fixed seed (all of them on a smaller grid), with their
+    column-major flat indices, so that two builds run with the same arguments can be compared output for output."""
+    phi = eq.state.peek().ravel(order="F")
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(phi.size, min(DUMP_NODES, phi.size), replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "phi_sample.npy"), phi[idx].astype(np.float64))
+    np.save(os.path.join(out_dir, "phi_sample_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "t.npy"), np.array([eq.t], dtype=np.float64))
 
 
 def invariance_check(m, ctx, dist, rank, world, local):
@@ -279,11 +294,15 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="N > 1: skip the C5 1024^3 strong-scaling attachment and the invariance check")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a seeded sample of the final level set and the "
+                                                         "final time to DIR/*.npy (float64); single GPU only")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (args.impl == "reference" or world > 1):
+        raise SystemExit("--dump-outputs writes the outputs of the single-GPU device path (--impl ours, --gpus 1)")
     if args.impl == "reference":
         run_reference(args, rank)
         return
@@ -339,6 +358,8 @@ def main():
     ms, cnt, low = timed_steps(m, ctx, eq, args.steps, args.warmup, dist, barrier)
     clocks = sampler.stop() if sampler else None
     value = nodes_total * args.steps / (ms * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, eq)              # before the e2e leg, which integrates the same state again from phi0
 
     # ---- e2e: the public API with pinned HOST buffers ------------------------------------------------------------------
     # cold  = what a first integrate! sees: H2D of phi AND of the stored velocity (AoS -> SoA on the device), K steps, D2H of phi

@@ -1,7 +1,7 @@
 """Pins the CPU oracle against every exact-value / known-answer check the reference's own
 test-suite and doctests hold for the dense-grid integration path (SURVEY.md §8c).
 
-Each test names the reference test it re-expresses (paths relative to /root/reference).
+Each test names the reference test it re-expresses (paths relative to the root of the LevelSetMethods.jl repository).
 """
 import json
 import math

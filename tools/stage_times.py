@@ -1,6 +1,7 @@
 """Per-step stage-kernel time (CUDA events) of C3 at 512^3 for a dtype; env LSM_B200_NO_FUSE_CFL=1 disables the fused CFL."""
-import sys, ctypes as C
-sys.path[:0] = ["/root/repo", "/root/repo/tests"]
+import os, sys, ctypes as C
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path[:0] = [ROOT, os.path.join(ROOT, "tests")]
 import numpy as np, lsm_b200 as m, helpers as H
 L = m._lib
 dt = np.float32 if len(sys.argv) > 1 and sys.argv[1] == "f32" else np.float64

@@ -60,7 +60,9 @@ enum {
     LSM_COEF_CONST = 0,       /* cval[0..N-1] (velocity) or cval[0]                                        */
     LSM_COEF_FIELD = 1,       /* device field (ncomp = N for a velocity, 1 otherwise)                      */
     LSM_COEF_SEPARABLE = 2,   /* field made by lsm_field_create_separable: u_d = s_d X_d[i1] Y_d[i2] Z_d[i3] */
-    LSM_COEF_NONE = 3         /* EikonalReinitializationTerm() — live sign (levelsetterms.jl:222)           */
+    LSM_COEF_NONE = 3,        /* EikonalReinitializationTerm() — live sign (levelsetterms.jl:222)           */
+    LSM_COEF_EXPR = 4         /* field with expressions attached (lsm_field_set_expr): f(x, t) of levelsetterms.jl:42-43,
+                                 materialised on the device at every time a term needs it; no time factor (t is in the expression) */
 };
 /* time factor g(t) multiplying the coefficient (device-side stand-in for update_func / f(x,t)) */
 enum { LSM_TS_NONE = 0, LSM_TS_COS = 1 /* cos(pi t / tparam) */, LSM_TS_HOST = 2 /* caller passes g per call */ };
@@ -257,6 +259,28 @@ int32_t lsm_field_fill_shape(lsm_field* f, int32_t shape, const double* params, 
 /* Materialise a separable velocity (lsm_field_create_separable) into a stored vector field:
  * u_d[i,j,k] = ((scale_d * X_d[i]) * Y_d[j]) * Z_d[k] — rigid rotation, shear, the Enright field ... from 3 x ndim small tables. */
 int32_t lsm_field_fill_separable(lsm_field* dst, const lsm_field* sep);
+
+/* Function-valued coefficients f(x, t) (_eval_field, levelsetterms.jl:42-43) on the device.  One CUDA C++ expression per component
+ * (ncomp = 1 for a speed or b, ndim for a velocity), evaluated in double with these names in scope: x1 .. xN (the node coordinate
+ * lc_d + i_d h_d, i_d the 0-based global index), t (the evaluation time), pi (the double nearest pi, numpy.pi) and CUDA's
+ * double-precision math functions.  The list `exprs` holds ncomp pointers followed by a NULL pointer.  Rejected with LSM_ERR_ARG
+ * and a message naming the reason: an empty expression, the characters ; { } # " ' \ and the backtick, identifiers starting with
+ * lsm_ or __, an integer-literal division such as 1/3 (0 in C++, 0.333... in Julia and Python), an expression count other than
+ * ncomp, ncomp not in {1, ndim}; an expression NVRTC does not compile (lsm_last_error holds NVRTC's log).  The expressions are
+ * compiled once per process for sm_100a with --fmad=false and without fast-math, so + - * / sqrt fabs fmin fmax give results
+ * bit-identical to the same formula in NumPy float64; values are rounded to the field's dtype on store.  NVRTC is loaded at run
+ * time: without it these entry points fail with LSM_ERR_UNSUPPORTED and the rest of the library is unaffected.
+ * Pure host function (no GPU needed): validate and compile. */
+int32_t lsm_expr_check(int32_t ndim, int32_t ncomp, const char* const* exprs);
+/* Attach f->ncomp expressions to a stored field (compiled, or taken from the process-wide cache).  The field is then usable as an
+ * LSM_COEF_EXPR coefficient: lsm_compute_cfl, lsm_stage, lsm_advance and lsm_integrate materialise it at the time the reference
+ * calls f (the CFL at tc; the stage times tc / tc + dt / tc + dt/2), and the same pass reduces the CFL maximum of the values, so
+ * no separate reduction runs.  An expression set that does not use `t` is materialised once and then behaves exactly like
+ * LSM_COEF_FIELD.  A field whose data was overwritten (upload, copy) is materialised again when a term next needs it. */
+int32_t lsm_field_set_expr(lsm_field* f, const char* const* exprs);
+/* Materialise the attached expressions at time t: MeshField(f, grid) (meshfield.jl:208-211) for any f, the general form of
+ * lsm_field_fill_shape. */
+int32_t lsm_field_fill_expr(lsm_field* f, double t);
 
 /* ---- diagnostics (test harness; SURVEY.md §2.2 K6) -------------------------------------------- */
 /* max |a - b| over all owned nodes, all-reduced over ranks. */

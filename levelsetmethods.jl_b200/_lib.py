@@ -19,7 +19,7 @@ F32, F64 = 0, 1
 BC_NONE, BC_PERIODIC, BC_EXTRAP, BC_SYMMETRY = -1, 0, 1, 2
 TERM_ADVECTION, TERM_NORMAL, TERM_CURVATURE, TERM_EIKONAL = 0, 1, 2, 3
 UPWIND, WENO5 = 0, 1
-COEF_CONST, COEF_FIELD, COEF_SEPARABLE, COEF_NONE = 0, 1, 2, 3
+COEF_CONST, COEF_FIELD, COEF_SEPARABLE, COEF_NONE, COEF_EXPR = 0, 1, 2, 3, 4
 TS_NONE, TS_COS, TS_HOST = 0, 1, 2
 SHAPE_SPHERE, SHAPE_BOX, SHAPE_PLANE, SHAPE_CONST = 0, 1, 2, 3
 FORWARD_EULER, RK2, RK3 = 0, 1, 2
@@ -91,6 +91,9 @@ SYMBOLS = {
     "lsm_field_destroy": (_i32, [_vp]),
     "lsm_field_fill_shape": (_i32, [_vp, _i32, _pdbl, _i32]),
     "lsm_field_fill_separable": (_i32, [_vp, _vp]),
+    "lsm_expr_check": (_i32, [_i32, _i32, C.POINTER(C.c_char_p)]),
+    "lsm_field_set_expr": (_i32, [_vp, C.POINTER(C.c_char_p)]),
+    "lsm_field_fill_expr": (_i32, [_vp, _dbl]),
     "lsm_field_set_bc": (_i32, [_vp, C.POINTER(lsm_bc)]),
     "lsm_field_local_extent": (_i32, [_vp, _pi32, _pi32]),
     "lsm_field_upload": (_i32, [_vp, _vp]),

@@ -15,6 +15,7 @@ from __future__ import annotations
 import ctypes as C
 import math
 import os
+import re
 from typing import Callable, Optional, Sequence
 
 import numpy as np
@@ -398,6 +399,16 @@ class MeshField:
         L.check(L.lib().lsm_field_fill_separable(f._dev, sep.device()))
         return f
 
+    @classmethod
+    def from_expr(cls, grid: CartesianGrid, expr, bc=None, dtype=None, ctx: Optional[Context] = None) -> "MeshField":
+        """Engine extension: ``MeshField(f, grid)`` (meshfield.jl:208-211) for any ``f`` written as a :class:`DeviceExpr` (or its
+        expression strings), evaluated on the device at ``t = 0`` (``lsm_field_fill_expr``)."""
+        expr = expr if isinstance(expr, DeviceExpr) else DeviceExpr(expr)
+        f = cls._device_only(grid, expr.ncomp, bc, dtype, ctx)
+        L.check(L.lib().lsm_field_set_expr(f._dev, expr._carray()))
+        L.check(L.lib().lsm_field_fill_expr(f._dev, 0.0))
+        return f
+
     def _host(self) -> np.ndarray:
         if self._vals is None:
             self._vals = np.empty(self._shape, dtype=self._dtype, order="F")
@@ -570,7 +581,48 @@ class TimeScaled:
     inside the library (so the whole step loop stays on the device)."""
 
     def __init__(self, base, g):
+        if isinstance(base, DeviceExpr):
+            raise ValueError("TimeScaled(DeviceExpr(...)): write the time factor into the expression, which already sees t")
         self.base, self.g = base, g
+
+
+class DeviceExpr:
+    """Engine extension: a function-valued coefficient ``f(x, t)`` (levelsetterms.jl:42-43) evaluated on the DEVICE.  ``exprs`` is
+    one CUDA C++ expression (a speed or ``b``) or a tuple of ``N`` (a velocity) in ``x1 .. xN``, ``t``, ``pi`` and CUDA's double
+    math functions, e.g. ``AdvectionTerm(DeviceExpr(("-x2", "x1")))`` for ``(x, t) -> SVector(-x[2], x[1])``.  The expressions are
+    checked and compiled (NVRTC, sm_100a, once per process) here, so a bad one fails before any GPU work; the engine then
+    materialises the coefficient in HBM at every time the reference would call ``f``.  Without ``t`` the coefficient is
+    materialised once and runs exactly like a stored field."""
+
+    def __init__(self, exprs):
+        self.exprs = (exprs,) if isinstance(exprs, str) else tuple(exprs)
+        if not all(isinstance(e, str) for e in self.exprs):
+            raise TypeError("DeviceExpr takes a string or a tuple of strings")
+        self.ncomp = len(self.exprs)
+        # a velocity has one component per dimension; a scalar is checked for the highest coordinate it names
+        used = [int(k) for e in self.exprs for k in re.findall(r"\bx([1-3])\b", e)]
+        ndim = self.ncomp if self.ncomp > 1 else max(used, default=1)
+        L.check(L.lib().lsm_expr_check(ndim, self.ncomp, self._carray()))
+        self._fields = {}         # (context, grid, dtype) -> MeshField carrying these expressions
+
+    def _carray(self):
+        return (C.c_char_p * (self.ncomp + 1))(*[e.encode() for e in self.exprs], None)
+
+    def _field(self, phi: MeshField, ncomp: int) -> MeshField:
+        """The device field of this coefficient for ``phi``'s context, grid and dtype (created on first use)."""
+        if ncomp != self.ncomp:
+            raise ValueError(f"this coefficient needs {ncomp} expression(s), the DeviceExpr has {self.ncomp}")
+        ctx, g = phi._context(), phi.mesh
+        key = (ctx, g.lc, g.hc, g.n, np.dtype(phi.valtype).str)
+        f = self._fields.get(key)
+        if f is None:
+            f = MeshField._device_only(g, ncomp, None, phi.valtype, ctx)
+            L.check(L.lib().lsm_field_set_expr(f._dev, self._carray()))
+            self._fields[key] = f
+        return f
+
+    def __repr__(self):
+        return f"DeviceExpr({self.exprs!r})"
 
 
 class SeparableVelocity:
@@ -722,6 +774,11 @@ class _Lowered:
         elif isinstance(coef, SeparableVelocity):
             d.coef_kind, d.field = L.COEF_SEPARABLE, coef.device()
             self.keep.append(coef)
+        elif isinstance(coef, DeviceExpr):
+            # f(x, t) on the device: materialised by the library at the CFL and stage times (no host evaluation)
+            f = coef._field(phi, ncomp)
+            d.coef_kind, d.field = L.COEF_EXPR, f.device()
+            self.keep.append(f)
         elif callable(coef):
             # Function-valued coefficient f(x, t) (levelsetterms.jl:43): evaluated on the HOST at the
             # stage time (slow path, like every host callback).  A result that does not depend on x

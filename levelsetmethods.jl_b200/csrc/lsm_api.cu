@@ -130,6 +130,15 @@ struct lsm_field {
     double scale[3] = {1, 1, 1};
     double* d_tabs = nullptr;
     const double* tab[3][3] = {};
+    // expressions attached by lsm_field_set_expr (LSM_COEF_EXPR)
+    const ExprKernel* expr = nullptr;
+    bool expr_filled = false;    // the data holds the expressions at expr_t, materialised at version expr_ver
+    double expr_t = 0;
+    uint64_t expr_ver = 0;
+    int expr_cfl_kind = 0;       // CFL quantity the last fill reduced into d_expr_cfl (ExprArgs::cfl_kind)
+    bool expr_cfl_read = false;  // expr_cfl_bits holds that maximum, all-reduced over ranks
+    unsigned long long expr_cfl_bits = 0;
+    unsigned long long* d_expr_cfl = nullptr;
 };
 
 namespace {
@@ -211,6 +220,7 @@ void field_free(lsm_field* f) {
     if (f->buf2) field_free(f->buf2);
     if (f->base) cudaFree(f->base);
     if (f->d_tabs) cudaFree(f->d_tabs);
+    if (f->d_expr_cfl) cudaFree(f->d_expr_cfl);
     delete f;
 }
 
@@ -279,7 +289,7 @@ int32_t make_term_dev(const lsm_field* phi, const lsm_term& t, double g, TermDev
     if (t.kind == LSM_TERM_EIKONAL && t.coef_kind != LSM_COEF_NONE && t.coef_kind != LSM_COEF_FIELD)
         return fail(LSM_ERR_ARG, "eikonal term takes a frozen S0 field or no coefficient");
     if (t.kind != LSM_TERM_EIKONAL && t.coef_kind == LSM_COEF_NONE) return fail(LSM_ERR_ARG, "term %d needs a coefficient", t.kind);
-    if (t.coef_kind == LSM_COEF_FIELD || t.coef_kind == LSM_COEF_SEPARABLE) {
+    if (t.coef_kind == LSM_COEF_FIELD || t.coef_kind == LSM_COEF_SEPARABLE || t.coef_kind == LSM_COEF_EXPR) {
         const lsm_field* cf = t.field;
         if (!cf) return fail(LSM_ERR_ARG, "coefficient field is NULL");
         if (cf->ctx != phi->ctx) return fail(LSM_ERR_ARG, "coefficient field belongs to another context");
@@ -297,9 +307,59 @@ int32_t make_term_dev(const lsm_field* phi, const lsm_term& t, double g, TermDev
                 else return fail(LSM_ERR_UNSUPPORTED, "Float32 coefficient with a Float64 state is not supported");
             }
             d.coef = cf->p; d.cstride = cf->cstride;
+            d.coef_kind = COEF_FIELD;       // an expression field is read like a stored one once materialised
         }
     }
     *out = d;
+    return LSM_OK;
+}
+
+// ---- expression coefficients (lsm_field_set_expr; the kernel is generated in lsm_expr.cu) ----------------------------------
+// Materialise the expressions of f at time t; cfl_kind != 0 also reduces that CFL quantity of the rounded values into d_expr_cfl.
+int32_t expr_fill(lsm_field* f, double t, int cfl_kind) {
+    lsm_ctx* c = f->ctx;
+    ExprArgs A{};
+    A.dst = f->p; A.cfl = f->d_expr_cfl; A.cstride = f->cstride; A.first_last = f->first_last;
+    A.f64 = f->dtype == LSM_F64; A.cfl_kind = cfl_kind; A.t = t;
+    for (int d = 0; d < 3; ++d) { A.n[d] = f->n[d]; A.lc[d] = f->lc[d]; A.h[d] = d < f->ndim ? f->h[d] : 0.0; }
+    if (cfl_kind) CU(cudaMemsetAsync(f->d_expr_cfl, 0, 8, c->stream));
+    cudaError_t e = launch_expr_fill(f->expr, A, c->sm_count, c->stream);
+    if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "expression kernel launch failed: %s", cudaGetErrorString(e));
+    c->cnt.kernel_launches += 1;
+    f->version++; f->halo_valid = false;
+    f->expr_filled = true; f->expr_t = t; f->expr_ver = f->version;
+    f->expr_cfl_kind = cfl_kind; f->expr_cfl_read = false;
+    return LSM_OK;
+}
+
+// Make f hold its expressions' values at time t for a term of kind term_kind: nothing to do when it already holds them (same
+// time, or no `t` in the expressions, and not overwritten since) and, with need_cfl, the last fill reduced this kind's CFL
+// quantity.  Otherwise one fill, which also reduces that quantity for the next CFL request at t.
+int32_t expr_ensure(lsm_field* f, double t, int term_kind, bool need_cfl) {
+    const int kind = term_kind == LSM_TERM_ADVECTION ? 1 : 2;
+    const bool fresh = f->expr_filled && f->version == f->expr_ver &&
+                       (!expr_uses_t(f->expr) || std::memcmp(&f->expr_t, &t, sizeof t) == 0);
+    if (fresh && (!need_cfl || f->expr_cfl_kind == kind)) return LSM_OK;
+    return expr_fill(f, t, kind);
+}
+
+// LSM_COEF_EXPR terms are checked like stored fields.  An expression set without `t` is materialised once and from then on lowered
+// to LSM_COEF_FIELD, so the CFL cache, graph replay, the resident and the x-pair kernels apply to it unchanged.  A time-dependent
+// one stays LSM_COEF_EXPR: run_stage_t and cfl_term materialise it at the times they need.
+int32_t prepare_terms(lsm_field* phi, const lsm_term* terms, int nterms, lsm_term* out) {
+    for (int k = 0; k < nterms; ++k) {
+        out[k] = terms[k];
+        if (terms[k].coef_kind != LSM_COEF_EXPR) continue;
+        if (terms[k].tscale_kind != LSM_TS_NONE) return fail(LSM_ERR_ARG, "an expression coefficient takes no time factor: t is already in the expression");
+        TermDev td;
+        TRY(make_term_dev(phi, terms[k], 1.0, &td));
+        lsm_field* f = terms[k].field;
+        if (!f->expr) return fail(LSM_ERR_ARG, "LSM_COEF_EXPR needs a field with attached expressions (lsm_field_set_expr)");
+        if (!expr_uses_t(f->expr)) {
+            TRY(expr_ensure(f, 0.0, terms[k].kind, false));
+            out[k].coef_kind = LSM_COEF_FIELD;
+        }
+    }
     return LSM_OK;
 }
 
@@ -387,6 +447,8 @@ int32_t run_stage_t(lsm_ctx* c, lsm_field* in, lsm_field* p0, lsm_field* out, ls
     for (int d = 0; d < 3; ++d) { P.h[d] = in->h[d]; if (d < in->ndim) dxmin = std::min(dxmin, in->h[d]); }
     P.dxmin = dxmin;
     for (int k = 0; k < nterms; ++k) TRY(make_term_dev(in, terms[k], term_scale(terms[k], tstage, gscale, k), &P.terms[k]));
+    for (int k = 0; k < nterms; ++k)
+        if (terms[k].coef_kind == LSM_COEF_EXPR) TRY(expr_ensure(terms[k].field, tstage, terms[k].kind, false));
     P.cfl_out = nullptr; P.cfl_g = 0; P.cfl_tau = 0;
     P.skip_zero_u = c->stage_skip_zero_u;
     if (c->fuse_req.on) {
@@ -751,8 +813,24 @@ int32_t cfl_bits(lsm_ctx* ctx, lsm_field* phi, const lsm_term& t, double g, unsi
 
 double bits_to_double(unsigned long long b) { double d; std::memcpy(&d, &b, 8); return d; }
 
+// CFL maximum of a time-dependent expression coefficient at time t: reduced by the fill that materialised it (at this CFL request,
+// or earlier by a stage at the same time), read once (one 8-byte D2H and a sync, like any coefficient that changes between steps)
+int32_t expr_cfl_bits(lsm_ctx* ctx, lsm_field* f, double t, int term_kind, unsigned long long* bits_out) {
+    TRY(expr_ensure(f, t, term_kind, true));
+    if (!f->expr_cfl_read) {
+        if (ctx->nranks > 1) NC(nccl().AllReduce(f->d_expr_cfl, f->d_expr_cfl, 1, ncclUint64, ncclMax, ctx->nccl_comm, ctx->stream));
+        CU(cudaMemcpyAsync(ctx->h_scalar + 3, f->d_expr_cfl, 8, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaStreamSynchronize(ctx->stream));
+        ctx->cnt.d2h_bytes += 8;
+        f->expr_cfl_bits = ctx->h_scalar[3];
+        f->expr_cfl_read = true;
+    }
+    *bits_out = f->expr_cfl_bits;
+    return LSM_OK;
+}
+
 // _compute_cfl(term, phi, t) for one term (levelsetterms.jl:30-37 + per-node rules)
-int32_t cfl_term(lsm_ctx* ctx, lsm_field* phi, const lsm_term& t, double g, double* dt_out) {
+int32_t cfl_term(lsm_ctx* ctx, lsm_field* phi, const lsm_term& t, double time, double g, double* dt_out) {
     const int N = phi->ndim;
     double dxmin = phi->h[0];
     for (int d = 1; d < N; ++d) dxmin = std::min(dxmin, phi->h[d]);
@@ -772,6 +850,10 @@ int32_t cfl_term(lsm_ctx* ctx, lsm_field* phi, const lsm_term& t, double g, doub
             double v = t.cval[0]; if (scaled) v = v * g;
             m = std::fabs(v);
         }
+    } else if (t.coef_kind == LSM_COEF_EXPR) {
+        unsigned long long bits = 0;
+        TRY(expr_cfl_bits(ctx, t.field, time, t.kind, &bits));
+        m = bits_to_double(bits);
     } else {
         unsigned long long bits = 0;
         TRY(cfl_bits(ctx, phi, t, g, &bits));
@@ -792,7 +874,7 @@ int32_t compute_cfl_impl(lsm_ctx* ctx, lsm_field* phi, const lsm_term* terms, in
     double dt = std::numeric_limits<double>::infinity();
     for (int k = 0; k < nterms; ++k) {
         double d;
-        TRY(cfl_term(ctx, phi, terms[k], term_scale(terms[k], t, gs, k), &d));
+        TRY(cfl_term(ctx, phi, terms[k], t, term_scale(terms[k], t, gs, k), &d));
         dt = k == 0 ? d : jl_min(dt, d);
     }
     *dt_out = dt;
@@ -1267,7 +1349,9 @@ int32_t lsm_compute_cfl(lsm_ctx* ctx, lsm_field* phi, const lsm_term* terms, int
                         const double* gscale, double* dt_out) {
     if (!dt_out) return fail(LSM_ERR_ARG, "null argument");
     TRY(check_state(ctx, phi, terms, nterms));
-    return compute_cfl_impl(ctx, phi, terms, nterms, t, gscale, dt_out);
+    lsm_term tl[LSM_MAX_TERMS];
+    TRY(prepare_terms(phi, terms, nterms, tl));
+    return compute_cfl_impl(ctx, phi, tl, nterms, t, gscale, dt_out);
 }
 
 int32_t lsm_nstages(int32_t integrator) { return nstages(integrator); }
@@ -1275,14 +1359,18 @@ int32_t lsm_nstages(int32_t integrator) { return nstages(integrator); }
 int32_t lsm_stage(lsm_ctx* ctx, int32_t integrator, int32_t stage, lsm_field* phi, const lsm_term* terms,
                   int32_t nterms, double tc, double dt, const double* gscale) {
     TRY(check_state(ctx, phi, terms, nterms));
-    return stage_impl(ctx, integrator, stage, phi, terms, nterms, tc, dt, gscale);
+    lsm_term tl[LSM_MAX_TERMS];
+    TRY(prepare_terms(phi, terms, nterms, tl));
+    return stage_impl(ctx, integrator, stage, phi, tl, nterms, tc, dt, gscale);
 }
 
 int32_t lsm_advance(lsm_ctx* ctx, int32_t integrator, lsm_field* phi, const lsm_term* terms, int32_t nterms,
                     double tc, double dt) {
     TRY(check_state(ctx, phi, terms, nterms));
     if (integrator < LSM_FORWARD_EULER || integrator > LSM_RK3) return fail(LSM_ERR_ARG, "bad integrator %d", integrator);
-    for (int s = 1; s <= nstages(integrator); ++s) TRY(stage_impl(ctx, integrator, s, phi, terms, nterms, tc, dt, nullptr));
+    lsm_term tl[LSM_MAX_TERMS];
+    TRY(prepare_terms(phi, terms, nterms, tl));
+    for (int s = 1; s <= nstages(integrator); ++s) TRY(stage_impl(ctx, integrator, s, phi, tl, nterms, tc, dt, nullptr));
     return LSM_OK;
 }
 
@@ -1294,6 +1382,9 @@ int32_t lsm_integrate(lsm_ctx* ctx, int32_t integrator, double cfl, lsm_field* p
     if (integrator < LSM_FORWARD_EULER || integrator > LSM_RK3) return fail(LSM_ERR_ARG, "bad integrator %d", integrator);
     if (!(tf >= t0))     // levelsetequation.jl:196
         return fail(LSM_ERR_TIME, "final time %g must be >= initial time %g: the level-set equation cannot be solved back in time", tf, t0);
+    lsm_term tl[LSM_MAX_TERMS];
+    TRY(prepare_terms(phi, terms, nterms, tl));
+    terms = tl;
     double tc = t0;
     int64_t steps = 0;
     bool finished = true;
@@ -1304,7 +1395,8 @@ int32_t lsm_integrate(lsm_ctx* ctx, int32_t integrator, double cfl, lsm_field* p
     // dt replays it (one graph launch instead of 2-3 kernel launches plus their host-side setup).
     bool graph_ok = ctx->opt_graph && ctx->nranks == 1 && integrator != LSM_FORWARD_EULER && !ctx->opt_time &&
                     phi->owned <= (1L << 22);
-    for (int k = 0; k < nterms && graph_ok; ++k) if (terms[k].tscale_kind != LSM_TS_NONE) graph_ok = false;
+    // (a time-dependent expression coefficient is materialised at each stage time: a captured fill would freeze t)
+    for (int k = 0; k < nterms && graph_ok; ++k) if (terms[k].tscale_kind != LSM_TS_NONE || terms[k].coef_kind == LSM_COEF_EXPR) graph_ok = false;
     cudaGraphExec_t gexec = nullptr;
     double gdt = 0.0;
     lsm_counters gdelta{};          // counters of one captured step
@@ -1565,6 +1657,35 @@ int32_t lsm_field_fill_separable(lsm_field* dst, const lsm_field* sep) {
     ctx->cnt.kernel_launches += 1;
     dst->version++; dst->halo_valid = false;
     return LSM_OK;
+}
+
+int32_t lsm_expr_check(int32_t ndim, int32_t ncomp, const char* const* exprs) {
+    const ExprKernel* k = nullptr;
+    std::string err;
+    const int32_t rc = expr_get(ndim, ncomp, exprs, false, &k, &err);
+    if (rc != LSM_OK) g_err = err;
+    return rc;
+}
+
+int32_t lsm_field_set_expr(lsm_field* f, const char* const* exprs) {
+    if (!f) return fail(LSM_ERR_ARG, "null field");
+    if (f->separable) return fail(LSM_ERR_ARG, "a separable field cannot carry expressions");
+    CU(cudaSetDevice(f->ctx->device));
+    const ExprKernel* k = nullptr;
+    std::string err;
+    const int32_t rc = expr_get(f->ndim, f->ncomp, exprs, true, &k, &err);
+    if (rc != LSM_OK) { g_err = err; return rc; }
+    if (!f->d_expr_cfl) CU(cudaMalloc(&f->d_expr_cfl, 8));
+    f->expr = k;
+    f->expr_filled = false;
+    return LSM_OK;
+}
+
+int32_t lsm_field_fill_expr(lsm_field* f, double t) {
+    if (!f) return fail(LSM_ERR_ARG, "null field");
+    if (!f->expr) return fail(LSM_ERR_ARG, "no expressions attached: call lsm_field_set_expr first");
+    CU(cudaSetDevice(f->ctx->device));
+    return expr_fill(f, t, 0);
 }
 
 int32_t lsm_max_abs_diff(lsm_ctx* ctx, const lsm_field* a, const lsm_field* b, double* out) {

@@ -1,5 +1,6 @@
 // lsm_kernels.h — launchers implemented by the .cu translation units, called by lsm_api.cu.
 #pragma once
+#include <string>
 #include "lsm_dev.cuh"
 
 namespace lsm {
@@ -44,6 +45,25 @@ struct ShapeParams {
 cudaError_t launch_fill_shape(int f64, void* dst, const ShapeParams& P, cudaStream_t s);
 cudaError_t launch_fill_separable(int f64, void* dst, long cstride, const int* n, int ndim, const double* scale, const double* const (*tab)[3], cudaStream_t s);
 cudaError_t launch_csg(int f64, void* dst, const void* src, long n, int op, cudaStream_t s);
+
+// lsm_expr.cu: coefficients given as CUDA C++ expressions in x1..xN and t, compiled at run time with NVRTC (lsm_field_set_expr)
+struct ExprKernel;             // one compiled pointwise kernel of the process-wide cache (never freed)
+struct ExprArgs {              // the generated kernel's parameter (its device twin is generated in lsm_expr.cu)
+    void* dst;                 // first owned node of component 0 (SoA, components cstride apart)
+    unsigned long long* cfl;   // CFL maximum of the rounded values (IEEE bits, atomicMax), zeroed by the caller; unused when cfl_kind == 0
+    long long cstride;
+    int n[3];                  // owned nodes
+    int first_last;            // global index of the first owned plane of the last dimension
+    int f64;                   // dtype of dst
+    int cfl_kind;              // 0 none, 1 advection (sum_d |u_d| / h_d), 2 normal motion / curvature (|v|)
+    double lc[3], h[3];
+    double t;
+};
+// Validates, generates and compiles (or finds in the cache) the kernel of `exprs` (ncomp pointers, then NULL); load != 0 also
+// loads it for launching (needs a device).  On failure returns an LSM_ERR_* status and the reason in *err.
+int32_t expr_get(int ndim, int ncomp, const char* const* exprs, bool load, const ExprKernel** out, std::string* err);
+bool expr_uses_t(const ExprKernel* k);
+cudaError_t launch_expr_fill(const ExprKernel* k, const ExprArgs& A, int sm_count, cudaStream_t s);
 cudaError_t launch_max_abs_diff(int f64, const void* a, const void* b, long n, unsigned long long* out, cudaStream_t s);
 
 // The five Float64 constants of the WENO5 evaluation that do not fit an instruction immediate travel in the kernel parameters

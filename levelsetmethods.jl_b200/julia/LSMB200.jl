@@ -35,7 +35,7 @@ const LSM_OK, LSM_ERR_ARG, LSM_ERR_CFL, LSM_ERR_TIME, LSM_ERR_BC = Int32(0), Int
 const F32, F64 = Int32(0), Int32(1)
 const BC_PERIODIC, BC_EXTRAP, BC_SYMMETRY = Int32(0), Int32(1), Int32(2)
 const TERM_ADVECTION, TERM_NORMAL, TERM_CURVATURE, TERM_EIKONAL = Int32(0), Int32(1), Int32(2), Int32(3)
-const COEF_CONST, COEF_FIELD, COEF_SEPARABLE, COEF_NONE = Int32(0), Int32(1), Int32(2), Int32(3)
+const COEF_CONST, COEF_FIELD, COEF_SEPARABLE, COEF_NONE, COEF_EXPR = Int32(0), Int32(1), Int32(2), Int32(3), Int32(4)
 const TS_NONE, TS_COS, TS_HOST = Int32(0), Int32(1), Int32(2)
 const SHAPE_SPHERE, SHAPE_BOX, SHAPE_PLANE, SHAPE_CONST = Int32(0), Int32(1), Int32(2), Int32(3)
 
@@ -287,6 +287,56 @@ function from_separable(s::SeparableVelocity{N, T}; S::Type = Float64) where {N,
     return d
 end
 
+"""
+    DeviceFunction(exprs...)
+
+A function-valued coefficient `f(x, t)` (`_eval_field`, levelsetterms.jl:42-43) evaluated on the DEVICE: one CUDA C++ expression per
+component in `x1 .. xN`, `t`, `pi` and CUDA's double math functions, e.g. `AdvectionTerm(DeviceFunction("-x2", "x1"))` for
+`(x, t) -> SVector(-x[2], x[1])`.  Checked and compiled (NVRTC, sm_100a, once per process) by the constructor; the library then
+materialises the coefficient in HBM at every time the reference would call `f`, so `integrate!` stays one `lsm_integrate` call.
+"""
+struct DeviceFunction
+    exprs::Vector{String}
+    fields::Vector{Any}       # [(ctx, grid, V, DeviceMeshField), ...]: one device field per context, grid and valtype
+end
+function _cexprs(f, exprs::Vector{String})
+    ptrs = Ptr{UInt8}[pointer(e) for e in exprs]
+    push!(ptrs, C_NULL)       # the list ends with a NULL pointer
+    return GC.@preserve exprs ptrs f(ptrs)
+end
+function DeviceFunction(exprs::AbstractString...)
+    ex = String[exprs...]
+    used = [parse(Int, m.captures[1]) for e in ex for m in eachmatch(r"\bx([1-3])\b", e)]
+    ndim = length(ex) > 1 ? length(ex) : maximum(used; init = 1)
+    _cexprs(ex) do p
+        check(ccall((:lsm_expr_check, LIB), Int32, (Int32, Int32, Ptr{Ptr{UInt8}}), ndim, length(ex), p))
+    end
+    return DeviceFunction(ex, Any[])
+end
+function _set_expr(d::DeviceMeshField, f::DeviceFunction)
+    _cexprs(f.exprs) do p
+        check(ccall((:lsm_field_set_expr, LIB), Int32, (Ptr{Cvoid}, Ptr{Ptr{UInt8}}), d.handle, p))
+    end
+    return d
+end
+"The device field of `f` for this context, grid and valtype (created on first use; the library fills it when a term needs it)."
+function device_field(f::DeviceFunction, ctx::Context, g::LSM.CartesianGrid{N}, ::Type{V}) where {N, V}
+    for (c, gg, VV, d) in f.fields
+        c === ctx && gg == g && VV === V && return d
+    end
+    d = _set_expr(_device_only(g, V, nothing, ctx), f)
+    push!(f.fields, (ctx, g, V, d))
+    return d
+end
+"`MeshField(f, grid)` (meshfield.jl:208-211) for any `f` written as a `DeviceFunction`, evaluated on the device at `t = 0`."
+function from_expr(g::LSM.CartesianGrid{N, T}, expr; bc = nothing, V::Type = Float64, ctx::Context = default_context()) where {N, T}
+    f = expr isa DeviceFunction ? expr : DeviceFunction((expr isa AbstractString ? (expr,) : expr)...)
+    bcs = isnothing(bc) ? nothing : LSM._normalize_bc(bc, N)
+    d = _set_expr(_device_only(g, length(f.exprs) == 1 ? V : SVector{N, V}, bcs, ctx), f)
+    check(ccall((:lsm_field_fill_expr, LIB), Int32, (Ptr{Cvoid}, Float64), d.handle, 0.0))
+    return d
+end
+
 # ---- device mirrors of host coefficient fields, cached per host array -------------------------------------------------------
 # A MeshField coefficient (velocity, speed, b, S₀) is uploaded ONCE per (context, host array) and reused by every later
 # compute_cfl / stage / integrate! call.  A term with a non-default update_func may rewrite its coefficient: its mirror is
@@ -319,7 +369,7 @@ struct Lowered
     device_only::Bool         # nothing needs the host between steps
 end
 
-function lower(terms, ϕ::DeviceMeshField{N}, t) where {N}
+function lower(terms, ϕ::DeviceMeshField{N, T, V}, t) where {N, T, V}
     ctx = ϕ.ctx
     out, gs, keep, device_only = CTerm[], Float64[], Any[], true
     for term in terms
@@ -328,6 +378,7 @@ function lower(terms, ϕ::DeviceMeshField{N}, t) where {N}
         custom && (device_only = false)
         ts, tp, g = TS_NONE, 1.0, 1.0
         if coef isa TimeScaled
+            coef.base isa DeviceFunction && throw(ArgumentError("TimeScaled(DeviceFunction): write the time factor into the expression, which already sees t"))
             if coef.g isa CosScale
                 ts, tp = TS_COS, coef.g.period
             else
@@ -345,6 +396,13 @@ function lower(terms, ϕ::DeviceMeshField{N}, t) where {N}
             d = mirror(ctx, coef)
             custom && coef isa LSM.MeshField && refresh!(d)
             ck, fld = COEF_FIELD, handle!(d)
+            push!(keep, d)
+        elseif coef isa DeviceFunction
+            # f(x, t) on the device: the library materialises it at the CFL and stage times
+            nc = kind == TERM_ADVECTION ? N : 1
+            length(coef.exprs) == nc || throw(ArgumentError("this coefficient needs $nc expression(s), the DeviceFunction has $(length(coef.exprs))"))
+            d = device_field(coef, ctx, LSM.mesh(ϕ), nc == 1 ? V : SVector{N, V})
+            ck, fld = COEF_EXPR, d.handle
             push!(keep, d)
         elseif coef isa Function
             # f(x, t) (levelsetterms.jl:43): evaluated on the host at the stage time, like every host callback (slow path)

@@ -282,6 +282,39 @@ int32_t lsm_field_set_expr(lsm_field* f, const char* const* exprs);
  * lsm_field_fill_shape. */
 int32_t lsm_field_fill_expr(lsm_field* f, double t);
 
+/* ---- zero-level-set extraction: the interface {phi = level} as a compact mesh, so that only the mesh leaves the device ------
+ * The reference draws the interface from values(phi) on the host (ext/MakieExt.jl); these entry points replace that download.
+ * Marching simplices on the Freudenthal–Kuhn triangulation of the node lattice (no case tables, no ambiguous cases, watertight):
+ *  - s = double(phi) - level; a node is inside if s <= 0, outside if s > 0, invalid if s is NaN.  level must be finite and every
+ *    n_d >= 2 (else LSM_ERR_ARG).
+ *  - cells are the global lower corners c, 0 <= c_d <= n_d - 2, in column-major order; cell c is split into N! simplices, one per
+ *    permutation pi of the axes in lexicographic order: w_0 = c, w_k = w_{k-1} + e_pi(k).  A simplex with an invalid vertex emits
+ *    nothing.
+ *  - vertices: the edge (a, b) = (w_i, w_j), i < j, e = b - a in {0,1}^N, is cut when one end is inside and the other outside.  Its
+ *    key is lin(a) (2^N - 1) + sum_d e_d 2^(d-1) - 1 (lin: global 0-based column-major node index, d = 1..N).  With
+ *    t = s_a / (s_a - s_b):  x_d = lc_d + (a_d + t) h_d where e_d = 1,  x_d = lc_d + a_d h_d where e_d = 0 (double, each operation
+ *    rounded, no FMA).  Vertices are sorted by key, one per cut lattice edge of the grid.
+ *  - primitives, N vertex indices each (0-based int32), in cell order, then simplex order, then as listed:
+ *      1-D: a point;  2-D: one segment per cut triangle, with the inside on its left;
+ *      3-D: a lone inside or outside vertex q: one triangle (qr, qs, qu), r < s < u in chain order, last two swapped if needed;
+ *           inside {a < b}, outside {c < d}: the quad (ac, ad, bd, bc) as (ac, ad, bd), (ac, bd, bc), or (ac, bd, ad), (ac, bc, bd);
+ *      every triangle is oriented so that (v1 - v0) x (v2 - v0) points toward s > 0, by a rule on pi, the inside mask and the signs
+ *      of h only, so triangles made degenerate by exact zeros at nodes are oriented consistently too.
+ *    This makes about 9 triangles per h^2 of interface against about 2 for marching cubes: the price of having no ambiguity.
+ *  - periodic axes: node n duplicates node 1, so no cell wraps; boundary conditions play no role.
+ * More than 2^31 - 1 vertices: LSM_ERR_UNSUPPORTED.  Scalar, non-separable fields only.
+ * With nranks > 1 rank r extracts the cells whose lower corner it owns (the call exchanges the ghost planes first when they are
+ * stale, so it is collective); a piece's vertices are the cut edges of its cells, so edges in a slab-boundary plane appear in two
+ * pieces with the same global key: welding the pieces by key gives the single-GPU mesh bit for bit.
+ * Blocking: one synchronisation and a 16-byte copy of the two counts; the mesh stays on the device in the context's persistent
+ * scratch (grown on demand) until the next extraction on this context replaces it. */
+int32_t lsm_interface_extract(lsm_ctx* ctx, lsm_field* phi, double level, int64_t* nverts_out, int64_t* nprims_out);
+/* Copy the last extraction of this context to the host: verts (nverts x ndim doubles, AoS), keys (nverts, may be NULL) and prims
+ * (nprims x ndim int32).  An array may be NULL when its count is 0.  LSM_ERR_ARG if nothing has been extracted on this context. */
+int32_t lsm_interface_fetch(lsm_ctx* ctx, double* verts, int64_t* keys, int32_t* prims);
+/* lsm_interface_extract on every rank of a lsm_ctx_create_multi box, on one host thread per GPU; counts per rank (n entries each). */
+int32_t lsm_multi_interface_extract(int32_t n, lsm_ctx* const* ctx, lsm_field* const* phi, double level, int64_t* nverts_out, int64_t* nprims_out);
+
 /* ---- diagnostics (test harness; SURVEY.md §2.2 K6) -------------------------------------------- */
 /* max |a - b| over all owned nodes, all-reduced over ranks. */
 int32_t lsm_max_abs_diff(lsm_ctx* ctx, const lsm_field* a, const lsm_field* b, double* out);

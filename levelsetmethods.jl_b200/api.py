@@ -16,7 +16,7 @@ import ctypes as C
 import math
 import os
 import re
-from typing import Callable, Optional, Sequence
+from typing import Callable, NamedTuple, Optional, Sequence
 
 import numpy as np
 
@@ -965,6 +965,60 @@ def perimeter(phi) -> float:
     out = C.c_double()
     L.check(L.lib().lsm_perimeter(phi._context().handle, phi.device(), C.byref(out)))
     return out.value
+
+
+class InterfaceMesh(NamedTuple):
+    """The zero level set as a piecewise-linear mesh (``lsm_interface_extract``): ``vertices`` (nv, N) float64, ``faces`` (np, N)
+    int32 0-based vertex indices (triangles in 3-D, segments in 2-D, points in 1-D), and ``keys`` (nv,) int64, the global id of
+    the lattice edge each vertex lies on (sorted; what :func:`merge_interfaces` welds on)."""
+    vertices: np.ndarray
+    faces: np.ndarray
+    keys: np.ndarray
+
+
+def _fetch_interface(ctx: Context, ndim: int, nv: int, nf: int) -> InterfaceMesh:
+    V = np.empty((nv, ndim), dtype=np.float64)
+    K = np.empty(nv, dtype=np.int64)
+    F = np.empty((nf, ndim), dtype=np.int32)
+    ptr = lambda a, t: C.cast(a.ctypes.data, C.POINTER(t)) if a.size else None
+    L.check(L.lib().lsm_interface_fetch(ctx.handle, ptr(V, C.c_double), ptr(K, C.c_int64), ptr(F, C.c_int32)))
+    return InterfaceMesh(V, F, K)
+
+
+def extract_interface(phi, level: float = 0.0) -> InterfaceMesh:
+    """Engine extension: the interface {phi = level} extracted on the device (marching simplices on the Freudenthal–Kuhn
+    triangulation, include/lsm_b200.h); only the mesh is copied to the host, not the field.  Triangles are oriented so that their
+    normal points toward phi > level; segments have phi <= level on their left.  The reference draws the interface from
+    ``values(phi)`` (ext/MakieExt.jl)."""
+    phi = current_state(phi)
+    ctx = phi._context()
+    nv, nf = C.c_int64(), C.c_int64()
+    L.check(L.lib().lsm_interface_extract(ctx.handle, phi.device(), float(level), C.byref(nv), C.byref(nf)))
+    return _fetch_interface(ctx, phi.ndim, nv.value, nf.value)
+
+
+def merge_interfaces(pieces: Sequence[InterfaceMesh]) -> InterfaceMesh:
+    """Weld the per-rank pieces of an extraction (in rank order) into one mesh: vertices with the same key are one vertex.  The
+    result equals the single-GPU extraction of the whole field."""
+    if not pieces:
+        raise ValueError("merge_interfaces needs at least one piece")
+    keys = np.concatenate([p.keys for p in pieces])
+    uniq, first, inv = np.unique(keys, return_index=True, return_inverse=True)
+    V = np.concatenate([p.vertices for p in pieces], axis=0)[first]
+    base = np.cumsum([0] + [len(p.keys) for p in pieces[:-1]])
+    F = np.concatenate([inv[p.faces.astype(np.int64) + b] for p, b in zip(pieces, base)], axis=0).astype(np.int32)
+    return InterfaceMesh(V, F.reshape(-1, pieces[0].faces.shape[1]), uniq.astype(np.int64))
+
+
+def extract_interface_multi(mc: MultiContext, phis, level: float = 0.0) -> InterfaceMesh:
+    """:func:`extract_interface` of a field slab-decomposed over ``mc`` (collective): each rank extracts the cells it owns, and the
+    pieces are welded on the host (:func:`merge_interfaces`)."""
+    n = len(mc)
+    phis = [current_state(p) for p in phis]
+    nv, nf = (C.c_int64 * n)(), (C.c_int64 * n)()
+    L.check(L.lib().lsm_multi_interface_extract(
+        n, (C.c_void_p * n)(*[c.handle for c in mc.ranks]), (C.c_void_p * n)(*[p.device() for p in phis]), float(level), nv, nf))
+    return merge_interfaces([_fetch_interface(mc.ranks[r], phis[r].ndim, nv[r], nf[r]) for r in range(n)])
 
 
 def _csg(dst: MeshField, src: Optional[MeshField], op: int) -> MeshField:

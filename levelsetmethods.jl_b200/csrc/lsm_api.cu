@@ -105,6 +105,11 @@ struct lsm_ctx {
     struct { bool valid = false; const void* field = nullptr; uint64_t version = 0; double g = 0; } fused;
     int opt_fuse_cfl = 1;
     int opt_graph = 1;          // lsm_integrate replays a captured CUDA graph of the stage launches on small grids
+    // the mesh of the last lsm_interface_extract (persistent, grown on demand): nverts x ndim doubles, nverts keys, nprims x ndim int32
+    void* d_iface = nullptr; size_t d_iface_bytes = 0;
+    bool iface_valid = false;
+    int iface_ndim = 0;
+    int64_t iface_nv = 0, iface_np = 0;
 };
 
 struct lsm_field {
@@ -882,6 +887,63 @@ int32_t compute_cfl_impl(lsm_ctx* ctx, lsm_field* phi, const lsm_term* terms, in
     return LSM_OK;
 }
 
+// ---- zero-level-set extraction (lsm_interface.cu) ----------------------------------------------
+int32_t interface_extract_impl(lsm_ctx* ctx, lsm_field* phi, double level, int64_t* nverts_out, int64_t* nprims_out) {
+    if (!ctx || !phi || !nverts_out || !nprims_out) return fail(LSM_ERR_ARG, "null argument");
+    ctx->iface_valid = false;                   // a failed extraction leaves nothing to fetch
+    if (phi->ctx != ctx || phi->ncomp != 1 || phi->separable) return fail(LSM_ERR_ARG, "interface extraction needs a real-valued field of this context");
+    if (!std::isfinite(level)) return fail(LSM_ERR_ARG, "level must be finite (got %g)", level);
+    for (int d = 0; d < phi->ndim; ++d)
+        if (phi->nglob[d] < 2) return fail(LSM_ERR_ARG, "interface extraction needs at least 2 nodes along every dimension (n[%d] = %d)", d, phi->nglob[d]);
+    CU(cudaSetDevice(ctx->device));
+    CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_halo, 0));
+    // the cells of the rank's last owned plane reach into the next rank's first plane (the upper ghost plane); the exchange is
+    // collective, so every rank takes part
+    const int last = phi->ndim - 1;
+    const bool ghost = ctx->nranks > 1 && ctx->rank < ctx->nranks - 1;
+    if (ctx->nranks > 1 && !phi->halo_valid) TRY(exchange_halo(phi, ctx->stream));
+    IfaceArgs A{};
+    A.phi = phi->p; A.f64 = phi->dtype == LSM_F64; A.ndim = phi->ndim; A.level = level;
+    A.first_last = phi->first_last;
+    A.hsign = 1;
+    for (int d = 0; d < 3; ++d) {
+        A.m[d] = phi->n[d] + (d == last && ghost ? 1 : 0);
+        A.lc[d] = phi->lc[d]; A.h[d] = d < phi->ndim ? phi->h[d] : 0.0;
+        if (d < phi->ndim && phi->h[d] < 0) A.hsign = -A.hsign;
+    }
+    A.s1 = A.m[0]; A.s2 = (long long)A.m[0] * A.m[1];
+    A.nodes = (long long)A.m[0] * A.m[1] * A.m[2];
+    A.ntiles = iface_tiles(A.nodes);
+    A.lin0 = (long long)phi->first_last * phi->plane;
+    void* work = nullptr;
+    TRY(ctx_scratch(ctx, iface_scratch_bytes(A.ntiles), &work));
+    CU(launch_iface(A, 0, work, nullptr, nullptr, nullptr, ctx->stream));
+    CU(cudaMemcpyAsync(ctx->h_scalar, iface_totals(A, work), 16, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    ctx->cnt.kernel_launches += 2; ctx->cnt.d2h_bytes += 16;
+    const int64_t nv = (int64_t)ctx->h_scalar[0], np = (int64_t)ctx->h_scalar[1];
+    if (nv > (int64_t)std::numeric_limits<int32_t>::max())
+        return fail(LSM_ERR_UNSUPPORTED, "the interface has %lld vertices; int32 vertex indices hold at most 2^31 - 1", (long long)nv);
+    const int N = phi->ndim;
+    const size_t vbytes = (size_t)nv * N * sizeof(double), kbytes = (size_t)nv * sizeof(int64_t), pbytes = (size_t)np * N * sizeof(int32_t);
+    const size_t need = vbytes + kbytes + pbytes;
+    if (need > ctx->d_iface_bytes) {
+        if (ctx->d_iface) cudaFree(ctx->d_iface);           // implicit synchronisation: nothing in flight reads it
+        ctx->d_iface = nullptr; ctx->d_iface_bytes = 0;
+        CU(cudaMalloc(&ctx->d_iface, need));
+        ctx->d_iface_bytes = need;
+    }
+    char* base = static_cast<char*>(ctx->d_iface);
+    double* verts = reinterpret_cast<double*>(base);
+    long long* keys = reinterpret_cast<long long*>(base + vbytes);
+    int* prims = reinterpret_cast<int*>(base + vbytes + kbytes);
+    if (nv > 0) { CU(launch_iface(A, 1, work, verts, keys, prims, ctx->stream)); ctx->cnt.kernel_launches += 1; }
+    if (np > 0) { CU(launch_iface(A, 2, work, verts, keys, prims, ctx->stream)); ctx->cnt.kernel_launches += 1; }
+    ctx->iface_valid = true; ctx->iface_ndim = N; ctx->iface_nv = nv; ctx->iface_np = np;
+    *nverts_out = nv; *nprims_out = np;
+    return LSM_OK;
+}
+
 }  // namespace
 
 // =================================================================================================
@@ -1008,6 +1070,11 @@ int32_t lsm_multi_integrate(int32_t n, lsm_ctx* const* ctx, int32_t integrator, 
     return LSM_OK;
 }
 
+int32_t lsm_multi_interface_extract(int32_t n, lsm_ctx* const* ctx, lsm_field* const* phi, double level, int64_t* nverts_out, int64_t* nprims_out) {
+    if (!ctx || !phi || !nverts_out || !nprims_out || n < 1) return fail(LSM_ERR_ARG, "bad argument");
+    return fan_out(n, [&](int r) { return interface_extract_impl(ctx[r], phi[r], level, &nverts_out[r], &nprims_out[r]); });
+}
+
 int32_t lsm_ctx_destroy(lsm_ctx* c) {
     if (!c) return LSM_OK;
     cudaSetDevice(c->device);
@@ -1020,6 +1087,7 @@ int32_t lsm_ctx_destroy(lsm_ctx* c) {
     if (c->h_scalar) cudaFreeHost(c->h_scalar);
     for (int b = 0; b < 2; ++b) { if (c->stage[b]) cudaFree(c->stage[b]); if (c->ev_stage[b]) cudaEventDestroy(c->ev_stage[b]); if (c->ev_free[b]) cudaEventDestroy(c->ev_free[b]); }
     if (c->d_work) cudaFree(c->d_work);
+    if (c->d_iface) cudaFree(c->d_iface);
     if (c->d_cand) cudaFree(c->d_cand);
     if (c->d_cand_count) cudaFree(c->d_cand_count);
     if (c->h_cand) cudaFreeHost(c->h_cand);
@@ -1605,6 +1673,27 @@ int32_t lsm_extend_along_normals(lsm_ctx* ctx, lsm_field* F, lsm_field* phi, int
     if (rc != LSM_OK) return rc;
     if (e != cudaSuccess || e2 != cudaSuccess) return fail(LSM_ERR_CUDA, "extend_along_normals failed: %s", cudaGetErrorString(e != cudaSuccess ? e : e2));
     F->version++;
+    return LSM_OK;
+}
+
+int32_t lsm_interface_extract(lsm_ctx* ctx, lsm_field* phi, double level, int64_t* nverts_out, int64_t* nprims_out) {
+    return interface_extract_impl(ctx, phi, level, nverts_out, nprims_out);
+}
+
+int32_t lsm_interface_fetch(lsm_ctx* ctx, double* verts, int64_t* keys, int32_t* prims) {
+    if (!ctx) return fail(LSM_ERR_ARG, "null context");
+    if (!ctx->iface_valid) return fail(LSM_ERR_ARG, "no interface has been extracted on this context");
+    const int64_t nv = ctx->iface_nv, np = ctx->iface_np;
+    if ((nv > 0 && !verts) || (np > 0 && !prims)) return fail(LSM_ERR_ARG, "null output array");
+    CU(cudaSetDevice(ctx->device));
+    const size_t vbytes = (size_t)nv * ctx->iface_ndim * sizeof(double), kbytes = (size_t)nv * sizeof(int64_t);
+    const size_t pbytes = (size_t)np * ctx->iface_ndim * sizeof(int32_t);
+    const char* base = static_cast<const char*>(ctx->d_iface);
+    if (vbytes) CU(cudaMemcpyAsync(verts, base, vbytes, cudaMemcpyDeviceToHost, ctx->stream));
+    if (kbytes && keys) CU(cudaMemcpyAsync(keys, base + vbytes, kbytes, cudaMemcpyDeviceToHost, ctx->stream));
+    if (pbytes) CU(cudaMemcpyAsync(prims, base + vbytes + kbytes, pbytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    ctx->cnt.d2h_bytes += (int64_t)(vbytes + (keys ? kbytes : 0) + pbytes);
     return LSM_OK;
 }
 

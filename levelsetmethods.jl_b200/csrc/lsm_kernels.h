@@ -66,6 +66,26 @@ bool expr_uses_t(const ExprKernel* k);
 cudaError_t launch_expr_fill(const ExprKernel* k, const ExprArgs& A, int sm_count, cudaStream_t s);
 cudaError_t launch_max_abs_diff(int f64, const void* a, const void* b, long n, unsigned long long* out, cudaStream_t s);
 
+// lsm_interface.cu: zero-level-set extraction (lsm_interface_extract).  The node box is this rank's owned nodes plus, below the
+// last rank, the first plane of the next rank (the upper ghost plane), so that every cell whose lower corner the rank owns is whole.
+struct IfaceArgs {
+    const void* phi;           // first node of the box (dense column-major, dim 1 contiguous)
+    int f64, ndim;
+    int m[3];                  // box nodes per dim (1 for unused dims)
+    int first_last;            // global index of the box's first plane of the last dimension
+    int hsign;                 // sign of prod_d h_d: a mirrored grid mirrors every simplex
+    long long s1, s2;          // element strides of dims 2 and 3
+    long long nodes, ntiles;   // nodes in the box, tiles of the passes
+    long long lin0;            // global column-major index of the box's first node
+    double level;
+    double lc[3], h[3];
+};
+long long iface_tiles(long long nodes);
+size_t iface_scratch_bytes(long long ntiles);
+long long* iface_totals(const IfaceArgs& A, void* scratch);     // device address of (nverts, nprims) after pass 0
+// pass 0: count + scan (totals at iface_totals); pass 1: vertices and keys; pass 2: primitives (needs the keys of pass 1)
+cudaError_t launch_iface(const IfaceArgs& A, int pass, void* scratch, double* verts, long long* keys, int* prims, cudaStream_t s);
+
 // The five Float64 constants of the WENO5 evaluation that do not fit an instruction immediate travel in the kernel parameters
 // (constant bank): as literals the compiler re-materialises them with 10 UMOV per node, from the constant bank it takes 3 uniform loads.
 struct WenoK { double c133, c56, cm13, e6, fl, pad; };

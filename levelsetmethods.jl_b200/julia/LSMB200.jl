@@ -523,6 +523,59 @@ function LSM.perimeter(ϕ::DeviceMeshField)
     return out[]
 end
 
+"""
+    interface_mesh(ϕ::DeviceMeshField{N}; level = 0) -> (vertices, faces, keys)
+
+The interface {ϕ = level} extracted on the device (`lsm_interface_extract`: marching simplices on the Freudenthal–Kuhn
+triangulation, watertight, triangles oriented toward ϕ > level, segments with ϕ <= level on their left); only the mesh is copied
+back, not `values(ϕ)`.  `vertices::Vector{SVector{N,Float64}}`, `faces::Vector{NTuple{N,Int32}}` (1-based): the arrays
+`Makie.mesh` (3-D) and `linesegments` (2-D) take.  `keys` are the global lattice-edge ids of the vertices (sorted).
+"""
+function interface_mesh(ϕ::DeviceMeshField{N}; level::Real = 0) where {N}
+    nv, np = Ref{Int64}(0), Ref{Int64}(0)
+    check(ccall((:lsm_interface_extract, LIB), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Float64, Ref{Int64}, Ref{Int64}),
+                ϕ.ctx.handle, handle!(ϕ), Float64(level), nv, np))
+    return _fetch_interface(ϕ.ctx, Val(N), nv[], np[])
+end
+
+function _fetch_interface(ctx::Context, ::Val{N}, nv::Integer, np::Integer) where {N}
+    V = Matrix{Float64}(undef, N, nv)          # AoS: vertex-major, N coordinates each
+    K = Vector{Int64}(undef, nv)
+    P = Matrix{Int32}(undef, N, np)
+    check(ccall((:lsm_interface_fetch, LIB), Int32, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Int64}, Ptr{Int32}),
+                ctx.handle, nv == 0 ? C_NULL : pointer(V), nv == 0 ? C_NULL : pointer(K), np == 0 ? C_NULL : pointer(P)))
+    verts = [SVector{N, Float64}(ntuple(d -> V[d, j], N)) for j in 1:nv]
+    faces = [ntuple(d -> P[d, j] + Int32(1), N) for j in 1:np]
+    return verts, faces, K
+end
+
+"`interface_mesh` of a field slab-decomposed over `mc` (collective, `lsm_multi_interface_extract`): the per-rank pieces welded by key."
+function interface_mesh(mc::MultiContext, ϕs::Vector{<:DeviceMeshField{N}}; level::Real = 0) where {N}
+    n = length(mc.ranks)
+    nv, np = zeros(Int64, n), zeros(Int64, n)
+    check(ccall((:lsm_multi_interface_extract, LIB), Int32, (Int32, Ptr{Ptr{Cvoid}}, Ptr{Ptr{Cvoid}}, Float64, Ptr{Int64}, Ptr{Int64}),
+                n, [c.handle for c in mc.ranks], [handle!(ϕ) for ϕ in ϕs], Float64(level), nv, np))
+    pieces = [_fetch_interface(mc.ranks[r], Val(N), nv[r], np[r]) for r in 1:n]
+    keys = reduce(vcat, [p[3] for p in pieces])
+    verts_all = reduce(vcat, [p[1] for p in pieces])
+    perm = sortperm(keys; alg = MergeSort)
+    newidx = Vector{Int32}(undef, length(keys))
+    verts, ukeys = SVector{N, Float64}[], Int64[]
+    for j in perm
+        if isempty(ukeys) || keys[j] != ukeys[end]
+            push!(verts, verts_all[j]); push!(ukeys, keys[j])
+        end
+        newidx[j] = length(ukeys)
+    end
+    faces = NTuple{N, Int32}[]
+    off = 0
+    for p in pieces
+        append!(faces, [ntuple(d -> newidx[f[d] + off], N) for f in p[2]])
+        off += length(p[3])
+    end
+    return verts, faces, ukeys
+end
+
 "`extend_along_normals!(F, ϕ; …)` — src/velocityextension.jl:20-78 on device fields."
 function LSM.extend_along_normals!(F::DeviceMeshField, ϕ::DeviceMeshField; nb_iters::Integer = 50, cfl::Real = 0.45, frozen = nothing,
                                    interface_band::Real = 1.5, min_norm::Real = 1.0e-14)

@@ -315,6 +315,44 @@ int32_t lsm_interface_fetch(lsm_ctx* ctx, double* verts, int64_t* keys, int32_t*
 /* lsm_interface_extract on every rank of a lsm_ctx_create_multi box, on one host thread per GPU; counts per rank (n entries each). */
 int32_t lsm_multi_interface_extract(int32_t n, lsm_ctx* const* ctx, lsm_field* const* phi, double level, int64_t* nverts_out, int64_t* nprims_out);
 
+/* ---- closest-point redistancing: phi <- the signed distance to its own zero-level-set mesh, on the device ----------------------
+ * The reference reinitialises phi between steps with reinitialize! (reinitializer.jl:12-42: Newton on Bernstein patches found with
+ * a KD-tree, on the host, after downloading values(phi)).  lsm_redistance does the same on the device with the linear interface:
+ * it replaces phi in place by the signed distance to the mesh that lsm_interface_extract(ctx, phi, 0.0, ...) would return, without
+ * building or fetching that mesh and without touching the context's last extraction.
+ *  - s = double(phi); inside s <= 0, outside s > 0, invalid s NaN (the extraction's rules); node coordinates x_d = lc_d + i_d h_d.
+ *  - primitives are the extraction's, rebuilt from phi with the same crossing formula and quad split, so their vertices are
+ *    bit-identical to lsm_interface_extract's.  All arithmetic in double, each operation rounded, no FMA; dot(u, v) =
+ *    (u1 v1 + u2 v2) + u3 v3 and dist(x, p) = sqrt(((x1 - p1)^2 + (x2 - p2)^2) + (x3 - p3)^2) (fewer terms in 1-D / 2-D).
+ *  - closest point p of a primitive to x: 1-D the vertex; 2-D the segment projection a + t (b - a), t = clamp(dot(x - a, b - a) /
+ *    dot(b - a, b - a), 0, 1), or a if a == b; 3-D Ericson's ClosestPtPointTriangle (Real-Time Collision Detection 5.1.5) in its
+ *    operation order, on the triangle's vertices in the extraction's order.  Where the divisor of the region it reaches is 0
+ *    (d1 - d3, d2 - d6, (d4 - d3) + (d5 - d6), or (va + vb) + vc: a triangle made degenerate by exact zeros at nodes), p is the
+ *    closest of the segment projections on ab, ac, bc, in that order (a later one only if strictly closer).
+ *  1. band: node i scans the cells c with max(0, i_d - band) <= c_d <= min(n_d - 2, i_d + band - 1) in increasing column-major order
+ *     and, within a cell, the primitives in the extraction's order; a candidate replaces the current point only if dist(x, p) is
+ *     strictly smaller.  A node whose window holds at least one primitive is a band node; every other node has no point yet.
+ *  2. propagation: jump flooding over the whole box with k = 2^(ceil(log2 max_d n_d) - 1), ..., 2, 1, then once more k = 1.  Each
+ *     pass reads one point buffer and writes the other; a node's candidates are its own point, then the points of the nodes
+ *     i + k o, o in {-1,0,1}^N \ {0} in column-major order of o, inside the box (no wrap on any axis); nodes without a point are
+ *     skipped and the strictly closest candidate wins, so a tie keeps the node's own point.
+ *  3. write: with d = dist(x, p), an inside node gets -d, an outside node +d, raised to the smallest positive subnormal of the
+ *     field's dtype if it rounds to 0, so that every node keeps its classification; values are rounded to the dtype on store.  NaN
+ *     nodes keep NaN; a node without a point keeps its value, which happens only when there is no interface, and then nothing
+ *     changes.
+ * Guarantee: a band node with d < band * min_d |h_d| holds the minimum over the whole mesh (any primitive outside its window is at
+ * least band |h_d| away along some axis); propagation can only replace it by a point whose computed distance is smaller in the last
+ * bits.  Elsewhere |phi| is the distance to a point on the mesh, never less than the true distance up to rounding.  band >= 1
+ * (3 in the Python and Julia wrappers: WENO5 reads 3 nodes on each side, so every value a stage reads near the interface is
+ * exact), else LSM_ERR_ARG.  Scalar, non-separable fields with every n_d >= 2, else LSM_ERR_ARG; nranks > 1: LSM_ERR_UNSUPPORTED
+ * (slab decomposition is not supported).  Boundary conditions play no role and are not required; on a periodic axis nodes 1 and
+ * n can therefore get different values.
+ * Asynchronous when band_nodes_out is NULL (no synchronisation, no copy: cheap in a prehook); otherwise one synchronisation and
+ * an 8-byte copy of the number of band nodes.  Bumps the field's version like every other write, so CFL caches, halos and
+ * expression fills see the new data.  Scratch: 16 N + 16 bytes per node (two point buffers of N doubles, two 8-byte keys of the band
+ * scan), persistent in the context and grown on demand (8.6 GB for a 512^3 3-D field). */
+int32_t lsm_redistance(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* band_nodes_out);
+
 /* ---- diagnostics (test harness; SURVEY.md §2.2 K6) -------------------------------------------- */
 /* max |a - b| over all owned nodes, all-reduced over ranks. */
 int32_t lsm_max_abs_diff(lsm_ctx* ctx, const lsm_field* a, const lsm_field* b, double* out);

@@ -1021,6 +1021,26 @@ def extract_interface_multi(mc: MultiContext, phis, level: float = 0.0) -> Inter
     return merge_interfaces([_fetch_interface(mc.ranks[r], phis[r].ndim, nv[r], nf[r]) for r in range(n)])
 
 
+def redistance(phi, band: int = 3):
+    """Engine extension: replace phi, in place on the device, by the signed distance to its zero level set (``lsm_redistance``).
+
+    The interface is the piecewise-linear mesh :func:`extract_interface` returns, but the mesh is never built: nodes within ``band``
+    cells of it scan the nearby primitives for their exact closest point, and jump flooding carries closest points to the rest of
+    the grid.  Every node keeps its inside / outside classification, so the interface does not move beyond the linear
+    reconstruction; NaN nodes stay NaN and a field without an interface is left unchanged.  No boundary conditions are needed,
+    nothing is copied to the host and the call does not synchronise, so it fits a ``prehook``:
+    ``integrate(eq, tf, prehook=lambda ls: redistance(ls.state))``.
+
+    This is the idea of the reference's Newton ``reinitialize!`` (reinitializer.jl:12-42: closest points on Bernstein patches found
+    from a KD-tree, on the host) with a linear instead of a Bernstein interface, so the two are not bit-compatible; unlike
+    :func:`eikonal_reinitialize` it is exact near the interface after one call.  ``phi`` is a field or an equation (its
+    ``current_state``); returns the field."""
+    phi = current_state(phi)
+    L.check(L.lib().lsm_redistance(phi._context().handle, phi.device(), int(band), None))
+    phi._mark_device_advanced()
+    return phi
+
+
 def _csg(dst: MeshField, src: Optional[MeshField], op: int) -> MeshField:
     for f in (dst, src):
         if f is not None and f.ncomp != 1:

@@ -110,6 +110,9 @@ struct lsm_ctx {
     bool iface_valid = false;
     int iface_ndim = 0;
     int64_t iface_nv = 0, iface_np = 0;
+    // lsm_redistance scratch (persistent, grown on demand): two point buffers of ndim doubles per node, the two 8-byte keys of the
+    // band scan per node, two counters
+    void* d_redist = nullptr; size_t d_redist_bytes = 0;
 };
 
 struct lsm_field {
@@ -944,6 +947,58 @@ int32_t interface_extract_impl(lsm_ctx* ctx, lsm_field* phi, double level, int64
     return LSM_OK;
 }
 
+
+// ---- closest-point redistancing (lsm_redistance.cu) ---------------------------------------------
+int32_t redistance_impl(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* band_nodes_out) {
+    if (band < 1) return fail(LSM_ERR_ARG, "band must be at least 1 (got %d)", band);
+    if (!ctx || !phi) return fail(LSM_ERR_ARG, "null argument");
+    if (phi->ctx != ctx || phi->ncomp != 1 || phi->separable) return fail(LSM_ERR_ARG, "redistancing needs a real-valued field of this context");
+    for (int d = 0; d < phi->ndim; ++d)
+        if (phi->nglob[d] < 2) return fail(LSM_ERR_ARG, "redistancing needs at least 2 nodes along every dimension (n[%d] = %d)", d, phi->nglob[d]);
+    if (ctx->nranks > 1) return fail(LSM_ERR_UNSUPPORTED, "redistancing a slab-decomposed field (nranks = %d) is not supported", ctx->nranks);
+    CU(cudaSetDevice(ctx->device));
+    RedistArgs R{};
+    IfaceArgs& A = R.g;
+    A.phi = phi->p; A.f64 = phi->dtype == LSM_F64; A.ndim = phi->ndim; A.level = 0.0;
+    A.hsign = 1;
+    for (int d = 0; d < 3; ++d) {
+        A.m[d] = phi->n[d];
+        A.lc[d] = phi->lc[d]; A.h[d] = d < phi->ndim ? phi->h[d] : 0.0;
+        if (d < phi->ndim && phi->h[d] < 0) A.hsign = -A.hsign;
+    }
+    A.s1 = A.m[0]; A.s2 = (long long)A.m[0] * A.m[1];
+    A.nodes = (long long)A.m[0] * A.m[1] * A.m[2];
+    R.band = band;
+    const size_t pbytes = (size_t)A.nodes * phi->ndim * sizeof(double), kbytes = (size_t)A.nodes * sizeof(unsigned long long);
+    const size_t need = 2 * pbytes + 2 * kbytes + 2 * sizeof(unsigned long long);
+    if (need > ctx->d_redist_bytes) {
+        if (ctx->d_redist) cudaFree(ctx->d_redist);         // implicit synchronisation: nothing in flight reads it
+        ctx->d_redist = nullptr; ctx->d_redist_bytes = 0;
+        CU(cudaMalloc(&ctx->d_redist, need));
+        ctx->d_redist_bytes = need;
+    }
+    char* base = static_cast<char*>(ctx->d_redist);
+    R.pa = reinterpret_cast<double*>(base);
+    R.pb = reinterpret_cast<double*>(base + pbytes);
+    R.list = reinterpret_cast<long long*>(R.pa);
+    R.dmin = reinterpret_cast<unsigned long long*>(base + 2 * pbytes);
+    R.ord = R.dmin + A.nodes;
+    R.ncells = R.ord + A.nodes;
+    R.count = R.ncells + 1;
+    CU(cudaMemsetAsync(R.ncells, 0, 2 * sizeof(unsigned long long), ctx->stream));
+    int launches = 0;
+    CU(launch_redistance(R, ctx->sm_count, ctx->stream, &launches));
+    ctx->cnt.kernel_launches += launches;
+    phi->version++; phi->halo_valid = false;
+    if (band_nodes_out) {
+        CU(cudaMemcpyAsync(ctx->h_scalar, R.count, 8, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaStreamSynchronize(ctx->stream));
+        ctx->cnt.d2h_bytes += 8;
+        *band_nodes_out = (int64_t)ctx->h_scalar[0];
+    }
+    return LSM_OK;
+}
+
 }  // namespace
 
 // =================================================================================================
@@ -1088,6 +1143,7 @@ int32_t lsm_ctx_destroy(lsm_ctx* c) {
     for (int b = 0; b < 2; ++b) { if (c->stage[b]) cudaFree(c->stage[b]); if (c->ev_stage[b]) cudaEventDestroy(c->ev_stage[b]); if (c->ev_free[b]) cudaEventDestroy(c->ev_free[b]); }
     if (c->d_work) cudaFree(c->d_work);
     if (c->d_iface) cudaFree(c->d_iface);
+    if (c->d_redist) cudaFree(c->d_redist);
     if (c->d_cand) cudaFree(c->d_cand);
     if (c->d_cand_count) cudaFree(c->d_cand_count);
     if (c->h_cand) cudaFreeHost(c->h_cand);
@@ -1695,6 +1751,10 @@ int32_t lsm_interface_fetch(lsm_ctx* ctx, double* verts, int64_t* keys, int32_t*
     CU(cudaStreamSynchronize(ctx->stream));
     ctx->cnt.d2h_bytes += (int64_t)(vbytes + (keys ? kbytes : 0) + pbytes);
     return LSM_OK;
+}
+
+int32_t lsm_redistance(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* band_nodes_out) {
+    return redistance_impl(ctx, phi, band, band_nodes_out);
 }
 
 int32_t lsm_field_csg(lsm_ctx* ctx, lsm_field* dst, const lsm_field* src, int32_t op) {

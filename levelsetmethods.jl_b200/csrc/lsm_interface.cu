@@ -18,90 +18,12 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 #include "lsm_kernels.h"
+#include "lsm_simplex.cuh"
 
 namespace lsm {
 namespace {
 
 constexpr int TPB = 256, NPT = 4, TILE = TPB * NPT;
-
-// corner k of a cell is c + sum_d bit_d(k) e_d.  Chain of simplex p (lexicographic permutation order) and the sign of p.
-__constant__ unsigned char c_chain3[6][4] = {{0, 1, 3, 7}, {0, 1, 5, 7}, {0, 2, 3, 7}, {0, 2, 6, 7}, {0, 4, 5, 7}, {0, 4, 6, 7}};
-__constant__ signed char c_sign3[6] = {1, -1, -1, 1, 1, -1};
-__constant__ unsigned char c_chain2[2][3] = {{0, 1, 3}, {0, 2, 3}};
-__constant__ signed char c_sign2[2] = {1, -1};
-
-template <int N> __device__ __forceinline__ int nsimplices() { return N == 3 ? 6 : N == 2 ? 2 : 1; }
-template <int N> __device__ __forceinline__ int chain(int p, int k) {
-    if (N == 3) return c_chain3[p][k];
-    if (N == 2) return c_chain2[p][k];
-    return k;
-}
-template <int N> __device__ __forceinline__ int psign(int p) { return N == 3 ? c_sign3[p] : N == 2 ? c_sign2[p] : 1; }
-template <int N> __device__ __forceinline__ unsigned chain_mask(int p) {
-    unsigned m = 0;
-    for (int k = 0; k <= N; ++k) m |= 1u << chain<N>(p, k);
-    return m;
-}
-
-__device__ __forceinline__ long long corner_off(const IfaceArgs& A, int k) {
-    return (long long)(k & 1) + ((k >> 1) & 1) * A.s1 + ((k >> 2) & 1) * A.s2;
-}
-
-template <class T> __device__ __forceinline__ double sval(const IfaceArgs& A, long long j) {
-    return double(static_cast<const T*>(A.phi)[j]) - A.level;
-}
-
-// corner classification of the cell of node idx: in-box, inside (s <= 0) and NaN bit masks over the 2^N corners
-struct Masks { unsigned box, in, nan; };
-
-template <class T, int N>
-__device__ __forceinline__ Masks classify(const IfaceArgs& A, long long idx, const int* i) {
-    unsigned up = 0;                      // axes along which the node has an upper neighbour in the box
-    for (int d = 0; d < N; ++d) if (i[d] + 1 < A.m[d]) up |= 1u << d;
-    Masks M{0, 0, 0};
-    for (int k = 0; k < (1 << N); ++k) {
-        if ((k & up) != k) continue;
-        const double s = sval<T>(A, idx + corner_off(A, k));
-        M.box |= 1u << k;
-        if (s <= 0.0) M.in |= 1u << k;
-        if (s != s) M.nan |= 1u << k;
-    }
-    return M;
-}
-
-// cut edges owned by the node: (a, a + e) for the in-box corners e != 0, both ends valid, one inside and one outside
-template <int N> __device__ __forceinline__ unsigned cut_edges(const Masks& M) {
-    if (M.nan & 1u) return 0;
-    const unsigned valid = M.box & ~M.nan;
-    return valid & ((M.in & 1u) ? ~M.in : M.in) & ~1u;
-}
-
-template <int N> __device__ __forceinline__ int prims_of_simplex(const Masks& M, int p) {
-    const unsigned cm = chain_mask<N>(p);
-    if (cm & M.nan) return 0;
-    const int k = __popc(cm & M.in);
-    if (k == 0 || k == N + 1) return 0;
-    return (N == 3 && k == 2) ? 2 : 1;
-}
-
-template <int N> __device__ __forceinline__ int cell_prims(const Masks& M) {
-    constexpr unsigned full = (1u << (1 << N)) - 1u;
-    const unsigned valid = M.box & ~M.nan;
-    if (M.box != full || !(valid & M.in) || !(valid & ~M.in)) return 0;
-    int np = 0;
-    for (int p = 0; p < nsimplices<N>(); ++p) np += prims_of_simplex<N>(M, p);
-    return np;
-}
-
-__device__ __forceinline__ void node_index(const IfaceArgs& A, long long idx, int* i) {
-    i[0] = (int)(idx % A.m[0]);
-    const long long q = idx / A.m[0];
-    i[1] = (int)(q % A.m[1]);
-    i[2] = (int)(q / A.m[1]);
-}
-__device__ __forceinline__ void next_index(const IfaceArgs& A, int* i) {
-    if (++i[0] == A.m[0]) { i[0] = 0; if (++i[1] == A.m[1]) { i[1] = 0; ++i[2]; } }
-}
 
 // block-wide exclusive scan of (a, b) pairs over TPB threads; also returns the block totals
 template <int BS, class V>
@@ -233,53 +155,15 @@ __global__ void __launch_bounds__(TPB) iface_prims_kernel(const __grid_constant_
         const Masks& M = Ms[j];
         for (int p = 0; p < nsimplices<N>(); ++p) {
             if (!prims_of_simplex<N>(M, p)) continue;
-            int w[N + 1], inside = 0;
-            for (int k = 0; k <= N; ++k) { w[k] = chain<N>(p, k); inside |= ((M.in >> w[k]) & 1) << k; }
-            // vertex index of simplex edge (w_x, w_y): bisection over the keys of the tile that owns the edge's lower node
-            auto vid = [&](int x, int y) {
-                const int a = x < y ? w[x] : w[y], b = x < y ? w[y] : w[x];
-                const long long na = idx + corner_off(A, a), ta = na / TILE;
-                return find_key(keys, off_v[ta], off_v[ta + 1], (A.lin0 + na) * ncode + ((a ^ b) - 1));
-            };
-            const int sgn = psign<N>(p) * A.hsign;
-            if constexpr (N == 1) {
-                prims[out++] = vid(0, 1);
-                continue;
-            }
-            const int k = __popc(inside);
-            if (N == 2 || k != 2) {
-                // lone vertex q (the only inside or the only outside one); r < s (< u) the others in chain order.  The
-                // simplex (q, r, s[, u]) has orientation sgn (-1)^q: with a positive one, (qr, qs[, qu]) has q on its left
-                // (2-D) / its normal pointing away from q (3-D); the normal must point outside and the inside must lie left.
-                const int q = __ffs(k == 1 ? inside : (~inside & ((1 << (N + 1)) - 1))) - 1;
-                int o[3], no = 0;
-                for (int x = 0; x <= N; ++x) if (x != q) o[no++] = x;
-                const int sigma = (q & 1) ? -sgn : sgn;
-                const bool q_outside = k == N;
-                const bool flip = (sigma < 0) != q_outside;
-                if constexpr (N == 2) {
-                    const int v0 = vid(q, o[0]), v1 = vid(q, o[1]);
-                    prims[out * 2] = flip ? v1 : v0; prims[out * 2 + 1] = flip ? v0 : v1;
-                } else {
-                    const int v0 = vid(q, o[0]), v1 = vid(q, o[1]), v2 = vid(q, o[2]);
-                    prims[out * 3] = v0; prims[out * 3 + 1] = flip ? v2 : v1; prims[out * 3 + 2] = flip ? v1 : v2;
+            simplex_prims<N>(M, p, A.hsign, [&](const int* w, const int2* e) {
+                // vertex index of simplex edge (w_x, w_y): bisection over the keys of the tile that owns the edge's lower node
+                for (int j = 0; j < N; ++j) {
+                    const int a = w[e[j].x], b = w[e[j].y];
+                    const long long na = idx + corner_off(A, a), ta = na / TILE;
+                    prims[out * N + j] = find_key(keys, off_v[ta], off_v[ta + 1], (A.lin0 + na) * ncode + ((a ^ b) - 1));
                 }
                 ++out;
-            } else if constexpr (N == 3) {
-                // 3-D, inside {a < b}, outside {c < d}: quad (ac, ad, bd, bc) split into (ac, ad, bd), (ac, bd, bc); with
-                // (a, b, c, d) positively oriented that ordering has its normal pointing to c, d (outside)
-                int ins[2], outs[2], ni = 0, nu = 0;
-                for (int x = 0; x <= 3; ++x) { if ((inside >> x) & 1) ins[ni++] = x; else outs[nu++] = x; }
-                const int seq[4] = {ins[0], ins[1], outs[0], outs[1]};
-                int inv = 0;
-                for (int x = 0; x < 4; ++x) for (int y = x + 1; y < 4; ++y) inv += seq[x] > seq[y];
-                const int sigma = (inv & 1) ? -sgn : sgn;
-                const int ac = vid(ins[0], outs[0]), ad = vid(ins[0], outs[1]), bd = vid(ins[1], outs[1]), bc = vid(ins[1], outs[0]);
-                int* P = prims + out * 3;
-                if (sigma > 0) { P[0] = ac; P[1] = ad; P[2] = bd; P[3] = ac; P[4] = bd; P[5] = bc; }
-                else           { P[0] = ac; P[1] = bd; P[2] = ad; P[3] = ac; P[4] = bc; P[5] = bd; }
-                out += 2;
-            }
+            });
         }
     }
 }

@@ -86,6 +86,21 @@ long long* iface_totals(const IfaceArgs& A, void* scratch);     // device addres
 // pass 0: count + scan (totals at iface_totals); pass 1: vertices and keys; pass 2: primitives (needs the keys of pass 1)
 cudaError_t launch_iface(const IfaceArgs& A, int pass, void* scratch, double* verts, long long* keys, int* prims, cudaStream_t s);
 
+// lsm_redistance.cu: closest-point redistancing (lsm_redistance), single-rank fields.  The box is the whole field.
+struct RedistArgs {
+    IfaceArgs g;               // the field (level 0; ntiles and lin0 unused); the write pass stores through g.phi
+    int band;                  // cell window half-width
+    double* pa;                // point buffers: N components of g.nodes doubles each (SoA); NaN = no point
+    double* pb;
+    long long* list;           // cut cells (up to g.nodes entries; aliases pa until the pick pass writes it)
+    unsigned long long* dmin;  // per node: smallest candidate distance (IEEE bits) of the band scan
+    unsigned long long* ord;   // per node: order key (cell * 16 + primitive) of the first candidate at that distance
+    unsigned long long* ncells;// listed cells, zeroed by the caller
+    unsigned long long* count; // band nodes, zeroed by the caller
+};
+// enqueues flag, the two cell passes, pick, the jump-flooding passes and the write pass on s; *launches = kernels enqueued
+cudaError_t launch_redistance(const RedistArgs& R, int sm_count, cudaStream_t s, int* launches);
+
 // The five Float64 constants of the WENO5 evaluation that do not fit an instruction immediate travel in the kernel parameters
 // (constant bank): as literals the compiler re-materialises them with 10 UMOV per node, from the constant bank it takes 3 uniform loads.
 struct WenoK { double c133, c56, cm13, e6, fl, pad; };

@@ -1,0 +1,379 @@
+// lsm_redistance.cu — closest-point redistancing (lsm_redistance): phi <- the signed distance to the piecewise-linear mesh that
+// lsm_interface_extract(phi, 0) returns, without building that mesh.
+//
+// Kernels:
+//   flag  : one thread per node; classifies the node's cell (lsm_simplex.cuh) and appends it to a list when it holds a primitive;
+//   cells : one block per listed cell, twice; the cell's primitives are rebuilt from phi exactly as the extraction builds them, then
+//           every node whose window holds the cell evaluates them: pass 0 takes the atomic minimum of the distance bits, pass 1 the
+//           atomic minimum of the (cell, primitive) order key among the candidates at that distance.  Together that is the first
+//           strictly closest primitive of the node's column-major scan, independent of the list order.  (A node-centric scan of the
+//           window, the direct form of the contract, leaves most lanes of a warp idle: along x only one or two of 32 nodes' cells
+//           are cut at a time.)
+//   pick  : one thread per node; the closest point of the winning primitive (NaN when there is none);
+//   flood : jump flooding over closest points, launched once per step k (2^(L-1), ..., 2, 1, then 1 again), reading one point
+//           buffer and writing the other; candidates are the node's own point, then its 3^N - 1 neighbours at +-k in column-major
+//           order of the offset, and the strictly closest one wins;
+//   write : phi = -d inside, +d outside (at least the smallest positive subnormal of the dtype), NaN nodes and nodes without a
+//           point unchanged.
+// The operation order of every distance and closest point is the one include/lsm_b200.h states; tests/redistance_ref.py restates
+// it in NumPy and the two agree bit for bit (this file is compiled with -fmad=false).
+#include <cstdint>
+#include <cuda_runtime.h>
+#include <math_constants.h>
+#include "lsm_kernels.h"
+#include "lsm_simplex.cuh"
+
+namespace lsm {
+namespace {
+
+constexpr int TPB = 256;
+constexpr int CTPB = 128;      // threads of a cell block (redist_cells_kernel)
+
+template <int N> __device__ __forceinline__ double dot(const double* a, const double* b) {
+    double r = a[0] * b[0];
+    for (int d = 1; d < N; ++d) r = r + a[d] * b[d];
+    return r;
+}
+
+// sqrt(((x1 - p1)^2 + (x2 - p2)^2) + (x3 - p3)^2)
+template <int N> __device__ __forceinline__ double dist(const double* x, const double* p) {
+    double r = (x[0] - p[0]) * (x[0] - p[0]);
+    for (int d = 1; d < N; ++d) r = r + (x[d] - p[d]) * (x[d] - p[d]);
+    return sqrt(r);
+}
+
+// closest point of segment [a, b] to x: t = clamp(dot(x - a, b - a) / dot(b - a, b - a), 0, 1); a when a == b
+template <int N> __device__ __forceinline__ void closest_seg(const double* x, const double* a, const double* b, double* q) {
+    double ab[N], ax[N];
+    bool same = true;
+    for (int d = 0; d < N; ++d) { ab[d] = b[d] - a[d]; ax[d] = x[d] - a[d]; same = same && a[d] == b[d]; }
+    if (same) { for (int d = 0; d < N; ++d) q[d] = a[d]; return; }
+    double t = dot<N>(ax, ab) / dot<N>(ab, ab);
+    t = t < 0.0 ? 0.0 : (t > 1.0 ? 1.0 : t);
+    for (int d = 0; d < N; ++d) q[d] = a[d] + t * ab[d];
+}
+
+// Ericson, Real-Time Collision Detection 5.1.5, ClosestPtPointTriangle, in its operation order.  Where the region's divisor is 0
+// (a triangle made degenerate by exact zeros at nodes), the closest of the projections on ab, ac, bc, in that order.
+__device__ __forceinline__ void closest_tri(const double* p, const double* a, const double* b, const double* c, double* q) {
+    double ab[3], ac[3], ap[3], bp[3], cp[3];
+    for (int d = 0; d < 3; ++d) { ab[d] = b[d] - a[d]; ac[d] = c[d] - a[d]; ap[d] = p[d] - a[d]; }
+    const double d1 = dot<3>(ab, ap), d2 = dot<3>(ac, ap);
+    if (d1 <= 0.0 && d2 <= 0.0) { for (int d = 0; d < 3; ++d) q[d] = a[d]; return; }
+    for (int d = 0; d < 3; ++d) bp[d] = p[d] - b[d];
+    const double d3 = dot<3>(ab, bp), d4 = dot<3>(ac, bp);
+    if (d3 >= 0.0 && d4 <= d3) { for (int d = 0; d < 3; ++d) q[d] = b[d]; return; }
+    const double vc = d1 * d4 - d3 * d2;
+    bool degenerate = false;
+    if (vc <= 0.0 && d1 >= 0.0 && d3 <= 0.0) {
+        const double den = d1 - d3;
+        if (den != 0.0) { const double v = d1 / den; for (int d = 0; d < 3; ++d) q[d] = a[d] + v * ab[d]; return; }
+        degenerate = true;
+    }
+    if (!degenerate) {
+        for (int d = 0; d < 3; ++d) cp[d] = p[d] - c[d];
+        const double d5 = dot<3>(ab, cp), d6 = dot<3>(ac, cp);
+        if (d6 >= 0.0 && d5 <= d6) { for (int d = 0; d < 3; ++d) q[d] = c[d]; return; }
+        const double vb = d5 * d2 - d1 * d6;
+        if (vb <= 0.0 && d2 >= 0.0 && d6 <= 0.0) {
+            const double den = d2 - d6;
+            if (den != 0.0) { const double w = d2 / den; for (int d = 0; d < 3; ++d) q[d] = a[d] + w * ac[d]; return; }
+            degenerate = true;
+        }
+        if (!degenerate) {
+            const double va = d3 * d6 - d5 * d4;
+            if (va <= 0.0 && (d4 - d3) >= 0.0 && (d5 - d6) >= 0.0) {
+                const double den = (d4 - d3) + (d5 - d6);
+                if (den != 0.0) {
+                    const double w = (d4 - d3) / den;
+                    for (int d = 0; d < 3; ++d) q[d] = b[d] + w * (c[d] - b[d]);
+                    return;
+                }
+                degenerate = true;
+            }
+            if (!degenerate) {
+                const double den = (va + vb) + vc;
+                if (den != 0.0) {
+                    const double denom = 1.0 / den, v = vb * denom, w = vc * denom;
+                    for (int d = 0; d < 3; ++d) q[d] = (a[d] + ab[d] * v) + ac[d] * w;
+                    return;
+                }
+            }
+        }
+    }
+    double s[3], best;
+    closest_seg<3>(p, a, b, q);
+    best = dist<3>(p, q);
+    closest_seg<3>(p, a, c, s);
+    double ds = dist<3>(p, s);
+    if (ds < best) { best = ds; for (int d = 0; d < 3; ++d) q[d] = s[d]; }
+    closest_seg<3>(p, b, c, s);
+    ds = dist<3>(p, s);
+    if (ds < best) { for (int d = 0; d < 3; ++d) q[d] = s[d]; }
+}
+
+__device__ __forceinline__ void node_coords(const IfaceArgs& A, const int* i, double* x) {
+    for (int d = 0; d < 3; ++d) x[d] = A.lc[d] + double(i[d]) * A.h[d];
+}
+
+// corner values of cell c (all corners in the box) and their classification
+template <class T, int N>
+__device__ __forceinline__ Masks cell_corners(const IfaceArgs& A, long long cidx, double* s) {
+    Masks M{(1u << (1 << N)) - 1u, 0, 0};
+    for (int k = 0; k < (1 << N); ++k) {
+        s[k] = sval<T>(A, cidx + corner_off(A, k));
+        if (s[k] <= 0.0) M.in |= 1u << k;
+        if (s[k] != s[k]) M.nan |= 1u << k;
+    }
+    return M;
+}
+
+// vertices V[j][d] of the primitives of simplex p of cell c, as lsm_interface.cu computes them on the lattice edge (c + w_x, c + w_y)
+template <int N, class F>
+__device__ __forceinline__ void simplex_vertices(const IfaceArgs& A, const int* c, const double* s, const Masks& M, int p, F&& f) {
+    simplex_prims<N>(M, p, A.hsign, [&](const int* w, const int2* e) {
+        double V[N][3];
+        for (int j = 0; j < N; ++j) {
+            const int a = w[e[j].x], b = w[e[j].y];
+            const double t = s[a] / (s[a] - s[b]);
+            for (int d = 0; d < N; ++d) {
+                const double g = double(c[d] + ((a >> d) & 1));
+                V[j][d] = (((a ^ b) >> d) & 1) ? A.lc[d] + (g + t) * A.h[d] : A.lc[d] + g * A.h[d];
+            }
+        }
+        f(V);
+    });
+}
+
+template <int N> __device__ __forceinline__ void closest(const double* x, const double (*V)[3], double* q) {
+    if constexpr (N == 1) q[0] = V[0][0];
+    else if constexpr (N == 2) closest_seg<2>(x, V[0], V[1], q);
+    else closest_tri(x, V[0], V[1], V[2], q);
+}
+
+constexpr unsigned long long NONE = ~0ull;                    // dmin / ord of a node outside every window
+constexpr unsigned long long INF_BITS = 0x7ff0000000000000ull; // dmin of a band node whose candidates are all NaN
+
+// every node: dmin = ord = NONE; a node whose cell holds a primitive appends the cell to the list
+template <class T, int N>
+__global__ void __launch_bounds__(TPB) redist_flag_kernel(const __grid_constant__ RedistArgs R) {
+    const IfaceArgs& A = R.g;
+    const long long idx = (long long)blockIdx.x * TPB + threadIdx.x;
+    bool cut = false;
+    if (idx < A.nodes) {
+        int i[3];
+        node_index(A, idx, i);
+        cut = cell_prims<N>(classify<T, N>(A, idx, i)) > 0;
+        R.dmin[idx] = NONE;
+        R.ord[idx] = NONE;
+    }
+    const unsigned bal = __ballot_sync(0xffffffffu, cut);
+    if (!bal) return;
+    const int lane = threadIdx.x & 31;
+    unsigned long long base = 0;
+    if (lane == 0) base = atomicAdd(R.ncells, (unsigned long long)__popc(bal));
+    base = __shfl_sync(0xffffffffu, base, 0);
+    if (cut) R.list[base + __popc(bal & ((1u << lane) - 1u))] = idx;
+}
+
+// One block per cut cell (grid-stride over the list): the cell's primitives go to shared memory, then every node whose window holds
+// the cell evaluates them.  pass 0: dmin = min over the node's candidates of the IEEE bits of dist (NaN as +inf);  pass 1: ord = the
+// smallest (cell, primitive) order key among the candidates whose distance equals dmin.  Both are atomicMin, so the result does not
+// depend on the order of the list: it is the first strictly closest candidate of the column-major scan the contract states.
+template <class T, int N>
+__global__ void __launch_bounds__(CTPB) redist_cells_kernel(const __grid_constant__ RedistArgs R, int pass) {
+    constexpr int MAXP = N == 3 ? 12 : N == 2 ? 2 : 1;
+    __shared__ double sV[MAXP][N][3];
+    const IfaceArgs& A = R.g;
+    const long long ncells = (long long)*R.ncells;
+    const int W = 2 * R.band;
+    int nwin = W;
+    for (int d = 1; d < N; ++d) nwin *= W;
+    for (long long t = blockIdx.x; t < ncells; t += gridDim.x) {
+        const long long cidx = R.list[t];
+        int c[3];
+        node_index(A, cidx, c);
+        double s[1 << N];
+        const Masks M = cell_corners<T, N>(A, cidx, s);
+        if (threadIdx.x < nsimplices<N>() && prims_of_simplex<N>(M, threadIdx.x)) {
+            int off = 0;
+            for (int q = 0; q < (int)threadIdx.x; ++q) off += prims_of_simplex<N>(M, q);
+            simplex_vertices<N>(A, c, s, M, threadIdx.x, [&](const double (*V)[3]) {
+                for (int j = 0; j < N; ++j) for (int d = 0; d < N; ++d) sV[off][j][d] = V[j][d];
+                ++off;
+            });
+        }
+        const int P = cell_prims<N>(M);
+        __syncthreads();
+        for (int r = threadIdx.x; r < nwin; r += CTPB) {
+            int j[3] = {0, 0, 0}, rr = r;
+            bool inbox = true;
+            for (int d = 0; d < N; ++d) {
+                j[d] = c[d] + (rr % W) - R.band + 1;
+                rr /= W;
+                inbox = inbox && j[d] >= 0 && j[d] < A.m[d];
+            }
+            if (!inbox) continue;
+            const long long jdx = j[0] + j[1] * A.s1 + j[2] * A.s2;
+            double x[3];
+            node_coords(A, j, x);
+            if (pass == 0) {
+                unsigned long long best = INF_BITS;
+                for (int k = 0; k < P; ++k) {
+                    double q[3];
+                    closest<N>(x, sV[k], q);
+                    const double dq = dist<N>(x, q);
+                    if (dq < CUDART_INF) { const unsigned long long b = __double_as_longlong(dq); best = b < best ? b : best; }
+                }
+                atomicMin(&R.dmin[jdx], best);
+            } else {
+                const unsigned long long dm = R.dmin[jdx];
+                if (dm == INF_BITS) continue;
+                for (int k = 0; k < P; ++k) {
+                    double q[3];
+                    closest<N>(x, sV[k], q);
+                    const double dq = dist<N>(x, q);
+                    if (dq < CUDART_INF && (unsigned long long)__double_as_longlong(dq) == dm) {
+                        atomicMin(&R.ord[jdx], (unsigned long long)cidx * 16ull + (unsigned long long)k);
+                        break;
+                    }
+                }
+            }
+        }
+        __syncthreads();
+    }
+}
+
+// every node: the closest point of the winning primitive (NaN when there is none) into pa; counts the band nodes
+template <class T, int N>
+__global__ void __launch_bounds__(TPB) redist_pick_kernel(const __grid_constant__ RedistArgs R) {
+    const IfaceArgs& A = R.g;
+    const long long idx = (long long)blockIdx.x * TPB + threadIdx.x;
+    bool band = false;
+    if (idx < A.nodes) {
+        band = R.dmin[idx] != NONE;
+        const unsigned long long o = R.ord[idx];
+        double P[3] = {CUDART_NAN, CUDART_NAN, CUDART_NAN};
+        if (o != NONE) {
+            const long long cidx = (long long)(o >> 4);
+            int want = (int)(o & 15ull), c[3], i[3];
+            node_index(A, cidx, c);
+            node_index(A, idx, i);
+            double s[1 << N], x[3];
+            node_coords(A, i, x);
+            const Masks M = cell_corners<T, N>(A, cidx, s);
+            for (int p = 0; p < nsimplices<N>() && want >= 0; ++p) {
+                if (!prims_of_simplex<N>(M, p)) continue;
+                simplex_vertices<N>(A, c, s, M, p, [&](const double (*V)[3]) {
+                    if (want-- == 0) closest<N>(x, V, P);
+                });
+            }
+        }
+        for (int d = 0; d < N; ++d) R.pa[d * A.nodes + idx] = P[d];
+    }
+    const unsigned bal = __ballot_sync(0xffffffffu, band);
+    if ((threadIdx.x & 31) == 0 && bal) atomicAdd(R.count, (unsigned long long)__popc(bal));
+}
+
+template <int N>
+__global__ void __launch_bounds__(TPB) redist_flood_kernel(const __grid_constant__ RedistArgs R, int k, const double* __restrict__ src,
+                                                           double* __restrict__ dst) {
+    const IfaceArgs& A = R.g;
+    const long long idx = (long long)blockIdx.x * TPB + threadIdx.x;
+    if (idx >= A.nodes) return;
+    int i[3];
+    node_index(A, idx, i);
+    double x[3], P[3] = {CUDART_NAN, CUDART_NAN, CUDART_NAN}, best = CUDART_INF;
+    node_coords(A, i, x);
+    auto consider = [&](long long j) {
+        double q[3];
+        q[0] = src[j];
+        if (q[0] != q[0]) return;                 // no point
+        for (int d = 1; d < N; ++d) q[d] = src[d * A.nodes + j];
+        const double dq = dist<N>(x, q);
+        if (dq < best) { best = dq; for (int d = 0; d < N; ++d) P[d] = q[d]; }
+    };
+    consider(idx);
+    const int r2 = N > 2 ? 1 : 0, r1 = N > 1 ? 1 : 0;
+    for (int o2 = -r2; o2 <= r2; ++o2) {
+        const int j2 = i[2] + o2 * k;
+        if (j2 < 0 || j2 >= A.m[2]) continue;
+        for (int o1 = -r1; o1 <= r1; ++o1) {
+            const int j1 = i[1] + o1 * k;
+            if (j1 < 0 || j1 >= A.m[1]) continue;
+            for (int o0 = -1; o0 <= 1; ++o0) {
+                const int j0 = i[0] + o0 * k;
+                if ((o0 | o1 | o2) == 0 || j0 < 0 || j0 >= A.m[0]) continue;
+                consider(j0 + j1 * A.s1 + j2 * A.s2);
+            }
+        }
+    }
+    for (int d = 0; d < N; ++d) dst[d * A.nodes + idx] = P[d];
+}
+
+template <class T> __device__ __forceinline__ T smallest_subnormal();
+template <> __device__ __forceinline__ float smallest_subnormal<float>() { return 1.40129846e-45f; }
+template <> __device__ __forceinline__ double smallest_subnormal<double>() { return 4.9406564584124654e-324; }
+
+template <class T, int N>
+__global__ void __launch_bounds__(TPB) redist_write_kernel(const __grid_constant__ RedistArgs R, const double* __restrict__ pts) {
+    const IfaceArgs& A = R.g;
+    const long long idx = (long long)blockIdx.x * TPB + threadIdx.x;
+    if (idx >= A.nodes) return;
+    T* phi = static_cast<T*>(const_cast<void*>(A.phi));
+    const double s = double(phi[idx]);
+    double q[3];
+    q[0] = pts[idx];
+    if (s != s || q[0] != q[0]) return;           // NaN node, or no interface at all
+    for (int d = 1; d < N; ++d) q[d] = pts[d * A.nodes + idx];
+    int i[3];
+    node_index(A, idx, i);
+    double x[3];
+    node_coords(A, i, x);
+    const double dq = dist<N>(x, q);
+    if (s <= 0.0) { phi[idx] = T(-dq); return; }
+    T v = T(dq);
+    if (v == T(0)) v = smallest_subnormal<T>();   // an outside node stays outside
+    phi[idx] = v;
+}
+
+template <class T, int N>
+cudaError_t launch_n(const RedistArgs& R, int cell_blocks, cudaStream_t s, int* launches) {
+    const unsigned grid = (unsigned)((R.g.nodes + TPB - 1) / TPB);
+    redist_flag_kernel<T, N><<<grid, TPB, 0, s>>>(R);
+    for (int pass = 0; pass < 2; ++pass) redist_cells_kernel<T, N><<<cell_blocks, CTPB, 0, s>>>(R, pass);
+    redist_pick_kernel<T, N><<<grid, TPB, 0, s>>>(R);
+    *launches = 4;
+    int maxn = 1, L = 0;
+    for (int d = 0; d < N; ++d) maxn = R.g.m[d] > maxn ? R.g.m[d] : maxn;
+    while ((1 << L) < maxn) ++L;
+    double *src = R.pa, *dst = R.pb;
+    for (int k = 1 << (L - 1); ; k >>= 1) {
+        const int kk = k > 0 ? k : 1;             // k = 2^(L-1), ..., 2, 1, then one more pass with k = 1
+        redist_flood_kernel<N><<<grid, TPB, 0, s>>>(R, kk, src, dst);
+        ++*launches;
+        double* t = src; src = dst; dst = t;
+        if (k == 0) break;
+    }
+    redist_write_kernel<T, N><<<grid, TPB, 0, s>>>(R, src);
+    ++*launches;
+    return cudaGetLastError();
+}
+
+template <class T>
+cudaError_t launch_t(const RedistArgs& R, int cell_blocks, cudaStream_t s, int* launches) {
+    switch (R.g.ndim) {
+        case 1: return launch_n<T, 1>(R, cell_blocks, s, launches);
+        case 2: return launch_n<T, 2>(R, cell_blocks, s, launches);
+        default: return launch_n<T, 3>(R, cell_blocks, s, launches);
+    }
+}
+
+}  // namespace
+
+cudaError_t launch_redistance(const RedistArgs& R, int sm_count, cudaStream_t s, int* launches) {
+    const int cell_blocks = sm_count * 16;
+    return R.g.f64 ? launch_t<double>(R, cell_blocks, s, launches) : launch_t<float>(R, cell_blocks, s, launches);
+}
+
+}  // namespace lsm

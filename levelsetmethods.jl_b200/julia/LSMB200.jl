@@ -576,6 +576,21 @@ function interface_mesh(mc::MultiContext, ϕs::Vector{<:DeviceMeshField{N}}; lev
     return verts, faces, ukeys
 end
 
+"""
+    redistance!(ϕ::DeviceMeshField; band = 3) -> ϕ
+
+Replace ϕ, in place on the device, by the signed distance to its zero level set (`lsm_redistance`): the piecewise-linear mesh
+`interface_mesh(ϕ)` returns, which is never built.  Nodes within `band` cells of it get their exact closest point, jump flooding
+carries closest points to the rest of the grid; every node keeps its sign, NaN nodes stay NaN.  No boundary conditions needed, no
+copy to the host and no synchronisation, so it fits a prehook: `integrate!(eq, tf; prehook = ls -> redistance!(current_state(ls)))`.
+The same idea as `LevelSetMethods.reinitialize!` (reinitializer.jl:12-42, Newton on Bernstein patches, host) with a linear
+interface, so the two are not bit-compatible; that is why this is not a method of `reinitialize!`.
+"""
+function redistance!(ϕ::DeviceMeshField; band::Integer = 3)
+    check(ccall((:lsm_redistance, LIB), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Int32, Ptr{Int64}), ϕ.ctx.handle, handle!(ϕ), band, C_NULL))
+    return _device_advanced!(ϕ)
+end
+
 "`extend_along_normals!(F, ϕ; …)` — src/velocityextension.jl:20-78 on device fields."
 function LSM.extend_along_normals!(F::DeviceMeshField, ϕ::DeviceMeshField; nb_iters::Integer = 50, cfl::Real = 0.45, frozen = nothing,
                                    interface_band::Real = 1.5, min_norm::Real = 1.0e-14)

@@ -353,6 +353,33 @@ int32_t lsm_multi_interface_extract(int32_t n, lsm_ctx* const* ctx, lsm_field* c
  * scan), persistent in the context and grown on demand (8.6 GB for a 512^3 3-D field). */
 int32_t lsm_redistance(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* band_nodes_out);
 
+/* ---- closest-point extension: F(x) <- F at the closest point of x on phi's zero-level-set mesh, on the device -----------------
+ * The reference extends a speed off the interface with extend_along_normals! (velocityextension.jl:20-78, upwind pseudo-time steps;
+ * lsm_extend_along_normals here), usually next to reinitialize! in the loop.  lsm_extend_closest_point gives each node the value of
+ * F, interpolated linearly on the mesh, at the closest point lsm_redistance(ctx, phi, band, ...) finds for it, in one call.
+ *  - geometry: exactly lsm_redistance's (the same primitives, band scan and winning primitive, closest point, jump-flooding passes
+ *    and tie rule), so every node ends up with the point lsm_redistance uses, bit for bit.  Arithmetic in double, each operation
+ *    rounded, no FMA.
+ *  - vertex value: a mesh vertex lies on the lattice edge (a, b), a = w_i, b = w_j, i < j, as the extraction defines them, at
+ *    t = s_a / (s_a - s_b), the t of its coordinates; its value is F_v = Fa + t (Fb - Fa), Fa = double(F[a]), Fb = double(F[b]).
+ *  - value at the closest point, following the branch the closest-point routine took, with F0, F1, F2 the values of the
+ *    primitive's vertices in the extraction's order: 1-D F_v; 2-D F0 + t (F1 - F0) with the clamped t of the projection, or F0 when
+ *    a == b; 3-D, Ericson's regions: vertex a / b / c F0 / F1 / F2, edge ab F0 + v (F1 - F0), edge ac F0 + w (F2 - F0), edge bc
+ *    F1 + w (F2 - F1), the interior (F0 + (F1 - F0) v) + (F2 - F0) w, with the routine's own v and w; the degenerate fallback
+ *    uses the segment it picked with that segment's t (its first vertex's value when the segment is a point).  These forms return
+ *    a constant F exactly, which barycentric u F0 + v F1 + w F2 would not.  A NaN in F gives NaN wherever it enters.
+ *  - propagation: each jump-flooding pass carries the value with the point; the winning candidate's value wins.
+ *  - write: every node that has a point and a non-NaN phi gets F = value, rounded to F's dtype.  NaN-phi nodes keep their F, and
+ *    so does every node when there is no interface.  With redistance_phi != 0 the same call also writes phi exactly as
+ *    lsm_redistance(ctx, phi, band, ...) would (bit for bit): one scan for the usual reinitialise-and-extend prehook.
+ * F and phi are scalar, non-separable fields of this context on the same grid (n, lc, h), F is not phi, band >= 1 and every
+ * n_d >= 2, else LSM_ERR_ARG; F's dtype may differ from phi's.  nranks > 1: LSM_ERR_UNSUPPORTED (slab decomposition is not
+ * supported).  No boundary conditions are needed.  Asynchronous when band_nodes_out is NULL; otherwise one synchronisation and an
+ * 8-byte copy of the number of band nodes.  Bumps F's version, and phi's when phi is written, so CFL caches and expression fills
+ * see the new data.  Scratch: lsm_redistance's plus two value buffers, 16 N + 32 bytes per node in the same context buffer
+ * (10.7 GB for a 512^3 3-D field). */
+int32_t lsm_extend_closest_point(lsm_ctx* ctx, lsm_field* F, lsm_field* phi, int32_t band, int32_t redistance_phi, int64_t* band_nodes_out);
+
 /* ---- diagnostics (test harness; SURVEY.md §2.2 K6) -------------------------------------------- */
 /* max |a - b| over all owned nodes, all-reduced over ranks. */
 int32_t lsm_max_abs_diff(lsm_ctx* ctx, const lsm_field* a, const lsm_field* b, double* out);

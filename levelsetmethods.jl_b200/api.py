@@ -1041,6 +1041,29 @@ def redistance(phi, band: int = 3):
     return phi
 
 
+def extend_closest_point(F: MeshField, phi, band: int = 3, redistance: bool = False) -> MeshField:
+    """Engine extension: give every node of ``F``, in place on the device, the value of ``F`` at its closest point on the zero level
+    set of ``phi`` (``lsm_extend_closest_point``): a speed known on or near the interface becomes constant along the normals, so a
+    ``NormalMotionTerm(F)`` moves the interface with it.
+
+    The closest points are exactly those :func:`redistance` finds (the piecewise-linear mesh of :func:`extract_interface`, never
+    built); ``F`` there is interpolated linearly on the mesh from its values at the lattice nodes, so a constant ``F`` comes back
+    unchanged.  NaN nodes of ``phi`` keep their ``F``, and so does every node when ``phi`` has no interface.  With
+    ``redistance=True`` the same call also replaces ``phi`` by its signed distance, bit for bit what :func:`redistance` writes, so
+    ``integrate(eq, tf, prehook=lambda ls: extend_closest_point(v, ls.state, redistance=True))`` reinitialises and extends in one
+    scan.  No boundary conditions are needed, nothing is copied to the host and the call does not synchronise.
+
+    Unlike :func:`extend_along_normals` (the reference's upwind pseudo-time PDE, velocityextension.jl:20-78) the result does not
+    depend on a number of iterations and is not smeared at the interface.  ``phi`` is a field or an equation (its
+    ``current_state``); ``F`` is a scalar field on the same grid, of either dtype; returns ``F``."""
+    phi = current_state(phi)
+    L.check(L.lib().lsm_extend_closest_point(phi._context().handle, F.device(), phi.device(), int(band), int(bool(redistance)), None))
+    F._mark_device_advanced()
+    if redistance:
+        phi._mark_device_advanced()
+    return F
+
+
 def _csg(dst: MeshField, src: Optional[MeshField], op: int) -> MeshField:
     for f in (dst, src):
         if f is not None and f.ncomp != 1:

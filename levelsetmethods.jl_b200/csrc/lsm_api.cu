@@ -110,8 +110,8 @@ struct lsm_ctx {
     bool iface_valid = false;
     int iface_ndim = 0;
     int64_t iface_nv = 0, iface_np = 0;
-    // lsm_redistance scratch (persistent, grown on demand): two point buffers of ndim doubles per node, the two 8-byte keys of the
-    // band scan per node, two counters
+    // lsm_redistance scratch (persistent, grown on demand): two point buffers of ndim doubles per node (ndim + 1 for
+    // lsm_extend_closest_point: the value at the point), the two 8-byte keys of the band scan per node, two counters
     void* d_redist = nullptr; size_t d_redist_bytes = 0;
 };
 
@@ -948,16 +948,11 @@ int32_t interface_extract_impl(lsm_ctx* ctx, lsm_field* phi, double level, int64
 }
 
 
-// ---- closest-point redistancing (lsm_redistance.cu) ---------------------------------------------
-int32_t redistance_impl(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* band_nodes_out) {
-    if (band < 1) return fail(LSM_ERR_ARG, "band must be at least 1 (got %d)", band);
-    if (!ctx || !phi) return fail(LSM_ERR_ARG, "null argument");
-    if (phi->ctx != ctx || phi->ncomp != 1 || phi->separable) return fail(LSM_ERR_ARG, "redistancing needs a real-valued field of this context");
-    for (int d = 0; d < phi->ndim; ++d)
-        if (phi->nglob[d] < 2) return fail(LSM_ERR_ARG, "redistancing needs at least 2 nodes along every dimension (n[%d] = %d)", d, phi->nglob[d]);
-    if (ctx->nranks > 1) return fail(LSM_ERR_UNSUPPORTED, "redistancing a slab-decomposed field (nranks = %d) is not supported", ctx->nranks);
+// ---- closest-point redistancing and extension (lsm_redistance.cu) --------------------------------
+// The arguments and scratch of the redistancing passes on phi (checked by the caller), with `values` extra components per point
+// (the value of F that lsm_extend_closest_point carries); zeroes the two counters on the context's stream.
+int32_t redist_setup(lsm_ctx* ctx, lsm_field* phi, int32_t band, int values, RedistArgs& R) {
     CU(cudaSetDevice(ctx->device));
-    RedistArgs R{};
     IfaceArgs& A = R.g;
     A.phi = phi->p; A.f64 = phi->dtype == LSM_F64; A.ndim = phi->ndim; A.level = 0.0;
     A.hsign = 1;
@@ -969,7 +964,7 @@ int32_t redistance_impl(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* ban
     A.s1 = A.m[0]; A.s2 = (long long)A.m[0] * A.m[1];
     A.nodes = (long long)A.m[0] * A.m[1] * A.m[2];
     R.band = band;
-    const size_t pbytes = (size_t)A.nodes * phi->ndim * sizeof(double), kbytes = (size_t)A.nodes * sizeof(unsigned long long);
+    const size_t pbytes = (size_t)A.nodes * (phi->ndim + values) * sizeof(double), kbytes = (size_t)A.nodes * sizeof(unsigned long long);
     const size_t need = 2 * pbytes + 2 * kbytes + 2 * sizeof(unsigned long long);
     if (need > ctx->d_redist_bytes) {
         if (ctx->d_redist) cudaFree(ctx->d_redist);         // implicit synchronisation: nothing in flight reads it
@@ -986,10 +981,11 @@ int32_t redistance_impl(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* ban
     R.ncells = R.ord + A.nodes;
     R.count = R.ncells + 1;
     CU(cudaMemsetAsync(R.ncells, 0, 2 * sizeof(unsigned long long), ctx->stream));
-    int launches = 0;
-    CU(launch_redistance(R, ctx->sm_count, ctx->stream, &launches));
-    ctx->cnt.kernel_launches += launches;
-    phi->version++; phi->halo_valid = false;
+    return LSM_OK;
+}
+
+// after the passes are enqueued: without band_nodes_out nothing (asynchronous); with it one sync and an 8-byte copy of the count
+int32_t redist_band_nodes(lsm_ctx* ctx, const RedistArgs& R, int64_t* band_nodes_out) {
     if (band_nodes_out) {
         CU(cudaMemcpyAsync(ctx->h_scalar, R.count, 8, cudaMemcpyDeviceToHost, ctx->stream));
         CU(cudaStreamSynchronize(ctx->stream));
@@ -997,6 +993,46 @@ int32_t redistance_impl(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* ban
         *band_nodes_out = (int64_t)ctx->h_scalar[0];
     }
     return LSM_OK;
+}
+
+int32_t redistance_impl(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* band_nodes_out) {
+    if (band < 1) return fail(LSM_ERR_ARG, "band must be at least 1 (got %d)", band);
+    if (!ctx || !phi) return fail(LSM_ERR_ARG, "null argument");
+    if (phi->ctx != ctx || phi->ncomp != 1 || phi->separable) return fail(LSM_ERR_ARG, "redistancing needs a real-valued field of this context");
+    for (int d = 0; d < phi->ndim; ++d)
+        if (phi->nglob[d] < 2) return fail(LSM_ERR_ARG, "redistancing needs at least 2 nodes along every dimension (n[%d] = %d)", d, phi->nglob[d]);
+    if (ctx->nranks > 1) return fail(LSM_ERR_UNSUPPORTED, "redistancing a slab-decomposed field (nranks = %d) is not supported", ctx->nranks);
+    RedistArgs R{};
+    TRY(redist_setup(ctx, phi, band, 0, R));
+    int launches = 0;
+    CU(launch_redistance(R, ctx->sm_count, ctx->stream, &launches));
+    ctx->cnt.kernel_launches += launches;
+    phi->version++; phi->halo_valid = false;
+    return redist_band_nodes(ctx, R, band_nodes_out);
+}
+
+int32_t extend_closest_impl(lsm_ctx* ctx, lsm_field* F, lsm_field* phi, int32_t band, int32_t redistance_phi, int64_t* band_nodes_out) {
+    if (band < 1) return fail(LSM_ERR_ARG, "band must be at least 1 (got %d)", band);
+    if (!ctx || !F || !phi) return fail(LSM_ERR_ARG, "null argument");
+    if (F == phi) return fail(LSM_ERR_ARG, "the extended field F must not be phi");
+    for (const lsm_field* f : {F, phi})
+        if (f->ctx != ctx || f->ncomp != 1 || f->separable) return fail(LSM_ERR_ARG, "the closest-point extension needs real-valued fields of this context");
+    bool same = F->ndim == phi->ndim;
+    for (int d = 0; same && d < phi->ndim; ++d)
+        same = F->nglob[d] == phi->nglob[d] && F->n[d] == phi->n[d] && F->lc[d] == phi->lc[d] && F->h[d] == phi->h[d];
+    if (!same) return fail(LSM_ERR_ARG, "F and phi must be on the same grid (n, lc and h)");
+    for (int d = 0; d < phi->ndim; ++d)
+        if (phi->nglob[d] < 2) return fail(LSM_ERR_ARG, "the closest-point extension needs at least 2 nodes along every dimension (n[%d] = %d)", d, phi->nglob[d]);
+    if (ctx->nranks > 1) return fail(LSM_ERR_UNSUPPORTED, "extending a slab-decomposed field (nranks = %d) is not supported", ctx->nranks);
+    ExtendArgs E{};
+    TRY(redist_setup(ctx, phi, band, 1, E));
+    E.F = F->p; E.f64 = F->dtype == LSM_F64; E.write_phi = redistance_phi != 0;
+    int launches = 0;
+    CU(launch_extend_closest(E, ctx->sm_count, ctx->stream, &launches));
+    ctx->cnt.kernel_launches += launches;
+    F->version++; F->halo_valid = false;
+    if (E.write_phi) { phi->version++; phi->halo_valid = false; }
+    return redist_band_nodes(ctx, E, band_nodes_out);
 }
 
 }  // namespace
@@ -1755,6 +1791,10 @@ int32_t lsm_interface_fetch(lsm_ctx* ctx, double* verts, int64_t* keys, int32_t*
 
 int32_t lsm_redistance(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* band_nodes_out) {
     return redistance_impl(ctx, phi, band, band_nodes_out);
+}
+
+int32_t lsm_extend_closest_point(lsm_ctx* ctx, lsm_field* F, lsm_field* phi, int32_t band, int32_t redistance_phi, int64_t* band_nodes_out) {
+    return extend_closest_impl(ctx, F, phi, band, redistance_phi, band_nodes_out);
 }
 
 int32_t lsm_field_csg(lsm_ctx* ctx, lsm_field* dst, const lsm_field* src, int32_t op) {

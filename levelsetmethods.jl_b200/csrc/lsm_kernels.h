@@ -101,6 +101,16 @@ struct RedistArgs {
 // enqueues flag, the two cell passes, pick, the jump-flooding passes and the write pass on s; *launches = kernels enqueued
 cudaError_t launch_redistance(const RedistArgs& R, int sm_count, cudaStream_t s, int* launches);
 
+// lsm_redistance.cu, extension variant (lsm_extend_closest_point): the same passes, with the value of F at each closest point carried
+// along.  The point buffers pa / pb hold N + 1 components of g.nodes doubles each: the point, then the value at it (NaN = no point).
+struct ExtendArgs : RedistArgs {
+    void* F;                   // scalar field on g's grid, read by the pick pass and written by the write pass
+    bool f64;                  // F's dtype
+    int write_phi;             // the write pass also stores the signed distance through g.phi, as lsm_redistance does
+};
+// enqueues the same kernels as launch_redistance on s; *launches = kernels enqueued
+cudaError_t launch_extend_closest(const ExtendArgs& E, int sm_count, cudaStream_t s, int* launches);
+
 // The five Float64 constants of the WENO5 evaluation that do not fit an instruction immediate travel in the kernel parameters
 // (constant bank): as literals the compiler re-materialises them with 10 UMOV per node, from the constant bank it takes 3 uniform loads.
 struct WenoK { double c133, c56, cm13, e6, fl, pad; };

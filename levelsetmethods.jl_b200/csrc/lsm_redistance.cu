@@ -15,9 +15,14 @@
 //           order of the offset, and the strictly closest one wins;
 //   write : phi = -d inside, +d outside (at least the smallest positive subnormal of the dtype), NaN nodes and nodes without a
 //           point unchanged.
-// The operation order of every distance and closest point is the one include/lsm_b200.h states; tests/redistance_ref.py restates
-// it in NumPy and the two agree bit for bit (this file is compiled with -fmad=false).
+// The closest-point extension (lsm_extend_closest_point) is a compile-time variant of pick / flood / write (TF, the dtype of F, not
+// void; EXT in the flood): pick also interpolates F at the winning closest point, the flood carries that value with the point (as
+// an (N+1)-th component of the point buffers), and write stores it into F, and the signed distance into phi when asked.  flag and
+// the cell passes are shared as they are, so the points are the ones lsm_redistance computes.
+// The operation order of every distance, closest point and value is the one include/lsm_b200.h states; tests/redistance_ref.py and
+// tests/extension_ref.py restate it in NumPy and agree with this file bit for bit (it is compiled with -fmad=false).
 #include <cstdint>
+#include <type_traits>
 #include <cuda_runtime.h>
 #include <math_constants.h>
 #include "lsm_kernels.h"
@@ -42,42 +47,80 @@ template <int N> __device__ __forceinline__ double dist(const double* x, const d
     return sqrt(r);
 }
 
-// closest point of segment [a, b] to x: t = clamp(dot(x - a, b - a) / dot(b - a, b - a), 0, 1); a when a == b
-template <int N> __device__ __forceinline__ void closest_seg(const double* x, const double* a, const double* b, double* q) {
+// Where a closest point lies on its primitive, for the value of F there: vertex a, b or c; edge ab, ac or bc at parameter t from its
+// first vertex; or the face at Ericson's (v, w) = (t, w).  Only the WHERE variants of the routines below report it.
+enum : int { AT_A, AT_B, AT_C, ON_AB, ON_AC, ON_BC, ON_FACE };
+struct Where { int at; double t, w; };
+
+// closest point of segment [a, b] to x: t = clamp(dot(x - a, b - a) / dot(b - a, b - a), 0, 1); a when a == b.  WHERE: *W = (at_a)
+// when a == b, else (on_ab, t).
+template <int N, bool WHERE = false>
+__device__ __forceinline__ void closest_seg(const double* x, const double* a, const double* b, double* q, Where* W = nullptr,
+                                            int at_a = AT_A, int on_ab = ON_AB) {
     double ab[N], ax[N];
     bool same = true;
     for (int d = 0; d < N; ++d) { ab[d] = b[d] - a[d]; ax[d] = x[d] - a[d]; same = same && a[d] == b[d]; }
-    if (same) { for (int d = 0; d < N; ++d) q[d] = a[d]; return; }
+    if (same) {
+        for (int d = 0; d < N; ++d) q[d] = a[d];
+        if constexpr (WHERE) W->at = at_a;
+        return;
+    }
     double t = dot<N>(ax, ab) / dot<N>(ab, ab);
     t = t < 0.0 ? 0.0 : (t > 1.0 ? 1.0 : t);
     for (int d = 0; d < N; ++d) q[d] = a[d] + t * ab[d];
+    if constexpr (WHERE) { W->at = on_ab; W->t = t; }
 }
 
 // Ericson, Real-Time Collision Detection 5.1.5, ClosestPtPointTriangle, in its operation order.  Where the region's divisor is 0
-// (a triangle made degenerate by exact zeros at nodes), the closest of the projections on ab, ac, bc, in that order.
-__device__ __forceinline__ void closest_tri(const double* p, const double* a, const double* b, const double* c, double* q) {
+// (a triangle made degenerate by exact zeros at nodes), the closest of the projections on ab, ac, bc, in that order.  WHERE: *W is
+// the region and its parameters (for the fallback, those of the segment it picked).
+template <bool WHERE = false>
+__device__ __forceinline__ void closest_tri(const double* p, const double* a, const double* b, const double* c, double* q,
+                                            Where* W = nullptr) {
     double ab[3], ac[3], ap[3], bp[3], cp[3];
     for (int d = 0; d < 3; ++d) { ab[d] = b[d] - a[d]; ac[d] = c[d] - a[d]; ap[d] = p[d] - a[d]; }
     const double d1 = dot<3>(ab, ap), d2 = dot<3>(ac, ap);
-    if (d1 <= 0.0 && d2 <= 0.0) { for (int d = 0; d < 3; ++d) q[d] = a[d]; return; }
+    if (d1 <= 0.0 && d2 <= 0.0) {
+        for (int d = 0; d < 3; ++d) q[d] = a[d];
+        if constexpr (WHERE) W->at = AT_A;
+        return;
+    }
     for (int d = 0; d < 3; ++d) bp[d] = p[d] - b[d];
     const double d3 = dot<3>(ab, bp), d4 = dot<3>(ac, bp);
-    if (d3 >= 0.0 && d4 <= d3) { for (int d = 0; d < 3; ++d) q[d] = b[d]; return; }
+    if (d3 >= 0.0 && d4 <= d3) {
+        for (int d = 0; d < 3; ++d) q[d] = b[d];
+        if constexpr (WHERE) W->at = AT_B;
+        return;
+    }
     const double vc = d1 * d4 - d3 * d2;
     bool degenerate = false;
     if (vc <= 0.0 && d1 >= 0.0 && d3 <= 0.0) {
         const double den = d1 - d3;
-        if (den != 0.0) { const double v = d1 / den; for (int d = 0; d < 3; ++d) q[d] = a[d] + v * ab[d]; return; }
+        if (den != 0.0) {
+            const double v = d1 / den;
+            for (int d = 0; d < 3; ++d) q[d] = a[d] + v * ab[d];
+            if constexpr (WHERE) { W->at = ON_AB; W->t = v; }
+            return;
+        }
         degenerate = true;
     }
     if (!degenerate) {
         for (int d = 0; d < 3; ++d) cp[d] = p[d] - c[d];
         const double d5 = dot<3>(ab, cp), d6 = dot<3>(ac, cp);
-        if (d6 >= 0.0 && d5 <= d6) { for (int d = 0; d < 3; ++d) q[d] = c[d]; return; }
+        if (d6 >= 0.0 && d5 <= d6) {
+            for (int d = 0; d < 3; ++d) q[d] = c[d];
+            if constexpr (WHERE) W->at = AT_C;
+            return;
+        }
         const double vb = d5 * d2 - d1 * d6;
         if (vb <= 0.0 && d2 >= 0.0 && d6 <= 0.0) {
             const double den = d2 - d6;
-            if (den != 0.0) { const double w = d2 / den; for (int d = 0; d < 3; ++d) q[d] = a[d] + w * ac[d]; return; }
+            if (den != 0.0) {
+                const double w = d2 / den;
+                for (int d = 0; d < 3; ++d) q[d] = a[d] + w * ac[d];
+                if constexpr (WHERE) { W->at = ON_AC; W->t = w; }
+                return;
+            }
             degenerate = true;
         }
         if (!degenerate) {
@@ -87,6 +130,7 @@ __device__ __forceinline__ void closest_tri(const double* p, const double* a, co
                 if (den != 0.0) {
                     const double w = (d4 - d3) / den;
                     for (int d = 0; d < 3; ++d) q[d] = b[d] + w * (c[d] - b[d]);
+                    if constexpr (WHERE) { W->at = ON_BC; W->t = w; }
                     return;
                 }
                 degenerate = true;
@@ -96,20 +140,46 @@ __device__ __forceinline__ void closest_tri(const double* p, const double* a, co
                 if (den != 0.0) {
                     const double denom = 1.0 / den, v = vb * denom, w = vc * denom;
                     for (int d = 0; d < 3; ++d) q[d] = (a[d] + ab[d] * v) + ac[d] * w;
+                    if constexpr (WHERE) { W->at = ON_FACE; W->t = v; W->w = w; }
                     return;
                 }
             }
         }
     }
     double s[3], best;
-    closest_seg<3>(p, a, b, q);
+    Where Ws;
+    closest_seg<3, WHERE>(p, a, b, q, W, AT_A, ON_AB);
     best = dist<3>(p, q);
-    closest_seg<3>(p, a, c, s);
+    closest_seg<3, WHERE>(p, a, c, s, &Ws, AT_A, ON_AC);
     double ds = dist<3>(p, s);
-    if (ds < best) { best = ds; for (int d = 0; d < 3; ++d) q[d] = s[d]; }
-    closest_seg<3>(p, b, c, s);
+    if (ds < best) {
+        best = ds;
+        for (int d = 0; d < 3; ++d) q[d] = s[d];
+        if constexpr (WHERE) *W = Ws;
+    }
+    closest_seg<3, WHERE>(p, b, c, s, &Ws, AT_B, ON_BC);
     ds = dist<3>(p, s);
-    if (ds < best) { for (int d = 0; d < 3; ++d) q[d] = s[d]; }
+    if (ds < best) {
+        for (int d = 0; d < 3; ++d) q[d] = s[d];
+        if constexpr (WHERE) *W = Ws;
+    }
+}
+
+// F at a closest point from the values f[j] at the primitive's vertices, in the form of its region (a constant F comes back exactly)
+template <int N> __device__ __forceinline__ double value_at(const Where& W, const double* f) {
+    if constexpr (N == 1) return f[0];
+    else if constexpr (N == 2) return W.at == AT_A ? f[0] : f[0] + W.t * (f[1] - f[0]);
+    else {
+        switch (W.at) {
+            case AT_A: return f[0];
+            case AT_B: return f[1];
+            case AT_C: return f[2];
+            case ON_AB: return f[0] + W.t * (f[1] - f[0]);
+            case ON_AC: return f[0] + W.t * (f[2] - f[0]);
+            case ON_BC: return f[1] + W.t * (f[2] - f[1]);
+            default: return (f[0] + (f[1] - f[0]) * W.t) + (f[2] - f[0]) * W.w;
+        }
+    }
 }
 
 __device__ __forceinline__ void node_coords(const IfaceArgs& A, const int* i, double* x) {
@@ -128,11 +198,15 @@ __device__ __forceinline__ Masks cell_corners(const IfaceArgs& A, long long cidx
     return M;
 }
 
-// vertices V[j][d] of the primitives of simplex p of cell c, as lsm_interface.cu computes them on the lattice edge (c + w_x, c + w_y)
-template <int N, class F>
-__device__ __forceinline__ void simplex_vertices(const IfaceArgs& A, const int* c, const double* s, const Masks& M, int p, F&& f) {
+// vertices V[j][d] of the primitives of simplex p of cell c, as lsm_interface.cu computes them on the lattice edge (c + w_x, c + w_y),
+// passed to f(V).  With a field F of dtype TF (cell c at index cidx), f(V, Fv) also gets the vertex values Fv[j] = Fa + t (Fb - Fa),
+// Fa = double(F[c + w_x]), Fb = double(F[c + w_y]), with the t of the coordinates.
+template <int N, class TF = void, class Fn>
+__device__ __forceinline__ void simplex_vertices(const IfaceArgs& A, const int* c, const double* s, const Masks& M, int p, Fn&& f,
+                                                 const TF* F = nullptr, long long cidx = 0) {
     simplex_prims<N>(M, p, A.hsign, [&](const int* w, const int2* e) {
         double V[N][3];
+        [[maybe_unused]] double Fv[N];
         for (int j = 0; j < N; ++j) {
             const int a = w[e[j].x], b = w[e[j].y];
             const double t = s[a] / (s[a] - s[b]);
@@ -140,16 +214,29 @@ __device__ __forceinline__ void simplex_vertices(const IfaceArgs& A, const int* 
                 const double g = double(c[d] + ((a >> d) & 1));
                 V[j][d] = (((a ^ b) >> d) & 1) ? A.lc[d] + (g + t) * A.h[d] : A.lc[d] + g * A.h[d];
             }
+            if constexpr (!std::is_void_v<TF>) {
+                const double fa = double(F[cidx + corner_off(A, a)]), fb = double(F[cidx + corner_off(A, b)]);
+                Fv[j] = fa + t * (fb - fa);
+            }
         }
-        f(V);
+        if constexpr (std::is_void_v<TF>) f(V);
+        else f(V, Fv);
     });
 }
 
-template <int N> __device__ __forceinline__ void closest(const double* x, const double (*V)[3], double* q) {
-    if constexpr (N == 1) q[0] = V[0][0];
-    else if constexpr (N == 2) closest_seg<2>(x, V[0], V[1], q);
-    else closest_tri(x, V[0], V[1], V[2], q);
+template <int N, bool WHERE = false>
+__device__ __forceinline__ void closest(const double* x, const double (*V)[3], double* q, Where* W = nullptr) {
+    if constexpr (N == 1) {
+        q[0] = V[0][0];
+        if constexpr (WHERE) W->at = AT_A;
+    }
+    else if constexpr (N == 2) closest_seg<2, WHERE>(x, V[0], V[1], q, W);
+    else closest_tri<WHERE>(x, V[0], V[1], V[2], q, W);
 }
+
+// kernel arguments: RedistArgs for lsm_redistance (TF void), ExtendArgs for the extension with F of dtype TF
+template <class TF> struct ArgsOf { using type = ExtendArgs; };
+template <> struct ArgsOf<void> { using type = RedistArgs; };
 
 constexpr unsigned long long NONE = ~0ull;                    // dmin / ord of a node outside every window
 constexpr unsigned long long INF_BITS = 0x7ff0000000000000ull; // dmin of a band node whose candidates are all NaN
@@ -244,9 +331,10 @@ __global__ void __launch_bounds__(CTPB) redist_cells_kernel(const __grid_constan
     }
 }
 
-// every node: the closest point of the winning primitive (NaN when there is none) into pa; counts the band nodes
-template <class T, int N>
-__global__ void __launch_bounds__(TPB) redist_pick_kernel(const __grid_constant__ RedistArgs R) {
+// every node: the closest point of the winning primitive (NaN when there is none) into pa, with the extension also the value of F
+// there; counts the band nodes
+template <class T, int N, class TF = void>
+__global__ void __launch_bounds__(TPB) redist_pick_kernel(const __grid_constant__ typename ArgsOf<TF>::type R) {
     const IfaceArgs& A = R.g;
     const long long idx = (long long)blockIdx.x * TPB + threadIdx.x;
     bool band = false;
@@ -254,6 +342,7 @@ __global__ void __launch_bounds__(TPB) redist_pick_kernel(const __grid_constant_
         band = R.dmin[idx] != NONE;
         const unsigned long long o = R.ord[idx];
         double P[3] = {CUDART_NAN, CUDART_NAN, CUDART_NAN};
+        [[maybe_unused]] double val = CUDART_NAN;
         if (o != NONE) {
             const long long cidx = (long long)(o >> 4);
             int want = (int)(o & 15ull), c[3], i[3];
@@ -264,18 +353,30 @@ __global__ void __launch_bounds__(TPB) redist_pick_kernel(const __grid_constant_
             const Masks M = cell_corners<T, N>(A, cidx, s);
             for (int p = 0; p < nsimplices<N>() && want >= 0; ++p) {
                 if (!prims_of_simplex<N>(M, p)) continue;
-                simplex_vertices<N>(A, c, s, M, p, [&](const double (*V)[3]) {
-                    if (want-- == 0) closest<N>(x, V, P);
-                });
+                if constexpr (std::is_void_v<TF>) {
+                    simplex_vertices<N>(A, c, s, M, p, [&](const double (*V)[3]) {
+                        if (want-- == 0) closest<N>(x, V, P);
+                    });
+                } else {
+                    simplex_vertices<N, TF>(A, c, s, M, p, [&](const double (*V)[3], const double* Fv) {
+                        if (want-- == 0) {
+                            Where W;
+                            closest<N, true>(x, V, P, &W);
+                            val = value_at<N>(W, Fv);
+                        }
+                    }, static_cast<const TF*>(R.F), cidx);
+                }
             }
         }
         for (int d = 0; d < N; ++d) R.pa[d * A.nodes + idx] = P[d];
+        if constexpr (!std::is_void_v<TF>) R.pa[N * A.nodes + idx] = val;
     }
     const unsigned bal = __ballot_sync(0xffffffffu, band);
     if ((threadIdx.x & 31) == 0 && bal) atomicAdd(R.count, (unsigned long long)__popc(bal));
 }
 
-template <int N>
+// EXT: the value at the point (component N) goes with it; it is read once, from the winning candidate
+template <int N, bool EXT = false>
 __global__ void __launch_bounds__(TPB) redist_flood_kernel(const __grid_constant__ RedistArgs R, int k, const double* __restrict__ src,
                                                            double* __restrict__ dst) {
     const IfaceArgs& A = R.g;
@@ -284,6 +385,7 @@ __global__ void __launch_bounds__(TPB) redist_flood_kernel(const __grid_constant
     int i[3];
     node_index(A, idx, i);
     double x[3], P[3] = {CUDART_NAN, CUDART_NAN, CUDART_NAN}, best = CUDART_INF;
+    [[maybe_unused]] long long from = -1;
     node_coords(A, i, x);
     auto consider = [&](long long j) {
         double q[3];
@@ -291,7 +393,11 @@ __global__ void __launch_bounds__(TPB) redist_flood_kernel(const __grid_constant
         if (q[0] != q[0]) return;                 // no point
         for (int d = 1; d < N; ++d) q[d] = src[d * A.nodes + j];
         const double dq = dist<N>(x, q);
-        if (dq < best) { best = dq; for (int d = 0; d < N; ++d) P[d] = q[d]; }
+        if (dq < best) {
+            best = dq;
+            for (int d = 0; d < N; ++d) P[d] = q[d];
+            if constexpr (EXT) from = j;
+        }
     };
     consider(idx);
     const int r2 = N > 2 ? 1 : 0, r1 = N > 1 ? 1 : 0;
@@ -309,14 +415,17 @@ __global__ void __launch_bounds__(TPB) redist_flood_kernel(const __grid_constant
         }
     }
     for (int d = 0; d < N; ++d) dst[d * A.nodes + idx] = P[d];
+    if constexpr (EXT) dst[N * A.nodes + idx] = from >= 0 ? src[N * A.nodes + from] : CUDART_NAN;
 }
 
 template <class T> __device__ __forceinline__ T smallest_subnormal();
 template <> __device__ __forceinline__ float smallest_subnormal<float>() { return 1.40129846e-45f; }
 template <> __device__ __forceinline__ double smallest_subnormal<double>() { return 4.9406564584124654e-324; }
 
-template <class T, int N>
-__global__ void __launch_bounds__(TPB) redist_write_kernel(const __grid_constant__ RedistArgs R, const double* __restrict__ pts) {
+// with the extension (TF not void) F = the value at the point, rounded to TF, on the same nodes; phi only when R.write_phi
+template <class T, int N, class TF = void>
+__global__ void __launch_bounds__(TPB) redist_write_kernel(const __grid_constant__ typename ArgsOf<TF>::type R,
+                                                           const double* __restrict__ pts) {
     const IfaceArgs& A = R.g;
     const long long idx = (long long)blockIdx.x * TPB + threadIdx.x;
     if (idx >= A.nodes) return;
@@ -325,6 +434,10 @@ __global__ void __launch_bounds__(TPB) redist_write_kernel(const __grid_constant
     double q[3];
     q[0] = pts[idx];
     if (s != s || q[0] != q[0]) return;           // NaN node, or no interface at all
+    if constexpr (!std::is_void_v<TF>) {
+        static_cast<TF*>(R.F)[idx] = TF(pts[N * A.nodes + idx]);
+        if (!R.write_phi) return;
+    }
     for (int d = 1; d < N; ++d) q[d] = pts[d * A.nodes + idx];
     int i[3];
     node_index(A, idx, i);
@@ -337,12 +450,13 @@ __global__ void __launch_bounds__(TPB) redist_write_kernel(const __grid_constant
     phi[idx] = v;
 }
 
-template <class T, int N>
-cudaError_t launch_n(const RedistArgs& R, int cell_blocks, cudaStream_t s, int* launches) {
+template <class T, int N, class TF>
+cudaError_t launch_n(const typename ArgsOf<TF>::type& R, int cell_blocks, cudaStream_t s, int* launches) {
+    constexpr bool EXT = !std::is_void_v<TF>;
     const unsigned grid = (unsigned)((R.g.nodes + TPB - 1) / TPB);
     redist_flag_kernel<T, N><<<grid, TPB, 0, s>>>(R);
     for (int pass = 0; pass < 2; ++pass) redist_cells_kernel<T, N><<<cell_blocks, CTPB, 0, s>>>(R, pass);
-    redist_pick_kernel<T, N><<<grid, TPB, 0, s>>>(R);
+    redist_pick_kernel<T, N, TF><<<grid, TPB, 0, s>>>(R);
     *launches = 4;
     int maxn = 1, L = 0;
     for (int d = 0; d < N; ++d) maxn = R.g.m[d] > maxn ? R.g.m[d] : maxn;
@@ -350,30 +464,38 @@ cudaError_t launch_n(const RedistArgs& R, int cell_blocks, cudaStream_t s, int* 
     double *src = R.pa, *dst = R.pb;
     for (int k = 1 << (L - 1); ; k >>= 1) {
         const int kk = k > 0 ? k : 1;             // k = 2^(L-1), ..., 2, 1, then one more pass with k = 1
-        redist_flood_kernel<N><<<grid, TPB, 0, s>>>(R, kk, src, dst);
+        redist_flood_kernel<N, EXT><<<grid, TPB, 0, s>>>(R, kk, src, dst);
         ++*launches;
         double* t = src; src = dst; dst = t;
         if (k == 0) break;
     }
-    redist_write_kernel<T, N><<<grid, TPB, 0, s>>>(R, src);
+    redist_write_kernel<T, N, TF><<<grid, TPB, 0, s>>>(R, src);
     ++*launches;
     return cudaGetLastError();
 }
 
-template <class T>
-cudaError_t launch_t(const RedistArgs& R, int cell_blocks, cudaStream_t s, int* launches) {
+template <class T, class TF>
+cudaError_t launch_t(const typename ArgsOf<TF>::type& R, int cell_blocks, cudaStream_t s, int* launches) {
     switch (R.g.ndim) {
-        case 1: return launch_n<T, 1>(R, cell_blocks, s, launches);
-        case 2: return launch_n<T, 2>(R, cell_blocks, s, launches);
-        default: return launch_n<T, 3>(R, cell_blocks, s, launches);
+        case 1: return launch_n<T, 1, TF>(R, cell_blocks, s, launches);
+        case 2: return launch_n<T, 2, TF>(R, cell_blocks, s, launches);
+        default: return launch_n<T, 3, TF>(R, cell_blocks, s, launches);
     }
+}
+
+template <class TF>
+cudaError_t launch_tf(const typename ArgsOf<TF>::type& R, int cell_blocks, cudaStream_t s, int* launches) {
+    return R.g.f64 ? launch_t<double, TF>(R, cell_blocks, s, launches) : launch_t<float, TF>(R, cell_blocks, s, launches);
 }
 
 }  // namespace
 
 cudaError_t launch_redistance(const RedistArgs& R, int sm_count, cudaStream_t s, int* launches) {
-    const int cell_blocks = sm_count * 16;
-    return R.g.f64 ? launch_t<double>(R, cell_blocks, s, launches) : launch_t<float>(R, cell_blocks, s, launches);
+    return launch_tf<void>(R, sm_count * 16, s, launches);
+}
+
+cudaError_t launch_extend_closest(const ExtendArgs& E, int sm_count, cudaStream_t s, int* launches) {
+    return E.f64 ? launch_tf<double>(E, sm_count * 16, s, launches) : launch_tf<float>(E, sm_count * 16, s, launches);
 }
 
 }  // namespace lsm

@@ -591,6 +591,24 @@ function redistance!(ϕ::DeviceMeshField; band::Integer = 3)
     return _device_advanced!(ϕ)
 end
 
+"""
+    extend_closest_point!(F::DeviceMeshField, ϕ::DeviceMeshField; band = 3, redistance = false) -> F
+
+Give every node of F, in place on the device, the value of F at its closest point on the zero level set of ϕ
+(`lsm_extend_closest_point`): the closest points `redistance!(ϕ)` finds, with F interpolated linearly on the mesh, so a speed known
+near the interface becomes constant along the normals and a constant F comes back unchanged.  NaN nodes of ϕ keep their F.  With
+`redistance = true` the same call also makes ϕ its signed distance, bit for bit what `redistance!` writes:
+`integrate!(eq, tf; prehook = ls -> extend_closest_point!(v, current_state(ls); redistance = true))`.  No boundary conditions, no
+copy to the host, no synchronisation.  Deliberately not a method of `LevelSetMethods.extend_along_normals!`, which solves the
+upwind extension PDE for a number of pseudo-time iterations.
+"""
+function extend_closest_point!(F::DeviceMeshField, ϕ::DeviceMeshField; band::Integer = 3, redistance::Bool = false)
+    check(ccall((:lsm_extend_closest_point, LIB), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, Int32, Int32, Ptr{Int64}),
+                ϕ.ctx.handle, handle!(F), handle!(ϕ), band, redistance ? 1 : 0, C_NULL))
+    redistance && _device_advanced!(ϕ)
+    return _device_advanced!(F)
+end
+
 "`extend_along_normals!(F, ϕ; …)` — src/velocityextension.jl:20-78 on device fields."
 function LSM.extend_along_normals!(F::DeviceMeshField, ϕ::DeviceMeshField; nb_iters::Integer = 50, cfl::Real = 0.45, frozen = nothing,
                                    interface_band::Real = 1.5, min_norm::Real = 1.0e-14)

@@ -113,6 +113,7 @@ cudaError_t launch_extend_closest(const ExtendArgs& E, int sm_count, cudaStream_
 
 // The five Float64 constants of the WENO5 evaluation that do not fit an instruction immediate travel in the kernel parameters
 // (constant bank): as literals the compiler re-materialises them with 10 UMOV per node, from the constant bank it takes 3 uniform loads.
+// The 3-D x-pair kernel's default form scales e6 and fl by 3/16 once per thread (lsm_pair_common.cuh: weno_regs).
 struct WenoK { double c133, c56, cm13, e6, fl, pad; };
 inline WenoK weno_constants() { return {13.0 / 3.0, 5.0 / 6.0, -1.0 / 3.0, 4.0e-6, 1.0e-70, 0.0}; }
 

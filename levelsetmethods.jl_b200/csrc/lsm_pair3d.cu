@@ -48,29 +48,6 @@ struct PairGeom {
     static size_t smem_bytes(int naux) { return ((size_t)RING * PLANE + (size_t)NBUF * naux * TILE) * sizeof(T) + 128 + 16; }
 };
 
-// The same evaluation on first differences d0..d4 AND their differences e1..e4 computed by the caller (so that other terms can
-// share them).  Float64 only.
-template <bool XMAX>
-__device__ __forceinline__ double weno_core_de(const WenoK& K, double d0, double d1, double d2, double d3, double d4,
-                                               double e1, double e2, double e3, double e4) {
-    const double m = XMAX ? absmax5(d0, d1, d2, d3, d4) : absmax5_hi(d0, d1, d2, d3, d4);
-    const double eps = fma(K.e6, m * m, K.fl);
-    const double c133 = K.c133;
-    const double t1a = e2 - e1, t1b = e3 - e2, t1c = e4 - e3;
-    const double t2a = fma(3.0, e2, -e1), t2b = e2 + e3, t2c = fma(-3.0, e3, e4);
-    const double b1 = fma(t2a, t2a, fma(c133, t1a * t1a, eps));
-    const double b2 = fma(t2b, t2b, fma(c133, t1b * t1b, eps));
-    const double b3 = fma(t2c, t2c, fma(c133, t1c * t1c, eps));
-    const double p12 = b1 * b2, p13 = b1 * b3, p23 = b2 * b3;
-    const double w1 = p23 * p23, w2 = p13 * p13, w3 = p12 * p12;
-    const double den = fma(3.0, w3, fma(6.0, w2, w1));
-    const double G1 = fma(K.c56, e2, K.cm13 * e1);
-    const double G2 = fma(2.0, e3, e2);
-    const double G3 = fma(2.0, e3, -0.5 * e4);
-    const double num = fma(w3, G3, fma(w2, G2, w1 * G1));
-    return fma(num, fast_rcp<1>(den), d2);
-}
-
 // One dimension of "NormalMotionTerm + AdvectionTerm(WENO5)" (BASELINE config 5) for two nodes.  The six first differences
 // D[k] = phi[k-2] - phi[k-3] and five second differences E[k] = D[k+1] - D[k] of a node feed BOTH terms:
 //   * the second-order ENO pair of the Godunov norm (levelsetterms.jl:156-170): D-  = D[2], D+ = D[3], D2-- = E[1], D20 = E[2],
@@ -231,12 +208,7 @@ pair3d_kernel(const __grid_constant__ StageParams<T> P, const __grid_constant__ 
                 for (int d = 0; d < 3; ++d) pxy[r][c][d] = (P.terms[TA].cval[d] * __ldg(P.terms[TA].tab[d][0] + ii)) * __ldg(P.terms[TA].tab[d][1] + jj);
             }
     }
-    // The five WENO constants that do not fit an instruction immediate are made opaque to ptxas (threadIdx.z is always 0, which
-    // the compiler cannot know): as plain kernel parameters it re-materialises them from the constant bank with ~12 moves in every
-    // one of the six evaluation blocks of a plane (36 issue slots per node, measured in SASS); this way they stay in 10 registers.
-    const double zopq = __longlong_as_double((long long)threadIdx.z);
-    WenoK KR;
-    KR.c133 = A.wk.c133 + zopq; KR.c56 = A.wk.c56 + zopq; KR.cm13 = A.wk.cm13 + zopq; KR.e6 = A.wk.e6 + zopq; KR.fl = A.wk.fl + zopq; KR.pad = 0.0;
+    const WenoK KR = weno_regs<XMAX>(A.wk);
     long lin = (long)i + (long)j0 * vs1 + (long)zbeg * vs2;       // output / phi^n element offset of node (i, j0, z)
     unsigned long long cfl_best = 0ULL;
 

@@ -24,30 +24,64 @@ __device__ __forceinline__ float2 lds_pair(unsigned addr, float) {
     return v;
 }
 
-// The reference's _weno5(v1..v5) (derivatives.jl:61-81) on UNDIVIDED first differences, restructured exactly like
-// weno5_up of lsm_tile_util.cuh (second differences, one reciprocal); returns h * weno.  The function is odd:
-// core(-v5..-v1 reversed) == -core(...) bit for bit, which is what makes the physical-order evaluation below
-// identical to the upwind-ordered one of lsm_tiled.cu.
-// XMAX: exact max|d| for eps (bit-identical to lsm_tiled.cu) instead of the 20-bit one (absmax5_hi).
+// The WENO constants as the x-pair kernels hold them in registers.  Those that do not fit an instruction immediate are made
+// opaque to ptxas (threadIdx.z is always 0, which the compiler cannot know): as plain kernel parameters it re-materialises them
+// from the constant bank with ~12 moves in every one of the six evaluation blocks of a plane (36 issue slots per node, measured
+// in SASS).  The default form (!XMAX) evaluates the smoothness indicators scaled by 3/16 (weno_core_de), so its eps constants
+// are scaled with them; it reads neither c133 nor c56, and the compiler drops their registers.
 template <bool XMAX>
-__device__ __forceinline__ double weno_core(const WenoK& K, double d0, double d1, double d2, double d3, double d4) {
-    const double e1 = d1 - d0, e2 = d2 - d1, e3 = d3 - d2, e4 = d4 - d3;
+__device__ __forceinline__ WenoK weno_regs(const WenoK& K) {
+    const double zopq = __longlong_as_double((long long)threadIdx.z);
+    const double s = XMAX ? 1.0 : 0.1875;
+    WenoK R;
+    R.c133 = K.c133 + zopq; R.c56 = K.c56 + zopq; R.cm13 = K.cm13 + zopq; R.e6 = K.e6 * s + zopq; R.fl = K.fl * s + zopq; R.pad = 0.0;
+    return R;
+}
+
+// The reference's _weno5(v1..v5) (derivatives.jl:61-81) on UNDIVIDED first differences d0..d4 and their differences e1..e4,
+// restructured like weno5_up of lsm_tile_util.cuh (second differences, one reciprocal); returns h * weno.  The function is
+// odd: core(-v5..-v1 reversed) == -core(...) bit for bit, which is what makes the physical-order evaluation below identical to
+// the upwind-ordered one of lsm_tiled.cu.  K comes from weno_regs<XMAX>.
+// XMAX: exact max|d| for eps and the operations of weno5_up (bit-identical to lsm_tiled.cu).  Otherwise the 20-bit maximum
+// (absmax5_hi) and the smoothness indicators as completed squares: the weights depend only on ratios of the b_k, so
+//   (3/16) b1 = (e1 - 11/8 e2)^2 + 39/64 e2^2 + eps',  (3/16) b2 = (e2 - 5/8 e3)^2 + 39/64 e3^2 + eps',
+//   (3/16) b3 = (e4 - 11/8 e3)^2 + 39/64 e3^2 + eps',  eps' = (3/16) eps
+// give the same result with dyadic coefficients (instruction immediates) in 10 FP64 instructions instead of 15; every term is
+// non-negative, so nothing cancels.  G1 = 5/6 e2 - 1/3 e1 = 3/8 e2 - 1/3 (e1 - 11/8 e2) reuses the first square's base.
+template <bool XMAX>
+__device__ __forceinline__ double weno_core_de(const WenoK& K, double d0, double d1, double d2, double d3, double d4,
+                                               double e1, double e2, double e3, double e4) {
     const double m = XMAX ? absmax5(d0, d1, d2, d3, d4) : absmax5_hi(d0, d1, d2, d3, d4);
     const double eps = fma(K.e6, m * m, K.fl);
-    const double c133 = K.c133;
-    const double t1a = e2 - e1, t1b = e3 - e2, t1c = e4 - e3;
-    const double t2a = fma(3.0, e2, -e1), t2b = e2 + e3, t2c = fma(-3.0, e3, e4);
-    const double b1 = fma(t2a, t2a, fma(c133, t1a * t1a, eps));
-    const double b2 = fma(t2b, t2b, fma(c133, t1b * t1b, eps));
-    const double b3 = fma(t2c, t2c, fma(c133, t1c * t1c, eps));
+    double b1, b2, b3, X1 = 0.0;
+    if constexpr (XMAX) {
+        const double c133 = K.c133;
+        const double t1a = e2 - e1, t1b = e3 - e2, t1c = e4 - e3;
+        const double t2a = fma(3.0, e2, -e1), t2b = e2 + e3, t2c = fma(-3.0, e3, e4);
+        b1 = fma(t2a, t2a, fma(c133, t1a * t1a, eps));
+        b2 = fma(t2b, t2b, fma(c133, t1b * t1b, eps));
+        b3 = fma(t2c, t2c, fma(c133, t1c * t1c, eps));
+    } else {
+        X1 = fma(-1.375, e2, e1);
+        const double X2 = fma(-0.625, e3, e2), X3 = fma(-1.375, e3, e4);
+        const double F2 = fma(0.609375, e2 * e2, eps), F3 = fma(0.609375, e3 * e3, eps);
+        b1 = fma(X1, X1, F2);
+        b2 = fma(X2, X2, F3);
+        b3 = fma(X3, X3, F3);
+    }
     const double p12 = b1 * b2, p13 = b1 * b3, p23 = b2 * b3;
     const double w1 = p23 * p23, w2 = p13 * p13, w3 = p12 * p12;
     const double den = fma(3.0, w3, fma(6.0, w2, w1));
-    const double G1 = fma(K.c56, e2, K.cm13 * e1);
+    const double G1 = XMAX ? fma(K.c56, e2, K.cm13 * e1) : fma(0.375, e2, K.cm13 * X1);
     const double G2 = fma(2.0, e3, e2);
     const double G3 = fma(2.0, e3, -0.5 * e4);
     const double num = fma(w3, G3, fma(w2, G2, w1 * G1));
     return fma(num, fast_rcp<1>(den), d2);
+}
+
+template <bool XMAX>
+__device__ __forceinline__ double weno_core(const WenoK& K, double d0, double d1, double d2, double d3, double d4) {
+    return weno_core_de<XMAX>(K, d0, d1, d2, d3, d4, d1 - d0, d2 - d1, d3 - d2, d4 - d3);
 }
 
 // Float32 fields: all-FP32 evaluation with the differences normalised by 1/max|d| (see weno5_up<float>)

@@ -319,7 +319,8 @@ int32_t lsm_multi_interface_extract(int32_t n, lsm_ctx* const* ctx, lsm_field* c
  * The reference reinitialises phi between steps with reinitialize! (reinitializer.jl:12-42: Newton on Bernstein patches found with
  * a KD-tree, on the host, after downloading values(phi)).  lsm_redistance does the same on the device with the linear interface:
  * it replaces phi in place by the signed distance to the mesh that lsm_interface_extract(ctx, phi, 0.0, ...) would return, without
- * building or fetching that mesh and without touching the context's last extraction.
+ * building or fetching that mesh and without touching the context's last extraction.  lsm_redistance_cubic (below) adds the
+ * reference's Newton step on the cubic interpolant, seeded with these closest points.
  *  - s = double(phi); inside s <= 0, outside s > 0, invalid s NaN (the extraction's rules); node coordinates x_d = lc_d + i_d h_d.
  *  - primitives are the extraction's, rebuilt from phi with the same crossing formula and quad split, so their vertices are
  *    bit-identical to lsm_interface_extract's.  All arithmetic in double, each operation rounded, no FMA; dot(u, v) =
@@ -379,6 +380,54 @@ int32_t lsm_redistance(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* band
  * see the new data.  Scratch: lsm_redistance's plus two value buffers, 16 N + 32 bytes per node in the same context buffer
  * (10.7 GB for a 512^3 3-D field). */
 int32_t lsm_extend_closest_point(lsm_ctx* ctx, lsm_field* F, lsm_field* phi, int32_t band, int32_t redistance_phi, int64_t* band_nodes_out);
+
+/* ---- cubic interpolant: phi between the nodes, as a degree-3 polynomial per cell, on the device --------------------------------
+ * The reference's reinitialize! (interpolation.jl, bernstein.jl) interpolates phi cell by cell with a tensor-product Bernstein patch
+ * of degree 3 fitted to the 4^N surrounding nodes.  With 4 nodes per axis that fit interpolates exactly, so the patch is the same
+ * polynomial as the tensor-product Lagrange interpolant below; the two agree as polynomials, not bit for bit (the reference solves
+ * with a pseudo-inverse of the Kronecker matrix).  In double, each operation rounded, no FMA:
+ *  - u_d = (y_d - lc_d) / h_d; y is inside the box when 0 <= u_d <= n_d - 1 for every d (mirrored grids, h_d < 0, included).
+ *  - cell c_d = min(floor(u_d), n_d - 2); stencil start s_d = min(max(c_d - 1, 0), n_d - 4): the 4 nodes s_d .. s_d + 3, one-sided
+ *    at the box faces, so no boundary conditions are used (needs n_d >= 4); xi = u_d - s_d, a = xi - 1, b = xi - 2, c = xi - 3.
+ *  - weights  L0 = ((a b) c) / -6, L1 = ((xi b) c) / 2, L2 = ((xi a) c) / -2, L3 = ((xi a) b) / 6;
+ *             L0' = ((a b + a c) + b c) / -6, L1' = ((xi b + xi c) + b c) / 2, L2' = ((xi a + xi c) + a c) / -2,
+ *             L3' = ((xi a + xi b) + a b) / 6;
+ *             L0'' = ((a + b) + c) / -3, L1'' = (xi + b) + c, L2'' = -((xi + a) + c), L3'' = ((xi + a) + b) / 3.
+ *    At integer xi the L are exactly 0 or 1, so the interpolant reproduces the node values.
+ *  - contraction over axis 1, then 2, then 3, each sum ((t0 + t1) + t2) + t3 with t_k = w_k * double(phi[s + k]).  The value uses L
+ *    on every axis; d/dy_d uses L' on axis d and is divided by h_d after the contraction; d2/dy_d dy_e uses L'' on axis d (d = e) or
+ *    L' on both axes (d < e) and is divided as (S / h_d) / h_e; the Hessian is symmetric (entry (e, d) = entry (d, e)).
+ *  - a NaN node in the stencil gives NaN.
+ * lsm_interpolate_cubic evaluates it at npts points: pts is npts x ndim (AoS, host), val npts, grad npts x ndim, hess
+ * npts x ndim x ndim (host); any output may be NULL.  A point outside the box gets NaN in every output.  Blocking: one host-to-
+ * device copy of the points, one kernel, device-to-host copies of the requested outputs, through the context's persistent scratch.
+ * Scalar, non-separable fields of this context with every n_d >= 4, npts >= 0 and pts not NULL when npts > 0, else LSM_ERR_ARG;
+ * nranks > 1: LSM_ERR_UNSUPPORTED (slab decomposition is not supported). */
+int32_t lsm_interpolate_cubic(lsm_ctx* ctx, lsm_field* phi, int64_t npts, const double* pts, double* val, double* grad, double* hess);
+
+/* ---- cubic closest-point redistancing: phi <- the signed distance to the zero set of its cubic interpolant, on the device --------
+ * lsm_redistance's passes, then a Newton refinement of every closest point on the interpolant P above, as the reference's
+ * reinitialize! refines its KD-tree seeds (reinitializer.jl:12-42, sdf.jl).  Here the seed of node x is the linear closest point y0
+ * lsm_redistance finds (an O(h^2)-accurate seed), so classification, NaN nodes and the no-interface case are lsm_redistance's.  In
+ * double, each operation rounded, no FMA, with lsm_redistance's dot and dist; P, g = grad P and H = the Hessian of P at y are the
+ * interpolant at y (the patch of the cell containing y):
+ *  - g = grad P(y0); lambda = dot(x - y0, g) / dot(g, g); y = y0.
+ *  - up to 20 iterations: evaluate P, g, H at y; solve the (N+1) x (N+1) system M z = r of the KKT conditions of min |y - x| on
+ *    P = 0, M = [[I + lambda H, g], [g^T, 0]] (diagonal 1 + lambda H_dd, off-diagonal lambda H_de), r = (-((y_d - x_d) + lambda g_d),
+ *    -P), by Gaussian elimination with partial pivoting (for column k the first row i >= k of largest |M_ik| is swapped into row k;
+ *    f = M_ik / M_kk, M_ij = M_ij - f M_kj for j > k, r_i = r_i - f r_k; then z_i = (((r_i - M_i,i+1 z_i+1) - ...) - M_iN z_N) / M_ii
+ *    for i = N .. 0); y_d = y_d + z_d, lambda = lambda + z_N; converged when dist(z, 0) <= 1e-10 min_d |h_d| (z's first N entries).
+ *  - fallback to y0 when: dot(g, g) is 0 or not finite at the start, or lambda is not finite; a value of P, g or H at y is not
+ *    finite; a pivot is 0; z, y or lambda is not finite; y leaves the box; dist(y, y0) > 2 max_d |h_d|; or 20 iterations pass
+ *    without convergence.  The node then gets exactly lsm_redistance's distance, so the call is never worse than lsm_redistance
+ *    on a node.
+ *  - NaN nodes and nodes without a point are not refined; lsm_redistance's write pass then stores -d / +d (raised to the smallest
+ *    subnormal) with d = dist(x, y).
+ * band >= 1, scalar non-separable fields of this context with every n_d >= 4, else LSM_ERR_ARG; nranks > 1: LSM_ERR_UNSUPPORTED
+ * (slab decomposition is not supported).  No boundary conditions are needed.  Asynchronous when both out-pointers are NULL;
+ * otherwise one synchronisation and a 16-byte copy of the number of band nodes (as lsm_redistance counts them) and of the nodes
+ * that fell back.  Bumps the field's version.  Scratch: lsm_redistance's (the refined points go to its spare point buffer). */
+int32_t lsm_redistance_cubic(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* band_nodes_out, int64_t* fallback_nodes_out);
 
 /* ---- diagnostics (test harness; SURVEY.md §2.2 K6) -------------------------------------------- */
 /* max |a - b| over all owned nodes, all-reduced over ranks. */

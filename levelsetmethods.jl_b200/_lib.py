@@ -118,6 +118,8 @@ SYMBOLS = {
     "lsm_multi_interface_extract": (_i32, [_i32, C.POINTER(_vp), C.POINTER(_vp), _dbl, C.POINTER(_i64), C.POINTER(_i64)]),
     "lsm_redistance": (_i32, [_vp, _vp, _i32, C.POINTER(_i64)]),
     "lsm_extend_closest_point": (_i32, [_vp, _vp, _vp, _i32, _i32, C.POINTER(_i64)]),
+    "lsm_interpolate_cubic": (_i32, [_vp, _vp, _i64, _pdbl, _pdbl, _pdbl, _pdbl]),
+    "lsm_redistance_cubic": (_i32, [_vp, _vp, _i32, C.POINTER(_i64), C.POINTER(_i64)]),
     "lsm_max_abs_diff": (_i32, [_vp, _vp, _vp, _pdbl]),
 }
 

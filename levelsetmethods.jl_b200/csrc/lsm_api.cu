@@ -111,7 +111,8 @@ struct lsm_ctx {
     int iface_ndim = 0;
     int64_t iface_nv = 0, iface_np = 0;
     // lsm_redistance scratch (persistent, grown on demand): two point buffers of ndim doubles per node (ndim + 1 for
-    // lsm_extend_closest_point: the value at the point), the two 8-byte keys of the band scan per node, two counters
+    // lsm_extend_closest_point: the value at the point), the two 8-byte keys of the band scan per node, three counters (listed
+    // cells, band nodes, lsm_redistance_cubic's fallbacks); lsm_interpolate_cubic's points and results use the same buffer
     void* d_redist = nullptr; size_t d_redist_bytes = 0;
 };
 
@@ -949,8 +950,19 @@ int32_t interface_extract_impl(lsm_ctx* ctx, lsm_field* phi, double level, int64
 
 
 // ---- closest-point redistancing and extension (lsm_redistance.cu) --------------------------------
+// grows the context's redistancing scratch to at least `need` bytes
+int32_t redist_scratch(lsm_ctx* ctx, size_t need) {
+    if (need > ctx->d_redist_bytes) {
+        if (ctx->d_redist) cudaFree(ctx->d_redist);         // implicit synchronisation: nothing in flight reads it
+        ctx->d_redist = nullptr; ctx->d_redist_bytes = 0;
+        CU(cudaMalloc(&ctx->d_redist, need));
+        ctx->d_redist_bytes = need;
+    }
+    return LSM_OK;
+}
+
 // The arguments and scratch of the redistancing passes on phi (checked by the caller), with `values` extra components per point
-// (the value of F that lsm_extend_closest_point carries); zeroes the two counters on the context's stream.
+// (the value of F that lsm_extend_closest_point carries); zeroes the three counters on the context's stream.
 int32_t redist_setup(lsm_ctx* ctx, lsm_field* phi, int32_t band, int values, RedistArgs& R) {
     CU(cudaSetDevice(ctx->device));
     IfaceArgs& A = R.g;
@@ -965,13 +977,7 @@ int32_t redist_setup(lsm_ctx* ctx, lsm_field* phi, int32_t band, int values, Red
     A.nodes = (long long)A.m[0] * A.m[1] * A.m[2];
     R.band = band;
     const size_t pbytes = (size_t)A.nodes * (phi->ndim + values) * sizeof(double), kbytes = (size_t)A.nodes * sizeof(unsigned long long);
-    const size_t need = 2 * pbytes + 2 * kbytes + 2 * sizeof(unsigned long long);
-    if (need > ctx->d_redist_bytes) {
-        if (ctx->d_redist) cudaFree(ctx->d_redist);         // implicit synchronisation: nothing in flight reads it
-        ctx->d_redist = nullptr; ctx->d_redist_bytes = 0;
-        CU(cudaMalloc(&ctx->d_redist, need));
-        ctx->d_redist_bytes = need;
-    }
+    TRY(redist_scratch(ctx, 2 * pbytes + 2 * kbytes + 3 * sizeof(unsigned long long)));
     char* base = static_cast<char*>(ctx->d_redist);
     R.pa = reinterpret_cast<double*>(base);
     R.pb = reinterpret_cast<double*>(base + pbytes);
@@ -980,7 +986,7 @@ int32_t redist_setup(lsm_ctx* ctx, lsm_field* phi, int32_t band, int values, Red
     R.ord = R.dmin + A.nodes;
     R.ncells = R.ord + A.nodes;
     R.count = R.ncells + 1;
-    CU(cudaMemsetAsync(R.ncells, 0, 2 * sizeof(unsigned long long), ctx->stream));
+    CU(cudaMemsetAsync(R.ncells, 0, 3 * sizeof(unsigned long long), ctx->stream));
     return LSM_OK;
 }
 
@@ -1033,6 +1039,68 @@ int32_t extend_closest_impl(lsm_ctx* ctx, lsm_field* F, lsm_field* phi, int32_t 
     F->version++; F->halo_valid = false;
     if (E.write_phi) { phi->version++; phi->halo_valid = false; }
     return redist_band_nodes(ctx, E, band_nodes_out);
+}
+
+// the checks lsm_redistance_cubic and lsm_interpolate_cubic share: a scalar field of this context with n_d >= 4, single rank
+int32_t cubic_check(lsm_ctx* ctx, lsm_field* phi, const char* what) {
+    if (!ctx || !phi) return fail(LSM_ERR_ARG, "null argument");
+    if (phi->ctx != ctx || phi->ncomp != 1 || phi->separable) return fail(LSM_ERR_ARG, "%s needs a real-valued field of this context", what);
+    for (int d = 0; d < phi->ndim; ++d)
+        if (phi->nglob[d] < 4) return fail(LSM_ERR_ARG, "%s needs at least 4 nodes along every dimension (n[%d] = %d)", what, d, phi->nglob[d]);
+    if (ctx->nranks > 1) return fail(LSM_ERR_UNSUPPORTED, "%s of a slab-decomposed field (nranks = %d) is not supported", what, ctx->nranks);
+    return LSM_OK;
+}
+
+int32_t redistance_cubic_impl(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* band_nodes_out, int64_t* fallback_nodes_out) {
+    if (band < 1) return fail(LSM_ERR_ARG, "band must be at least 1 (got %d)", band);
+    TRY(cubic_check(ctx, phi, "cubic redistancing"));
+    RedistArgs R{};
+    TRY(redist_setup(ctx, phi, band, 0, R));
+    int launches = 0;
+    CU(launch_redistance_cubic(R, R.count + 1, ctx->sm_count, ctx->stream, &launches));
+    ctx->cnt.kernel_launches += launches;
+    phi->version++; phi->halo_valid = false;
+    if (band_nodes_out || fallback_nodes_out) {                  // band nodes and fallbacks are adjacent: one 16-byte copy
+        CU(cudaMemcpyAsync(ctx->h_scalar, R.count, 16, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaStreamSynchronize(ctx->stream));
+        ctx->cnt.d2h_bytes += 16;
+        if (band_nodes_out) *band_nodes_out = (int64_t)ctx->h_scalar[0];
+        if (fallback_nodes_out) *fallback_nodes_out = (int64_t)ctx->h_scalar[1];
+    }
+    return LSM_OK;
+}
+
+int32_t interpolate_cubic_impl(lsm_ctx* ctx, lsm_field* phi, int64_t npts, const double* pts, double* val, double* grad, double* hess) {
+    TRY(cubic_check(ctx, phi, "cubic interpolation"));
+    if (npts < 0) return fail(LSM_ERR_ARG, "npts must not be negative (got %lld)", (long long)npts);
+    if (npts > 0 && !pts) return fail(LSM_ERR_ARG, "null points");
+    if (npts == 0) return LSM_OK;
+    CU(cudaSetDevice(ctx->device));
+    const int N = phi->ndim;
+    IfaceArgs A{};
+    A.phi = phi->p; A.f64 = phi->dtype == LSM_F64; A.ndim = N; A.hsign = 1;
+    for (int d = 0; d < 3; ++d) { A.m[d] = phi->n[d]; A.lc[d] = phi->lc[d]; A.h[d] = d < N ? phi->h[d] : 0.0; }
+    A.s1 = A.m[0]; A.s2 = (long long)A.m[0] * A.m[1];
+    A.nodes = (long long)A.m[0] * A.m[1] * A.m[2];
+    // scratch: points, then values, gradients and Hessians (only the requested ones)
+    const size_t pb = (size_t)npts * N * sizeof(double), vb = val ? (size_t)npts * sizeof(double) : 0,
+                 gb = grad ? pb : 0, hb = hess ? pb * N : 0;
+    TRY(redist_scratch(ctx, pb + vb + gb + hb));
+    char* base = static_cast<char*>(ctx->d_redist);
+    double* dp = reinterpret_cast<double*>(base);
+    double* dv = val ? reinterpret_cast<double*>(base + pb) : nullptr;
+    double* dg = grad ? reinterpret_cast<double*>(base + pb + vb) : nullptr;
+    double* dh = hess ? reinterpret_cast<double*>(base + pb + vb + gb) : nullptr;
+    CU(cudaMemcpyAsync(dp, pts, pb, cudaMemcpyHostToDevice, ctx->stream));
+    ctx->cnt.h2d_bytes += pb;
+    CU(launch_interp_cubic(A, npts, dp, dv, dg, dh, ctx->stream));
+    ctx->cnt.kernel_launches += 1;
+    if (val) CU(cudaMemcpyAsync(val, dv, vb, cudaMemcpyDeviceToHost, ctx->stream));
+    if (grad) CU(cudaMemcpyAsync(grad, dg, gb, cudaMemcpyDeviceToHost, ctx->stream));
+    if (hess) CU(cudaMemcpyAsync(hess, dh, hb, cudaMemcpyDeviceToHost, ctx->stream));
+    ctx->cnt.d2h_bytes += vb + gb + hb;
+    CU(cudaStreamSynchronize(ctx->stream));
+    return LSM_OK;
 }
 
 }  // namespace
@@ -1795,6 +1863,14 @@ int32_t lsm_redistance(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* band
 
 int32_t lsm_extend_closest_point(lsm_ctx* ctx, lsm_field* F, lsm_field* phi, int32_t band, int32_t redistance_phi, int64_t* band_nodes_out) {
     return extend_closest_impl(ctx, F, phi, band, redistance_phi, band_nodes_out);
+}
+
+int32_t lsm_interpolate_cubic(lsm_ctx* ctx, lsm_field* phi, int64_t npts, const double* pts, double* val, double* grad, double* hess) {
+    return interpolate_cubic_impl(ctx, phi, npts, pts, val, grad, hess);
+}
+
+int32_t lsm_redistance_cubic(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* band_nodes_out, int64_t* fallback_nodes_out) {
+    return redistance_cubic_impl(ctx, phi, band, band_nodes_out, fallback_nodes_out);
 }
 
 int32_t lsm_field_csg(lsm_ctx* ctx, lsm_field* dst, const lsm_field* src, int32_t op) {

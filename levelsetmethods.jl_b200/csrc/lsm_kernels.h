@@ -111,6 +111,15 @@ struct ExtendArgs : RedistArgs {
 // enqueues the same kernels as launch_redistance on s; *launches = kernels enqueued
 cudaError_t launch_extend_closest(const ExtendArgs& E, int sm_count, cudaStream_t s, int* launches);
 
+// lsm_redistance.cu, cubic variant (lsm_redistance_cubic): launch_redistance's passes with the Newton refinement on the cubic
+// interpolant (lsm_cubic.cuh) between the last flooding pass and the write; *fallbacks (zeroed by the caller) counts the nodes that
+// keep their linear closest point.
+cudaError_t launch_redistance_cubic(const RedistArgs& R, unsigned long long* fallbacks, int sm_count, cudaStream_t s, int* launches);
+// lsm_interpolate_cubic: the interpolant of A's field at npts points (pts AoS, npts x ndim); val (npts), grad (npts x ndim) and
+// hess (npts x ndim x ndim) may each be null
+cudaError_t launch_interp_cubic(const IfaceArgs& A, long long npts, const double* pts, double* val, double* grad, double* hess,
+                                cudaStream_t s);
+
 // The five Float64 constants of the WENO5 evaluation that do not fit an instruction immediate travel in the kernel parameters
 // (constant bank): as literals the compiler re-materialises them with 10 UMOV per node, from the constant bank it takes 3 uniform loads.
 // The 3-D x-pair kernel's default form scales e6 and fl by 3/16 once per thread (lsm_pair_common.cuh: weno_regs).

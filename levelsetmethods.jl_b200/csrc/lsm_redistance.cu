@@ -19,14 +19,21 @@
 // void; EXT in the flood): pick also interpolates F at the winning closest point, the flood carries that value with the point (as
 // an (N+1)-th component of the point buffers), and write stores it into F, and the signed distance into phi when asked.  flag and
 // the cell passes are shared as they are, so the points are the ones lsm_redistance computes.
+// Cubic redistancing (lsm_redistance_cubic) runs lsm_redistance's kernels unchanged with one more between the last flood and the
+// write:
+//   refine: one thread per node; Newton on the KKT system of the closest point on the cubic interpolant (lsm_cubic.cuh), from the
+//           node's linear closest point, into the spare point buffer; a node that falls back keeps the linear point and is counted.
+// cubic_interp_kernel evaluates the same interpolant at arbitrary points for lsm_interpolate_cubic.
 // The operation order of every distance, closest point and value is the one include/lsm_b200.h states; tests/redistance_ref.py and
-// tests/extension_ref.py restate it in NumPy and agree with this file bit for bit (it is compiled with -fmad=false).
+// tests/extension_ref.py (and tests/cubic_ref.py for the cubic kernels) restate it in NumPy and agree with this file bit for bit (it
+// is compiled with -fmad=false).
 #include <cstdint>
 #include <type_traits>
 #include <cuda_runtime.h>
 #include <math_constants.h>
 #include "lsm_kernels.h"
 #include "lsm_simplex.cuh"
+#include "lsm_cubic.cuh"
 
 namespace lsm {
 namespace {
@@ -450,8 +457,141 @@ __global__ void __launch_bounds__(TPB) redist_write_kernel(const __grid_constant
     phi[idx] = v;
 }
 
+// ---- lsm_redistance_cubic: Newton refinement of the closest points on the cubic interpolant (lsm_cubic.cuh) -------------------
+constexpr int NEWTON_ITERS = 20;
+
+__device__ __forceinline__ bool finite(double v) { return fabs(v) < CUDART_INF; }
+
+// Solves M z = r, M (K x K), by Gaussian elimination with partial pivoting (the first row of largest |entry| wins; columns left to
+// right; then back substitution).  Rows are swapped with compile-time indices only, so M stays in registers.  false on a zero pivot.
+template <int K> __device__ __forceinline__ bool solve(double (*M)[K], double* r, double* z) {
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+        int p = k;
+        double big = fabs(M[k][k]);
+#pragma unroll
+        for (int i = k + 1; i < K; ++i) if (fabs(M[i][k]) > big) { big = fabs(M[i][k]); p = i; }
+        if (big == 0.0) return false;
+#pragma unroll
+        for (int i = k + 1; i < K; ++i) {
+            if (i == p) {
+#pragma unroll
+                for (int j = k; j < K; ++j) { const double t = M[k][j]; M[k][j] = M[i][j]; M[i][j] = t; }
+                const double t = r[k]; r[k] = r[i]; r[i] = t;
+            }
+        }
+#pragma unroll
+        for (int i = k + 1; i < K; ++i) {
+            const double f = M[i][k] / M[k][k];
+#pragma unroll
+            for (int j = k + 1; j < K; ++j) M[i][j] = M[i][j] - f * M[k][j];
+            r[i] = r[i] - f * r[k];
+        }
+    }
+#pragma unroll
+    for (int i = K - 1; i >= 0; --i) {
+        double s = r[i];
+#pragma unroll
+        for (int j = i + 1; j < K; ++j) s = s - M[i][j] * z[j];
+        z[i] = s / M[i][i];
+    }
+    return true;
+}
+
+// Newton on the KKT system of min |y - x| subject to P(y) = 0, from the linear closest point y0 (include/lsm_b200.h states the
+// iteration).  Returns true with the refined point in y, or false (fall back to y0).
+template <class T, int N>
+__device__ __forceinline__ bool newton(const IfaceArgs& A, const double* x, const double* y0, double* y) {
+    double P, g[N], H[3][3];
+    cubic::eval<T, N, 1>(A, y0, P, g, H);
+    const double gg = dot<N>(g, g);
+    if (!finite(gg) || gg == 0.0) return false;
+    double xy[N];
+    for (int d = 0; d < N; ++d) { xy[d] = x[d] - y0[d]; y[d] = y0[d]; }
+    double lam = dot<N>(xy, g) / gg;
+    if (!finite(lam)) return false;
+    double hmin = fabs(A.h[0]), hmax = fabs(A.h[0]);
+    for (int d = 1; d < N; ++d) { hmin = fmin(hmin, fabs(A.h[d])); hmax = fmax(hmax, fabs(A.h[d])); }
+    const double tol = 1e-10 * hmin, reach = 2.0 * hmax;
+    for (int it = 0; it < NEWTON_ITERS; ++it) {
+        if (!cubic::eval<T, N, 2>(A, y, P, g, H)) return false;
+        bool fin = finite(P);
+        double M[N + 1][N + 1], r[N + 1], z[N + 1];
+#pragma unroll
+        for (int i = 0; i < N; ++i) {
+#pragma unroll
+            for (int j = 0; j < N; ++j) { M[i][j] = i == j ? 1.0 + lam * H[i][j] : lam * H[i][j]; fin = fin && finite(H[i][j]); }
+            M[i][N] = g[i];
+            M[N][i] = g[i];
+            r[i] = -((y[i] - x[i]) + lam * g[i]);
+            fin = fin && finite(g[i]);
+        }
+        M[N][N] = 0.0;
+        r[N] = -P;
+        if (!fin) return false;
+        if (!solve<N + 1>(M, r, z)) return false;
+        bool zf = true;
+        for (int d = 0; d <= N; ++d) zf = zf && finite(z[d]);
+        if (!zf) return false;
+        for (int d = 0; d < N; ++d) y[d] = y[d] + z[d];
+        lam = lam + z[N];
+        bool ok = finite(lam);
+        for (int d = 0; d < N; ++d) {
+            const double u = (y[d] - A.lc[d]) / A.h[d];
+            ok = ok && finite(y[d]) && u >= 0.0 && u <= double(A.m[d] - 1);
+        }
+        if (!ok || dist<N>(y, y0) > reach) return false;
+        const double zero[N] = {};
+        if (dist<N>(z, zero) <= tol) return true;
+    }
+    return false;
+}
+
+// every node: the refined closest point from the linear one in src (NaN = no point) into dst; a NaN node keeps its point (the write
+// pass leaves it alone).  Counts the nodes that fall back to the linear point.
+template <class T, int N>
+__global__ void __launch_bounds__(TPB) redist_refine_kernel(const __grid_constant__ RedistArgs R, const double* __restrict__ src,
+                                                            double* __restrict__ dst, unsigned long long* fallbacks) {
+    const IfaceArgs& A = R.g;
+    const long long idx = (long long)blockIdx.x * TPB + threadIdx.x;
+    bool fell = false;
+    if (idx < A.nodes) {
+        double y0[N], y[N];
+        for (int d = 0; d < N; ++d) y0[d] = src[d * A.nodes + idx];
+        const double s = double(static_cast<const T*>(A.phi)[idx]);
+        if (y0[0] == y0[0] && s == s) {
+            int i[3];
+            node_index(A, idx, i);
+            double x[3];
+            node_coords(A, i, x);
+            fell = !newton<T, N>(A, x, y0, y);
+            if (fell) for (int d = 0; d < N; ++d) y[d] = y0[d];
+        } else {
+            for (int d = 0; d < N; ++d) y[d] = y0[d];
+        }
+        for (int d = 0; d < N; ++d) dst[d * A.nodes + idx] = y[d];
+    }
+    const unsigned bal = __ballot_sync(0xffffffffu, fell);
+    if ((threadIdx.x & 31) == 0 && bal) atomicAdd(fallbacks, (unsigned long long)__popc(bal));
+}
+
+// lsm_interpolate_cubic: one thread per point; pts AoS (npts x N), outputs AoS and optional
+template <class T, int N>
+__global__ void __launch_bounds__(TPB) cubic_interp_kernel(const __grid_constant__ IfaceArgs A, long long npts,
+                                                           const double* __restrict__ pts, double* val, double* grad, double* hess) {
+    const long long p = (long long)blockIdx.x * TPB + threadIdx.x;
+    if (p >= npts) return;
+    double y[N], P, g[N], H[3][3];
+    for (int d = 0; d < N; ++d) y[d] = pts[p * N + d];
+    cubic::eval<T, N, 2>(A, y, P, g, H);
+    if (val) val[p] = P;
+    if (grad) for (int d = 0; d < N; ++d) grad[p * N + d] = g[d];
+    if (hess) for (int d = 0; d < N; ++d) for (int e = 0; e < N; ++e) hess[(p * N + d) * N + e] = H[d][e];
+}
+
 template <class T, int N, class TF>
-cudaError_t launch_n(const typename ArgsOf<TF>::type& R, int cell_blocks, cudaStream_t s, int* launches) {
+cudaError_t launch_n(const typename ArgsOf<TF>::type& R, int cell_blocks, cudaStream_t s, int* launches,
+                     unsigned long long* fallbacks = nullptr) {
     constexpr bool EXT = !std::is_void_v<TF>;
     const unsigned grid = (unsigned)((R.g.nodes + TPB - 1) / TPB);
     redist_flag_kernel<T, N><<<grid, TPB, 0, s>>>(R);
@@ -469,23 +609,45 @@ cudaError_t launch_n(const typename ArgsOf<TF>::type& R, int cell_blocks, cudaSt
         double* t = src; src = dst; dst = t;
         if (k == 0) break;
     }
+    if constexpr (std::is_void_v<TF>) {
+        if (fallbacks) {                          // the cubic refinement: the spare point buffer takes the refined points
+            redist_refine_kernel<T, N><<<grid, TPB, 0, s>>>(R, src, dst, fallbacks);
+            ++*launches;
+            src = dst;
+        }
+    }
     redist_write_kernel<T, N, TF><<<grid, TPB, 0, s>>>(R, src);
     ++*launches;
     return cudaGetLastError();
 }
 
 template <class T, class TF>
-cudaError_t launch_t(const typename ArgsOf<TF>::type& R, int cell_blocks, cudaStream_t s, int* launches) {
+cudaError_t launch_t(const typename ArgsOf<TF>::type& R, int cell_blocks, cudaStream_t s, int* launches,
+                     unsigned long long* fallbacks = nullptr) {
     switch (R.g.ndim) {
-        case 1: return launch_n<T, 1, TF>(R, cell_blocks, s, launches);
-        case 2: return launch_n<T, 2, TF>(R, cell_blocks, s, launches);
-        default: return launch_n<T, 3, TF>(R, cell_blocks, s, launches);
+        case 1: return launch_n<T, 1, TF>(R, cell_blocks, s, launches, fallbacks);
+        case 2: return launch_n<T, 2, TF>(R, cell_blocks, s, launches, fallbacks);
+        default: return launch_n<T, 3, TF>(R, cell_blocks, s, launches, fallbacks);
     }
 }
 
 template <class TF>
-cudaError_t launch_tf(const typename ArgsOf<TF>::type& R, int cell_blocks, cudaStream_t s, int* launches) {
-    return R.g.f64 ? launch_t<double, TF>(R, cell_blocks, s, launches) : launch_t<float, TF>(R, cell_blocks, s, launches);
+cudaError_t launch_tf(const typename ArgsOf<TF>::type& R, int cell_blocks, cudaStream_t s, int* launches,
+                      unsigned long long* fallbacks = nullptr) {
+    return R.g.f64 ? launch_t<double, TF>(R, cell_blocks, s, launches, fallbacks)
+                   : launch_t<float, TF>(R, cell_blocks, s, launches, fallbacks);
+}
+
+template <class T>
+cudaError_t launch_interp_t(const IfaceArgs& A, long long npts, const double* pts, double* val, double* grad, double* hess,
+                            cudaStream_t s) {
+    const unsigned grid = (unsigned)((npts + TPB - 1) / TPB);
+    switch (A.ndim) {
+        case 1: cubic_interp_kernel<T, 1><<<grid, TPB, 0, s>>>(A, npts, pts, val, grad, hess); break;
+        case 2: cubic_interp_kernel<T, 2><<<grid, TPB, 0, s>>>(A, npts, pts, val, grad, hess); break;
+        default: cubic_interp_kernel<T, 3><<<grid, TPB, 0, s>>>(A, npts, pts, val, grad, hess); break;
+    }
+    return cudaGetLastError();
 }
 
 }  // namespace
@@ -496,6 +658,16 @@ cudaError_t launch_redistance(const RedistArgs& R, int sm_count, cudaStream_t s,
 
 cudaError_t launch_extend_closest(const ExtendArgs& E, int sm_count, cudaStream_t s, int* launches) {
     return E.f64 ? launch_tf<double>(E, sm_count * 16, s, launches) : launch_tf<float>(E, sm_count * 16, s, launches);
+}
+
+cudaError_t launch_redistance_cubic(const RedistArgs& R, unsigned long long* fallbacks, int sm_count, cudaStream_t s, int* launches) {
+    return launch_tf<void>(R, sm_count * 16, s, launches, fallbacks);
+}
+
+cudaError_t launch_interp_cubic(const IfaceArgs& A, long long npts, const double* pts, double* val, double* grad, double* hess,
+                                cudaStream_t s) {
+    if (npts <= 0) return cudaSuccess;
+    return A.f64 ? launch_interp_t<double>(A, npts, pts, val, grad, hess, s) : launch_interp_t<float>(A, npts, pts, val, grad, hess, s);
 }
 
 }  // namespace lsm

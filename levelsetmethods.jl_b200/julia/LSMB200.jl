@@ -577,18 +577,48 @@ function interface_mesh(mc::MultiContext, ϕs::Vector{<:DeviceMeshField{N}}; lev
 end
 
 """
-    redistance!(ϕ::DeviceMeshField; band = 3) -> ϕ
+    redistance!(ϕ::DeviceMeshField; band = 3, order = 1) -> ϕ
 
 Replace ϕ, in place on the device, by the signed distance to its zero level set (`lsm_redistance`): the piecewise-linear mesh
 `interface_mesh(ϕ)` returns, which is never built.  Nodes within `band` cells of it get their exact closest point, jump flooding
 carries closest points to the rest of the grid; every node keeps its sign, NaN nodes stay NaN.  No boundary conditions needed, no
 copy to the host and no synchronisation, so it fits a prehook: `integrate!(eq, tf; prehook = ls -> redistance!(current_state(ls)))`.
-The same idea as `LevelSetMethods.reinitialize!` (reinitializer.jl:12-42, Newton on Bernstein patches, host) with a linear
-interface, so the two are not bit-compatible; that is why this is not a method of `reinitialize!`.
+`order = 3` (`lsm_redistance_cubic`) refines every closest point by Newton's method on the zero set of the cubic interpolant of ϕ
+(`interpolate_cubic`), third-order accurate; a node where Newton fails keeps its linear closest point.
+The same idea as `LevelSetMethods.reinitialize!` (reinitializer.jl:12-42, Newton on Bernstein patches from KD-tree seeds, host),
+but the seeds (the linear mesh) and the one-sided stencils at the box faces are not verified against it, so the two are not
+bit-compatible; that is why this is not a method of `reinitialize!`.
 """
-function redistance!(ϕ::DeviceMeshField; band::Integer = 3)
-    check(ccall((:lsm_redistance, LIB), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Int32, Ptr{Int64}), ϕ.ctx.handle, handle!(ϕ), band, C_NULL))
+function redistance!(ϕ::DeviceMeshField; band::Integer = 3, order::Integer = 1)
+    if order == 1
+        check(ccall((:lsm_redistance, LIB), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Int32, Ptr{Int64}), ϕ.ctx.handle, handle!(ϕ), band, C_NULL))
+    elseif order == 3
+        check(ccall((:lsm_redistance_cubic, LIB), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Int32, Ptr{Int64}, Ptr{Int64}),
+                    ϕ.ctx.handle, handle!(ϕ), band, C_NULL, C_NULL))
+    else
+        throw(ArgumentError("redistance!: order must be 1 or 3 (got $order)"))
+    end
     return _device_advanced!(ϕ)
+end
+
+"""
+    interpolate_cubic(ϕ::DeviceMeshField, X::AbstractMatrix) -> (values, gradients, hessians)
+
+The tensor-product cubic interpolant of ϕ (`lsm_interpolate_cubic`) at the columns of X (N × npts): `values` (npts),
+`gradients` (N × npts) and `hessians` (N × N × npts), evaluated on the device; NaN at points outside the grid.  The same
+polynomial per cell as the reference's Bernstein patch of an `InterpolatedField` (interpolation.jl, bernstein.jl), not the same
+bits; one-sided stencils at the box faces, no boundary conditions.
+"""
+function interpolate_cubic(ϕ::DeviceMeshField{N}, X::AbstractMatrix) where {N}
+    size(X, 1) == N || throw(DimensionMismatch("interpolate_cubic: X must have $N rows (one column per point), got $(size(X, 1))"))
+    pts = Matrix{Float64}(X)
+    npts = size(pts, 2)
+    val = Vector{Float64}(undef, npts)
+    grad = Matrix{Float64}(undef, N, npts)
+    hess = Array{Float64, 3}(undef, N, N, npts)
+    check(ccall((:lsm_interpolate_cubic, LIB), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+                ϕ.ctx.handle, handle!(ϕ), npts, pts, val, grad, hess))
+    return val, grad, hess
 end
 
 """

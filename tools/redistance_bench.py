@@ -1,16 +1,18 @@
 #!/usr/bin/env python
-"""tools/redistance_bench.py — closest-point redistancing on the device (redistance, lsm_redistance, band 3) against the PDE
-reinitialisation eikonal_reinitialize(iterations=20) on the same Float64 states:
+"""tools/redistance_bench.py — closest-point redistancing on the device (redistance, lsm_redistance, band 3; and order=3,
+lsm_redistance_cubic, with its fallback count) against the PDE reinitialisation eikonal_reinitialize(iterations=20) on the same
+Float64 states:
 
   sphere  a 512^3 sphere of radius 0.35 on [-0.5, 0.5]^3, generated on the device (lsm_field_fill_shape), NeumannBC;
   c3      bench.py's C3 state (Enright sphere, WENO5 + TVD-RK3, NeumannBC) after --c3-steps RK3 steps.
 
 Time: CUDA events on the library's stream around each call, the median of --reps after --warmup calls (each call works on the
 output of the previous one; the working set, 8.6 GB of scratch at 512^3, is far larger than the L2).  Quality, from one call
-on a copy of the state: the interface shift (the largest distance from a vertex of extract_interface after the call to the mesh
+on a copy of the state: the mean Newton iterations of order 3 within 3h (newton_iterations: the NumPy restatement of the device's
+arithmetic on a sample of the state's nodes), the interface shift (the largest distance from a vertex of extract_interface after the call to the mesh
 before, over the 8 primitives nearest by centroid: an upper bound) and max | |grad phi| - 1 | over the nodes with |phi| < 3 h whose
 second differences are below 0.5 / h on every axis (centred differences; away from kinks).  --profile: mean CUDA time per kernel of
-redistance under torch.profiler, in a separate run.  The card's name and power limit are read in the same run.  One JSON line per
+redistance and of redistance(order=3) under torch.profiler, in a separate run.  The card's name and power limit are read in the same run.  One JSON line per
 state.
 
     python tools/redistance_bench.py [--n 512] [--c3-steps 20] [--reps 10] [--warmup 2] [--profile]
@@ -90,6 +92,35 @@ def quality(m, phi, fn):
     return out
 
 
+def newton_iterations(phi, mesh, sample=20000, k=16, seed=0):
+    """Newton iterations of redistance(order=3) within 3h, from tests/cubic_ref.py (the device's arithmetic) on the same state: up
+    to `sample` random nodes whose distance to the extracted mesh is below 3h, seeded with their closest point on that mesh (the
+    band scan's point; the first primitive in mesh order among equally close ones, over the k nearest by centroid).  Returns
+    (mean iterations of the converged nodes, nodes that fell back, nodes sampled)."""
+    import cubic_ref as CR
+    import redistance_ref as R
+    from scipy.spatial import cKDTree
+    vals = np.asarray(phi.peek())
+    g = phi.mesh
+    h, lc = g.meshsize(), g.lc
+    h3 = 3 * min(abs(v) for v in h)
+    cand = np.flatnonzero(np.abs(vals) < 2 * h3)
+    cand = np.random.default_rng(seed).permutation(cand)[:4 * sample]
+    idx = np.stack(np.unravel_index(cand, vals.shape), axis=-1)
+    x = np.stack([float(lc[d]) + idx[:, d].astype(np.float64) * float(h[d]) for d in range(vals.ndim)], axis=-1)
+    V = mesh.vertices[mesh.faces.astype(np.int64)]
+    _, j = cKDTree(V.mean(axis=1)).query(x, k=k)
+    j = np.sort(j.reshape(len(x), k), axis=1)
+    X = np.repeat(x[:, None, :], k, axis=1)
+    q = R.closest_point(X, V[j])
+    d = R.dist(X, q)
+    best = np.argmin(d, axis=1)
+    dmin = d[np.arange(len(x)), best]
+    keep = np.flatnonzero(dmin < h3)[:sample]
+    y, fell, iters = CR.refine(vals, lc, h, x[keep], q[keep, best[keep]])
+    return float(iters[~fell].mean()), int(fell.sum()), int(len(keep))
+
+
 def measure(m, ctx, phi, reps, warmup):
     lib = m._lib.lib()
     nb = C.c_int64()
@@ -98,11 +129,20 @@ def measure(m, ctx, phi, reps, warmup):
     work = phi.copy()
     red_ms, red_min = timed(ctx, lambda: m.redistance(work, band=3), reps, warmup)
     work = phi.copy()
+    nf = C.c_int64()
+    m._lib.check(lib.lsm_redistance_cubic(ctx.handle, work.device(), 3, None, C.byref(nf)))     # fallbacks on the state itself
+    work = phi.copy()
+    cub_ms, cub_min = timed(ctx, lambda: m.redistance(work, band=3, order=3), reps, warmup)
+    work = phi.copy()
     eik_ms, eik_min = timed(ctx, lambda: m.eikonal_reinitialize(work, iterations=20), reps, warmup)
     del work
-    return {"nodes": list(phi.mesh.n), "band_nodes": int(nb.value),
-            "redistance_ms": red_ms, "redistance_ms_min": red_min, "eikonal20_ms": eik_ms, "eikonal20_ms_min": eik_min,
+    it, it_fell, it_nodes = newton_iterations(phi, m.extract_interface(phi))
+    return {"nodes": list(phi.mesh.n), "band_nodes": int(nb.value), "newton_iters_3h": it, "newton_fallbacks_3h": it_fell,
+            "newton_sampled_3h": it_nodes,
+            "redistance_ms": red_ms, "redistance_ms_min": red_min, "cubic_ms": cub_ms, "cubic_ms_min": cub_min,
+            "cubic_fallbacks": int(nf.value), "eikonal20_ms": eik_ms, "eikonal20_ms_min": eik_min,
             "redistance": quality(m, phi, lambda f: m.redistance(f, band=3)),
+            "cubic": quality(m, phi, lambda f: m.redistance(f, band=3, order=3)),
             "eikonal20": quality(m, phi, lambda f: m.eikonal_reinitialize(f, iterations=20))}
 
 
@@ -126,14 +166,17 @@ def main():
     if args.profile:
         import torch
         from torch.profiler import ProfilerActivity, profile
+        cub = phi.copy()                       # each order works on its own output, as in the timed runs
         m.redistance(phi)
+        m.redistance(cub, order=3)
         ctx.sync()
         with profile(activities=[ProfilerActivity.CUDA]) as prof:
             for _ in range(args.reps):
                 m.redistance(phi)
+                m.redistance(cub, order=3)
             ctx.sync()
         torch.cuda.synchronize()
-        kern = {e.key[:60]: {"calls": e.count, "mean_us": e.device_time} for e in prof.key_averages() if "redist" in e.key}
+        kern = {e.key[:70]: {"calls": e.count, "mean_us": e.device_time} for e in prof.key_averages() if "redist" in e.key or "refine" in e.key}
         print(json.dumps({"state": f"sphere r=0.35, {n}^3, Float64 (profiled)", "card": name, "power_limit": limit, "kernels": kern}), flush=True)
         return
     res = measure(m, ctx, phi, args.reps, args.warmup)

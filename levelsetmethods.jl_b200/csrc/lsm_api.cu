@@ -96,7 +96,7 @@ struct lsm_ctx {
     unsigned* d_cand_count = nullptr; double* d_cand = nullptr; double* h_cand = nullptr;   // candidate staging (device / pinned)
     void* stage[2] = {nullptr, nullptr};        // AoS <-> SoA staging chunks of vector-field transfers (allocated on first use)
     cudaEvent_t ev_stage[2] = {nullptr, nullptr}, ev_free[2] = {nullptr, nullptr};
-    double* d_work = nullptr; size_t d_work_bytes = 0;     // persistent scratch of the reductions / getindex (grown on demand)
+    void* d_work = nullptr; size_t d_work_bytes = 0;       // persistent scratch of the reductions / getindex (grown on demand)
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> timed;     // pending stage timings
     std::vector<cudaEvent_t> ev_pool;
     cudaEvent_t ev_user[8] = {};
@@ -233,16 +233,22 @@ void field_free(lsm_field* f) {
     delete f;
 }
 
+// grows one of the context's persistent device buffers (*buf, *size bytes) to at least `need` bytes; the old buffer is freed once
+// the context's stream has drained, so no work in flight still reads it
+int32_t grow_scratch(lsm_ctx* c, void** buf, size_t* size, size_t need) {
+    if (need > *size) {
+        CU(cudaStreamSynchronize(c->stream));
+        if (*buf) cudaFree(*buf);
+        *buf = nullptr; *size = 0;
+        CU(cudaMalloc(buf, need));
+        *size = need;
+    }
+    return LSM_OK;
+}
+
 // persistent device scratch of the context (reductions, getindex): grown on demand, never freed per call
 int32_t ctx_scratch(lsm_ctx* c, size_t bytes, void** out) {
-    if (bytes > c->d_work_bytes) {
-        CU(cudaStreamSynchronize(c->stream));
-        if (c->d_work) cudaFree(c->d_work);
-        c->d_work = nullptr; c->d_work_bytes = 0;
-        const size_t want = std::max<size_t>(bytes, 1u << 16);
-        CU(cudaMalloc(reinterpret_cast<void**>(&c->d_work), want));
-        c->d_work_bytes = want;
-    }
+    TRY(grow_scratch(c, &c->d_work, &c->d_work_bytes, std::max<size_t>(bytes, 1u << 16)));
     *out = c->d_work;
     return LSM_OK;
 }
@@ -891,215 +897,81 @@ int32_t compute_cfl_impl(lsm_ctx* ctx, lsm_field* phi, const lsm_term* terms, in
     return LSM_OK;
 }
 
-// ---- zero-level-set extraction (lsm_interface.cu) ----------------------------------------------
-int32_t interface_extract_impl(lsm_ctx* ctx, lsm_field* phi, double level, int64_t* nverts_out, int64_t* nprims_out) {
-    if (!ctx || !phi || !nverts_out || !nprims_out) return fail(LSM_ERR_ARG, "null argument");
-    ctx->iface_valid = false;                   // a failed extraction leaves nothing to fetch
-    if (phi->ctx != ctx || phi->ncomp != 1 || phi->separable) return fail(LSM_ERR_ARG, "interface extraction needs a real-valued field of this context");
-    if (!std::isfinite(level)) return fail(LSM_ERR_ARG, "level must be finite (got %g)", level);
+// ---- zero-level-set operations (lsm_interface.cu, lsm_redistance.cu) ------------------------------
+// The checks every operation on a level set makes: a real-valued field of this context with at least min_n nodes along every
+// dimension and, for the operations that have no multi-rank form, a context of one rank.  `what` names the operation.
+int32_t check_level_set(lsm_ctx* ctx, const lsm_field* phi, const char* what, int min_n, bool single_rank) {
+    if (!ctx || !phi) return fail(LSM_ERR_ARG, "null argument");
+    if (phi->ctx != ctx || phi->ncomp != 1 || phi->separable) return fail(LSM_ERR_ARG, "%s needs a real-valued field of this context", what);
     for (int d = 0; d < phi->ndim; ++d)
-        if (phi->nglob[d] < 2) return fail(LSM_ERR_ARG, "interface extraction needs at least 2 nodes along every dimension (n[%d] = %d)", d, phi->nglob[d]);
-    CU(cudaSetDevice(ctx->device));
-    CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_halo, 0));
-    // the cells of the rank's last owned plane reach into the next rank's first plane (the upper ghost plane); the exchange is
-    // collective, so every rank takes part
-    const int last = phi->ndim - 1;
-    const bool ghost = ctx->nranks > 1 && ctx->rank < ctx->nranks - 1;
-    if (ctx->nranks > 1 && !phi->halo_valid) TRY(exchange_halo(phi, ctx->stream));
+        if (phi->nglob[d] < min_n)
+            return fail(LSM_ERR_ARG, "%s needs at least %d nodes along every dimension (n[%d] = %d)", what, min_n, d, phi->nglob[d]);
+    if (single_rank && ctx->nranks > 1)
+        return fail(LSM_ERR_UNSUPPORTED, "%s: slab decomposition is not supported (nranks = %d)", what, ctx->nranks);
+    return LSM_OK;
+}
+
+// The node box of phi for the kernels: this rank's owned nodes and, with `ghost`, the first plane of the next rank.  Level 0,
+// ntiles unset.
+IfaceArgs field_box(const lsm_field* phi, bool ghost) {
     IfaceArgs A{};
-    A.phi = phi->p; A.f64 = phi->dtype == LSM_F64; A.ndim = phi->ndim; A.level = level;
+    A.phi = phi->p; A.f64 = phi->dtype == LSM_F64; A.ndim = phi->ndim;
     A.first_last = phi->first_last;
     A.hsign = 1;
     for (int d = 0; d < 3; ++d) {
-        A.m[d] = phi->n[d] + (d == last && ghost ? 1 : 0);
+        A.m[d] = phi->n[d] + (d == phi->ndim - 1 && ghost ? 1 : 0);
         A.lc[d] = phi->lc[d]; A.h[d] = d < phi->ndim ? phi->h[d] : 0.0;
         if (d < phi->ndim && phi->h[d] < 0) A.hsign = -A.hsign;
     }
     A.s1 = A.m[0]; A.s2 = (long long)A.m[0] * A.m[1];
     A.nodes = (long long)A.m[0] * A.m[1] * A.m[2];
-    A.ntiles = iface_tiles(A.nodes);
     A.lin0 = (long long)phi->first_last * phi->plane;
-    void* work = nullptr;
-    TRY(ctx_scratch(ctx, iface_scratch_bytes(A.ntiles), &work));
-    CU(launch_iface(A, 0, work, nullptr, nullptr, nullptr, ctx->stream));
-    CU(cudaMemcpyAsync(ctx->h_scalar, iface_totals(A, work), 16, cudaMemcpyDeviceToHost, ctx->stream));
+    return A;
+}
+
+// one synchronisation and one copy of n adjacent 8-byte device counters into ctx->h_scalar[0 .. n-1]
+int32_t read_counts(lsm_ctx* ctx, const void* d_counts, int n) {
+    CU(cudaMemcpyAsync(ctx->h_scalar, d_counts, 8 * n, cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
-    ctx->cnt.kernel_launches += 2; ctx->cnt.d2h_bytes += 16;
-    const int64_t nv = (int64_t)ctx->h_scalar[0], np = (int64_t)ctx->h_scalar[1];
-    if (nv > (int64_t)std::numeric_limits<int32_t>::max())
-        return fail(LSM_ERR_UNSUPPORTED, "the interface has %lld vertices; int32 vertex indices hold at most 2^31 - 1", (long long)nv);
-    const int N = phi->ndim;
-    const size_t vbytes = (size_t)nv * N * sizeof(double), kbytes = (size_t)nv * sizeof(int64_t), pbytes = (size_t)np * N * sizeof(int32_t);
-    const size_t need = vbytes + kbytes + pbytes;
-    if (need > ctx->d_iface_bytes) {
-        if (ctx->d_iface) cudaFree(ctx->d_iface);           // implicit synchronisation: nothing in flight reads it
-        ctx->d_iface = nullptr; ctx->d_iface_bytes = 0;
-        CU(cudaMalloc(&ctx->d_iface, need));
-        ctx->d_iface_bytes = need;
-    }
-    char* base = static_cast<char*>(ctx->d_iface);
-    double* verts = reinterpret_cast<double*>(base);
-    long long* keys = reinterpret_cast<long long*>(base + vbytes);
-    int* prims = reinterpret_cast<int*>(base + vbytes + kbytes);
-    if (nv > 0) { CU(launch_iface(A, 1, work, verts, keys, prims, ctx->stream)); ctx->cnt.kernel_launches += 1; }
-    if (np > 0) { CU(launch_iface(A, 2, work, verts, keys, prims, ctx->stream)); ctx->cnt.kernel_launches += 1; }
-    ctx->iface_valid = true; ctx->iface_ndim = N; ctx->iface_nv = nv; ctx->iface_np = np;
-    *nverts_out = nv; *nprims_out = np;
+    ctx->cnt.d2h_bytes += 8 * n;
     return LSM_OK;
 }
 
-
-// ---- closest-point redistancing and extension (lsm_redistance.cu) --------------------------------
-// grows the context's redistancing scratch to at least `need` bytes
-int32_t redist_scratch(lsm_ctx* ctx, size_t need) {
-    if (need > ctx->d_redist_bytes) {
-        if (ctx->d_redist) cudaFree(ctx->d_redist);         // implicit synchronisation: nothing in flight reads it
-        ctx->d_redist = nullptr; ctx->d_redist_bytes = 0;
-        CU(cudaMalloc(&ctx->d_redist, need));
-        ctx->d_redist_bytes = need;
-    }
-    return LSM_OK;
-}
-
-// The arguments and scratch of the redistancing passes on phi (checked by the caller), with `values` extra components per point
-// (the value of F that lsm_extend_closest_point carries); zeroes the three counters on the context's stream.
-int32_t redist_setup(lsm_ctx* ctx, lsm_field* phi, int32_t band, int values, RedistArgs& R) {
+// The closest-point passes on phi (checked by the caller): the extension of F unless F is null, redistancing of phi when write_phi
+// (the caller sets it when F is null), with `cubic` the Newton refinement before the write.  Scratch: two point buffers of N doubles
+// per node (N + 1 with F: the value at the point), the two 8-byte keys of the band scan per node, and three counters (listed
+// cells, band nodes, fallbacks).  Asynchronous unless an out-pointer is given; then one synchronisation and one copy of the band-node
+// count, and with `cubic` of the fallback count next to it.
+int32_t closest_points(lsm_ctx* ctx, lsm_field* phi, int32_t band, lsm_field* F, bool write_phi, bool cubic,
+                       int64_t* band_nodes_out, int64_t* fallback_nodes_out) {
     CU(cudaSetDevice(ctx->device));
-    IfaceArgs& A = R.g;
-    A.phi = phi->p; A.f64 = phi->dtype == LSM_F64; A.ndim = phi->ndim; A.level = 0.0;
-    A.hsign = 1;
-    for (int d = 0; d < 3; ++d) {
-        A.m[d] = phi->n[d];
-        A.lc[d] = phi->lc[d]; A.h[d] = d < phi->ndim ? phi->h[d] : 0.0;
-        if (d < phi->ndim && phi->h[d] < 0) A.hsign = -A.hsign;
-    }
-    A.s1 = A.m[0]; A.s2 = (long long)A.m[0] * A.m[1];
-    A.nodes = (long long)A.m[0] * A.m[1] * A.m[2];
+    RedistArgs R{};
+    R.g = field_box(phi, false);
     R.band = band;
-    const size_t pbytes = (size_t)A.nodes * (phi->ndim + values) * sizeof(double), kbytes = (size_t)A.nodes * sizeof(unsigned long long);
-    TRY(redist_scratch(ctx, 2 * pbytes + 2 * kbytes + 3 * sizeof(unsigned long long)));
+    R.F = F ? F->p : nullptr; R.F_f64 = F && F->dtype == LSM_F64; R.write_phi = write_phi;
+    const long long nodes = R.g.nodes;
+    const size_t pbytes = (size_t)nodes * (phi->ndim + (F ? 1 : 0)) * sizeof(double), kbytes = (size_t)nodes * sizeof(unsigned long long);
+    TRY(grow_scratch(ctx, &ctx->d_redist, &ctx->d_redist_bytes, 2 * pbytes + 2 * kbytes + 3 * sizeof(unsigned long long)));
     char* base = static_cast<char*>(ctx->d_redist);
     R.pa = reinterpret_cast<double*>(base);
     R.pb = reinterpret_cast<double*>(base + pbytes);
     R.list = reinterpret_cast<long long*>(R.pa);
     R.dmin = reinterpret_cast<unsigned long long*>(base + 2 * pbytes);
-    R.ord = R.dmin + A.nodes;
-    R.ncells = R.ord + A.nodes;
+    R.ord = R.dmin + nodes;
+    R.ncells = R.ord + nodes;
     R.count = R.ncells + 1;
+    R.fallbacks = cubic ? R.count + 1 : nullptr;
     CU(cudaMemsetAsync(R.ncells, 0, 3 * sizeof(unsigned long long), ctx->stream));
-    return LSM_OK;
-}
-
-// after the passes are enqueued: without band_nodes_out nothing (asynchronous); with it one sync and an 8-byte copy of the count
-int32_t redist_band_nodes(lsm_ctx* ctx, const RedistArgs& R, int64_t* band_nodes_out) {
-    if (band_nodes_out) {
-        CU(cudaMemcpyAsync(ctx->h_scalar, R.count, 8, cudaMemcpyDeviceToHost, ctx->stream));
-        CU(cudaStreamSynchronize(ctx->stream));
-        ctx->cnt.d2h_bytes += 8;
-        *band_nodes_out = (int64_t)ctx->h_scalar[0];
-    }
-    return LSM_OK;
-}
-
-int32_t redistance_impl(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* band_nodes_out) {
-    if (band < 1) return fail(LSM_ERR_ARG, "band must be at least 1 (got %d)", band);
-    if (!ctx || !phi) return fail(LSM_ERR_ARG, "null argument");
-    if (phi->ctx != ctx || phi->ncomp != 1 || phi->separable) return fail(LSM_ERR_ARG, "redistancing needs a real-valued field of this context");
-    for (int d = 0; d < phi->ndim; ++d)
-        if (phi->nglob[d] < 2) return fail(LSM_ERR_ARG, "redistancing needs at least 2 nodes along every dimension (n[%d] = %d)", d, phi->nglob[d]);
-    if (ctx->nranks > 1) return fail(LSM_ERR_UNSUPPORTED, "redistancing a slab-decomposed field (nranks = %d) is not supported", ctx->nranks);
-    RedistArgs R{};
-    TRY(redist_setup(ctx, phi, band, 0, R));
     int launches = 0;
-    CU(launch_redistance(R, ctx->sm_count, ctx->stream, &launches));
+    CU(launch_closest_points(R, ctx->sm_count, ctx->stream, &launches));
     ctx->cnt.kernel_launches += launches;
-    phi->version++; phi->halo_valid = false;
-    return redist_band_nodes(ctx, R, band_nodes_out);
-}
-
-int32_t extend_closest_impl(lsm_ctx* ctx, lsm_field* F, lsm_field* phi, int32_t band, int32_t redistance_phi, int64_t* band_nodes_out) {
-    if (band < 1) return fail(LSM_ERR_ARG, "band must be at least 1 (got %d)", band);
-    if (!ctx || !F || !phi) return fail(LSM_ERR_ARG, "null argument");
-    if (F == phi) return fail(LSM_ERR_ARG, "the extended field F must not be phi");
-    for (const lsm_field* f : {F, phi})
-        if (f->ctx != ctx || f->ncomp != 1 || f->separable) return fail(LSM_ERR_ARG, "the closest-point extension needs real-valued fields of this context");
-    bool same = F->ndim == phi->ndim;
-    for (int d = 0; same && d < phi->ndim; ++d)
-        same = F->nglob[d] == phi->nglob[d] && F->n[d] == phi->n[d] && F->lc[d] == phi->lc[d] && F->h[d] == phi->h[d];
-    if (!same) return fail(LSM_ERR_ARG, "F and phi must be on the same grid (n, lc and h)");
-    for (int d = 0; d < phi->ndim; ++d)
-        if (phi->nglob[d] < 2) return fail(LSM_ERR_ARG, "the closest-point extension needs at least 2 nodes along every dimension (n[%d] = %d)", d, phi->nglob[d]);
-    if (ctx->nranks > 1) return fail(LSM_ERR_UNSUPPORTED, "extending a slab-decomposed field (nranks = %d) is not supported", ctx->nranks);
-    ExtendArgs E{};
-    TRY(redist_setup(ctx, phi, band, 1, E));
-    E.F = F->p; E.f64 = F->dtype == LSM_F64; E.write_phi = redistance_phi != 0;
-    int launches = 0;
-    CU(launch_extend_closest(E, ctx->sm_count, ctx->stream, &launches));
-    ctx->cnt.kernel_launches += launches;
-    F->version++; F->halo_valid = false;
-    if (E.write_phi) { phi->version++; phi->halo_valid = false; }
-    return redist_band_nodes(ctx, E, band_nodes_out);
-}
-
-// the checks lsm_redistance_cubic and lsm_interpolate_cubic share: a scalar field of this context with n_d >= 4, single rank
-int32_t cubic_check(lsm_ctx* ctx, lsm_field* phi, const char* what) {
-    if (!ctx || !phi) return fail(LSM_ERR_ARG, "null argument");
-    if (phi->ctx != ctx || phi->ncomp != 1 || phi->separable) return fail(LSM_ERR_ARG, "%s needs a real-valued field of this context", what);
-    for (int d = 0; d < phi->ndim; ++d)
-        if (phi->nglob[d] < 4) return fail(LSM_ERR_ARG, "%s needs at least 4 nodes along every dimension (n[%d] = %d)", what, d, phi->nglob[d]);
-    if (ctx->nranks > 1) return fail(LSM_ERR_UNSUPPORTED, "%s of a slab-decomposed field (nranks = %d) is not supported", what, ctx->nranks);
-    return LSM_OK;
-}
-
-int32_t redistance_cubic_impl(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* band_nodes_out, int64_t* fallback_nodes_out) {
-    if (band < 1) return fail(LSM_ERR_ARG, "band must be at least 1 (got %d)", band);
-    TRY(cubic_check(ctx, phi, "cubic redistancing"));
-    RedistArgs R{};
-    TRY(redist_setup(ctx, phi, band, 0, R));
-    int launches = 0;
-    CU(launch_redistance_cubic(R, R.count + 1, ctx->sm_count, ctx->stream, &launches));
-    ctx->cnt.kernel_launches += launches;
-    phi->version++; phi->halo_valid = false;
-    if (band_nodes_out || fallback_nodes_out) {                  // band nodes and fallbacks are adjacent: one 16-byte copy
-        CU(cudaMemcpyAsync(ctx->h_scalar, R.count, 16, cudaMemcpyDeviceToHost, ctx->stream));
-        CU(cudaStreamSynchronize(ctx->stream));
-        ctx->cnt.d2h_bytes += 16;
+    if (F) { F->version++; F->halo_valid = false; }
+    if (R.write_phi) { phi->version++; phi->halo_valid = false; }
+    if (band_nodes_out || fallback_nodes_out) {
+        TRY(read_counts(ctx, R.count, cubic ? 2 : 1));
         if (band_nodes_out) *band_nodes_out = (int64_t)ctx->h_scalar[0];
         if (fallback_nodes_out) *fallback_nodes_out = (int64_t)ctx->h_scalar[1];
     }
-    return LSM_OK;
-}
-
-int32_t interpolate_cubic_impl(lsm_ctx* ctx, lsm_field* phi, int64_t npts, const double* pts, double* val, double* grad, double* hess) {
-    TRY(cubic_check(ctx, phi, "cubic interpolation"));
-    if (npts < 0) return fail(LSM_ERR_ARG, "npts must not be negative (got %lld)", (long long)npts);
-    if (npts > 0 && !pts) return fail(LSM_ERR_ARG, "null points");
-    if (npts == 0) return LSM_OK;
-    CU(cudaSetDevice(ctx->device));
-    const int N = phi->ndim;
-    IfaceArgs A{};
-    A.phi = phi->p; A.f64 = phi->dtype == LSM_F64; A.ndim = N; A.hsign = 1;
-    for (int d = 0; d < 3; ++d) { A.m[d] = phi->n[d]; A.lc[d] = phi->lc[d]; A.h[d] = d < N ? phi->h[d] : 0.0; }
-    A.s1 = A.m[0]; A.s2 = (long long)A.m[0] * A.m[1];
-    A.nodes = (long long)A.m[0] * A.m[1] * A.m[2];
-    // scratch: points, then values, gradients and Hessians (only the requested ones)
-    const size_t pb = (size_t)npts * N * sizeof(double), vb = val ? (size_t)npts * sizeof(double) : 0,
-                 gb = grad ? pb : 0, hb = hess ? pb * N : 0;
-    TRY(redist_scratch(ctx, pb + vb + gb + hb));
-    char* base = static_cast<char*>(ctx->d_redist);
-    double* dp = reinterpret_cast<double*>(base);
-    double* dv = val ? reinterpret_cast<double*>(base + pb) : nullptr;
-    double* dg = grad ? reinterpret_cast<double*>(base + pb + vb) : nullptr;
-    double* dh = hess ? reinterpret_cast<double*>(base + pb + vb + gb) : nullptr;
-    CU(cudaMemcpyAsync(dp, pts, pb, cudaMemcpyHostToDevice, ctx->stream));
-    ctx->cnt.h2d_bytes += pb;
-    CU(launch_interp_cubic(A, npts, dp, dv, dg, dh, ctx->stream));
-    ctx->cnt.kernel_launches += 1;
-    if (val) CU(cudaMemcpyAsync(val, dv, vb, cudaMemcpyDeviceToHost, ctx->stream));
-    if (grad) CU(cudaMemcpyAsync(grad, dg, gb, cudaMemcpyDeviceToHost, ctx->stream));
-    if (hess) CU(cudaMemcpyAsync(hess, dh, hb, cudaMemcpyDeviceToHost, ctx->stream));
-    ctx->cnt.d2h_bytes += vb + gb + hb;
-    CU(cudaStreamSynchronize(ctx->stream));
     return LSM_OK;
 }
 
@@ -1231,7 +1103,7 @@ int32_t lsm_multi_integrate(int32_t n, lsm_ctx* const* ctx, int32_t integrator, 
 
 int32_t lsm_multi_interface_extract(int32_t n, lsm_ctx* const* ctx, lsm_field* const* phi, double level, int64_t* nverts_out, int64_t* nprims_out) {
     if (!ctx || !phi || !nverts_out || !nprims_out || n < 1) return fail(LSM_ERR_ARG, "bad argument");
-    return fan_out(n, [&](int r) { return interface_extract_impl(ctx[r], phi[r], level, &nverts_out[r], &nprims_out[r]); });
+    return fan_out(n, [&](int r) { return lsm_interface_extract(ctx[r], phi[r], level, &nverts_out[r], &nprims_out[r]); });
 }
 
 int32_t lsm_ctx_destroy(lsm_ctx* c) {
@@ -1837,7 +1709,38 @@ int32_t lsm_extend_along_normals(lsm_ctx* ctx, lsm_field* F, lsm_field* phi, int
 }
 
 int32_t lsm_interface_extract(lsm_ctx* ctx, lsm_field* phi, double level, int64_t* nverts_out, int64_t* nprims_out) {
-    return interface_extract_impl(ctx, phi, level, nverts_out, nprims_out);
+    if (!ctx || !phi || !nverts_out || !nprims_out) return fail(LSM_ERR_ARG, "null argument");
+    ctx->iface_valid = false;                   // a failed extraction leaves nothing to fetch
+    TRY(check_level_set(ctx, phi, "interface extraction", 2, false));
+    if (!std::isfinite(level)) return fail(LSM_ERR_ARG, "level must be finite (got %g)", level);
+    CU(cudaSetDevice(ctx->device));
+    CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_halo, 0));
+    // the cells of the rank's last owned plane reach into the next rank's first plane (the upper ghost plane); the exchange is
+    // collective, so every rank takes part
+    if (ctx->nranks > 1 && !phi->halo_valid) TRY(exchange_halo(phi, ctx->stream));
+    IfaceArgs A = field_box(phi, ctx->nranks > 1 && ctx->rank < ctx->nranks - 1);
+    A.level = level;
+    A.ntiles = iface_tiles(A.nodes);
+    void* work = nullptr;
+    TRY(ctx_scratch(ctx, iface_scratch_bytes(A.ntiles), &work));
+    CU(launch_iface(A, 0, work, nullptr, nullptr, nullptr, ctx->stream));
+    TRY(read_counts(ctx, iface_totals(A, work), 2));
+    ctx->cnt.kernel_launches += 2;
+    const int64_t nv = (int64_t)ctx->h_scalar[0], np = (int64_t)ctx->h_scalar[1];
+    if (nv > (int64_t)std::numeric_limits<int32_t>::max())
+        return fail(LSM_ERR_UNSUPPORTED, "the interface has %lld vertices; int32 vertex indices hold at most 2^31 - 1", (long long)nv);
+    const int N = phi->ndim;
+    const size_t vbytes = (size_t)nv * N * sizeof(double), kbytes = (size_t)nv * sizeof(int64_t), pbytes = (size_t)np * N * sizeof(int32_t);
+    TRY(grow_scratch(ctx, &ctx->d_iface, &ctx->d_iface_bytes, vbytes + kbytes + pbytes));
+    char* base = static_cast<char*>(ctx->d_iface);
+    double* verts = reinterpret_cast<double*>(base);
+    long long* keys = reinterpret_cast<long long*>(base + vbytes);
+    int* prims = reinterpret_cast<int*>(base + vbytes + kbytes);
+    if (nv > 0) { CU(launch_iface(A, 1, work, verts, keys, prims, ctx->stream)); ctx->cnt.kernel_launches += 1; }
+    if (np > 0) { CU(launch_iface(A, 2, work, verts, keys, prims, ctx->stream)); ctx->cnt.kernel_launches += 1; }
+    ctx->iface_valid = true; ctx->iface_ndim = N; ctx->iface_nv = nv; ctx->iface_np = np;
+    *nverts_out = nv; *nprims_out = np;
+    return LSM_OK;
 }
 
 int32_t lsm_interface_fetch(lsm_ctx* ctx, double* verts, int64_t* keys, int32_t* prims) {
@@ -1858,19 +1761,54 @@ int32_t lsm_interface_fetch(lsm_ctx* ctx, double* verts, int64_t* keys, int32_t*
 }
 
 int32_t lsm_redistance(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* band_nodes_out) {
-    return redistance_impl(ctx, phi, band, band_nodes_out);
+    if (band < 1) return fail(LSM_ERR_ARG, "band must be at least 1 (got %d)", band);
+    TRY(check_level_set(ctx, phi, "redistancing", 2, true));
+    return closest_points(ctx, phi, band, nullptr, true, false, band_nodes_out, nullptr);
 }
 
 int32_t lsm_extend_closest_point(lsm_ctx* ctx, lsm_field* F, lsm_field* phi, int32_t band, int32_t redistance_phi, int64_t* band_nodes_out) {
-    return extend_closest_impl(ctx, F, phi, band, redistance_phi, band_nodes_out);
+    if (band < 1) return fail(LSM_ERR_ARG, "band must be at least 1 (got %d)", band);
+    if (F && F == phi) return fail(LSM_ERR_ARG, "the extended field F must not be phi");
+    for (const lsm_field* f : {F, phi}) TRY(check_level_set(ctx, f, "the closest-point extension", 2, true));
+    bool same = F->ndim == phi->ndim;
+    for (int d = 0; same && d < phi->ndim; ++d)
+        same = F->nglob[d] == phi->nglob[d] && F->n[d] == phi->n[d] && F->lc[d] == phi->lc[d] && F->h[d] == phi->h[d];
+    if (!same) return fail(LSM_ERR_ARG, "F and phi must be on the same grid (n, lc and h)");
+    return closest_points(ctx, phi, band, F, redistance_phi != 0, false, band_nodes_out, nullptr);
 }
 
 int32_t lsm_interpolate_cubic(lsm_ctx* ctx, lsm_field* phi, int64_t npts, const double* pts, double* val, double* grad, double* hess) {
-    return interpolate_cubic_impl(ctx, phi, npts, pts, val, grad, hess);
+    TRY(check_level_set(ctx, phi, "cubic interpolation", 4, true));
+    if (npts < 0) return fail(LSM_ERR_ARG, "npts must not be negative (got %lld)", (long long)npts);
+    if (npts > 0 && !pts) return fail(LSM_ERR_ARG, "null points");
+    if (npts == 0) return LSM_OK;
+    CU(cudaSetDevice(ctx->device));
+    const int N = phi->ndim;
+    // scratch: points, then values, gradients and Hessians (only the requested ones)
+    const size_t pb = (size_t)npts * N * sizeof(double), vb = val ? (size_t)npts * sizeof(double) : 0,
+                 gb = grad ? pb : 0, hb = hess ? pb * N : 0;
+    TRY(grow_scratch(ctx, &ctx->d_redist, &ctx->d_redist_bytes, pb + vb + gb + hb));
+    char* base = static_cast<char*>(ctx->d_redist);
+    double* dp = reinterpret_cast<double*>(base);
+    double* dv = val ? reinterpret_cast<double*>(base + pb) : nullptr;
+    double* dg = grad ? reinterpret_cast<double*>(base + pb + vb) : nullptr;
+    double* dh = hess ? reinterpret_cast<double*>(base + pb + vb + gb) : nullptr;
+    CU(cudaMemcpyAsync(dp, pts, pb, cudaMemcpyHostToDevice, ctx->stream));
+    ctx->cnt.h2d_bytes += pb;
+    CU(launch_interp_cubic(field_box(phi, false), npts, dp, dv, dg, dh, ctx->stream));
+    ctx->cnt.kernel_launches += 1;
+    if (val) CU(cudaMemcpyAsync(val, dv, vb, cudaMemcpyDeviceToHost, ctx->stream));
+    if (grad) CU(cudaMemcpyAsync(grad, dg, gb, cudaMemcpyDeviceToHost, ctx->stream));
+    if (hess) CU(cudaMemcpyAsync(hess, dh, hb, cudaMemcpyDeviceToHost, ctx->stream));
+    ctx->cnt.d2h_bytes += vb + gb + hb;
+    CU(cudaStreamSynchronize(ctx->stream));
+    return LSM_OK;
 }
 
 int32_t lsm_redistance_cubic(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* band_nodes_out, int64_t* fallback_nodes_out) {
-    return redistance_cubic_impl(ctx, phi, band, band_nodes_out, fallback_nodes_out);
+    if (band < 1) return fail(LSM_ERR_ARG, "band must be at least 1 (got %d)", band);
+    TRY(check_level_set(ctx, phi, "cubic redistancing", 4, true));
+    return closest_points(ctx, phi, band, nullptr, true, true, band_nodes_out, fallback_nodes_out);
 }
 
 int32_t lsm_field_csg(lsm_ctx* ctx, lsm_field* dst, const lsm_field* src, int32_t op) {

@@ -86,35 +86,27 @@ long long* iface_totals(const IfaceArgs& A, void* scratch);     // device addres
 // pass 0: count + scan (totals at iface_totals); pass 1: vertices and keys; pass 2: primitives (needs the keys of pass 1)
 cudaError_t launch_iface(const IfaceArgs& A, int pass, void* scratch, double* verts, long long* keys, int* prims, cudaStream_t s);
 
-// lsm_redistance.cu: closest-point redistancing (lsm_redistance), single-rank fields.  The box is the whole field.
+// lsm_redistance.cu: closest-point redistancing (lsm_redistance), its closest-point extension (lsm_extend_closest_point) and its
+// cubic refinement (lsm_redistance_cubic), single-rank fields.  The box is the whole field.
 struct RedistArgs {
     IfaceArgs g;               // the field (level 0; ntiles and lin0 unused); the write pass stores through g.phi
     int band;                  // cell window half-width
-    double* pa;                // point buffers: N components of g.nodes doubles each (SoA); NaN = no point
-    double* pb;
+    double* pa;                // point buffers: N components of g.nodes doubles each (SoA), N + 1 with F (the value at the point
+    double* pb;                // last); NaN = no point
     long long* list;           // cut cells (up to g.nodes entries; aliases pa until the pick pass writes it)
     unsigned long long* dmin;  // per node: smallest candidate distance (IEEE bits) of the band scan
     unsigned long long* ord;   // per node: order key (cell * 16 + primitive) of the first candidate at that distance
     unsigned long long* ncells;// listed cells, zeroed by the caller
     unsigned long long* count; // band nodes, zeroed by the caller
+    void* F;                   // the extension: scalar field on g's grid, read by the pick pass and written by the write pass; null
+                               // for redistancing
+    bool F_f64;                // F's dtype
+    int write_phi;             // with F: the write pass also stores the signed distance through g.phi, as it does without F
+    unsigned long long* fallbacks; // the cubic refinement (null: none): nodes that keep their linear closest point, zeroed by the caller
 };
-// enqueues flag, the two cell passes, pick, the jump-flooding passes and the write pass on s; *launches = kernels enqueued
-cudaError_t launch_redistance(const RedistArgs& R, int sm_count, cudaStream_t s, int* launches);
-
-// lsm_redistance.cu, extension variant (lsm_extend_closest_point): the same passes, with the value of F at each closest point carried
-// along.  The point buffers pa / pb hold N + 1 components of g.nodes doubles each: the point, then the value at it (NaN = no point).
-struct ExtendArgs : RedistArgs {
-    void* F;                   // scalar field on g's grid, read by the pick pass and written by the write pass
-    bool f64;                  // F's dtype
-    int write_phi;             // the write pass also stores the signed distance through g.phi, as lsm_redistance does
-};
-// enqueues the same kernels as launch_redistance on s; *launches = kernels enqueued
-cudaError_t launch_extend_closest(const ExtendArgs& E, int sm_count, cudaStream_t s, int* launches);
-
-// lsm_redistance.cu, cubic variant (lsm_redistance_cubic): launch_redistance's passes with the Newton refinement on the cubic
-// interpolant (lsm_cubic.cuh) between the last flooding pass and the write; *fallbacks (zeroed by the caller) counts the nodes that
-// keep their linear closest point.
-cudaError_t launch_redistance_cubic(const RedistArgs& R, unsigned long long* fallbacks, int sm_count, cudaStream_t s, int* launches);
+// enqueues flag, the two cell passes, pick, the jump-flooding passes, with fallbacks set the Newton refinement on the cubic
+// interpolant (lsm_cubic.cuh), and the write pass on s; *launches = kernels enqueued
+cudaError_t launch_closest_points(const RedistArgs& R, int sm_count, cudaStream_t s, int* launches);
 // lsm_interpolate_cubic: the interpolant of A's field at npts points (pts AoS, npts x ndim); val (npts), grad (npts x ndim) and
 // hess (npts x ndim x ndim) may each be null
 cudaError_t launch_interp_cubic(const IfaceArgs& A, long long npts, const double* pts, double* val, double* grad, double* hess,

@@ -23,7 +23,8 @@
 // write:
 //   refine: one thread per node; Newton on the KKT system of the closest point on the cubic interpolant (lsm_cubic.cuh), from the
 //           node's linear closest point, into the spare point buffer; a node that falls back keeps the linear point and is counted.
-// cubic_interp_kernel evaluates the same interpolant at arbitrary points for lsm_interpolate_cubic.
+// One launcher, launch_closest_points, enqueues all three: the extension's variant when RedistArgs::F is set, the refinement when
+// RedistArgs::fallbacks is.  cubic_interp_kernel evaluates the same interpolant at arbitrary points for lsm_interpolate_cubic.
 // The operation order of every distance, closest point and value is the one include/lsm_b200.h states; tests/redistance_ref.py and
 // tests/extension_ref.py (and tests/cubic_ref.py for the cubic kernels) restate it in NumPy and agree with this file bit for bit (it
 // is compiled with -fmad=false).
@@ -241,10 +242,6 @@ __device__ __forceinline__ void closest(const double* x, const double (*V)[3], d
     else closest_tri<WHERE>(x, V[0], V[1], V[2], q, W);
 }
 
-// kernel arguments: RedistArgs for lsm_redistance (TF void), ExtendArgs for the extension with F of dtype TF
-template <class TF> struct ArgsOf { using type = ExtendArgs; };
-template <> struct ArgsOf<void> { using type = RedistArgs; };
-
 constexpr unsigned long long NONE = ~0ull;                    // dmin / ord of a node outside every window
 constexpr unsigned long long INF_BITS = 0x7ff0000000000000ull; // dmin of a band node whose candidates are all NaN
 
@@ -341,7 +338,7 @@ __global__ void __launch_bounds__(CTPB) redist_cells_kernel(const __grid_constan
 // every node: the closest point of the winning primitive (NaN when there is none) into pa, with the extension also the value of F
 // there; counts the band nodes
 template <class T, int N, class TF = void>
-__global__ void __launch_bounds__(TPB) redist_pick_kernel(const __grid_constant__ typename ArgsOf<TF>::type R) {
+__global__ void __launch_bounds__(TPB) redist_pick_kernel(const __grid_constant__ RedistArgs R) {
     const IfaceArgs& A = R.g;
     const long long idx = (long long)blockIdx.x * TPB + threadIdx.x;
     bool band = false;
@@ -431,7 +428,7 @@ template <> __device__ __forceinline__ double smallest_subnormal<double>() { ret
 
 // with the extension (TF not void) F = the value at the point, rounded to TF, on the same nodes; phi only when R.write_phi
 template <class T, int N, class TF = void>
-__global__ void __launch_bounds__(TPB) redist_write_kernel(const __grid_constant__ typename ArgsOf<TF>::type R,
+__global__ void __launch_bounds__(TPB) redist_write_kernel(const __grid_constant__ RedistArgs R,
                                                            const double* __restrict__ pts) {
     const IfaceArgs& A = R.g;
     const long long idx = (long long)blockIdx.x * TPB + threadIdx.x;
@@ -590,8 +587,7 @@ __global__ void __launch_bounds__(TPB) cubic_interp_kernel(const __grid_constant
 }
 
 template <class T, int N, class TF>
-cudaError_t launch_n(const typename ArgsOf<TF>::type& R, int cell_blocks, cudaStream_t s, int* launches,
-                     unsigned long long* fallbacks = nullptr) {
+cudaError_t launch_n(const RedistArgs& R, int cell_blocks, cudaStream_t s, int* launches) {
     constexpr bool EXT = !std::is_void_v<TF>;
     const unsigned grid = (unsigned)((R.g.nodes + TPB - 1) / TPB);
     redist_flag_kernel<T, N><<<grid, TPB, 0, s>>>(R);
@@ -609,9 +605,9 @@ cudaError_t launch_n(const typename ArgsOf<TF>::type& R, int cell_blocks, cudaSt
         double* t = src; src = dst; dst = t;
         if (k == 0) break;
     }
-    if constexpr (std::is_void_v<TF>) {
-        if (fallbacks) {                          // the cubic refinement: the spare point buffer takes the refined points
-            redist_refine_kernel<T, N><<<grid, TPB, 0, s>>>(R, src, dst, fallbacks);
+    if constexpr (!EXT) {
+        if (R.fallbacks) {                        // the cubic refinement: the spare point buffer takes the refined points
+            redist_refine_kernel<T, N><<<grid, TPB, 0, s>>>(R, src, dst, R.fallbacks);
             ++*launches;
             src = dst;
         }
@@ -622,20 +618,17 @@ cudaError_t launch_n(const typename ArgsOf<TF>::type& R, int cell_blocks, cudaSt
 }
 
 template <class T, class TF>
-cudaError_t launch_t(const typename ArgsOf<TF>::type& R, int cell_blocks, cudaStream_t s, int* launches,
-                     unsigned long long* fallbacks = nullptr) {
+cudaError_t launch_t(const RedistArgs& R, int cell_blocks, cudaStream_t s, int* launches) {
     switch (R.g.ndim) {
-        case 1: return launch_n<T, 1, TF>(R, cell_blocks, s, launches, fallbacks);
-        case 2: return launch_n<T, 2, TF>(R, cell_blocks, s, launches, fallbacks);
-        default: return launch_n<T, 3, TF>(R, cell_blocks, s, launches, fallbacks);
+        case 1: return launch_n<T, 1, TF>(R, cell_blocks, s, launches);
+        case 2: return launch_n<T, 2, TF>(R, cell_blocks, s, launches);
+        default: return launch_n<T, 3, TF>(R, cell_blocks, s, launches);
     }
 }
 
 template <class TF>
-cudaError_t launch_tf(const typename ArgsOf<TF>::type& R, int cell_blocks, cudaStream_t s, int* launches,
-                      unsigned long long* fallbacks = nullptr) {
-    return R.g.f64 ? launch_t<double, TF>(R, cell_blocks, s, launches, fallbacks)
-                   : launch_t<float, TF>(R, cell_blocks, s, launches, fallbacks);
+cudaError_t launch_tf(const RedistArgs& R, int cell_blocks, cudaStream_t s, int* launches) {
+    return R.g.f64 ? launch_t<double, TF>(R, cell_blocks, s, launches) : launch_t<float, TF>(R, cell_blocks, s, launches);
 }
 
 template <class T>
@@ -652,16 +645,9 @@ cudaError_t launch_interp_t(const IfaceArgs& A, long long npts, const double* pt
 
 }  // namespace
 
-cudaError_t launch_redistance(const RedistArgs& R, int sm_count, cudaStream_t s, int* launches) {
-    return launch_tf<void>(R, sm_count * 16, s, launches);
-}
-
-cudaError_t launch_extend_closest(const ExtendArgs& E, int sm_count, cudaStream_t s, int* launches) {
-    return E.f64 ? launch_tf<double>(E, sm_count * 16, s, launches) : launch_tf<float>(E, sm_count * 16, s, launches);
-}
-
-cudaError_t launch_redistance_cubic(const RedistArgs& R, unsigned long long* fallbacks, int sm_count, cudaStream_t s, int* launches) {
-    return launch_tf<void>(R, sm_count * 16, s, launches, fallbacks);
+cudaError_t launch_closest_points(const RedistArgs& R, int sm_count, cudaStream_t s, int* launches) {
+    if (!R.F) return launch_tf<void>(R, sm_count * 16, s, launches);
+    return R.F_f64 ? launch_tf<double>(R, sm_count * 16, s, launches) : launch_tf<float>(R, sm_count * 16, s, launches);
 }
 
 cudaError_t launch_interp_cubic(const IfaceArgs& A, long long npts, const double* pts, double* val, double* grad, double* hess,

@@ -15,13 +15,7 @@ import pytest
 
 import extension_ref as E
 import redistance_ref as R
-from test_redistance import BAND_CASES, CASES, bits_equal, grid_h, sphere, zalesak
-
-
-@pytest.fixture(scope="module")
-def m():
-    import lsm_b200
-    return lsm_b200
+from zero_set_helpers import BAND_CASES, CASES, bits_equal, grid_h, m, on_device, sphere, zalesak  # noqa: F401 (m is a fixture)
 
 
 def same(a, b):
@@ -196,10 +190,6 @@ def test_abi_argument_checks_without_a_device(m):
 # ================================================================================================
 # device == restatement, bit for bit
 # ================================================================================================
-def _device(m, vals, lc, hc, dtype, ctx=None, bc=None):
-    return m.MeshField(np.asfortranarray(np.asarray(vals).astype(dtype)), m.CartesianGrid(lc, hc, np.shape(vals)), bc=bc, ctx=ctx)
-
-
 def _run(m, F, phi, band, redistance=0):
     """lsm_extend_closest_point through the C ABI with the band-node count; returns (F, phi, band nodes)."""
     ctx = phi._context()
@@ -233,7 +223,7 @@ def test_device_equals_restatement(m, name, dt, band):
     vals = vals.astype(pd)
     F, h = _f_case(name, vals, lc, hc)
     F = F.astype(fd)
-    got, phi_got, nb = _run(m, _device(m, F, lc, hc, fd), _device(m, vals, lc, hc, pd), band)
+    got, phi_got, nb = _run(m, on_device(m, F, lc, hc, fd), on_device(m, vals, lc, hc, pd), band)
     want, _, nb_want = E.extend(F, vals, lc, h, band)
     assert nb == nb_want
     assert same(got, want)
@@ -248,7 +238,7 @@ def test_device_equals_restatement_wider_bands(m, band):
     for name in ("1d", "2d_odd_aniso", "3d_notched_sphere"):
         vals, lc, hc = CASES[name]
         F, h = _f_case(name, vals, lc, hc)
-        got, _, nb = _run(m, _device(m, F, lc, hc, np.float64), _device(m, vals, lc, hc, np.float64), band)
+        got, _, nb = _run(m, on_device(m, F, lc, hc, np.float64), on_device(m, vals, lc, hc, np.float64), band)
         want, _, nb_want = E.extend(F, vals, lc, h, band)
         assert nb == nb_want and same(got, want), name
 
@@ -270,9 +260,9 @@ def test_zalesak_disk_equals_restatement(m, dtype):
 def test_redistance_flag_writes_lsm_redistance_phi(m, name):
     vals, lc, hc = CASES[name]
     F, _ = _f_case(name, vals, lc, hc)
-    f1, phi1, nb1 = _run(m, _device(m, F, lc, hc, np.float64), _device(m, vals, lc, hc, np.float64), 3, redistance=1)
-    f0, phi0, nb0 = _run(m, _device(m, F, lc, hc, np.float64), _device(m, vals, lc, hc, np.float64), 3, redistance=0)
-    ref = _device(m, vals, lc, hc, np.float64)
+    f1, phi1, nb1 = _run(m, on_device(m, F, lc, hc, np.float64), on_device(m, vals, lc, hc, np.float64), 3, redistance=1)
+    f0, phi0, nb0 = _run(m, on_device(m, F, lc, hc, np.float64), on_device(m, vals, lc, hc, np.float64), 3, redistance=0)
+    ref = on_device(m, vals, lc, hc, np.float64)
     m.redistance(ref)
     assert bits_equal(phi1, np.array(ref.peek()))     # phi is lsm_redistance's, bit for bit
     assert same(f1, f0) and nb1 == nb0 and bits_equal(phi0, vals)
@@ -284,8 +274,8 @@ def test_constant_F_is_kept(m):
         vals, lc, hc = CASES[name]
         for dtype in (np.float64, np.float32):
             F0 = np.full(vals.shape, -1.25, dtype=dtype)
-            F = _device(m, F0, lc, hc, dtype)
-            m.extend_closest_point(F, _device(m, vals, lc, hc, np.float64), redistance=True)
+            F = on_device(m, F0, lc, hc, dtype)
+            m.extend_closest_point(F, on_device(m, vals, lc, hc, np.float64), redistance=True)
             assert bits_equal(np.array(F.peek()), F0), name
 
 
@@ -320,8 +310,8 @@ def test_deterministic_and_asynchronous(m):
     vals, lc, hc = CASES["3d_notched_sphere"]
     F0, _ = _f_case("3d_notched_sphere", vals, lc, hc)
     ctx = m.default_context()
-    fa, fb = _device(m, F0, lc, hc, np.float64), _device(m, F0, lc, hc, np.float64)
-    pa, pb = _device(m, vals, lc, hc, np.float64), _device(m, vals, lc, hc, np.float64)
+    fa, fb = on_device(m, F0, lc, hc, np.float64), on_device(m, F0, lc, hc, np.float64)
+    pa, pb = on_device(m, vals, lc, hc, np.float64), on_device(m, vals, lc, hc, np.float64)
     for f in (fa, fb, pa, pb):
         f.device()
     ctx.reset_counters()
@@ -414,20 +404,3 @@ def test_error_codes(m):
     finally:
         fresh.close()
 
-
-@pytest.mark.gpu
-def test_slab_decomposition_is_refused(m):
-    n = C.c_int32(0)
-    m._lib.lib().lsm_device_count(C.byref(n))
-    if n.value < 2:
-        pytest.skip("needs 2 GPUs")
-    mc = m.MultiContext([0, 1])
-    try:
-        phi, h = sphere((20, 18, 24))
-        f = m.MeshField(np.asfortranarray(phi), m.CartesianGrid((-0.5,) * 3, (0.5,) * 3, phi.shape), ctx=mc.ranks[0])
-        F = m.MeshField(np.asfortranarray(np.ones(phi.shape)), m.CartesianGrid((-0.5,) * 3, (0.5,) * 3, phi.shape), ctx=mc.ranks[0])
-        assert m._lib.lib().lsm_extend_closest_point(mc.ranks[0].handle, F.device(), f.device(), 3, 0, None) == m._lib.ERR_UNSUPPORTED
-        assert "slab decomposition is not supported" in m._lib.last_error()
-        del f, F
-    finally:
-        mc.close()

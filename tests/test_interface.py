@@ -15,27 +15,12 @@ import pytest
 
 import helpers as H
 import interface_ref as R
-
-
-@pytest.fixture(scope="module")
-def m():
-    import lsm_b200
-    return lsm_b200
+from zero_set_helpers import m, on_device, sphere, torus  # noqa: F401 (m is a fixture)
 
 
 def grid_values(lc, hc, n):
     h = [(hc[d] - lc[d]) / (n[d] - 1) for d in range(len(n))]
     return H.coords(lc, hc, n), h
-
-
-def sphere(n, r=0.3507, lc=(-0.5,) * 3, hc=(0.5,) * 3, c=(0.0, 0.0, 0.0)):
-    (x, y, z), h = grid_values(lc, hc, n)
-    return np.sqrt(((x - c[0]) ** 2 + (y - c[1]) ** 2) + (z - c[2]) ** 2) - r, h
-
-
-def torus(n, R0=0.3, r=0.12):
-    (x, y, z), h = grid_values((-0.5,) * 3, (0.5,) * 3, n)
-    return np.sqrt((np.sqrt(x * x + y * y) - R0) ** 2 + z * z) - r, h
 
 
 # ================================================================================================
@@ -124,10 +109,10 @@ def test_closed_surfaces_converge_at_second_order(shape):
     errs = []
     for n in (24, 48):
         if shape == "sphere":
-            phi, h = sphere((n, n, n))
+            phi, h = sphere((n, n, n), r=0.3507, c=(0.0, 0.0, 0.0))
             A0, V0, chi = 4 * math.pi * 0.3507 ** 2, 4 / 3 * math.pi * 0.3507 ** 3, 2
         else:
-            phi, h = torus((n, n, n))
+            phi, h = torus((n, n, n), R0=0.3, r=0.12)
             A0, V0, chi = 4 * math.pi ** 2 * 0.3 * 0.12, 2 * math.pi ** 2 * 0.3 * 0.12 ** 2, 0
         X, F, K = R.extract(phi, (-0.5,) * 3, h)
         _closed_surface(X, F, chi)
@@ -183,11 +168,6 @@ def test_abi_argument_checks_without_a_device(m):
 # ================================================================================================
 # device mesh == restatement, bit for bit
 # ================================================================================================
-def _device(m, vals, lc, hc, dtype, ctx=None, bc=None):
-    n = vals.shape
-    return m.MeshField(np.asfortranarray(vals.astype(dtype)), m.CartesianGrid(lc, hc, n), bc=bc, ctx=ctx)
-
-
 def _same(got, want):
     X, F, K = want
     assert got.vertices.dtype == np.float64 and got.faces.dtype == np.int32 and got.keys.dtype == np.int64
@@ -231,7 +211,7 @@ CASES = _cases()
 @pytest.mark.parametrize("name", list(CASES))
 def test_device_mesh_equals_restatement(m, name, dtype):
     vals, lc, hc, level = CASES[name]
-    phi = _device(m, vals, lc, hc, dtype)
+    phi = on_device(m, vals, lc, hc, dtype)
     h = [(hc[d] - lc[d]) / (vals.shape[d] - 1) for d in range(vals.ndim)]
     got = m.extract_interface(phi, level)
     want = R.extract(vals.astype(dtype), lc, h, level)
@@ -247,7 +227,7 @@ def test_device_mesh_equals_restatement(m, name, dtype):
 
 @pytest.mark.gpu
 def test_empty_fetch_with_null_arrays(m):
-    phi = _device(m, np.ones((9, 7)), (0, 0), (1, 1), np.float64)
+    phi = on_device(m, np.ones((9, 7)), (0, 0), (1, 1), np.float64)
     lib, ctx = m._lib.lib(), m.default_context()
     nv, nf = C.c_int64(-1), C.c_int64(-1)
     m._lib.check(lib.lsm_interface_extract(ctx.handle, phi.device(), 0.0, C.byref(nv), C.byref(nf)))
@@ -344,7 +324,7 @@ def test_multi_gpu_weld_equals_single_gpu(m, periodic):
         bc = (m.NeumannBC(), m.NeumannBC(), m.PeriodicBC() if periodic else m.NeumannBC())
         eqs = []
         for ctx in mc.ranks:
-            f = _device(m, phi0, lc, hc, np.float64, ctx=ctx, bc=bc)
+            f = on_device(m, phi0, lc, hc, np.float64, ctx=ctx, bc=bc)
             eqs.append(m.LevelSetEquation(terms=(m.AdvectionTerm((0.3, -0.2, 0.5), m.WENO5()),), ic=f, integrator=m.RK3()))
         m.integrate_multi(mc, eqs, 0.02)
         for fresh_upload in (False, True):
@@ -354,7 +334,7 @@ def test_multi_gpu_weld_equals_single_gpu(m, periodic):
                     e.state.vals[...] = vals[..., e.state._first:e.state._first + e.state._count]
             glob = m.MultiContext.gather([e.state for e in eqs])
             got = m.extract_interface_multi(mc, [e.state for e in eqs])
-            ref = m.extract_interface(_device(m, glob, lc, hc, np.float64, ctx=solo, bc=bc))
+            ref = m.extract_interface(on_device(m, glob, lc, hc, np.float64, ctx=solo, bc=bc))
             for a, b in zip(got, ref):
                 assert a.dtype == b.dtype and np.array_equal(a, b)
             assert len(ref.faces) > 1000

@@ -5,7 +5,8 @@ dense sampling in every region of Ericson's algorithm and on degenerate triangle
 whole mesh, the propagated distances against brute force, classification (with the subnormal raise), and the argument checks of
 the C ABI that need no device.  On the GPU: the device result equals the restatement bit for bit over dimensions, dtypes, odd
 sizes, anisotropic and mirrored grids, bands, kinked shapes, exact zeros, NaN nodes and a field without an interface; second-order
-accuracy on a sphere; the interface shift; determinism; asynchrony; invalidation of the CFL cache; the prehook; error codes."""
+accuracy on a sphere; the interface shift; determinism; asynchrony; invalidation of the CFL cache; the prehook; error codes.  On
+2 GPUs: every single-rank zero-level-set entry point refuses a slab-decomposed field."""
 import ctypes as C
 import math
 
@@ -13,35 +14,7 @@ import numpy as np
 import pytest
 
 import redistance_ref as R
-
-
-@pytest.fixture(scope="module")
-def m():
-    import lsm_b200
-    return lsm_b200
-
-
-def grid_h(lc, hc, n):
-    return [(hc[d] - lc[d]) / (n[d] - 1) for d in range(len(n))]
-
-
-def sphere(n, r=0.3, lc=(-0.5,) * 3, hc=(0.5,) * 3, c=(0.02, -0.01, 0.0)):
-    h = grid_h(lc, hc, n)
-    x = R.node_coords(n, lc, h)
-    return np.sqrt(((x[..., 0] - c[0]) ** 2 + (x[..., 1] - c[1]) ** 2) + (x[..., 2] - c[2]) ** 2) - r, h
-
-
-def torus(n, R0=0.28, r=0.11):
-    lc, hc = (-0.5,) * 3, (0.5,) * 3
-    h = grid_h(lc, hc, n)
-    x = R.node_coords(n, lc, h)
-    return np.sqrt((np.sqrt(x[..., 0] ** 2 + x[..., 1] ** 2) - R0) ** 2 + x[..., 2] ** 2) - r, h
-
-
-def bits_equal(a, b):
-    a, b = np.asarray(a), np.asarray(b)
-    return (a.dtype == b.dtype and a.shape == b.shape
-            and np.array_equal(np.ascontiguousarray(a).view(np.uint8), np.ascontiguousarray(b).view(np.uint8)))
+from zero_set_helpers import BAND_CASES, CASES, bits_equal, grid_h, m, on_device, sphere, zalesak  # noqa: F401 (m is a fixture)
 
 
 # ================================================================================================
@@ -115,24 +88,6 @@ def test_closest_point_on_degenerate_triangles(kind):
     assert np.all(d <= dmin + 1e-12) and np.all(d >= dmin - 1e-3)
 
 
-def _band_cases():
-    out = {}
-    phi, h = sphere((16, 17, 15), r=0.27)
-    out["sphere"] = (phi, (-0.5,) * 3, h)
-    phi, h = torus((20, 20, 14))
-    out["torus"] = (phi, (-0.5,) * 3, h)
-    lc, hc = (-0.5, -0.6, -0.4), (0.55, 0.6, 0.45)
-    phi, h = sphere((15, 26, 11), r=0.3, lc=lc, hc=hc)
-    out["aniso"] = (phi, lc, h)
-    lc, hc = (0.55, -0.6, -0.4), (-0.5, 0.6, 0.45)
-    phi, h = sphere((15, 19, 13), r=0.3, lc=lc, hc=hc)
-    out["mirrored"] = (phi, lc, h)
-    return out
-
-
-BAND_CASES = _band_cases()
-
-
 @pytest.mark.parametrize("name", list(BAND_CASES))
 def test_band_guarantee_against_brute_force(name):
     phi, lc, h = BAND_CASES[name]
@@ -201,40 +156,6 @@ def test_abi_argument_checks_without_a_device(m):
 # ================================================================================================
 # device == restatement, bit for bit
 # ================================================================================================
-def _cases():
-    out = {}
-    x = np.linspace(-1, 1, 37)
-    v1 = np.sin(7 * x) + 0.1
-    v1[5] = 0.0
-    v1[20] = np.nan
-    out["1d"] = (v1, (-1.0,), (1.0,))
-    h2 = grid_h((-1, -1.5), (1.2, 1.5), (37, 53))
-    x2 = R.node_coords((37, 53), (-1, -1.5), h2)
-    out["2d_odd_aniso"] = (np.hypot(x2[..., 0] - 0.1, x2[..., 1]) ** 2 - 0.55 ** 2, (-1, -1.5), (1.2, 1.5))
-    out["2d_mirrored"] = (np.hypot(x2[..., 0] - 0.1, x2[..., 1]) - 0.55, (1.2, -1.5), (-1, 1.5))
-    phi, _ = sphere((29, 33, 23), r=0.33, lc=(-0.5, -0.6, -0.4), hc=(0.55, 0.6, 0.45), c=(0.03, -0.02, 0.01))
-    out["3d_odd_aniso"] = (phi * (1.5 + phi), (-0.5, -0.6, -0.4), (0.55, 0.6, 0.45))
-    out["3d_mirrored"] = (phi, (0.55, -0.6, -0.4), (-0.5, 0.6, 0.45))
-    h3 = grid_h((-0.5,) * 3, (0.5,) * 3, (27, 25, 29))
-    x3 = R.node_coords((27, 25, 29), (-0.5,) * 3, h3)
-    ball = np.sqrt((x3[..., 0] ** 2 + x3[..., 1] ** 2) + x3[..., 2] ** 2) - 0.35
-    slot = np.maximum(np.maximum(np.abs(x3[..., 0]) - 0.06, np.abs(x3[..., 1] + 0.25) - 0.25), np.abs(x3[..., 2]) - 0.5)
-    out["3d_notched_sphere"] = (np.maximum(ball, -slot), (-0.5,) * 3, (0.5,) * 3)
-    q = np.round(ball * 16) / 16            # many exact zeros at nodes, and NaN nodes
-    q[3:6, 10:12, 4] = np.nan
-    q[13, 13, 20:23] = np.nan
-    out["3d_zeros_nan"] = (q, (-0.5,) * 3, (0.5,) * 3)
-    out["3d_all_positive"] = (ball + 2.0, (-0.5,) * 3, (0.5,) * 3)
-    return out
-
-
-CASES = _cases()
-
-
-def _device(m, vals, lc, hc, dtype, ctx=None, bc=None):
-    return m.MeshField(np.asfortranarray(vals.astype(dtype)), m.CartesianGrid(lc, hc, vals.shape), bc=bc, ctx=ctx)
-
-
 def _run(m, phi, band):
     """lsm_redistance through the C ABI with the band-node count; returns (values, band nodes)."""
     ctx = phi._context()
@@ -252,7 +173,7 @@ def test_device_equals_restatement(m, name, dtype, band):
     vals, lc, hc = CASES[name]
     vals = vals.astype(dtype)
     h = grid_h(lc, hc, vals.shape)
-    got, nb = _run(m, _device(m, vals, lc, hc, dtype), band)
+    got, nb = _run(m, on_device(m, vals, lc, hc, dtype), band)
     want, nb_want = R.redistance(vals, lc, h, band)
     assert nb == nb_want
     assert bits_equal(got, want)
@@ -265,17 +186,9 @@ def test_device_equals_restatement(m, name, dtype, band):
 def test_device_equals_restatement_wider_bands(m, band):
     for name in ("2d_odd_aniso", "3d_notched_sphere"):
         vals, lc, hc = CASES[name]
-        got, nb = _run(m, _device(m, vals, lc, hc, np.float64), band)
+        got, nb = _run(m, on_device(m, vals, lc, hc, np.float64), band)
         want, nb_want = R.redistance(vals, lc, grid_h(lc, hc, vals.shape), band)
         assert nb == nb_want and bits_equal(got, want), name
-
-
-def zalesak(m, n, dtype=np.float64):
-    """The Zalesak disk of docs/src/example-zalesak.md built on the device: a disk minus a slot."""
-    g = m.CartesianGrid((0.0, 0.0), (1.0, 1.0), (n, n))
-    disk = m.MeshField.from_shape(g, "sphere", (0.5, 0.75, 0.15), dtype=dtype)
-    slot = m.MeshField.from_shape(g, "box", (0.5, 0.725, 0.05, 0.25), dtype=dtype)
-    return m.setdiff_(disk, slot), g
 
 
 @pytest.mark.gpu
@@ -343,8 +256,8 @@ def test_interface_shift(m):
 def test_deterministic_and_asynchronous(m):
     vals, lc, hc = CASES["3d_notched_sphere"]
     ctx = m.default_context()
-    a = _device(m, vals, lc, hc, np.float64)
-    b = _device(m, vals, lc, hc, np.float64)
+    a = on_device(m, vals, lc, hc, np.float64)
+    b = on_device(m, vals, lc, hc, np.float64)
     a.device(), b.device()
     ctx.reset_counters()
     m.redistance(a)
@@ -426,17 +339,30 @@ def test_error_codes(m):
 
 
 @pytest.mark.gpu
-def test_slab_decomposition_is_refused(m):
+@pytest.mark.parametrize("entry", ["redistance", "extend_closest_point", "redistance_cubic", "interpolate_cubic"])
+def test_slab_decomposition_is_refused(m, entry):
+    """The single-rank zero-level-set operations refuse a slab-decomposed field with the header's wording."""
     n = C.c_int32(0)
     m._lib.lib().lsm_device_count(C.byref(n))
     if n.value < 2:
         pytest.skip("needs 2 GPUs")
+    lib = m._lib.lib()
     mc = m.MultiContext([0, 1])
     try:
-        phi, h = sphere((20, 18, 24))
-        f = _device(m, phi, (-0.5,) * 3, (0.5,) * 3, np.float64, ctx=mc.ranks[0])
-        assert m._lib.lib().lsm_redistance(mc.ranks[0].handle, f.device(), 3, None) == m._lib.ERR_UNSUPPORTED
+        ctx = mc.ranks[0]
+        phi, _ = sphere((20, 18, 24))
+        f = on_device(m, phi, (-0.5,) * 3, (0.5,) * 3, np.float64, ctx=ctx)
+        F = on_device(m, np.ones(phi.shape), (-0.5,) * 3, (0.5,) * 3, np.float64, ctx=ctx)
+        Y = np.zeros((1, 3))
+        call = {
+            "redistance": lambda: lib.lsm_redistance(ctx.handle, f.device(), 3, None),
+            "extend_closest_point": lambda: lib.lsm_extend_closest_point(ctx.handle, F.device(), f.device(), 3, 0, None),
+            "redistance_cubic": lambda: lib.lsm_redistance_cubic(ctx.handle, f.device(), 3, None, None),
+            "interpolate_cubic": lambda: lib.lsm_interpolate_cubic(ctx.handle, f.device(), 1, C.cast(Y.ctypes.data, C.POINTER(C.c_double)),
+                                                                   None, None, None),
+        }[entry]
+        assert call() == m._lib.ERR_UNSUPPORTED
         assert "slab decomposition is not supported" in m._lib.last_error()
-        del f
+        del f, F
     finally:
         mc.close()

@@ -16,22 +16,7 @@ import pytest
 
 import cubic_ref as CR
 import redistance_ref as R
-
-
-@pytest.fixture(scope="module")
-def m():
-    import lsm_b200
-    return lsm_b200
-
-
-def grid_h(lc, hc, n):
-    return [(hc[d] - lc[d]) / (n[d] - 1) for d in range(len(n))]
-
-
-def bits_equal(a, b):
-    a, b = np.asarray(a), np.asarray(b)
-    return (a.dtype == b.dtype and a.shape == b.shape
-            and np.array_equal(np.ascontiguousarray(a).view(np.uint8), np.ascontiguousarray(b).view(np.uint8)))
+from zero_set_helpers import bits_equal, grid_h, m, on_device, zalesak  # noqa: F401 (m is a fixture)
 
 
 def same_values(a, b):
@@ -275,10 +260,6 @@ def _cases():
 CASES = _cases()
 
 
-def _device(m, vals, lc, hc, dtype, ctx=None, bc=None):
-    return m.MeshField(np.asfortranarray(vals.astype(dtype)), m.CartesianGrid(lc, hc, vals.shape), bc=bc, ctx=ctx)
-
-
 def _points(vals, lc, hc, seed):
     """points inside the box, on cell faces (half-integer and integer u), on box faces, and outside"""
     rng = np.random.default_rng(seed)
@@ -311,14 +292,14 @@ def test_interpolate_equals_restatement(m, name, dtype):
     vals, lc, hc = CASES[name]
     vals = vals.astype(dtype)
     Y = _points(vals, lc, hc, len(name))
-    got = _interp(m, _device(m, vals, lc, hc, dtype), Y)
+    got = _interp(m, on_device(m, vals, lc, hc, dtype), Y)
     want = CR.evaluate(vals, lc, grid_h(lc, hc, vals.shape), Y)
     for a, b in zip(got, want):
         assert same_values(a, b)
     assert np.all(np.isnan(got[0][160:220]))
-    res = m.interpolate(_device(m, vals, lc, hc, dtype), Y)                  # the Python wrapper, and NULL outputs
+    res = m.interpolate(on_device(m, vals, lc, hc, dtype), Y)                  # the Python wrapper, and NULL outputs
     assert all(same_values(a, b) for a, b in zip(res, want))
-    ph = _device(m, vals, lc, hc, dtype)
+    ph = on_device(m, vals, lc, hc, dtype)
     v = np.empty(len(Y))
     m._lib.check(m._lib.lib().lsm_interpolate_cubic(ph._context().handle, ph.device(), len(Y),
                                                     C.cast(np.ascontiguousarray(Y).ctypes.data, C.POINTER(C.c_double)),
@@ -341,7 +322,7 @@ def _run(m, phi, band):
 def test_redistance_cubic_equals_restatement(m, name, dtype, band):
     vals, lc, hc = CASES[name]
     vals = vals.astype(dtype)
-    got, nb, nf = _run(m, _device(m, vals, lc, hc, dtype), band)
+    got, nb, nf = _run(m, on_device(m, vals, lc, hc, dtype), band)
     want, nb_want, nf_want = CR.redistance_cubic(vals, lc, grid_h(lc, hc, vals.shape), band)
     assert (nb, nf) == (nb_want, nf_want)
     assert bits_equal(got, want)
@@ -349,13 +330,6 @@ def test_redistance_cubic_equals_restatement(m, name, dtype, band):
         assert nb == 0 and nf == 0 and bits_equal(got, vals)
     if name == "3d_nan":
         assert nf > 0                                                          # stencils holding a NaN node fall back
-
-
-def zalesak(m, n, dtype=np.float64):
-    g = m.CartesianGrid((0.0, 0.0), (1.0, 1.0), (n, n))
-    disk = m.MeshField.from_shape(g, "sphere", (0.5, 0.75, 0.15), dtype=dtype)
-    slot = m.MeshField.from_shape(g, "box", (0.5, 0.725, 0.05, 0.25), dtype=dtype)
-    return m.setdiff_(disk, slot), g
 
 
 @pytest.mark.gpu
@@ -402,8 +376,8 @@ def test_third_order_on_a_sphere(m):
 def test_deterministic_and_asynchronous(m):
     vals, lc, hc = CASES["3d_odd_aniso"]
     ctx = m.default_context()
-    a = _device(m, vals, lc, hc, np.float64)
-    b = _device(m, vals, lc, hc, np.float64)
+    a = on_device(m, vals, lc, hc, np.float64)
+    b = on_device(m, vals, lc, hc, np.float64)
     a.device(), b.device()
     ctx.reset_counters()
     assert m.redistance(a, order=3) is a
@@ -493,22 +467,3 @@ def test_error_codes(m):
     finally:
         fresh.close()
 
-
-@pytest.mark.gpu
-def test_slab_decomposition_is_refused(m):
-    n = C.c_int32(0)
-    m._lib.lib().lsm_device_count(C.byref(n))
-    if n.value < 2:
-        pytest.skip("needs 2 GPUs")
-    mc = m.MultiContext([0, 1])
-    try:
-        vals, lc, hc = CASES["3d_odd_aniso"]
-        f = _device(m, vals, lc, hc, np.float64, ctx=mc.ranks[0])
-        assert m._lib.lib().lsm_redistance_cubic(mc.ranks[0].handle, f.device(), 3, None, None) == m._lib.ERR_UNSUPPORTED
-        assert "slab decomposition is not supported" in m._lib.last_error()
-        Y = np.zeros((1, 3))
-        assert m._lib.lib().lsm_interpolate_cubic(mc.ranks[0].handle, f.device(), 1, C.cast(Y.ctypes.data, C.POINTER(C.c_double)),
-                                                  None, None, None) == m._lib.ERR_UNSUPPORTED
-        del f
-    finally:
-        mc.close()

@@ -429,6 +429,57 @@ int32_t lsm_interpolate_cubic(lsm_ctx* ctx, lsm_field* phi, int64_t npts, const 
  * that fell back.  Bumps the field's version.  Scratch: lsm_redistance's (the refined points go to its spare point buffer). */
 int32_t lsm_redistance_cubic(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t* band_nodes_out, int64_t* fallback_nodes_out);
 
+/* ---- level-set integrals: how much region and interface the zero level set holds, and integrals of a field over them -----------
+ * The reference integrates over implicit domains on the host (ext/ImplicitIntegrationExt.jl); lsm_volume and lsm_perimeter above
+ * give its smoothed-Heaviside and smoothed-delta sums, whose values depend on the smoothing width.  lsm_level_set_integrals measures
+ * the sharp piecewise-linear geometry of lsm_interface_extract instead, on the device, and returns
+ *   out[0] = |{s <= 0}|,  out[1] = |{s = 0}|,  out[2] = integral of F over {s <= 0},  out[3] = integral of F over {s = 0}
+ * (out[2] and out[3] are NaN when F is NULL).  In double, each operation rounded, no FMA:
+ *  - geometry: s = double(phi) - level; a node is inside if s <= 0, outside if s > 0, invalid if s is NaN.  Cells, simplices, cut
+ *    edges, vertex coordinates and primitives are exactly those of lsm_interface_extract; a simplex with an invalid vertex
+ *    contributes nothing to any output.  The region is {P1(s) <= 0}, P1 the piecewise-linear interpolant on the triangulation.
+ *  - F is the P1 interpolant of its node values f = double(F): at the crossing of the simplex edge (w_x, w_y), x < y, its value is
+ *    Fa + t (Fb - Fa), t = s_a / (s_a - s_b), a = w_x, b = w_y (lsm_extend_closest_point's vertex value).  A sub-simplex contributes
+ *    its volume times the mean of F over its N+1 vertices, (((v0 + v1) + v2) + v3) / (N + 1); a primitive its measure times the mean
+ *    over its N vertices, (v0 + v1) / 2 or ((v0 + v1) + v2) / 3.  Both are exact for a linear F.  A NaN in F propagates.
+ *  - region (out[0], out[2]), with V = (|h1| |h2|) |h3| and Vs = V / N!:
+ *      a cell whose 2^N corners are all valid and inside contributes V, and V ((f0 + f7) / 4 + (((((f1 + f2) + f3) + f4) + f5) + f6) / 12)
+ *      to the integral of F (2-D: V ((f0 + f3) / 3 + (f1 + f2) / 6); 1-D: V ((f0 + f1) / 2); corner k = c + sum_d bit_d(k) e_d):
+ *      that is the sum over its simplices, and it makes a fully inside box exact;  a cell whose corners are all valid and outside
+ *      contributes nothing;  every other cell contributes its simplices in order:
+ *      a simplex whose vertices are all inside contributes Vs; a cut simplex the volume of its inside part, in fractions of Vs from
+ *      the crossing parameters of its cut edges:
+ *      - one lone vertex q (the only inside one; in 1-D always): with u_j = s_q / (s_q - s_oj) for the other vertices o_0 < o_1 < ..
+ *        in chain order, the corner simplex (q, P_qo0, ..) of volume Vs ((u_0 u_1) u_2).  1-D: the segment; 2-D and 3-D: a corner.
+ *      - 2-D, one lone outside vertex q, others r < s: the quad as the triangles (r, s, P_qs) of volume Vs (1 - u_s) and
+ *        (r, P_qs, P_qr) of volume Vs (u_s (1 - u_r)).
+ *      - 3-D, one lone outside vertex q: the tet minus the corner tet at q, volume Vs (1 - (u_0 u_1) u_2), integral of F
+ *        Vs mean(f over the tet) - (Vs ((u_0 u_1) u_2)) mean(corner tet).
+ *      - 3-D, inside {a < b}, outside {c < d} (the 2–2 prism), tau_xy = s_x / (s_x - s_y): the three tets (a, P_ac, P_ad, P_bd),
+ *        (a, P_ac, P_bc, P_bd), (a, b, P_bc, P_bd) of volumes Vs ((tau_ac tau_ad) (1 - tau_bd)), Vs ((tau_ac (1 - tau_bc)) tau_bd),
+ *        Vs (tau_bc tau_bd).
+ *  - interface (out[1], out[3]): the sum of the primitive measures, from the extraction's vertex coordinates v0, v1, v2: 1-D one per
+ *    point; 2-D sqrt(dx dx + dy dy), d = v1 - v0; 3-D sqrt((cx cx + cy cy) + cz cz) / 2, c = (v1 - v0) x (v2 - v0) with
+ *    cx = uy wz - uz wy, cy = uz wx - ux wz, cz = ux wy - uy wx, u = v1 - v0, w = v2 - v0.  This is the measure of the mesh
+ *    lsm_interface_extract returns, primitive by primitive; a lattice plane of exact zeros is counted once (from the cells on its
+ *    outside), since the cells on its inside have no cut edge.
+ *  - summation: each plane of cells (the cells sharing the index of the last axis) is summed to one partial per output, in a fixed
+ *    order that depends only on the plane's shape; then the planes are summed in increasing order.  The result does not depend
+ *    on the slab decomposition, bit for bit.
+ * F, when given, is a scalar, non-separable field of this context on phi's grid (n, lc and h), of either dtype, and may be phi itself;
+ * phi is a scalar, non-separable field of this context with every n_d >= 2; level is finite; out is not NULL; else LSM_ERR_ARG.
+ * Boundary conditions play no role (periodic axes: node n duplicates node 1, so no cell wraps).  With nranks > 1 the call is
+ * collective: rank r integrates the cell planes whose lower corner it owns (exchanging the ghost planes of phi, and of F, when they
+ * are stale), writes its plane partials into a buffer of n_last - 1 planes that is zero elsewhere, all-reduces the buffer (every
+ * entry has one non-zero contributor, so the sum is exact) and sums the planes as one GPU does: every rank returns the single-GPU
+ * value bit for bit.  Blocking: one synchronisation and a 32-byte copy; the plane partials (32 bytes per plane) live in the
+ * context's persistent reduction scratch, so the last extraction and the redistancing scratch are untouched.  Two kernel launches. */
+int32_t lsm_level_set_integrals(lsm_ctx* ctx, lsm_field* phi, lsm_field* F, double level, double* out);
+/* lsm_level_set_integrals on every rank of a lsm_ctx_create_multi box, on one host thread per GPU; F may be NULL (no F on any rank).
+ * out receives the 4 results, which are identical on every rank. */
+int32_t lsm_multi_level_set_integrals(int32_t n, lsm_ctx* const* ctx, lsm_field* const* phi, lsm_field* const* F,
+                                      double level, double* out);
+
 /* ---- diagnostics (test harness; SURVEY.md §2.2 K6) -------------------------------------------- */
 /* max |a - b| over all owned nodes, all-reduced over ranks. */
 int32_t lsm_max_abs_diff(lsm_ctx* ctx, const lsm_field* a, const lsm_field* b, double* out);

@@ -13,7 +13,7 @@ from .api import (Context, MultiContext, integrate_multi, compute_cfl_multi, def
                   EikonalReinitializationTerm, update_term, compute_cfl, step_plan, TimeIntegrator, ForwardEuler, RK2, RK3,
                   LevelSetEquation, current_state, current_time, integrate, integrate_bang, volume, perimeter, eikonal_reinitialize, extend_along_normals,
                   InterfaceMesh, extract_interface, merge_interfaces, extract_interface_multi, redistance, extend_closest_point,
-                  CubicInterpolation, interpolate,
+                  CubicInterpolation, interpolate, LevelSetIntegrals, level_set_integrals, level_set_integrals_multi,
     union, union_, intersect, intersect_, setdiff, setdiff_, complement, complement_,
                   _normalize_bc, _add_boundary_conditions)
 

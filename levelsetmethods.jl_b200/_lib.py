@@ -120,6 +120,8 @@ SYMBOLS = {
     "lsm_extend_closest_point": (_i32, [_vp, _vp, _vp, _i32, _i32, C.POINTER(_i64)]),
     "lsm_interpolate_cubic": (_i32, [_vp, _vp, _i64, _pdbl, _pdbl, _pdbl, _pdbl]),
     "lsm_redistance_cubic": (_i32, [_vp, _vp, _i32, C.POINTER(_i64), C.POINTER(_i64)]),
+    "lsm_level_set_integrals": (_i32, [_vp, _vp, _vp, _dbl, _pdbl]),
+    "lsm_multi_level_set_integrals": (_i32, [_i32, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), _dbl, _pdbl]),
     "lsm_max_abs_diff": (_i32, [_vp, _vp, _vp, _pdbl]),
 }
 

@@ -911,6 +911,16 @@ int32_t check_level_set(lsm_ctx* ctx, const lsm_field* phi, const char* what, in
     return LSM_OK;
 }
 
+// A second field F of an operation on phi (checked by check_level_set too) must lie on phi's grid: same node counts, same owned
+// slab, same lower corner and spacing.
+int32_t check_same_grid(const lsm_field* F, const lsm_field* phi) {
+    bool same = F->ndim == phi->ndim;
+    for (int d = 0; same && d < phi->ndim; ++d)
+        same = F->nglob[d] == phi->nglob[d] && F->n[d] == phi->n[d] && F->lc[d] == phi->lc[d] && F->h[d] == phi->h[d];
+    if (!same) return fail(LSM_ERR_ARG, "F and phi must be on the same grid (n, lc and h)");
+    return LSM_OK;
+}
+
 // The node box of phi for the kernels: this rank's owned nodes and, with `ghost`, the first plane of the next rank.  Level 0,
 // ntiles unset.
 IfaceArgs field_box(const lsm_field* phi, bool ghost) {
@@ -1770,10 +1780,7 @@ int32_t lsm_extend_closest_point(lsm_ctx* ctx, lsm_field* F, lsm_field* phi, int
     if (band < 1) return fail(LSM_ERR_ARG, "band must be at least 1 (got %d)", band);
     if (F && F == phi) return fail(LSM_ERR_ARG, "the extended field F must not be phi");
     for (const lsm_field* f : {F, phi}) TRY(check_level_set(ctx, f, "the closest-point extension", 2, true));
-    bool same = F->ndim == phi->ndim;
-    for (int d = 0; same && d < phi->ndim; ++d)
-        same = F->nglob[d] == phi->nglob[d] && F->n[d] == phi->n[d] && F->lc[d] == phi->lc[d] && F->h[d] == phi->h[d];
-    if (!same) return fail(LSM_ERR_ARG, "F and phi must be on the same grid (n, lc and h)");
+    TRY(check_same_grid(F, phi));
     return closest_points(ctx, phi, band, F, redistance_phi != 0, false, band_nodes_out, nullptr);
 }
 
@@ -1809,6 +1816,56 @@ int32_t lsm_redistance_cubic(lsm_ctx* ctx, lsm_field* phi, int32_t band, int64_t
     if (band < 1) return fail(LSM_ERR_ARG, "band must be at least 1 (got %d)", band);
     TRY(check_level_set(ctx, phi, "cubic redistancing", 4, true));
     return closest_points(ctx, phi, band, nullptr, true, true, band_nodes_out, fallback_nodes_out);
+}
+
+int32_t lsm_level_set_integrals(lsm_ctx* ctx, lsm_field* phi, lsm_field* F, double level, double* out) {
+    TRY(check_level_set(ctx, phi, "level-set integrals", 2, false));
+    if (F) {
+        TRY(check_level_set(ctx, F, "level-set integrals", 2, false));
+        TRY(check_same_grid(F, phi));
+    }
+    if (!std::isfinite(level)) return fail(LSM_ERR_ARG, "level must be finite (got %g)", level);
+    if (!out) return fail(LSM_ERR_ARG, "null argument");
+    CU(cudaSetDevice(ctx->device));
+    CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_halo, 0));
+    // the cells of the rank's last owned plane reach into the next rank's first plane (the upper ghost plane); the exchanges are
+    // collective, so every rank takes part
+    if (ctx->nranks > 1 && !phi->halo_valid) TRY(exchange_halo(phi, ctx->stream));
+    if (ctx->nranks > 1 && F && F != phi && !F->halo_valid) TRY(exchange_halo(F, ctx->stream));
+    const int N = phi->ndim, last = N - 1;
+    IntegArgs I{};
+    I.g = field_box(phi, ctx->nranks > 1 && ctx->rank < ctx->nranks - 1);
+    I.g.level = level;
+    I.F = F ? F->p : nullptr; I.F_f64 = F && F->dtype == LSM_F64;
+    I.planes = I.g.m[last] - 1;
+    I.plane0 = phi->first_last;
+    I.V = std::fabs(phi->h[0]);
+    for (int d = 1; d < N; ++d) I.V = I.V * std::fabs(phi->h[d]);
+    I.Vs = N == 3 ? I.V / 6.0 : N == 2 ? I.V / 2.0 : I.V;
+    // the partials of every cell plane of the grid (32 bytes each), then the four results
+    const long long nplanes = phi->nglob[last] - 1;
+    void* work = nullptr;
+    TRY(ctx_scratch(ctx, sizeof(double) * 4 * (size_t)(nplanes + 1), &work));
+    I.part = static_cast<double*>(work);
+    double* res = I.part + 4 * nplanes;
+    if (ctx->nranks > 1) CU(cudaMemsetAsync(I.part, 0, sizeof(double) * 4 * (size_t)nplanes, ctx->stream));
+    CU(launch_integral_planes(I, ctx->stream));
+    if (ctx->nranks > 1) NC(nccl().AllReduce(I.part, I.part, (size_t)(4 * nplanes), ncclDouble, ncclSum, ctx->nccl_comm, ctx->stream));
+    CU(launch_integral_sum(I.part, nplanes, res, ctx->stream));
+    ctx->cnt.kernel_launches += 2;
+    TRY(read_counts(ctx, res, 4));
+    std::memcpy(out, ctx->h_scalar, 4 * sizeof(double));
+    if (!F) out[2] = out[3] = std::numeric_limits<double>::quiet_NaN();
+    return LSM_OK;
+}
+
+int32_t lsm_multi_level_set_integrals(int32_t n, lsm_ctx* const* ctx, lsm_field* const* phi, lsm_field* const* F, double level,
+                                      double* out) {
+    if (!ctx || !phi || !out || n < 1) return fail(LSM_ERR_ARG, "bad argument");
+    std::vector<double> res(4 * (size_t)n, 0.0);
+    TRY(fan_out(n, [&](int r) { return lsm_level_set_integrals(ctx[r], phi[r], F ? F[r] : nullptr, level, &res[4 * (size_t)r]); }));
+    std::memcpy(out, res.data(), 4 * sizeof(double));       // identical on every rank
+    return LSM_OK;
 }
 
 int32_t lsm_field_csg(lsm_ctx* ctx, lsm_field* dst, const lsm_field* src, int32_t op) {

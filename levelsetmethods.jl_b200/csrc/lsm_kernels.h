@@ -112,6 +112,22 @@ cudaError_t launch_closest_points(const RedistArgs& R, int sm_count, cudaStream_
 cudaError_t launch_interp_cubic(const IfaceArgs& A, long long npts, const double* pts, double* val, double* grad, double* hess,
                                 cudaStream_t s);
 
+// lsm_integrals.cu: measures of {s <= 0} and {s = 0} and the integrals of F over them (lsm_level_set_integrals).  The box is
+// field_box's (with the upper ghost plane below the last rank); partials are 4 doubles per cell plane of the whole grid.
+struct IntegArgs {
+    IfaceArgs g;               // the box and the level (ntiles and lin0 unused)
+    const void* F;             // scalar field on g's grid, same box layout, or null
+    int F_f64;                 // F's dtype
+    long long planes;          // cell planes of the box (m_last - 1)
+    long long plane0;          // global index of the box's first cell plane
+    double V, Vs;              // prod_d |h_d| and V / N!
+    double* part;              // partials: part[4 plane + q], q = region, interface, F over the region, F over the interface
+};
+// one block per cell plane (one thread per cell in 1-D): writes the partials of the box's planes
+cudaError_t launch_integral_planes(const IntegArgs& I, cudaStream_t s);
+// one block: out[q] = sum of part[4 plane + q] over the planes in increasing order
+cudaError_t launch_integral_sum(const double* part, long long nplanes, double* out, cudaStream_t s);
+
 // The five Float64 constants of the WENO5 evaluation that do not fit an instruction immediate travel in the kernel parameters
 // (constant bank): as literals the compiler re-materialises them with 10 UMOV per node, from the constant bank it takes 3 uniform loads.
 // The 3-D x-pair kernel's default form scales e6 and fl by 3/16 once per thread (lsm_pair_common.cuh: weno_regs).

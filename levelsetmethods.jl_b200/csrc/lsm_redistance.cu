@@ -194,44 +194,6 @@ __device__ __forceinline__ void node_coords(const IfaceArgs& A, const int* i, do
     for (int d = 0; d < 3; ++d) x[d] = A.lc[d] + double(i[d]) * A.h[d];
 }
 
-// corner values of cell c (all corners in the box) and their classification
-template <class T, int N>
-__device__ __forceinline__ Masks cell_corners(const IfaceArgs& A, long long cidx, double* s) {
-    Masks M{(1u << (1 << N)) - 1u, 0, 0};
-    for (int k = 0; k < (1 << N); ++k) {
-        s[k] = sval<T>(A, cidx + corner_off(A, k));
-        if (s[k] <= 0.0) M.in |= 1u << k;
-        if (s[k] != s[k]) M.nan |= 1u << k;
-    }
-    return M;
-}
-
-// vertices V[j][d] of the primitives of simplex p of cell c, as lsm_interface.cu computes them on the lattice edge (c + w_x, c + w_y),
-// passed to f(V).  With a field F of dtype TF (cell c at index cidx), f(V, Fv) also gets the vertex values Fv[j] = Fa + t (Fb - Fa),
-// Fa = double(F[c + w_x]), Fb = double(F[c + w_y]), with the t of the coordinates.
-template <int N, class TF = void, class Fn>
-__device__ __forceinline__ void simplex_vertices(const IfaceArgs& A, const int* c, const double* s, const Masks& M, int p, Fn&& f,
-                                                 const TF* F = nullptr, long long cidx = 0) {
-    simplex_prims<N>(M, p, A.hsign, [&](const int* w, const int2* e) {
-        double V[N][3];
-        [[maybe_unused]] double Fv[N];
-        for (int j = 0; j < N; ++j) {
-            const int a = w[e[j].x], b = w[e[j].y];
-            const double t = s[a] / (s[a] - s[b]);
-            for (int d = 0; d < N; ++d) {
-                const double g = double(c[d] + ((a >> d) & 1));
-                V[j][d] = (((a ^ b) >> d) & 1) ? A.lc[d] + (g + t) * A.h[d] : A.lc[d] + g * A.h[d];
-            }
-            if constexpr (!std::is_void_v<TF>) {
-                const double fa = double(F[cidx + corner_off(A, a)]), fb = double(F[cidx + corner_off(A, b)]);
-                Fv[j] = fa + t * (fb - fa);
-            }
-        }
-        if constexpr (std::is_void_v<TF>) f(V);
-        else f(V, Fv);
-    });
-}
-
 template <int N, bool WHERE = false>
 __device__ __forceinline__ void closest(const double* x, const double (*V)[3], double* q, Where* W = nullptr) {
     if constexpr (N == 1) {
@@ -362,13 +324,14 @@ __global__ void __launch_bounds__(TPB) redist_pick_kernel(const __grid_constant_
                         if (want-- == 0) closest<N>(x, V, P);
                     });
                 } else {
-                    simplex_vertices<N, TF>(A, c, s, M, p, [&](const double (*V)[3], const double* Fv) {
+                    const TF* F = static_cast<const TF*>(R.F);
+                    simplex_vertices<N>(A, c, s, M, p, [&](const double (*V)[3], const double* Fv) {
                         if (want-- == 0) {
                             Where W;
                             closest<N, true>(x, V, P, &W);
                             val = value_at<N>(W, Fv);
                         }
-                    }, static_cast<const TF*>(R.F), cidx);
+                    }, [&](int k) { return double(F[cidx + corner_off(A, k)]); });
                 }
             }
         }

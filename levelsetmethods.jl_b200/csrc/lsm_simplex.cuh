@@ -1,8 +1,11 @@
 // lsm_simplex.cuh — the Freudenthal–Kuhn triangulation of the node lattice, shared by the zero-level-set extraction
-// (lsm_interface.cu) and the closest-point redistancing (lsm_redistance.cu): corner classification of a node's cell, the simplices
-// of a cell and the primitives (points / segments / triangles) each simplex contributes, in the order include/lsm_b200.h states.
+// (lsm_interface.cu), the closest-point redistancing (lsm_redistance.cu) and the level-set integrals (lsm_integrals.cu): corner
+// classification of a node's cell, the simplices of a cell, the primitives (points / segments / triangles) each simplex contributes,
+// in the order include/lsm_b200.h states, and their vertex coordinates.
 #pragma once
+#include <cstddef>
 #include <cstdint>
+#include <type_traits>
 #include <cuda_runtime.h>
 #include "lsm_kernels.h"
 
@@ -123,6 +126,45 @@ __device__ __forceinline__ void simplex_prims(const Masks& M, int p, int hsign, 
         if (sigma > 0) { const int2 t0[3] = {ac, ad, bd}, t1[3] = {ac, bd, bc}; emit(w, t0); emit(w, t1); }
         else           { const int2 t0[3] = {ac, bd, ad}, t1[3] = {ac, bc, bd}; emit(w, t0); emit(w, t1); }
     }
+}
+
+// corner values of cell c (all corners in the box) and their classification
+template <class T, int N>
+__device__ __forceinline__ Masks cell_corners(const IfaceArgs& A, long long cidx, double* s) {
+    Masks M{(1u << (1 << N)) - 1u, 0, 0};
+    for (int k = 0; k < (1 << N); ++k) {
+        s[k] = sval<T>(A, cidx + corner_off(A, k));
+        if (s[k] <= 0.0) M.in |= 1u << k;
+        if (s[k] != s[k]) M.nan |= 1u << k;
+    }
+    return M;
+}
+
+// vertices V[j][d] of the primitives of simplex p of cell c, as lsm_interface.cu computes them on the lattice edge (c + w_x, c + w_y),
+// passed to f(V).  With a field F, given as F_at(k) = double(F) at corner k of the cell, f(V, Fv) also gets the vertex values
+// Fv[j] = Fa + t (Fb - Fa), Fa = F_at(w_x), Fb = F_at(w_y), with the t of the coordinates.
+template <int N, class Fn, class FAt = std::nullptr_t>
+__device__ __forceinline__ void simplex_vertices(const IfaceArgs& A, const int* c, const double* s, const Masks& M, int p, Fn&& f,
+                                                 FAt&& F_at = nullptr) {
+    constexpr bool WITH_F = !std::is_same_v<std::decay_t<FAt>, std::nullptr_t>;
+    simplex_prims<N>(M, p, A.hsign, [&](const int* w, const int2* e) {
+        double V[N][3];
+        [[maybe_unused]] double Fv[N];
+        for (int j = 0; j < N; ++j) {
+            const int a = w[e[j].x], b = w[e[j].y];
+            const double t = s[a] / (s[a] - s[b]);
+            for (int d = 0; d < N; ++d) {
+                const double g = double(c[d] + ((a >> d) & 1));
+                V[j][d] = (((a ^ b) >> d) & 1) ? A.lc[d] + (g + t) * A.h[d] : A.lc[d] + g * A.h[d];
+            }
+            if constexpr (WITH_F) {
+                const double fa = F_at(a), fb = F_at(b);
+                Fv[j] = fa + t * (fb - fa);
+            }
+        }
+        if constexpr (WITH_F) f(V, Fv);
+        else f(V);
+    });
 }
 
 __device__ __forceinline__ void node_index(const IfaceArgs& A, long long idx, int* i) {

@@ -639,6 +639,34 @@ function extend_closest_point!(F::DeviceMeshField, ϕ::DeviceMeshField; band::In
     return _device_advanced!(F)
 end
 
+"""
+    level_set_integrals(ϕ::DeviceMeshField; F = nothing, level = 0) -> (inside, interface, F_inside, F_interface)
+
+The measures of {ϕ ≤ level} and {ϕ = level} and the integrals of F over both, on the device (`lsm_level_set_integrals`; 32 bytes
+reach the host).  The geometry is the sharp piecewise-linear interface of `interface_mesh` and the region it bounds, with F
+interpolated linearly (exact for a linear F); `F_inside` / `F_interface` are `nothing` without F.  Moments come from an F such as
+the device field of `x1`.  Deliberately not methods of `LevelSetMethods.volume` / `perimeter`, which keep the reference's smoothed
+Heaviside and delta sums (levelsetops.jl:27-33,139-149).
+"""
+function level_set_integrals(ϕ::DeviceMeshField; F::Union{DeviceMeshField, Nothing} = nothing, level::Real = 0)
+    out = zeros(Float64, 4)
+    check(ccall((:lsm_level_set_integrals, LIB), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, Float64, Ptr{Float64}),
+                ϕ.ctx.handle, handle!(ϕ), F === nothing ? C_NULL : handle!(F), Float64(level), out))
+    return (inside = out[1], interface = out[2], F_inside = F === nothing ? nothing : out[3],
+            F_interface = F === nothing ? nothing : out[4])
+end
+
+"`level_set_integrals` of a field slab-decomposed over `mc` (collective, `lsm_multi_level_set_integrals`): the single-GPU value bit for bit."
+function level_set_integrals(mc::MultiContext, ϕs::Vector{<:DeviceMeshField}; Fs = nothing, level::Real = 0)
+    n = length(mc.ranks)
+    out = zeros(Float64, 4)
+    check(ccall((:lsm_multi_level_set_integrals, LIB), Int32, (Int32, Ptr{Ptr{Cvoid}}, Ptr{Ptr{Cvoid}}, Ptr{Ptr{Cvoid}}, Float64, Ptr{Float64}),
+                n, [c.handle for c in mc.ranks], [handle!(ϕ) for ϕ in ϕs], Fs === nothing ? C_NULL : [handle!(F) for F in Fs],
+                Float64(level), out))
+    return (inside = out[1], interface = out[2], F_inside = Fs === nothing ? nothing : out[3],
+            F_interface = Fs === nothing ? nothing : out[4])
+end
+
 "`extend_along_normals!(F, ϕ; …)` — src/velocityextension.jl:20-78 on device fields."
 function LSM.extend_along_normals!(F::DeviceMeshField, ϕ::DeviceMeshField; nb_iters::Integer = 50, cfl::Real = 0.45, frozen = nothing,
                                    interface_band::Real = 1.5, min_norm::Real = 1.0e-14)

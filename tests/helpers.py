@@ -33,6 +33,10 @@ class Case:
         self.phi0 = np.asfortranarray(phi0.astype(dtype))
         self.terms, self.bc, self.dtype = terms, bc, dtype
 
+    def coef_field(self, t):
+        """A term's stored coefficient, in its own ``field_dtype`` when it sets one (a Float64 field with a Float32 state)."""
+        return np.asfortranarray(t["field"].astype(t.get("field_dtype", self.dtype)))
+
     # ---- oracle side ----
     def oracle_bc(self):
         def one(b):
@@ -57,15 +61,13 @@ class Case:
                     sc, tabs = t["separable"]
                     out.append(O.advection_separable(sc, tabs, scheme=sch, tscale=ts, tparam=tp))
                 elif "field" in t:
-                    out.append(O.advection(np.asfortranarray(t["field"].astype(self.dtype)), scheme=sch, tscale=ts, tparam=tp))
+                    out.append(O.advection(self.coef_field(t), scheme=sch, tscale=ts, tparam=tp))
                 else:
                     out.append(O.advection(t["const"], scheme=sch, tscale=ts, tparam=tp))
             elif k == "normal":
-                v = t["field"].astype(self.dtype) if "field" in t else t["const"]
-                out.append(O.normal_motion(np.asfortranarray(v) if "field" in t else v))
+                out.append(O.normal_motion(self.coef_field(t) if "field" in t else t["const"]))
             elif k == "curvature":
-                b = t["field"].astype(self.dtype) if "field" in t else t["const"]
-                out.append(O.curvature(np.asfortranarray(b) if "field" in t else b))
+                out.append(O.curvature(self.coef_field(t) if "field" in t else t["const"]))
             elif k == "eikonal":
                 if t.get("frozen", True):
                     out.append(O.eikonal(O.eikonal_s0(self.oracle_field()) if s0 is None else s0))
@@ -105,17 +107,17 @@ class Case:
                     sc, tabs = t["separable"]
                     base = m.SeparableVelocity(g, sc, tabs, ctx=ctx)
                 elif "field" in t:
-                    base = m.MeshField(np.asfortranarray(t["field"].astype(self.dtype)), g, ctx=ctx)
+                    base = m.MeshField(self.coef_field(t), g, ctx=ctx)
                 else:
                     base = tuple(t["const"])
                 if "cos_period" in t:
                     base = m.TimeScaled(base, ("cos", t["cos_period"]))
                 out.append(m.AdvectionTerm(base, sch))
             elif k == "normal":
-                v = m.MeshField(np.asfortranarray(t["field"].astype(self.dtype)), g, ctx=ctx) if "field" in t else t["const"]
+                v = m.MeshField(self.coef_field(t), g, ctx=ctx) if "field" in t else t["const"]
                 out.append(m.NormalMotionTerm(v))
             elif k == "curvature":
-                b = m.MeshField(np.asfortranarray(t["field"].astype(self.dtype)), g, ctx=ctx) if "field" in t else t["const"]
+                b = m.MeshField(self.coef_field(t), g, ctx=ctx) if "field" in t else t["const"]
                 out.append(m.CurvatureTerm(b))
             elif k == "eikonal":
                 out.append(m.EikonalReinitializationTerm(phi) if t.get("frozen", True) else m.EikonalReinitializationTerm())
@@ -185,6 +187,109 @@ def c5_normal_advection(n=64, dtype=np.float64):
     v = np.full(nn, 0.2)
     u = np.stack([bcast(-y, nn), bcast(x, nn), np.zeros(nn)], axis=0)
     return Case("C5", lc, hc, nn, phi, [dict(kind="normal", field=v), dict(kind="advection", field=u)], ("neumann",), dtype)
+
+
+# ---- the term / BC matrix of the stage-kernel parity tests ----------------------------------------------------------
+def small_problem(n):
+    """Grid corners, phi0 and the stored velocity u, speed v and curvature coefficient b of the term / BC matrix on an n grid
+    (1-, 2- or 3-D; anisotropic mesh sizes, sign changes of every coefficient)."""
+    N = len(n)
+    lc, hc = [-1.0] * N, [1.0 + 0.1 * d for d in range(N)]
+    X = coords(lc, hc, n)
+    r = np.sqrt(sum((x - 0.1) ** 2 for x in X))
+    phi = bcast((r - 0.5) * (1 + 0.3 * np.sin(3 * X[0])), n)
+    u = np.stack([bcast(np.sin(2 * X[d] + d) + 0.2, n) for d in range(N)], axis=0)
+    v = bcast(0.3 + 0.5 * np.cos(2 * X[0]), n)
+    b = bcast(-0.02 - 0.01 * np.sin(X[-1]), n)
+    return lc, hc, phi, u, v, b
+
+
+def small_termsets(u, v, b, N):
+    """Every term kind and coefficient kind alone, and the two- and three-term lists the stage kernels dispatch on."""
+    return {
+        "adv_weno": [dict(kind="advection", field=u)],
+        "adv_upwind": [dict(kind="advection", field=u, scheme="upwind")],
+        "adv_const_cos": [dict(kind="advection", const=tuple([0.7, -0.4, 0.5][:N]), cos_period=0.05)],
+        "normal": [dict(kind="normal", field=v)],
+        "normal_const": [dict(kind="normal", const=-0.8)],
+        "curv": [dict(kind="curvature", field=b)],
+        "curv_const": [dict(kind="curvature", const=-0.05)],
+        "eik_frozen": [dict(kind="eikonal", frozen=True)],
+        "eik_live": [dict(kind="eikonal", frozen=False)],
+        "three": [dict(kind="normal", field=v), dict(kind="advection", field=u), dict(kind="curvature", const=-0.01)],
+        # two-term lists: the BASELINE orders run the static-signature kernels (C5: normal+adv fields, C2: adv field + const
+        # curvature); the reversed orders / other coefficient kinds must take the runtime-dispatch kernels of the same masks
+        "normal_adv": [dict(kind="normal", field=v), dict(kind="advection", field=u)],
+        "adv_normal": [dict(kind="advection", field=u), dict(kind="normal", field=v)],
+        "normalc_adv": [dict(kind="normal", const=0.6), dict(kind="advection", field=u)],
+        "adv_curvc": [dict(kind="advection", field=u), dict(kind="curvature", const=-0.03)],
+        "curvc_adv": [dict(kind="curvature", const=-0.03), dict(kind="advection", field=u)],
+        "adv_curvf": [dict(kind="advection", field=u), dict(kind="curvature", field=b)],
+    }
+
+
+SMALL_BCS = (("periodic",), ("neumann",), ("extrap", 2), ("symmetry",), ("extrap", 1))
+SMALL_SPLIT = (("neumann",), ("extrap", 1))
+
+
+def small_bc(i, N, bcs=SMALL_BCS, split=SMALL_SPLIT):
+    """BC of the i-th term set: bcs[(i + d) % len(bcs)] along axis d; every third set (2-D and 3-D) has `split`'s two
+    different sides along y."""
+    bc = tuple(bcs[(i + d) % len(bcs)] for d in range(N))
+    if N > 1 and i % 3 == 0:
+        bc = (bc[0], split) + bc[2:]
+    return bc
+
+
+def small_cases(n, bcs=SMALL_BCS, split=SMALL_SPLIT):
+    """[(f"{N}d-{term set}", Case)] of the term / BC matrix on an n grid."""
+    N = len(n)
+    lc, hc, phi, u, v, b = small_problem(n)
+    return [(f"{N}d-{tn}", Case(tn, lc, hc, n, phi, ts, small_bc(i, N, bcs, split)))
+            for i, (tn, ts) in enumerate(small_termsets(u, v, b, N).items())]
+
+
+# ---- integration through the oracle and the engine -----------------------------------------------------------------
+INTEG = {"FE": 0, "RK2": 1, "RK3": 2}
+
+
+def run_oracle(O, case, integ="RK3", steps=100, tf=None, cfl=0.5):
+    """Integrate `case` with the oracle; return (phi, t, nsteps, tf).  Without `tf`, tf is chosen from the initial CFL step so
+    that exactly `steps` steps are taken when dt is constant."""
+    fo = case.oracle_field()
+    to = case.oracle_terms()
+    if tf is None:
+        dt0 = cfl * O.compute_cfl(fo, to, 0.0)
+        tf = dt0 * steps * (1 - 1e-12)
+    t_o, n_o = O.integrate(fo, INTEG[integ], to, tf, cfl=cfl)
+    return fo.vals, t_o, n_o, tf
+
+
+def run_engine(m, case, integ, tf, cfl=0.5):
+    """Integrate `case` to `tf` with the engine (the context's current kernel options); return the equation."""
+    phi = case.engine_field(m)
+    terms = case.engine_terms(m, phi)
+    eq = m.LevelSetEquation(terms=terms, ic=phi, integrator=getattr(m, {"FE": "ForwardEuler"}.get(integ, integ))(cfl))
+    m.integrate(eq, tf)
+    return eq
+
+
+def run_pair(m, O, case, integ="RK3", steps=100, tf=None, cfl=0.5):
+    """Integrate `case` with the oracle and the engine; return (phi_oracle, phi_engine, t, nsteps)."""
+    a, t_o, n_o, tf = run_oracle(O, case, integ, steps, tf, cfl)
+    eq = run_engine(m, case, integ, tf, cfl)
+    assert eq.t == t_o
+    assert eq.steps_taken == n_o
+    return a, eq.state.peek(), t_o, n_o
+
+
+def check_parity(a, b, tol):
+    assert not np.isnan(b).any()
+    d = np.abs(a.astype(np.float64) - b.astype(np.float64)).max()
+    assert d <= tol, f"max-abs difference {d:.3e} > {tol:.1e}"
+    assert np.array_equal(np.sign(a), np.sign(b)), "zero-level-set node classification differs"
+    assert np.array_equal(cut_cells(a), cut_cells(b)), "cut-cell classification differs"
+    return d
 
 
 def cut_cells(phi):

@@ -31,36 +31,6 @@ def strict(m):
     ctx.set_option(OPT_KERNEL, 0)
 
 
-INTEG = {"FE": 0, "RK2": 1, "RK3": 2}
-
-
-def run_pair(m, O, case, integ="RK3", steps=100, tf=None, cfl=0.5):
-    """Integrate `case` with the oracle and the engine; return (phi_oracle, phi_engine, t, nsteps)."""
-    fo = case.oracle_field()
-    to = case.oracle_terms()
-    # choose tf from the initial CFL step so that exactly `steps` steps are taken when dt is constant
-    if tf is None:
-        dt0 = cfl * O.compute_cfl(fo, to, 0.0)
-        tf = dt0 * steps * (1 - 1e-12)
-    t_o, n_o = O.integrate(fo, INTEG[integ], to, tf, cfl=cfl)
-    phi = case.engine_field(m)
-    terms = case.engine_terms(m, phi)
-    eq = m.LevelSetEquation(terms=terms, ic=phi, integrator=getattr(m, {"FE": "ForwardEuler"}.get(integ, integ))(cfl))
-    m.integrate(eq, tf)
-    assert eq.t == t_o
-    assert eq.steps_taken == n_o
-    return fo.vals, eq.state.peek(), t_o, n_o
-
-
-def check_parity(a, b, tol):
-    assert not np.isnan(b).any()
-    d = np.abs(a.astype(np.float64) - b.astype(np.float64)).max()
-    assert d <= tol, f"max-abs difference {d:.3e} > {tol:.1e}"
-    assert np.array_equal(np.sign(a), np.sign(b)), "zero-level-set node classification differs"
-    assert np.array_equal(H.cut_cells(a), H.cut_cells(b)), "cut-cell classification differs"
-    return d
-
-
 # ------------------------------------------------------------------------------------------------
 # ghost cells on the device (test/test-meshfield.jl:44-125) against the oracle
 # ------------------------------------------------------------------------------------------------
@@ -131,43 +101,7 @@ def test_cfl_bitexact_and_errors(m, O):
 # strict kernel: every term x BC x dim x dtype x integrator, a few steps, rounding-level agreement
 # ------------------------------------------------------------------------------------------------
 def _small_cases():
-    out = []
-    rng = np.random.default_rng(3)
-    for N, n in ((1, (40,)), (2, (26, 22)), (3, (14, 12, 13))):
-        lc, hc = [-1.0] * N, [1.0 + 0.1 * d for d in range(N)]
-        X = H.coords(lc, hc, n)
-        r = np.sqrt(sum((x - 0.1) ** 2 for x in X))
-        phi = H.bcast((r - 0.5) * (1 + 0.3 * np.sin(3 * X[0])), n)
-        u = np.stack([H.bcast(np.sin(2 * X[d] + d) + 0.2, n) for d in range(N)], axis=0)
-        v = H.bcast(0.3 + 0.5 * np.cos(2 * X[0]), n)
-        b = H.bcast(-0.02 - 0.01 * np.sin(X[-1]), n)
-        bcs = [("periodic",), ("neumann",), ("extrap", 2), ("symmetry",), ("extrap", 1)]
-        termsets = {
-            "adv_weno": [dict(kind="advection", field=u)],
-            "adv_upwind": [dict(kind="advection", field=u, scheme="upwind")],
-            "adv_const_cos": [dict(kind="advection", const=tuple([0.7, -0.4, 0.5][:N]), cos_period=0.05)],
-            "normal": [dict(kind="normal", field=v)],
-            "normal_const": [dict(kind="normal", const=-0.8)],
-            "curv": [dict(kind="curvature", field=b)],
-            "curv_const": [dict(kind="curvature", const=-0.05)],
-            "eik_frozen": [dict(kind="eikonal", frozen=True)],
-            "eik_live": [dict(kind="eikonal", frozen=False)],
-            "three": [dict(kind="normal", field=v), dict(kind="advection", field=u), dict(kind="curvature", const=-0.01)],
-            # two-term lists: the BASELINE orders run the static-signature kernels (C5: normal+adv fields, C2: adv field + const
-            # curvature); the reversed orders / other coefficient kinds must take the runtime-dispatch kernels of the same masks
-            "normal_adv": [dict(kind="normal", field=v), dict(kind="advection", field=u)],
-            "adv_normal": [dict(kind="advection", field=u), dict(kind="normal", field=v)],
-            "normalc_adv": [dict(kind="normal", const=0.6), dict(kind="advection", field=u)],
-            "adv_curvc": [dict(kind="advection", field=u), dict(kind="curvature", const=-0.03)],
-            "curvc_adv": [dict(kind="curvature", const=-0.03), dict(kind="advection", field=u)],
-            "adv_curvf": [dict(kind="advection", field=u), dict(kind="curvature", field=b)],
-        }
-        for i, (tn, ts) in enumerate(termsets.items()):
-            bc = tuple(bcs[(i + d) % len(bcs)] for d in range(N))
-            if N > 1 and i % 3 == 0:
-                bc = (bc[0],) + ((("neumann",), ("extrap", 1)),) + bc[2:]       # different left / right
-            out.append((f"{N}d-{tn}", H.Case(tn, lc, hc, n, phi, ts, bc)))
-    return out
+    return [c for n in ((40,), (26, 22), (14, 12, 13)) for c in H.small_cases(n)]
 
 
 @pytest.mark.parametrize("name,case", _small_cases(), ids=[c[0] for c in _small_cases()])
@@ -175,7 +109,7 @@ def _small_cases():
 def test_strict_kernel_all_terms(m, O, strict, name, case, dtype):
     case = H.Case(case.name, case.lc, case.hc, case.n, case.phi0, case.terms, case.bc, dtype)
     for integ in ("FE", "RK2", "RK3"):
-        a, b, _, n = run_pair(m, O, case, integ=integ, steps=4)
+        a, b, _, n = H.run_pair(m, O, case, integ=integ, steps=4)
         assert n == 4 or "cos" in name
         tol = 1e-13 if dtype == np.float64 else 2e-6
         d = np.abs(a.astype(np.float64) - b.astype(np.float64)).max()
@@ -186,12 +120,14 @@ def test_strict_kernel_all_terms(m, O, strict, name, case, dtype):
                          ids=[c[0] for c in _small_cases() if not c[0].startswith("1d")])
 @pytest.mark.parametrize("dtype", [np.float64, np.float32], ids=["f64", "f32"])
 def test_tiled_kernel_all_terms(m, O, name, case, dtype):
-    """The same matrix through the default kernel selection, i.e. the tiled cp.async/TMA kernels (2-D and 3-D): every
-    term, every BC kind (index-remap and polynomial-extrapolation instantiations), partial tiles on every side, all three
-    integrators.  Tolerance = the BASELINE bar (1e-10 / 1e-4), far above what 8 steps accumulate."""
+    """The same matrix through the default kernel selection, i.e. the tiled kernels (2-D and 3-D): every term, every BC
+    kind (index-remap and polynomial-extrapolation instantiations), all three integrators.  The grids are small: 26 x 22 is
+    one tile in x and two in y, 14 x 12 x 13 one tile and one z chunk, so every tile is partial and resolves its ghosts;
+    none takes the plain-copy or TMA fill.  Grids of many tiles are in test_tiled_multitile.py.  Tolerance = the BASELINE
+    bar (1e-10 / 1e-4), far above what 8 steps accumulate."""
     case = H.Case(case.name, case.lc, case.hc, case.n, case.phi0, case.terms, case.bc, dtype)
     for integ in ("FE", "RK2", "RK3"):
-        a, b, _, n = run_pair(m, O, case, integ=integ, steps=8)
+        a, b, _, n = H.run_pair(m, O, case, integ=integ, steps=8)
         tol = 1e-10 if dtype == np.float64 else 1e-4
         d = np.abs(a.astype(np.float64) - b.astype(np.float64)).max()
         assert not np.isnan(b).any() and d <= tol * max(1.0, np.abs(a).max()), (name, integ, d)
@@ -215,9 +151,9 @@ CONFIGS = [
 def test_config_parity_100_steps(m, O, name, mk, dtype):
     case = mk(dtype)
     steps = 50 if name.startswith("C4") else 100
-    a, b, t, n = run_pair(m, O, case, integ="RK3", steps=steps)
+    a, b, t, n = H.run_pair(m, O, case, integ="RK3", steps=steps)
     assert n >= 0.9 * steps
-    d = check_parity(a, b, 1e-10 if dtype == np.float64 else 1e-4)
+    d = H.check_parity(a, b, 1e-10 if dtype == np.float64 else 1e-4)
     print(f"{name} {np.dtype(dtype).name}: {n} steps, max-abs diff {d:.3e}")
 
 
@@ -240,9 +176,9 @@ def test_config_parity_survey_sizes(m, O, name, mk, dtype):
     case = mk(dtype)
     steps = 50 if name.startswith("C4") else 100
     O.set_threads(O.max_threads())
-    a, b, t, n = run_pair(m, O, case, integ="RK3", steps=steps)
+    a, b, t, n = H.run_pair(m, O, case, integ="RK3", steps=steps)
     assert n >= 0.9 * steps
-    d = check_parity(a, b, 1e-10 if dtype == np.float64 else 1e-4)
+    d = H.check_parity(a, b, 1e-10 if dtype == np.float64 else 1e-4)
     print(f"PARITY {name} {np.dtype(dtype).name}: {n} steps, max-abs diff {d:.3e} (bar {'1e-10' if dtype == np.float64 else '1e-4'})")
 
 
@@ -479,8 +415,8 @@ def test_pair_kernel_kinked_body_parity(m, O):
     """Default kernels on non-smooth data, 96^3 cube (isotropic mesh: folded scaling + 20-bit epsilon maximum), 100 RK3 steps
     against the oracle: the BASELINE bar with the observed value printed."""
     O.set_threads(O.max_threads())
-    a, b, t, n = run_pair(m, O, _notched_sphere_case(96), integ="RK3", steps=100)
-    d = check_parity(a, b, 1e-10)
+    a, b, t, n = H.run_pair(m, O, _notched_sphere_case(96), integ="RK3", steps=100)
+    d = H.check_parity(a, b, 1e-10)
     print(f"PARITY notched-sphere-96 float64: {n} steps, max-abs diff {d:.3e} (bar 1e-10)")
     assert d <= 2e-11
 
@@ -606,18 +542,18 @@ def test_against_committed_vectors(m):
             eq = m.LevelSetEquation(terms=case.engine_terms(m, phi), ic=phi, integrator={"RK2": m.RK2, "RK3": m.RK3}[integ]())
             m.integrate(eq, float(tf))
             assert eq.steps_taken == int(n), (name, tag)
-            check_parity(gold[f"{name}_{tag}"], eq.state.peek(), 1e-10 if dtype == np.float64 else 1e-4)
+            H.check_parity(gold[f"{name}_{tag}"], eq.state.peek(), 1e-10 if dtype == np.float64 else 1e-4)
 
 
 def test_c4_rk2_reference_default(m, O):
-    a, b, _, n = run_pair(m, O, H.c4_eikonal(40), integ="RK2", steps=50)
-    check_parity(a, b, 1e-10)
+    a, b, _, n = H.run_pair(m, O, H.c4_eikonal(40), integ="RK2", steps=50)
+    H.check_parity(a, b, 1e-10)
 
 
 def test_strict_and_default_kernels_agree(m, O, strict):
     """Same run through the strict generic kernel: must also be inside the tolerance (and is in fact at rounding level)."""
-    a, b, _, _ = run_pair(m, O, H.c3_enright(40), steps=60)
-    d = check_parity(a, b, 1e-10)
+    a, b, _, _ = H.run_pair(m, O, H.c3_enright(40), steps=60)
+    d = H.check_parity(a, b, 1e-10)
     assert d <= 1e-13
 
 

@@ -104,7 +104,7 @@ enum {
     LSM_OPT_TIME_STAGES = 1,  /* 1: bracket every stage launch with CUDA events, resolved at the next sync  */
     LSM_OPT_CFL_CACHE = 2,    /* 1 (default): reuse the CFL reduction while coefficient data/scale unchanged  */
     LSM_OPT_OVERLAP = 3,      /* 1 (default): overlap halo exchange with interior compute (multi-rank)        */
-    LSM_OPT_FUSE_CFL = 4,     /* 1 (default): lsm_integrate lets the last RK stage reduce the next step's CFL maximum (time-scaled stored velocity) */
+    /* 4 is retired and not reused: lsm_set_option rejects it with LSM_ERR_ARG */
     LSM_OPT_GRAPH = 5,        /* 1 (default): lsm_integrate replays a captured CUDA graph of one step's stage launches on small grids (launch-bound regime) */
     LSM_OPT_CFL_CANDIDATES = 6, /* 1 (default): the CFL maximum of a TIME-SCALED static coefficient field is evaluated on the host over the few nodes that
                                   can attain it for any scale (exact, see lsm_api.cu) - no reduction pass, D2H or host sync per step */

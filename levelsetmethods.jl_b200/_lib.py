@@ -23,7 +23,7 @@ COEF_CONST, COEF_FIELD, COEF_SEPARABLE, COEF_NONE, COEF_EXPR = 0, 1, 2, 3, 4
 TS_NONE, TS_COS, TS_HOST = 0, 1, 2
 SHAPE_SPHERE, SHAPE_BOX, SHAPE_PLANE, SHAPE_CONST = 0, 1, 2, 3
 FORWARD_EULER, RK2, RK3 = 0, 1, 2
-OPT_KERNEL, OPT_TIME_STAGES, OPT_CFL_CACHE, OPT_OVERLAP, OPT_FUSE_CFL, OPT_GRAPH, OPT_CFL_CANDIDATES, OPT_RESIDENT = 0, 1, 2, 3, 4, 5, 6, 7
+OPT_KERNEL, OPT_TIME_STAGES, OPT_CFL_CACHE, OPT_OVERLAP, OPT_GRAPH, OPT_CFL_CANDIDATES, OPT_RESIDENT = 0, 1, 2, 3, 5, 6, 7
 MAX_TERMS = 4
 
 

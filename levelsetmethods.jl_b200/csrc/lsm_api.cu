@@ -60,17 +60,18 @@ inline double jl_eps(double x) {    // Base.eps(::Float64)
     return std::nextafter(x, std::numeric_limits<double>::infinity()) - x;
 }
 
-struct CflCacheEntry { int kind; const void* field; uint64_t version; double g; int scaled; unsigned long long bits; };
-
-// Exact CFL maximum of a TIME-SCALED static coefficient field without touching the device again (replaces a per-step reduction
-// pass + 8-byte D2H + host sync).  The reference's per-node quantity is s_i(g) = sum_d fl(|fl(u_d g)| / h_d) (levelsetterms.jl:
-// 90-96) = |g| S_i (1 + theta), |theta| <= 4.5e-16, with S_i = sum_d |u_d| / h_d.  A node with S_i < (1 - 1e-12) max_j S_j can
-// therefore never attain max_i s_i(g) for ANY g, so the maximum over the (few) candidate nodes above that threshold, evaluated on
-// the host with the same IEEE operations, is bit-identical to the full reduction.  For the scalar coefficients (normal motion,
-// curvature) |fl(v g)| is monotone in |v|, and the same argument holds with S_i = |v_i|.
-struct CflCand {
+// What is known about the CFL maximum of one (term kind, stored or separable coefficient field) at one version of the field's data.
+//   * The last exact answer of a full reduction pass, for its scale g.
+//   * The candidate set of a TIME-SCALED field, which answers every scale without touching the device again (no reduction pass,
+//     no 8-byte D2H, no host sync per step).  The reference's per-node quantity is s_i(g) = sum_d fl(|fl(u_d g)| / h_d)
+//     (levelsetterms.jl:90-96) = |g| S_i (1 + theta), |theta| <= 4.5e-16, with S_i = sum_d |u_d| / h_d.  A node with
+//     S_i < (1 - 1e-12) max_j S_j can therefore never attain max_i s_i(g) for ANY g, so the maximum over the (few) candidate nodes
+//     above that threshold, evaluated on the host with the same IEEE operations, is bit-identical to the full reduction.  For the
+//     scalar coefficients (normal motion, curvature) |fl(v g)| is monotone in |v|, and the same argument holds with S_i = |v_i|.
+struct CflMemo {
     int kind = 0; const void* field = nullptr; uint64_t version = 0;
-    int ncomp = 0, seen = 0;
+    bool have_bits = false; int scaled = 0; double g = 0; unsigned long long bits = 0;     // last full pass
+    int ncomp = 0, seen = 0;     // candidates: coefficient components, time-scaled requests seen
     bool built = false, overflow = false;
     std::vector<double> tup;     // distinct raw coefficient tuples of the candidate nodes (all ranks)
 };
@@ -88,8 +89,7 @@ struct lsm_ctx {
     lsm_counters cnt{};
     int opt_kernel = 0, opt_time = 0, opt_cfl_cache = 1, opt_overlap = 1;
     int interior_first = 0;     // LSM_B200_INTERIOR_FIRST (experiments): round-2's original launch order of the overlapped stage
-    std::vector<CflCacheEntry> cfl_cache;
-    std::vector<CflCand> cfl_cand;
+    std::vector<CflMemo> cfl_memo;
     int opt_cand = 1;           // LSM_OPT_CFL_CANDIDATES
     int opt_resident = 1;       // LSM_OPT_RESIDENT
     int stage_skip_zero_u = 0;  // transient: set by lsm_extend_along_normals around its stages (StageParams::skip_zero_u)
@@ -100,10 +100,6 @@ struct lsm_ctx {
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> timed;     // pending stage timings
     std::vector<cudaEvent_t> ev_pool;
     cudaEvent_t ev_user[8] = {};
-    // fused CFL (lsm_integrate only): request for the last stage of the current step, and its pending result
-    struct { bool on = false; double g_next = 0, tau = 0; } fuse_req;
-    struct { bool valid = false; const void* field = nullptr; uint64_t version = 0; double g = 0; } fused;
-    int opt_fuse_cfl = 1;
     int opt_graph = 1;          // lsm_integrate replays a captured CUDA graph of the stage launches on small grids
     // the mesh of the last lsm_interface_extract (persistent, grown on demand): nverts x ndim doubles, nverts keys, nprims x ndim int32
     void* d_iface = nullptr; size_t d_iface_bytes = 0;
@@ -172,7 +168,6 @@ int32_t ctx_common_init(lsm_ctx* c) {
     CU(cudaEventCreateWithFlags(&c->ev_halo, cudaEventDisableTiming));
     CU(cudaMalloc(&c->d_scalar, 64));
     CU(cudaMallocHost(&c->h_scalar, 64));
-    if (getenv("LSM_B200_NO_FUSE_CFL")) c->opt_fuse_cfl = 0;
     if (getenv("LSM_B200_NO_OVERLAP")) c->opt_overlap = 0;
     if (getenv("LSM_B200_INTERIOR_FIRST")) c->interior_first = 1;
     if (getenv("LSM_B200_NO_GRAPH")) c->opt_graph = 0;
@@ -464,25 +459,7 @@ int32_t run_stage_t(lsm_ctx* c, lsm_field* in, lsm_field* p0, lsm_field* out, ls
     for (int k = 0; k < nterms; ++k) TRY(make_term_dev(in, terms[k], term_scale(terms[k], tstage, gscale, k), &P.terms[k]));
     for (int k = 0; k < nterms; ++k)
         if (terms[k].coef_kind == LSM_COEF_EXPR) TRY(expr_ensure(terms[k].field, tstage, terms[k].kind, false));
-    P.cfl_out = nullptr; P.cfl_g = 0; P.cfl_tau = 0;
     P.skip_zero_u = c->stage_skip_zero_u;
-    if (c->fuse_req.on) {
-        c->fuse_req.on = false;
-        const TermDev& t0 = P.terms[0];
-        if (nterms == 1 && t0.kind == TERM_ADVECTION && t0.scheme == SCHEME_WENO5 && (t0.coef_kind == COEF_SEPARABLE || (t0.coef_kind == COEF_FIELD && !t0.coef_f64)) &&
-            c->opt_kernel != 1 && in->ndim == 3 && stage_tiled_supported<T>(in->ndim, P)) {
-            bool remap = true;      // the fused variant exists for the index-remap instantiation only
-            for (int d = 0; d < 3; ++d) for (int sd = 0; sd < 2; ++sd) if (P.in.bc[d][sd].kind == BC_EXTRAP && P.in.bc[d][sd].P > 0) remap = false;
-            if (!remap) goto no_fuse;
-            P.cfl_out = c->d_scalar + 1; P.cfl_g = c->fuse_req.g_next;
-            // the kernel's cheap estimate is sum_d |u_d| (|g_stage| / h_d), which it already forms for the Hamiltonian; the bound
-            // tau on sum_d |u_d g_next| / h_d therefore becomes tau |g_stage / g_next| (inf / NaN -> no candidates -> full pass)
-            P.cfl_tau = (1.0 - 1e-13) * c->fuse_req.tau * std::fabs((t0.scaled ? t0.g : 1.0) / c->fuse_req.g_next);
-            CU(cudaMemsetAsync(c->d_scalar + 1, 0, 8, c->stream));
-            c->fused.valid = true; c->fused.field = terms[0].field; c->fused.version = terms[0].field->version; c->fused.g = c->fuse_req.g_next;
-        }
-    no_fuse:;
-    }
 
     const int last = in->ndim - 1, nl = in->n[last];
     if (c->nranks > 1 && !in->halo_valid) {        // e.g. right after an upload
@@ -646,43 +623,42 @@ unsigned long long dbits(double s) {
     return b;
 }
 
-// max over the candidate tuples of the reference's per-node CFL quantity at scale g — the expression of cfl_kernel, operation
-// for operation (this translation unit is compiled without FMA contraction)
-unsigned long long cand_eval(const CflCand& e, const lsm_field* phi, double g) {
+// The reference's CFL quantity of one node with coefficient tuple v (ndim velocity components, or one scalar coefficient):
+// sum_d fl(|fl(v_d g)| / h_d) for advection (levelsetterms.jl:90-96), |fl(v g)| otherwise; an unscaled term takes v as it is.
+// The expression of cfl_kernel, operation for operation (this translation unit is compiled without FMA contraction).
+double cfl_node(int kind, const double* v, int ndim, const double* h, bool scaled, double g) {
+    if (kind != LSM_TERM_ADVECTION) return std::fabs(scaled ? v[0] * g : v[0]);
+    double acc = 0.0;
+    for (int d = 0; d < ndim; ++d) {
+        const double w = scaled ? v[d] * g : v[d];
+        const double q = std::fabs(w) / h[d];
+        acc = d == 0 ? q : acc + q;
+    }
+    return acc;
+}
+
+// max over the candidate tuples of the CFL quantity at scale g
+unsigned long long cand_eval(const CflMemo& e, const lsm_field* phi, double g) {
     unsigned long long best = 0ULL;
     const size_t n = e.tup.size() / e.ncomp;
     for (size_t k = 0; k < n; ++k) {
-        const double* v = &e.tup[k * e.ncomp];
-        double acc;
-        if (e.kind == LSM_TERM_ADVECTION) {
-            acc = 0.0;
-            for (int d = 0; d < e.ncomp; ++d) {
-                const double w = v[d] * g;
-                const double q = std::fabs(w) / phi->h[d];
-                acc = d == 0 ? q : acc + q;
-            }
-        } else {
-            acc = std::fabs(v[0] * g);
-        }
-        const unsigned long long b = dbits(acc);
+        const unsigned long long b = dbits(cfl_node(e.kind, &e.tup[k * e.ncomp], e.ncomp, phi->h, true, g));
         best = b > best ? b : best;
     }
     return best;
 }
 
-CflCand* cand_find(lsm_ctx* ctx, const lsm_term& t) {
-    for (auto& e : ctx->cfl_cand) if (e.kind == t.kind && e.field == t.field) return &e;
-    return nullptr;
+// the memo of (t.kind, t.field), created on first use and emptied when the field's data has changed since it was filled
+CflMemo& cfl_memo(lsm_ctx* ctx, const lsm_term& t) {
+    CflMemo* e = nullptr;
+    for (auto& m : ctx->cfl_memo) if (m.kind == t.kind && m.field == t.field) { e = &m; break; }
+    if (!e) { ctx->cfl_memo.emplace_back(); e = &ctx->cfl_memo.back(); }
+    if (e->field != t.field || e->version != t.field->version) { *e = CflMemo{}; e->kind = t.kind; e->field = t.field; e->version = t.field->version; }
+    return *e;
 }
 
-// the candidate set answers (or is about to answer) this term's CFL requests: the fused in-kernel reduction is not needed
-bool cand_pending_or_ready(lsm_ctx* ctx, const lsm_term& t) {
-    if (!ctx->opt_cand || !ctx->opt_cfl_cache || !t.field) return false;
-    const CflCand* e = cand_find(ctx, t);
-    return e && !e->overflow && e->version == t.field->version;
-}
-
-int32_t raw_cfl_pass(lsm_ctx* ctx, lsm_field* phi, const TermDev& td, unsigned long long* bits_out) {
+// one reduction pass over every owned node (all ranks), read back: the exact maximum as IEEE bits (see lsm_generic.cu K3)
+int32_t full_cfl_pass(lsm_ctx* ctx, lsm_field* phi, const TermDev& td, unsigned long long* bits_out) {
     CflParams P{};
     P.term = td;
     for (int d = 0; d < 3; ++d) { P.n[d] = phi->n[d]; P.h[d] = phi->h[d]; }
@@ -702,13 +678,13 @@ int32_t raw_cfl_pass(lsm_ctx* ctx, lsm_field* phi, const TermDev& td, unsigned l
 // Build the candidate set of a scaled coefficient field: one unscaled reduction (global maximum M), one extraction pass
 // (nodes with S_i >= (1 - 1e-12) M), one gather.  Multi-rank: every rank contributes a fixed-size segment of a zero-filled
 // buffer and the segments are concatenated with an all-reduce(sum) (x + 0 = x exactly), so all ranks hold the same set.
-int32_t cand_build(lsm_ctx* ctx, lsm_field* phi, const lsm_term& t, const TermDev& td_scaled, CflCand* e) {
+int32_t cand_build(lsm_ctx* ctx, lsm_field* phi, const lsm_term& t, const TermDev& td_scaled, CflMemo* e) {
     TermDev td = td_scaled;
     td.scaled = 0; td.g = 1.0;
     e->ncomp = t.kind == LSM_TERM_ADVECTION ? phi->ndim : 1;
     e->built = false; e->overflow = false; e->tup.clear();
     unsigned long long mb = 0;
-    TRY(raw_cfl_pass(ctx, phi, td, &mb));
+    TRY(full_cfl_pass(ctx, phi, td, &mb));
     double M; std::memcpy(&M, &mb, 8);
     const int R = ctx->nranks;
     const size_t seg = 1 + (size_t)CAND_CAP * e->ncomp;          // [count, tuples...] per rank
@@ -774,55 +750,20 @@ int32_t cand_build(lsm_ctx* ctx, lsm_field* phi, const lsm_term& t, const TermDe
 int32_t cfl_bits(lsm_ctx* ctx, lsm_field* phi, const lsm_term& t, double g, unsigned long long* bits_out) {
     TermDev td;
     TRY(make_term_dev(phi, t, g, &td));
+    CflMemo* e = nullptr;
     if (ctx->opt_cfl_cache && (t.coef_kind == LSM_COEF_FIELD || t.coef_kind == LSM_COEF_SEPARABLE)) {
-        for (const auto& e : ctx->cfl_cache)
-            if (e.kind == t.kind && e.field == t.field && e.version == t.field->version && e.scaled == td.scaled &&
-                (!td.scaled || e.g == g)) { *bits_out = e.bits; return LSM_OK; }
-    }
-    if (ctx->opt_cand && ctx->opt_cfl_cache && td.scaled && (t.coef_kind == LSM_COEF_FIELD || t.coef_kind == LSM_COEF_SEPARABLE)) {
-        // time-scaled static coefficient: the second request for the same data builds the candidate set, every later one is
-        // answered on the host (no kernel, no D2H, no sync)
-        CflCand* e = cand_find(ctx, t);
-        if (!e) { ctx->cfl_cand.emplace_back(); e = &ctx->cfl_cand.back(); e->kind = t.kind; e->field = t.field; e->version = ~0ULL; }
-        if (e->version != t.field->version) { e->version = t.field->version; e->seen = 0; e->built = false; e->overflow = false; e->tup.clear(); }
-        e->seen++;
-        if (!e->built && !e->overflow && e->seen >= 2) { ctx->fused.valid = false; TRY(cand_build(ctx, phi, t, td, e)); }
-        if (e->built && !e->overflow) { *bits_out = cand_eval(*e, phi, g); return LSM_OK; }
-    }
-    if (ctx->fused.valid) {
-        ctx->fused.valid = false;
-        if (ctx->fused.field == t.field && ctx->fused.version == t.field->version && td.scaled && ctx->fused.g == g && t.kind == LSM_TERM_ADVECTION) {
-            if (ctx->nranks > 1) NC(nccl().AllReduce(ctx->d_scalar + 1, ctx->d_scalar + 1, 1, ncclUint64, ncclMax, ctx->nccl_comm, ctx->stream));
-            CU(cudaMemcpyAsync(ctx->h_scalar + 1, ctx->d_scalar + 1, 8, cudaMemcpyDeviceToHost, ctx->stream));
-            CU(cudaStreamSynchronize(ctx->stream));
-            ctx->cnt.d2h_bytes += 8;
-            if (ctx->h_scalar[1] != 0ULL) {      // a candidate was found (always, see StageParams::cfl_tau); else fall through to the full pass
-                *bits_out = ctx->h_scalar[1];
-                for (auto& en : ctx->cfl_cache)
-                    if (en.kind == t.kind && en.field == t.field) en = {t.kind, t.field, t.field->version, g, td.scaled, *bits_out};
-                return LSM_OK;
-            }
+        e = &cfl_memo(ctx, t);
+        if (e->have_bits && e->scaled == td.scaled && (!td.scaled || e->g == g)) { *bits_out = e->bits; return LSM_OK; }
+        if (ctx->opt_cand && td.scaled) {
+            // time-scaled static coefficient: the second request for the same data builds the candidate set, every later one is
+            // answered on the host (no kernel, no D2H, no sync)
+            e->seen++;
+            if (!e->built && !e->overflow && e->seen >= 2) TRY(cand_build(ctx, phi, t, td, e));
+            if (e->built && !e->overflow) { *bits_out = cand_eval(*e, phi, g); return LSM_OK; }
         }
     }
-    CflParams P{};
-    P.term = td;
-    for (int d = 0; d < 3; ++d) { P.n[d] = phi->n[d]; P.h[d] = phi->h[d]; }
-    P.out = ctx->d_scalar;
-    CU(cudaMemsetAsync(ctx->d_scalar, 0, 8, ctx->stream));
-    cudaError_t e = launch_cfl(phi->ndim, phi->dtype == LSM_F64, P, ctx->sm_count, ctx->stream);
-    if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "CFL kernel launch failed: %s", cudaGetErrorString(e));
-    ctx->cnt.kernel_launches += 1; ctx->cnt.cfl_passes += 1;
-    if (ctx->nranks > 1) NC(nccl().AllReduce(ctx->d_scalar, ctx->d_scalar, 1, ncclUint64, ncclMax, ctx->nccl_comm, ctx->stream));
-    CU(cudaMemcpyAsync(ctx->h_scalar, ctx->d_scalar, 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    ctx->cnt.d2h_bytes += 8;
-    *bits_out = *ctx->h_scalar;
-    if (ctx->opt_cfl_cache && (t.coef_kind == LSM_COEF_FIELD || t.coef_kind == LSM_COEF_SEPARABLE)) {
-        bool replaced = false;
-        for (auto& en : ctx->cfl_cache)
-            if (en.kind == t.kind && en.field == t.field) { en = {t.kind, t.field, t.field->version, g, td.scaled, *bits_out}; replaced = true; }
-        if (!replaced) ctx->cfl_cache.push_back({t.kind, t.field, t.field->version, g, td.scaled, *bits_out});
-    }
+    TRY(full_cfl_pass(ctx, phi, td, bits_out));
+    if (e) { e->have_bits = true; e->scaled = td.scaled; e->g = g; e->bits = *bits_out; }
     return LSM_OK;
 }
 
@@ -854,17 +795,7 @@ int32_t cfl_term(lsm_ctx* ctx, lsm_field* phi, const lsm_term& t, double time, d
     const bool scaled = t.tscale_kind != LSM_TS_NONE;
     double m;     // max over nodes of sum_d |u_d|/h_d (advection) or of |coefficient| (normal, curvature)
     if (t.coef_kind == LSM_COEF_CONST) {
-        if (t.kind == LSM_TERM_ADVECTION) {
-            m = 0;
-            for (int d = 0; d < N; ++d) {
-                double v = t.cval[d]; if (scaled) v = v * g;
-                const double q = std::fabs(v) / phi->h[d];
-                m = d == 0 ? q : m + q;
-            }
-        } else {
-            double v = t.cval[0]; if (scaled) v = v * g;
-            m = std::fabs(v);
-        }
+        m = cfl_node(t.kind, t.cval, N, phi->h, scaled, g);
     } else if (t.coef_kind == LSM_COEF_EXPR) {
         unsigned long long bits = 0;
         TRY(expr_cfl_bits(ctx, t.field, time, t.kind, &bits));
@@ -1156,11 +1087,13 @@ int32_t lsm_set_option(lsm_ctx* c, int32_t option, int32_t value) {
     switch (option) {
         case LSM_OPT_KERNEL: if (value < 0 || value > 4) return fail(LSM_ERR_ARG, "LSM_OPT_KERNEL takes 0..4"); c->opt_kernel = value; break;
         case LSM_OPT_TIME_STAGES: c->opt_time = value != 0; break;
-        case LSM_OPT_CFL_CACHE: c->opt_cfl_cache = value != 0; c->cfl_cache.clear(); c->cfl_cand.clear(); break;
-        case LSM_OPT_CFL_CANDIDATES: c->opt_cand = value != 0; c->cfl_cand.clear(); break;
+        case LSM_OPT_CFL_CACHE: c->opt_cfl_cache = value != 0; c->cfl_memo.clear(); break;
+        case LSM_OPT_CFL_CANDIDATES:
+            c->opt_cand = value != 0;
+            for (auto& e : c->cfl_memo) { e.ncomp = 0; e.seen = 0; e.built = false; e.overflow = false; e.tup.clear(); }
+            break;
         case LSM_OPT_RESIDENT: c->opt_resident = value != 0; break;
         case LSM_OPT_OVERLAP: c->opt_overlap = value != 0; break;
-        case LSM_OPT_FUSE_CFL: c->opt_fuse_cfl = value != 0; break;
         case LSM_OPT_GRAPH: c->opt_graph = value != 0; break;
         default: return fail(LSM_ERR_ARG, "unknown option %d", option);
     }
@@ -1283,12 +1216,9 @@ int32_t lsm_field_destroy(lsm_field* f) {
     cudaSetDevice(f->ctx->device);
     cudaStreamSynchronize(f->ctx->stream);
     cudaStreamSynchronize(f->ctx->comm);
-    // drop CFL cache entries that point at this field
-    auto& cc = f->ctx->cfl_cache;
-    for (size_t i = 0; i < cc.size();) { if (cc[i].field == f) cc.erase(cc.begin() + i); else ++i; }
-    auto& cd = f->ctx->cfl_cand;
-    for (size_t i = 0; i < cd.size();) { if (cd[i].field == f) cd.erase(cd.begin() + i); else ++i; }
-    if (f->ctx->fused.field == f) f->ctx->fused.valid = false;       // a new field at the same address must not consume a stale fused maximum
+    // drop the CFL memos of this field: a new field at the same address must not find them
+    auto& cm = f->ctx->cfl_memo;
+    for (size_t i = 0; i < cm.size();) { if (cm[i].field == f) cm.erase(cm.begin() + i); else ++i; }
     field_free(f);
     return LSM_OK;
 }
@@ -1553,20 +1483,7 @@ int32_t lsm_integrate(lsm_ctx* ctx, int32_t integrator, double cfl, lsm_field* p
         uint64_t vb[3] = {phi->version, phi->buf1 ? phi->buf1->version : 0, phi->buf2 ? phi->buf2->version : 0};
         if (capture && cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) { cudaGetLastError(); graph_ok = false; }
         const bool capturing = capture && graph_ok;
-        for (int s = 1; s <= nstages(integrator) && rc == LSM_OK; ++s) {
-            if (s == nstages(integrator) && ctx->opt_fuse_cfl && ctx->opt_cfl_cache && nterms == 1 && terms[0].kind == LSM_TERM_ADVECTION &&
-                (terms[0].coef_kind == LSM_COEF_FIELD || terms[0].coef_kind == LSM_COEF_SEPARABLE) && terms[0].tscale_kind == LSM_TS_COS && (tc + dt) <= tf - jl_eps(tc + dt) &&
-                !cand_pending_or_ready(ctx, terms[0])) {
-                // next step's CFL maximum from this stage's velocity traffic: max(g') >= (1 - 1e-13) * max(g) * |g'/g|
-                for (const auto& en : ctx->cfl_cache)
-                    if (en.kind == terms[0].kind && en.field == terms[0].field && en.version == terms[0].field->version && en.scaled && en.g != 0.0) {
-                        const double gn = term_scale(terms[0], tc + dt, nullptr, 0);
-                        ctx->fuse_req.on = true; ctx->fuse_req.g_next = gn;
-                        ctx->fuse_req.tau = (1.0 - 1e-13) * bits_to_double(en.bits) * std::fabs(gn / en.g);
-                    }
-            }
-            rc = stage_impl(ctx, integrator, s, phi, terms, nterms, tc, dt, nullptr);
-        }
+        for (int s = 1; s <= nstages(integrator) && rc == LSM_OK; ++s) rc = stage_impl(ctx, integrator, s, phi, terms, nterms, tc, dt, nullptr);
         if (capturing) {
             cudaGraph_t graph = nullptr;
             cudaError_t ge = cudaStreamEndCapture(ctx->stream, &graph);
@@ -1592,7 +1509,6 @@ int32_t lsm_integrate(lsm_ctx* ctx, int32_t integrator, double cfl, lsm_field* p
         tc += dt;
         ++steps;
     }
-    ctx->fuse_req.on = false;        // a request left behind by a failed stage must not leak into a later lsm_stage
     if (gexec) { cudaStreamSynchronize(ctx->stream); cudaGraphExecDestroy(gexec); }
     cudaStreamSynchronize(ctx->comm);
     cudaError_t e = cudaStreamSynchronize(ctx->stream);

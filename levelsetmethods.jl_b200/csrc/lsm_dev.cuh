@@ -62,11 +62,8 @@ struct StageParams {
     int r0, r1;          // range [r0, r1) of the LAST dimension to update (interior/boundary split)
     int skip_zero_u;     // upwind advection: a component with u_d == 0 contributes exactly 0 even when its one-sided difference is
     int _pad1;           // NaN / Inf (extend_along_normals!: frozen nodes keep their value, velocityextension.jl:53-56)
-    // Fused CFL for the NEXT step (single stored-velocity advection term whose time factor changes every step): the last
-    // stage also reduces max_nodes sum_d |u_d * cfl_g| / h_d.  Exact: only nodes whose cheap estimate reaches cfl_tau (a lower
-    // bound of the new maximum derived from the previous exact maximum) evaluate the reference expression with true divisions.
-    unsigned long long* cfl_out;   // device scalar (IEEE bits, atomicMax) or nullptr
-    double cfl_g, cfl_tau;         // g(t_next); candidate bound on the kernel's estimate sum_d |u_d| |g_stage| / h_d
+    double _pad2;        // keeps terms[] 8 bytes past a 16-byte boundary: that alignment decides which of its fields the stage
+                         // kernels fetch in pairs with 128-bit constant loads, and so the code they compile to
     TermDev terms[4];
 };
 

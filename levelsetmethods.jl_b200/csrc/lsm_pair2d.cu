@@ -305,7 +305,6 @@ template <class T>
 cudaError_t launch_stage_pair2d(const StageParams<T>& P, const AuxList& A, cudaStream_t s, bool force, int sm_count) {
     if (pair_kernel_disabled() || tma_disabled() || !encode_tiled_fn()) return cudaErrorNotSupported;
     if (P.nterms != 1 && P.nterms != 2) return cudaErrorNotSupported;
-    if (P.cfl_out) return cudaErrorNotSupported;
     const TermDev& ta = P.terms[0];
     if (ta.kind != TERM_ADVECTION || ta.scheme != SCHEME_WENO5 || ta.coef_kind != COEF_FIELD || ta.coef_f64 || A.first[0] != 0) return cudaErrorNotSupported;
     const bool curv = P.nterms == 2;

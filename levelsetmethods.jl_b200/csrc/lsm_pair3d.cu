@@ -87,8 +87,8 @@ __device__ __forceinline__ void pair_eval_n(const WenoK& K, const double (&a)[7]
 constexpr int PAIR_EIK = 100;    // value of the CK template parameter that selects the Eikonal variant
 
 // CK: COEF_FIELD (stored velocity, staged by TMA next to the phi ring) or COEF_SEPARABLE (u_d = s_d X_d[i] Y_d[j] Z_d[k] from tables).
-// SB: static RK base mode (SB_* of lsm_tile_util.cuh).  FCFL: also reduce the next step's CFL maximum (see StageParams).
-template <class T, int RY, int NT, int CK, bool FCFL, int SB, bool ISO, bool XMAX, bool HASN>
+// SB: static RK base mode (SB_* of lsm_tile_util.cuh).
+template <class T, int RY, int NT, int CK, int SB, bool ISO, bool XMAX, bool HASN>
 __global__ void __launch_bounds__(NT, 2)
 pair3d_kernel(const __grid_constant__ StageParams<T> P, const __grid_constant__ AuxList A, const __grid_constant__ TmaMaps M, const int cz) {
     using G = PairGeom<T, RY, NT>;
@@ -104,8 +104,8 @@ pair3d_kernel(const __grid_constant__ StageParams<T> P, const __grid_constant__ 
     constexpr int AU = HASN ? 1 : 0;                       // first velocity tile
     constexpr int NVEL = EIK ? 1 : (CK == COEF_FIELD ? 3 : 0) + AU;  // tiles before phi^n
     constexpr int NAUX = NVEL + (HAS_P0 ? 1 : 0);
-    static_assert(!HASN || (CK == COEF_FIELD && !FCFL && sizeof(T) == 8 && RY == 1), "the two-term variant is Float64, stored coefficients");
-    static_assert(!EIK || (!HASN && !FCFL && RY == 1), "the Eikonal variant is a single term without fused CFL");
+    static_assert(!HASN || (CK == COEF_FIELD && sizeof(T) == 8 && RY == 1), "the two-term variant is Float64, stored coefficients");
+    static_assert(!EIK || (!HASN && RY == 1), "the Eikonal variant is a single term");
     constexpr unsigned PHI_BYTES = (unsigned)(W * G::HH * sizeof(T));
     constexpr unsigned AUX_BYTES = (unsigned)(NAUX * TILE * sizeof(T));
 
@@ -192,7 +192,6 @@ pair3d_kernel(const __grid_constant__ StageParams<T> P, const __grid_constant__ 
     const double gih[3] = {g * (1.0 / P.h[0]), g * (1.0 / P.h[1]), g * (1.0 / P.h[2])};
     // ISO (equal mesh size in the three dimensions, the usual case): sum_d (u_d g / h) W_d = (g / h) sum_d u_d W_d, so the per-
     // dimension scaling (3 DMUL per node) folds into the stage coefficient: x -= (c g / h) * sum_d u_d W_d.
-    const double tau = ISO ? P.cfl_tau / fabs(gih[0]) * (1.0 - 1e-15) : P.cfl_tau;      // candidate bound on the unscaled estimate (ISO)
     const double cH = ISO ? P.c * gih[0] : P.c, cH2 = ISO ? P.c2 * gih[0] : P.c2;
     const double cN = ISO ? P.c * (1.0 / P.h[0]) : P.c, cN2 = ISO ? P.c2 * (1.0 / P.h[0]) : P.c2;     // normal term: sqrt(sum / h^2) = sqrt(sum) / h
     auto scl = [&](double u, int d) -> double { return ISO ? u : u * gih[d]; };
@@ -210,7 +209,6 @@ pair3d_kernel(const __grid_constant__ StageParams<T> P, const __grid_constant__ 
     }
     const WenoK KR = weno_regs<XMAX>(A.wk);
     long lin = (long)i + (long)j0 * vs1 + (long)zbeg * vs2;       // output / phi^n element offset of node (i, j0, z)
-    unsigned long long cfl_best = 0ULL;
 
     mbar_wait(bar, 0);
     unsigned phase = 1;
@@ -306,7 +304,6 @@ pair3d_kernel(const __grid_constant__ StageParams<T> P, const __grid_constant__ 
             }
         } else if (act[0]) {
             double H[RY][2];
-            double uraw[RY][2][3];
             V2 cc[RY];
             // normal-motion term (HASN): speed of the two nodes, which Godunov norm it selects, and the accumulated squares
             double vn[RY][2], gn[RY][2];
@@ -345,7 +342,6 @@ pair3d_kernel(const __grid_constant__ StageParams<T> P, const __grid_constant__ 
                     const V2 u = lds_pair(auxz + (AU * TILE + r * G::BX) * ES, T());
                     ua = double(u.x); ub = double(u.y);
                 } else { ua = pxy[r][0][0] * __ldg(P.terms[TA].tab[0][2] + z); ub = pxy[r][1][0] * __ldg(P.terms[TA].tab[0][2] + z); }
-                uraw[r][0][0] = ua; uraw[r][1][0] = ub;
                 double wa, wb;
                 evalp(a, b, ua, ub, 0, r, wa, wb);
                 H[r][0] = scl(ua, 0) * wa;
@@ -363,7 +359,6 @@ pair3d_kernel(const __grid_constant__ StageParams<T> P, const __grid_constant__ 
                         const V2 uu = lds_pair(auxz + ((AU + 1) * TILE + r * G::BX) * ES, T());
                         u[r][0] = double(uu.x); u[r][1] = double(uu.y);
                     } else { u[r][0] = pxy[r][0][1] * __ldg(P.terms[TA].tab[1][2] + z); u[r][1] = pxy[r][1][1] * __ldg(P.terms[TA].tab[1][2] + z); }
-                    uraw[r][0][1] = u[r][0]; uraw[r][1][1] = u[r][1];
                 }
                 if (RY == 1) {
                     const T a[7] = {yv[0].x, yv[1].x, yv[2].x, yv[3].x, yv[4].x, yv[5].x, yv[6].x};
@@ -400,7 +395,6 @@ pair3d_kernel(const __grid_constant__ StageParams<T> P, const __grid_constant__ 
                     const V2 u = lds_pair(auxz + ((AU + 2) * TILE + r * G::BX) * ES, T());
                     ua = double(u.x); ub = double(u.y);
                 } else { ua = pxy[r][0][2] * __ldg(P.terms[TA].tab[2][2] + z); ub = pxy[r][1][2] * __ldg(P.terms[TA].tab[2][2] + z); }
-                uraw[r][0][2] = ua; uraw[r][1][2] = ub;
                 double wa, wb;
                 evalp(a, b, ua, ub, 2, r, wa, wb);
                 H[r][0] = fma(scl(ua, 2), wa, H[r][0]);
@@ -444,25 +438,6 @@ pair3d_kernel(const __grid_constant__ StageParams<T> P, const __grid_constant__ 
                     o2.y = T(fma(-cH2, H[r][1], double(x2[1])));
                     *reinterpret_cast<V2*>(P.out2 + lin + r * vs1) = o2;
                 }
-                if (FCFL) {
-#pragma unroll
-                    for (int c = 0; c < 2; ++c) {
-                        // cheap estimate sum_d |u_d| |g_stage| / h_d against the candidate bound; candidates evaluate the reference
-                        // expression bit for bit (levelsetterms.jl:90-96)
-                        const double sest = ISO ? (fabs(uraw[r][c][0]) + fabs(uraw[r][c][1])) + fabs(uraw[r][c][2])
-                                                : (fabs(uraw[r][c][0] * gih[0]) + fabs(uraw[r][c][1] * gih[1])) + fabs(uraw[r][c][2] * gih[2]);
-                        if (!(sest < tau)) {
-                            double sx = 0.0;
-#pragma unroll
-                            for (int d = 0; d < 3; ++d) {
-                                const double q = __ddiv_rn(fabs(__dmul_rn(uraw[r][c][d], P.cfl_g)), P.h[d]);
-                                sx = d == 0 ? q : __dadd_rn(sx, q);
-                            }
-                            const unsigned long long bits = isnan(sx) ? 0x7FF8000000000000ULL : (unsigned long long)__double_as_longlong(sx);
-                            cfl_best = bits > cfl_best ? bits : cfl_best;
-                        }
-                    }
-                }
             }
         }
         if (fix) {
@@ -483,14 +458,6 @@ pair3d_kernel(const __grid_constant__ StageParams<T> P, const __grid_constant__ 
         ab = ABUF - ab;
         lin += vs2;
     }
-    if (FCFL) {
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const unsigned long long other = __shfl_xor_sync(0xffffffffu, cfl_best, o);
-            cfl_best = other > cfl_best ? other : cfl_best;
-        }
-        if ((tid & 31) == 0 && cfl_best) atomicMax(P.cfl_out, cfl_best);
-    }
 }
 
 #ifndef LSM_PAIR_RY
@@ -498,11 +465,11 @@ pair3d_kernel(const __grid_constant__ StageParams<T> P, const __grid_constant__ 
 #define LSM_PAIR_NT 256
 #endif
 
-template <class T, int CK, bool FCFL, int SB, bool ISO, bool XMAX, bool HASN = false>
+template <class T, int CK, int SB, bool ISO, bool XMAX, bool HASN = false>
 cudaError_t launch_pair_x(const StageParams<T>& P, const AuxList& A, cudaStream_t s) {
     constexpr int RY = LSM_PAIR_RY, NT = LSM_PAIR_NT;
     using G = PairGeom<T, RY, NT>;
-    auto kern = pair3d_kernel<T, RY, NT, CK, FCFL, SB, ISO, XMAX, HASN>;
+    auto kern = pair3d_kernel<T, RY, NT, CK, SB, ISO, XMAX, HASN>;
     constexpr bool HAS_P0 = SB == SB_S2 || SB == SB_S3 || SB == SB_P0;
     constexpr int NAUX = (CK == PAIR_EIK ? 1 : (CK == COEF_FIELD ? 3 : 0) + (HASN ? 1 : 0)) + (HAS_P0 ? 1 : 0);
     const size_t smem = G::smem_bytes(NAUX);
@@ -530,28 +497,28 @@ cudaError_t launch_pair_x(const StageParams<T>& P, const AuxList& A, cudaStream_
     return cudaGetLastError();
 }
 
-template <class T, int CK, bool FCFL, int SB, bool HASN>
+template <class T, int CK, int SB, bool HASN>
 cudaError_t launch_pair(const StageParams<T>& P, const AuxList& A, cudaStream_t s, bool exact_eps) {
-    if constexpr (CK == PAIR_EIK) return launch_pair_x<T, CK, FCFL, SB, false, false, false>(P, A, s);
+    if constexpr (CK == PAIR_EIK) return launch_pair_x<T, CK, SB, false, false, false>(P, A, s);
     const bool iso = P.h[0] == P.h[1] && P.h[1] == P.h[2];
     if (sizeof(T) == 4 || !exact_eps)      // (the Float32 evaluation normalises by the exact FP32 maximum either way)
-        return iso ? launch_pair_x<T, CK, FCFL, SB, true, false, HASN>(P, A, s) : launch_pair_x<T, CK, FCFL, SB, false, false, HASN>(P, A, s);
+        return iso ? launch_pair_x<T, CK, SB, true, false, HASN>(P, A, s) : launch_pair_x<T, CK, SB, false, false, HASN>(P, A, s);
     if constexpr (sizeof(T) == 8)
-        return iso ? launch_pair_x<T, CK, FCFL, SB, true, true, HASN>(P, A, s) : launch_pair_x<T, CK, FCFL, SB, false, true, HASN>(P, A, s);
+        return iso ? launch_pair_x<T, CK, SB, true, true, HASN>(P, A, s) : launch_pair_x<T, CK, SB, false, true, HASN>(P, A, s);
     return cudaErrorNotSupported;
 }
 
-template <class T, int CK, bool FCFL, bool HASN = false>
+template <class T, int CK, bool HASN = false>
 cudaError_t launch_pair_sb(const StageParams<T>& P, const AuxList& A, cudaStream_t s, bool exact_eps) {
     constexpr int SP0 = CK == PAIR_EIK ? 1 : (CK == COEF_FIELD ? 3 : 0) + (HASN ? 1 : 0);
     if (A.p0 >= 0 && A.p0 != SP0) return cudaErrorNotSupported;
     if (P.base == BASE_IN && !P.p0) {
-        if (!P.out2) return launch_pair<T, CK, FCFL, SB_IN, HASN>(P, A, s, exact_eps);
-        if (!FCFL) return launch_pair<T, CK, false, SB_IN_OUT2, HASN>(P, A, s, exact_eps);
+        if (!P.out2) return launch_pair<T, CK, SB_IN, HASN>(P, A, s, exact_eps);
+        return launch_pair<T, CK, SB_IN_OUT2, HASN>(P, A, s, exact_eps);
     }
-    if (P.base == BASE_RK3_S2 && P.p0 && !P.out2 && !FCFL) return launch_pair<T, CK, false, SB_S2, HASN>(P, A, s, exact_eps);
-    if (P.base == BASE_RK3_S3 && P.p0 && !P.out2) return launch_pair<T, CK, FCFL, SB_S3, HASN>(P, A, s, exact_eps);
-    if (P.base == BASE_P0 && P.p0 && !P.out2) return launch_pair<T, CK, FCFL, SB_P0, HASN>(P, A, s, exact_eps);
+    if (P.base == BASE_RK3_S2 && P.p0 && !P.out2) return launch_pair<T, CK, SB_S2, HASN>(P, A, s, exact_eps);
+    if (P.base == BASE_RK3_S3 && P.p0 && !P.out2) return launch_pair<T, CK, SB_S3, HASN>(P, A, s, exact_eps);
+    if (P.base == BASE_P0 && P.p0 && !P.out2) return launch_pair<T, CK, SB_P0, HASN>(P, A, s, exact_eps);
     return cudaErrorNotSupported;
 }
 
@@ -564,7 +531,7 @@ cudaError_t launch_stage_pair3d(const StageParams<T>& P, const AuxList& A, cudaS
     if (pair_kernel_disabled() || tma_disabled() || !encode_tiled_fn()) return cudaErrorNotSupported;
     if (P.nterms != 1 && P.nterms != 2) return cudaErrorNotSupported;
     const TermDev& ta = P.terms[P.nterms - 1];          // the advection term (last)
-    const bool eik = P.nterms == 1 && ta.kind == TERM_EIKONAL && ta.coef_kind == COEF_FIELD && !ta.coef_f64 && A.first[0] == 0 && !P.cfl_out;
+    const bool eik = P.nterms == 1 && ta.kind == TERM_EIKONAL && ta.coef_kind == COEF_FIELD && !ta.coef_f64 && A.first[0] == 0;
     if (!eik && (ta.kind != TERM_ADVECTION || ta.scheme != SCHEME_WENO5)) return cudaErrorNotSupported;
     const View<T>& v = P.in;
     if ((v.n[0] * sizeof(T)) % 16 != 0 || v.n[0] < 8 || v.n[1] < 8 || v.n[2] < 4) return cudaErrorNotSupported;
@@ -575,21 +542,19 @@ cudaError_t launch_stage_pair3d(const StageParams<T>& P, const AuxList& A, cudaS
             const bool index_map = b.kind == BC_PERIODIC || b.kind == BC_SYMMETRY || (b.kind == BC_EXTRAP && b.P == 0) || (b.kind == BC_HALO && d == 2);
             if (!index_map) return cudaErrorNotSupported;
         }
-    if (eik) return launch_pair_sb<T, PAIR_EIK, false>(P, A, s, exact_eps);
+    if (eik) return launch_pair_sb<T, PAIR_EIK>(P, A, s, exact_eps);
     if (P.nterms == 2) {
-        // (NormalMotionTerm(stored speed), AdvectionTerm(stored velocity)) in this order, Float64, no fused CFL
+        // (NormalMotionTerm(stored speed), AdvectionTerm(stored velocity)) in this order, Float64
         if constexpr (sizeof(T) == 8) {
             const TermDev& tn = P.terms[0];
             if (tn.kind != TERM_NORMAL || tn.coef_kind != COEF_FIELD || tn.coef_f64 != 0 || A.first[0] != 0) return cudaErrorNotSupported;
-            if (ta.coef_kind != COEF_FIELD || ta.coef_f64 != 0 || A.first[1] != 1 || P.cfl_out) return cudaErrorNotSupported;
-            return launch_pair_sb<T, COEF_FIELD, false, true>(P, A, s, exact_eps);
+            if (ta.coef_kind != COEF_FIELD || ta.coef_f64 != 0 || A.first[1] != 1) return cudaErrorNotSupported;
+            return launch_pair_sb<T, COEF_FIELD, true>(P, A, s, exact_eps);
         }
         return cudaErrorNotSupported;
     }
-    if (ta.coef_kind == COEF_FIELD && A.first[0] == 0 && !ta.coef_f64)
-        return P.cfl_out ? launch_pair_sb<T, COEF_FIELD, true>(P, A, s, exact_eps) : launch_pair_sb<T, COEF_FIELD, false>(P, A, s, exact_eps);
-    if (ta.coef_kind == COEF_SEPARABLE)
-        return P.cfl_out ? launch_pair_sb<T, COEF_SEPARABLE, true>(P, A, s, exact_eps) : launch_pair_sb<T, COEF_SEPARABLE, false>(P, A, s, exact_eps);
+    if (ta.coef_kind == COEF_FIELD && A.first[0] == 0 && !ta.coef_f64) return launch_pair_sb<T, COEF_FIELD>(P, A, s, exact_eps);
+    if (ta.coef_kind == COEF_SEPARABLE) return launch_pair_sb<T, COEF_SEPARABLE>(P, A, s, exact_eps);
     return cudaErrorNotSupported;
 }
 

@@ -38,7 +38,8 @@ namespace {
 #endif
 #ifndef LSM_MINB_EIK
 #define LSM_MINB_EIK 3    // Eikonal kernel: latency-bound at 16 warps/SM (ncu: 'wait' + short-scoreboard stalls lead); 3 blocks of 74 KB fit.
-                          // Also the Float32 advection kernels (45 KB each; the fused-CFL variant otherwise takes 84 registers -> 2 blocks)
+                          // Also the single-term Float32 WENO advection kernels: 45 KB each, so 3 blocks fit and the bound keeps their
+                          // registers from ruling that out
 #endif
 
 template <class T, int NDIM, int TX, int TY, int NY>
@@ -63,7 +64,7 @@ struct TileGeom {
 // Fused stage kernel.  MASK = which term kinds the instantiation carries code for; the terms themselves
 // (order, coefficients) are runtime data, applied one after the other like the reference
 // (x = base; x -= c*H_1; x -= c*H_2; ..., timestepping.jl:128-202).
-template <class T, int NDIM, int MASK, int NTS, int COEFK, bool REMAP, bool FCFL, int TX, int TY, int NY, int MINB, int TK, int SB>
+template <class T, int NDIM, int MASK, int NTS, int COEFK, bool REMAP, int TX, int TY, int NY, int MINB, int TK, int SB>
 __global__ void __launch_bounds__(TX * TY, (NDIM == 2 ? LSM_MINB_2D
                                                    : ((MASK == M_EIK && TK >= 0) || (sizeof(T) == 4 && MASK == M_ADV_WENO && NTS == 1) ? LSM_MINB_EIK : MINB)))
 stage_tiled_kernel(const __grid_constant__ StageParams<T> P, const __grid_constant__ AuxList A, const __grid_constant__ TmaMaps M, const int cz) {
@@ -209,8 +210,6 @@ stage_tiled_kernel(const __grid_constant__ StageParams<T> P, const __grid_consta
             for (int d = 0; d < NDIM; ++d) pxy[k][d] = (P.terms[0].cval[d] * __ldg(P.terms[0].tab[d][0] + ii)) * __ldg(P.terms[0].tab[d][1] + jj);
         }
     }
-    unsigned long long cfl_best = 0ULL;                       // fused CFL: this thread's exact maximum (IEEE bits)
-    constexpr bool do_cfl = FCFL;        // separate instantiation: the lean kernel carries none of this code
     int s0 = 0;        // ring slot of plane z - HAL
     int ab = 0;        // aux buffer of plane z
     // element offsets of the ring slots of planes z-3 .. z+3 (block-uniform); shifted by one entry per plane
@@ -333,11 +332,9 @@ stage_tiled_kernel(const __grid_constant__ StageParams<T> P, const __grid_consta
                         // levelsetterms.jl:73-82 : H = sum_d u_d * weno(d) = sum_d (|u_d| / h_d) * W_d, left to right
                         const double g = tm.scaled ? tm.g : 1.0;
                         const int ghi = __double2hiint(g);
-                        double uu[3] = {0, 0, 0}, sest = 0.0;
 #pragma unroll
                         for (int d = 0; d < NDIM; ++d) {
                             const double u = coef_raw(tm, kk, d, kc);             // velocity before the time factor g(t)
-                            if (do_cfl) uu[d] = u;
                             // v = u*g; v > 0 selects the minus-biased stencil.  sign(v) = sign(u)*sign(g); |v|/h = |u| * (|g|/h)
                             // s from the sign bits (integer ops instead of 8 DSETP): when u*g == 0 the reference takes the plus-biased
                             // stencil but multiplies it by zero, so either ordering yields the same 0 contribution (a == 0).
@@ -347,19 +344,7 @@ stage_tiled_kernel(const __grid_constant__ StageParams<T> P, const __grid_consta
                             const double w = (NDIM == 2 || !ONE) ? weno5_up_f64<T>(A.wk, up(d, -3, s), up(d, -2, s), up(d, -1, s), qc, up(d, 1, s), up(d, 2, s))
                                                                  : weno5_up<T>(A.wk, up(d, -3, s), up(d, -2, s), up(d, -1, s), qc, up(d, 1, s), up(d, 2, s));
                             const double a = fabs(u) * (fabs(g) * ih[d]);
-                            if (do_cfl) sest = d == 0 ? a : sest + a;       // = sum_d |u_d| |g_stage| / h_d, compared with tau |g_stage / g_next|
                             H = d == 0 ? a * w : fma(a, w, H);
-                        }
-                        if (do_cfl && !(sest < P.cfl_tau)) {
-                            // candidate for the maximum: the reference expression, bit for bit (levelsetterms.jl:90-96)
-                            double sx = 0.0;
-#pragma unroll
-                            for (int d = 0; d < NDIM; ++d) {
-                                const double q = __ddiv_rn(fabs(__dmul_rn(uu[d], P.cfl_g)), P.h[d]);
-                                sx = d == 0 ? q : __dadd_rn(sx, q);
-                            }
-                            const unsigned long long bits = isnan(sx) ? 0x7FF8000000000000ULL : (unsigned long long)__double_as_longlong(sx);
-                            cfl_best = bits > cfl_best ? bits : cfl_best;
                         }
                     } else if ((MASK & M_ADV_UPWIND) && k_upw) {
 #pragma unroll
@@ -457,14 +442,6 @@ stage_tiled_kernel(const __grid_constant__ StageParams<T> P, const __grid_consta
             for (int k = 0; k < NY; ++k) lin_k[k] += vs2;
         }
     }
-    if (do_cfl) {
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const unsigned long long other = __shfl_xor_sync(0xffffffffu, cfl_best, o);
-            cfl_best = other > cfl_best ? other : cfl_best;
-        }
-        if (lane == 0 && cfl_best) atomicMax(P.cfl_out, cfl_best);
-    }
 }
 
 #ifndef LSM_MINB_2D
@@ -478,11 +455,11 @@ stage_tiled_kernel(const __grid_constant__ StageParams<T> P, const __grid_consta
 #endif
 
 
-template <class T, int NDIM, int MASK, int NTS, int COEFK, bool REMAP, bool FCFL = false, int TK = -1, int SB = -1>
+template <class T, int NDIM, int MASK, int NTS, int COEFK, bool REMAP, int TK = -1, int SB = -1>
 cudaError_t launch_tiled(const StageParams<T>& P, const AuxList& A, cudaStream_t s) {
     constexpr int TX = LSM_TX, TY = LSM_TY, NY = LSM_NY;
     using G = TileGeom<T, NDIM, TX, TY, NY>;
-    auto kern = stage_tiled_kernel<T, NDIM, MASK, NTS, COEFK, REMAP, FCFL, TX, TY, NY, LSM_MINB, TK, SB>;
+    auto kern = stage_tiled_kernel<T, NDIM, MASK, NTS, COEFK, REMAP, TX, TY, NY, LSM_MINB, TK, SB>;
     const size_t smem = G::smem_bytes(A.n);
     static size_t attr_smem[16] = {};
     { cudaError_t e = ensure_dyn_smem(kern, smem, attr_smem); if (e != cudaSuccess) return e; }
@@ -512,21 +489,20 @@ cudaError_t launch_tiled(const StageParams<T>& P, const AuxList& A, cudaStream_t
 
 // Static-signature kernels also fix the RK base mode at compile time (5 legal combinations of BASE_* and out2); anything
 // unexpected (phi^n staged in another aux slot) takes the runtime-base instantiation.
-template <class T, int NDIM, int MASK, int NTS, int COEFK, bool REMAP, bool FCFL, int TK>
+template <class T, int NDIM, int MASK, int NTS, int COEFK, bool REMAP, int TK>
 cudaError_t launch_static(const StageParams<T>& P, const AuxList& A, cudaStream_t s) {
     constexpr int SP0 = TK >= 0 ? sig_first(TK, COEFK, NTS, NDIM) : (COEFK == COEF_FIELD ? NDIM : 0);
     const bool p0_ok = A.p0 < 0 || A.p0 == SP0;
     if (p0_ok) {
         if (P.base == BASE_IN && !P.p0) {
-            if (!P.out2) return launch_tiled<T, NDIM, MASK, NTS, COEFK, REMAP, FCFL, TK, SB_IN>(P, A, s);
-            if (!FCFL) return launch_tiled<T, NDIM, MASK, NTS, COEFK, REMAP, false, TK, SB_IN_OUT2>(P, A, s);
+            if (!P.out2) return launch_tiled<T, NDIM, MASK, NTS, COEFK, REMAP, TK, SB_IN>(P, A, s);
+            return launch_tiled<T, NDIM, MASK, NTS, COEFK, REMAP, TK, SB_IN_OUT2>(P, A, s);
         }
-        if (P.base == BASE_RK3_S2 && P.p0 && !P.out2 && !FCFL) return launch_tiled<T, NDIM, MASK, NTS, COEFK, REMAP, false, TK, SB_S2>(P, A, s);
-        if (P.base == BASE_RK3_S3 && P.p0 && !P.out2) return launch_tiled<T, NDIM, MASK, NTS, COEFK, REMAP, FCFL, TK, SB_S3>(P, A, s);
-        if (P.base == BASE_P0 && P.p0 && !P.out2) return launch_tiled<T, NDIM, MASK, NTS, COEFK, REMAP, FCFL, TK, SB_P0>(P, A, s);
+        if (P.base == BASE_RK3_S2 && P.p0 && !P.out2) return launch_tiled<T, NDIM, MASK, NTS, COEFK, REMAP, TK, SB_S2>(P, A, s);
+        if (P.base == BASE_RK3_S3 && P.p0 && !P.out2) return launch_tiled<T, NDIM, MASK, NTS, COEFK, REMAP, TK, SB_S3>(P, A, s);
+        if (P.base == BASE_P0 && P.p0 && !P.out2) return launch_tiled<T, NDIM, MASK, NTS, COEFK, REMAP, TK, SB_P0>(P, A, s);
     }
-    // (cannot happen with the aux list launch_stage_tiled builds; the all-terms kernel handles anything, and a requested fused CFL
-    //  that is not delivered makes the host fall back to the separate reduction pass)
+    // (cannot happen with the aux list launch_stage_tiled builds; the all-terms kernel handles anything)
     return launch_tiled<T, NDIM, M_ALL, 0, -1, REMAP>(P, A, s);
 }
 
@@ -537,15 +513,9 @@ cudaError_t launch_by_mask(int mask, const StageParams<T>& P, const AuxList& A, 
             case M_ADV_WENO:
                 if (P.nterms == 1) {
                     const TermDev& t0 = P.terms[0];
-                    if (t0.coef_kind == COEF_FIELD && A.first[0] == 0) {
-                        if (NDIM == 3 && P.cfl_out) return launch_static<T, NDIM, M_ADV_WENO, 1, COEF_FIELD, REMAP, true, -1>(P, A, s);
-                        return launch_static<T, NDIM, M_ADV_WENO, 1, COEF_FIELD, REMAP, false, -1>(P, A, s);
-                    }
-                    if (t0.coef_kind == COEF_SEPARABLE) {
-                        if (NDIM == 3 && P.cfl_out) return launch_static<T, NDIM, M_ADV_WENO, 1, COEF_SEPARABLE, REMAP, true, -1>(P, A, s);
-                        return launch_static<T, NDIM, M_ADV_WENO, 1, COEF_SEPARABLE, REMAP, false, -1>(P, A, s);
-                    }
-                    if (t0.coef_kind == COEF_CONST) return launch_static<T, NDIM, M_ADV_WENO, 1, COEF_CONST, REMAP, false, -1>(P, A, s);
+                    if (t0.coef_kind == COEF_FIELD && A.first[0] == 0) return launch_static<T, NDIM, M_ADV_WENO, 1, COEF_FIELD, REMAP, -1>(P, A, s);
+                    if (t0.coef_kind == COEF_SEPARABLE) return launch_static<T, NDIM, M_ADV_WENO, 1, COEF_SEPARABLE, REMAP, -1>(P, A, s);
+                    if (t0.coef_kind == COEF_CONST) return launch_static<T, NDIM, M_ADV_WENO, 1, COEF_CONST, REMAP, -1>(P, A, s);
                 }
                 break;
             // static signatures (term kinds, coefficient kinds and aux-tile slots known at compile time) for the BASELINE
@@ -553,8 +523,8 @@ cudaError_t launch_by_mask(int mask, const StageParams<T>& P, const AuxList& A, 
             case M_EIK:
                 if (P.nterms == 1) {
                     const TermDev& t0 = P.terms[0];
-                    if (t0.coef_kind == COEF_FIELD && A.first[0] == 0) return launch_static<T, NDIM, M_EIK, 1, COEF_FIELD, REMAP, false, SK_EIK>(P, A, s);
-                    if (t0.coef_kind == COEF_NONE) return launch_static<T, NDIM, M_EIK, 1, COEF_NONE, REMAP, false, SK_EIK>(P, A, s);
+                    if (t0.coef_kind == COEF_FIELD && A.first[0] == 0) return launch_static<T, NDIM, M_EIK, 1, COEF_FIELD, REMAP, SK_EIK>(P, A, s);
+                    if (t0.coef_kind == COEF_NONE) return launch_static<T, NDIM, M_EIK, 1, COEF_NONE, REMAP, SK_EIK>(P, A, s);
                     return launch_tiled<T, NDIM, M_EIK, 1, -1, REMAP>(P, A, s);
                 }
                 break;
@@ -562,7 +532,7 @@ cudaError_t launch_by_mask(int mask, const StageParams<T>& P, const AuxList& A, 
                 if (P.nterms == 2) {
                     const TermDev &t0 = P.terms[0], &t1 = P.terms[1];
                     if (t0.kind == TERM_NORMAL && t0.coef_kind == COEF_FIELD && A.first[0] == 0 && t1.coef_kind == COEF_FIELD && A.first[1] == 1)
-                        return launch_static<T, NDIM, M_NORMAL | M_ADV_WENO, 2, COEF_FIELD | (COEF_FIELD << 2), REMAP, false, SK_NORMAL | (SK_ADV_WENO << 3)>(P, A, s);
+                        return launch_static<T, NDIM, M_NORMAL | M_ADV_WENO, 2, COEF_FIELD | (COEF_FIELD << 2), REMAP, SK_NORMAL | (SK_ADV_WENO << 3)>(P, A, s);
                     return launch_tiled<T, NDIM, M_NORMAL | M_ADV_WENO, 2, -1, REMAP>(P, A, s);
                 }
                 break;
@@ -570,7 +540,7 @@ cudaError_t launch_by_mask(int mask, const StageParams<T>& P, const AuxList& A, 
                 if (P.nterms == 2) {
                     const TermDev &t0 = P.terms[0], &t1 = P.terms[1];
                     if (t0.kind == TERM_ADVECTION && t0.coef_kind == COEF_FIELD && A.first[0] == 0 && t1.coef_kind == COEF_CONST)
-                        return launch_static<T, NDIM, M_ADV_WENO | M_CURV, 2, COEF_FIELD | (COEF_CONST << 2), REMAP, false, SK_ADV_WENO | (SK_CURV << 3)>(P, A, s);
+                        return launch_static<T, NDIM, M_ADV_WENO | M_CURV, 2, COEF_FIELD | (COEF_CONST << 2), REMAP, SK_ADV_WENO | (SK_CURV << 3)>(P, A, s);
                     return launch_tiled<T, NDIM, M_ADV_WENO | M_CURV, 2, -1, REMAP>(P, A, s);
                 }
                 break;
@@ -639,7 +609,7 @@ cudaError_t launch_stage_tiled(int ndim, const StageParams<T>& P, int sm_count, 
     return remap ? launch_by_mask<T, 2, true>(mask, P, A, s) : launch_by_mask<T, 2, false>(mask, P, A, s);
 }
 
-// The Makefile compiles this file twice (-DLSM_TILED_F32 / -DLSM_TILED_F64) so that the two halves of the ~180 kernel
+// The Makefile compiles this file twice (-DLSM_TILED_F32 / -DLSM_TILED_F64) so that the two halves of the ~160 kernel
 // instantiations build in parallel; without either macro both are instantiated here.
 #if !defined(LSM_TILED_F64)
 template bool stage_tiled_supported<float>(int, const StageParams<float>&);

@@ -37,7 +37,7 @@ def main():
     # thinner slabs fall back to the strict kernel, which is bit-equal to the oracle but not to the tiled kernel
     nc = max(24, 10 * world)
     cases = []
-    c = H.c3_enright(nc); cases.append(("C3 WENO5 advection x cos (fused CFL), Neumann", c, "RK3", 8))
+    c = H.c3_enright(nc); cases.append(("C3 WENO5 advection x cos (CFL candidates), Neumann", c, "RK3", 8))
     c = H.c5_normal_advection(nc); cases.append(("C5 normal motion + advection", c, "RK3", 6))
     c = H.c4_eikonal(nc); cases.append(("C4 eikonal RK2", c, "RK2", 6))
     # 2-D, decomposed along y: on 2 ranks every slab is large enough for the 2-D x-pair kernel (rows arrive through the halo rows)

@@ -423,11 +423,11 @@ def test_pair_kernel_kinked_body_parity(m, O):
 
 def test_cfl_candidates_are_exact(m, O):
     """Time-scaled static coefficients: from the third CFL request on, the maximum is evaluated on the HOST over the candidate
-    nodes (lsm_api.cu, CflCand) — no reduction pass, no D2H, no sync per step.  It must be bit-identical to the full reduction
+    nodes (lsm_api.cu, CflMemo) — no reduction pass, no D2H, no sync per step.  It must be bit-identical to the full reduction
     (LSM_OPT_CFL_CANDIDATES = 0) for every scale: stored and separable velocity, both dtypes, a scalar speed, a field of ties
-    (constant velocity stored as a field: the candidate list overflows and the regular path answers), and whole integrations
+    (constant velocity stored as a field: the candidate list overflows and the full pass answers), and whole integrations
     must take the same steps and produce the same bits."""
-    OPT_FUSE, OPT_CAND = 4, 6
+    OPT_CAND = 6
     ctx = m.default_context()
     cases = [H.c3_enright(40), H.c3_enright(40, separable=True), H.c3_enright(32, np.float32), H.c1_circle_rotation(96)]
     cases[3].terms[0]["cos_period"] = 2.0
@@ -456,17 +456,17 @@ def test_cfl_candidates_are_exact(m, O):
         ctx.set_option(OPT_CAND, opt)
         ref.append([m.compute_cfl((term,), phi, t) for t in ts])
     assert ref[0] == ref[1]
-    # whole integrations: identical step counts, times and states with and without candidates (and without the fused CFL)
+    # whole integrations: identical step counts, times and states with and without candidates
     for case in (H.c3_enright(40), H.c3_enright(40, separable=True)):
         outs = []
-        for cand, fuse in ((1, 1), (0, 1), (0, 0)):
-            ctx.set_option(OPT_CAND, cand); ctx.set_option(OPT_FUSE, fuse)
+        for cand in (1, 0):
+            ctx.set_option(OPT_CAND, cand)
             phi = case.engine_field(m)
             eq = m.LevelSetEquation(terms=case.engine_terms(m, phi), ic=phi, integrator=m.RK3())
             ctx.reset_counters()
             m.integrate(eq, 0.25)
             outs.append((eq.t, eq.steps_taken, eq.state.peek().copy(), ctx.counters()))
-        ctx.set_option(OPT_CAND, 1); ctx.set_option(OPT_FUSE, 1)
+        ctx.set_option(OPT_CAND, 1)
         assert outs[0][1] > 12
         for o in outs[1:]:
             assert o[:2] == outs[0][:2] and np.array_equal(o[2], outs[0][2])
@@ -883,18 +883,20 @@ def test_graph_replay_is_invisible(m, O):
 
 @pytest.mark.parametrize("integ", ["RK3", "RK2", "FE"])
 def test_counters_and_launch_accounting(m, integ):
-    """Launch accounting of the three ways the per-step CFL maximum of a time-scaled velocity is obtained, for all three
-    integrators (all exact, so the states are bit-identical): (a) default — host evaluation over the candidate nodes: one
+    """Launch accounting of the two ways the per-step CFL maximum of a time-scaled velocity is obtained, for all three
+    integrators (both exact, so the states are bit-identical): (a) default — host evaluation over the candidate nodes: one
     reduction for the first step, the unscaled reduction + one extraction kernel when the set is built, nothing afterwards;
-    (b) candidates off — the last stage of every step reduces the next step's maximum (fused-CFL instantiations: RK3 S3,
-    RK2 corrector, ForwardEuler); (c) both off — one reduction pass per step."""
+    (b) candidates off, which is also what a field with more ties at the maximum than the candidate list holds gets — one
+    reduction pass per step.  Option 4 (the retired next-step reduction in the last stage) is refused."""
     ctx = m.default_context()
+    with pytest.raises(m.LSMError) as ei:
+        ctx.set_option(4, 0)
+    assert ei.value.code == m._lib.ERR_ARG
     case = H.c3_enright(32)
     mk, nst = {"RK3": (m.RK3, 3), "RK2": (m.RK2, 2), "FE": (m.ForwardEuler, 1)}[integ]
     results = []
-    for cand, fuse in ((1, 1), (0, 1), (0, 0)):
+    for cand in (1, 0):
         ctx.set_option(m._lib.OPT_CFL_CANDIDATES, cand)
-        ctx.set_option(m._lib.OPT_FUSE_CFL, fuse)
         phi = case.engine_field(m)
         eq = m.LevelSetEquation(terms=case.engine_terms(m, phi), ic=phi, integrator=mk())
         eq.state.device()
@@ -907,11 +909,8 @@ def test_counters_and_launch_accounting(m, integ):
         if cand:
             assert c["cfl_passes"] == 2 and c["kernel_launches"] == c["stage_launches"] + 3
         else:
-            assert c["cfl_passes"] == (1 if fuse else eq.steps_taken)
+            assert c["cfl_passes"] == eq.steps_taken
             assert c["kernel_launches"] == c["stage_launches"] + c["cfl_passes"]
         results.append((eq.t, eq.steps_taken, eq.state.peek().copy()))
-    ctx.set_option(m._lib.OPT_FUSE_CFL, 1)
     ctx.set_option(m._lib.OPT_CFL_CANDIDATES, 1)
-    assert results[0][:2] == results[2][:2] and np.array_equal(results[0][2], results[2][2])
-    # the fused reduction is exact: identical step sizes, hence bit-identical states
     assert results[0][:2] == results[1][:2] and np.array_equal(results[0][2], results[1][2])

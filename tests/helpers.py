@@ -37,6 +37,25 @@ class Case:
         """A term's stored coefficient, in its own ``field_dtype`` when it sets one (a Float64 field with a Float32 state)."""
         return np.asfortranarray(t["field"].astype(t.get("field_dtype", self.dtype)))
 
+    # the keys each term kind understands; anything else raises, so that a spec is never dropped silently
+    TERM_KEYS = {
+        "advection": {"kind", "field", "const", "separable", "scheme", "cos_period", "field_dtype"},
+        "normal": {"kind", "field", "const", "cos_period", "field_dtype"},
+        "curvature": {"kind", "field", "const", "cos_period", "field_dtype"},
+        "eikonal": {"kind", "frozen"},
+    }
+
+    def check_term(self, t):
+        k = t.get("kind")
+        if k not in self.TERM_KEYS:
+            raise ValueError(f"unknown term kind {k!r}")
+        extra = set(t) - self.TERM_KEYS[k]
+        if extra:
+            raise ValueError(f"{k} term: unknown key(s) {sorted(extra)}")
+        if k != "eikonal" and sum(c in t for c in ("field", "const", "separable")) != 1:
+            raise ValueError(f"{k} term needs exactly one of field, const, separable")
+        return k
+
     # ---- oracle side ----
     def oracle_bc(self):
         def one(b):
@@ -52,11 +71,11 @@ class Case:
     def oracle_terms(self, s0=None):
         out = []
         for t in self.terms:
-            k = t["kind"]
+            k = self.check_term(t)
+            ts = O.TS_COS if "cos_period" in t else O.TS_NONE
+            tp = t.get("cos_period", 1.0)
             if k == "advection":
                 sch = O.UPWIND if t.get("scheme") == "upwind" else O.WENO5
-                ts = O.TS_COS if "cos_period" in t else O.TS_NONE
-                tp = t.get("cos_period", 1.0)
                 if "separable" in t:
                     sc, tabs = t["separable"]
                     out.append(O.advection_separable(sc, tabs, scheme=sch, tscale=ts, tparam=tp))
@@ -64,11 +83,13 @@ class Case:
                     out.append(O.advection(self.coef_field(t), scheme=sch, tscale=ts, tparam=tp))
                 else:
                     out.append(O.advection(t["const"], scheme=sch, tscale=ts, tparam=tp))
-            elif k == "normal":
-                out.append(O.normal_motion(self.coef_field(t) if "field" in t else t["const"]))
-            elif k == "curvature":
-                out.append(O.curvature(self.coef_field(t) if "field" in t else t["const"]))
-            elif k == "eikonal":
+            elif k in ("normal", "curvature"):
+                kind = O.TERM_NORMAL if k == "normal" else O.TERM_CURVATURE
+                if "field" in t:
+                    out.append(O.Term(kind, coef_kind=O.COEF_FIELD, field=self.coef_field(t), tscale=ts, tparam=tp))
+                else:
+                    out.append(O.Term(kind, coef_kind=O.COEF_CONST, cval=(t["const"],), tscale=ts, tparam=tp))
+            else:
                 if t.get("frozen", True):
                     out.append(O.eikonal(O.eikonal_s0(self.oracle_field()) if s0 is None else s0))
                 else:
@@ -100,27 +121,25 @@ class Case:
         out = []
         g = phi.mesh
         for t in self.terms:
-            k = t["kind"]
-            if k == "advection":
-                sch = m.Upwind() if t.get("scheme") == "upwind" else m.WENO5()
-                if "separable" in t:
-                    sc, tabs = t["separable"]
-                    base = m.SeparableVelocity(g, sc, tabs, ctx=ctx)
-                elif "field" in t:
-                    base = m.MeshField(self.coef_field(t), g, ctx=ctx)
-                else:
-                    base = tuple(t["const"])
-                if "cos_period" in t:
-                    base = m.TimeScaled(base, ("cos", t["cos_period"]))
-                out.append(m.AdvectionTerm(base, sch))
-            elif k == "normal":
-                v = m.MeshField(self.coef_field(t), g, ctx=ctx) if "field" in t else t["const"]
-                out.append(m.NormalMotionTerm(v))
-            elif k == "curvature":
-                b = m.MeshField(self.coef_field(t), g, ctx=ctx) if "field" in t else t["const"]
-                out.append(m.CurvatureTerm(b))
-            elif k == "eikonal":
+            k = self.check_term(t)
+            if k == "eikonal":
                 out.append(m.EikonalReinitializationTerm(phi) if t.get("frozen", True) else m.EikonalReinitializationTerm())
+                continue
+            if "separable" in t:
+                sc, tabs = t["separable"]
+                base = m.SeparableVelocity(g, sc, tabs, ctx=ctx)
+            elif "field" in t:
+                base = m.MeshField(self.coef_field(t), g, ctx=ctx)
+            else:
+                base = tuple(t["const"]) if k == "advection" else t["const"]
+            if "cos_period" in t:
+                base = m.TimeScaled(base, ("cos", t["cos_period"]))
+            if k == "advection":
+                out.append(m.AdvectionTerm(base, m.Upwind() if t.get("scheme") == "upwind" else m.WENO5()))
+            elif k == "normal":
+                out.append(m.NormalMotionTerm(base))
+            else:
+                out.append(m.CurvatureTerm(base))
         return tuple(out)
 
 

@@ -67,8 +67,8 @@ enum {
 /* time factor g(t) multiplying the coefficient (device-side stand-in for update_func / f(x,t)) */
 enum { LSM_TS_NONE = 0, LSM_TS_COS = 1 /* cos(pi t / tparam) */, LSM_TS_HOST = 2 /* caller passes g per call */ };
 
-/* timestepping.jl:26-28,46-48,65-67 */
-enum { LSM_FORWARD_EULER = 0, LSM_RK2 = 1, LSM_RK3 = 2 };
+/* timestepping.jl:26-28,46-48,65-67; LSM_SEMI_IMPLICIT: see "semi-implicit advection" below */
+enum { LSM_FORWARD_EULER = 0, LSM_RK2 = 1, LSM_RK3 = 2, LSM_SEMI_IMPLICIT = 3 };
 
 typedef struct lsm_ctx lsm_ctx;
 typedef struct lsm_field lsm_field;
@@ -95,12 +95,15 @@ typedef struct {
     int64_t timed_stages;
     int64_t pair_launches;    /* stage launches that took the x-pair kernel (3-D single-term WENO5 advection)  */
     int64_t resident_steps;   /* time steps taken inside the resident cluster kernel (small 2-D grids; one launch per lsm_integrate) */
+    int64_t jacobi_sweeps;    /* Jacobi sweeps of LSM_SEMI_IMPLICIT steps (k per step, see lsm_semi_implicit_sweeps)          */
 } lsm_counters;
 
 /* options for lsm_set_option */
 enum {
     LSM_OPT_KERNEL = 0,       /* 0 auto (x-pair / tiled where available), 1 force generic strict kernel, 2 force tiled / x-pair, 3 tiled without the x-pair kernel,
-                                 4 x-pair kernel with the exact WENO epsilon maximum (bit-identical to 3; default is a 20-bit maximum) */
+                                 4 x-pair kernel with the exact WENO epsilon maximum (bit-identical to 3; default is a 20-bit maximum).
+                                 LSM_SEMI_IMPLICIT: 2 runs the temporally blocked Jacobi sweeps, every other value one sweep per launch
+                                 (the faster form on a B200, see DESIGN.md 4.6); the two are bit-identical */
     LSM_OPT_TIME_STAGES = 1,  /* 1: bracket every stage launch with CUDA events, resolved at the next sync  */
     LSM_OPT_CFL_CACHE = 2,    /* 1 (default): reuse the CFL reduction while coefficient data/scale unchanged  */
     LSM_OPT_OVERLAP = 3,      /* 1 (default): overlap halo exchange with interior compute (multi-rank)        */
@@ -203,7 +206,7 @@ int32_t lsm_field_stage_buffer(lsm_field* phi, int32_t which, lsm_field** out);
  * over ranks.  gscale: per-term g for LSM_TS_HOST terms (may be NULL).  LSM_ERR_CFL unless dt > 0. */
 int32_t lsm_compute_cfl(lsm_ctx* ctx, lsm_field* phi, const lsm_term* terms, int32_t nterms, double t,
                         const double* gscale, double* dt_out);
-/* Number of stages of an integrator (1, 2, 3). */
+/* Number of stages of an integrator (1, 2, 3; 1 for LSM_SEMI_IMPLICIT). */
 int32_t lsm_nstages(int32_t integrator);
 /* One stage (1-based) of _advance! (timestepping.jl:128-137,143-164,170-202), so that a host can
  * run update_term! callbacks between stages like the reference does.  Asynchronous. */
@@ -218,6 +221,31 @@ int32_t lsm_advance(lsm_ctx* ctx, int32_t integrator, lsm_field* phi, const lsm_
 int32_t lsm_integrate(lsm_ctx* ctx, int32_t integrator, double cfl, lsm_field* phi, const lsm_term* terms,
                       int32_t nterms, double t0, double tf, double dt_max, int64_t max_steps,
                       double* t_out, int64_t* steps_out);
+
+/* ---- semi-implicit advection: LSM_SEMI_IMPLICIT, inflow implicit / outflow explicit ----------------------------------------
+ * An integrator for ONE AdvectionTerm phi_t + u.grad phi = 0 that stays stable at Courant numbers above 1, in the idea of the
+ * reference's SemiImplicitI2OE (not bit for bit: the two are different restatements of the scheme).  A step dt from tc:
+ *  - the velocity is taken at t* = tc + dt/2 (any coefficient kind: const, field, separable, time-scaled, expression); the
+ *    term's scheme tag is ignored;
+ *  - for each node I and dimension d: c_d = dt u_d(I, t*) / h_d, a_d = |c_d| / 2, s_d = +1 if c_d > 0 else -1 (zero or NaN: -1);
+ *  - (1 + sum_d a_d) x_I - sum_d a_d x_{I - s_d e_d} = phi_I - sum_d a_d (phi_{I + s_d e_d} - phi_I), sums left to right over d;
+ *    off-grid reads on both sides are the field's BC-aware reads (meshfield.jl:213-260) applied to the unknown too;
+ *  - phi^{n+1} = x after k Jacobi sweeps x_I <- (r_I + sum_d a_d x_{I - s_d e_d}) / (1 + sum_d a_d) from x = r, with k =
+ *    lsm_semi_implicit_sweeps(C, dtype), C = dt / compute_cfl(terms, phi, t*) = max_I sum_d |c_d| (up to rounding): no reduction, copy to the
+ *    host or synchronisation inside the solve.  The CFL evaluation at t* that fixes k is answered on the host for constant,
+ *    stored and separable velocities (the CFL memo) and for time-scaled ones once their candidate set is built (the second step);
+ *    an expression velocity that uses t, or any velocity with LSM_OPT_CFL_CACHE = 0, costs one reduction, an 8-byte copy and a
+ *    synchronisation per step there, as its CFL at tc does (for an expression the reduction is part of the fill the step needs
+ *    anyway).  Float32 states: differences in float, the rest in double, rounded on store.
+ * lsm_stage (stage 1), lsm_advance and lsm_integrate run whole steps; lsm_integrate takes dt = min(dt_max, cfl * compute_cfl at
+ * tc, tf - tc) like the explicit integrators (cfl 2 in the Python and Julia wrappers) and never uses its CUDA-graph or resident
+ * paths for it.  The stage buffers of phi hold r and the second iterate.  Refused: more than one term or a term that is not
+ * advection (LSM_ERR_ARG); ExtrapolationBC with P >= 1 (LSM_ERR_UNSUPPORTED: negative ghost weights); an axis with fewer than 2
+ * nodes (LSM_ERR_ARG); nranks > 1 (LSM_ERR_UNSUPPORTED, slab decomposition is not supported). */
+/* Pure host function (no GPU needed): the Jacobi sweeps of a semi-implicit step at Courant number C >= 0 (finite), k =
+ * max(1, ceil(log(tol) / log(q))), q = (C/2) / (1 + C/2) the contraction factor of a sweep, tol = 1e-15 (LSM_F64) or 1e-8
+ * (LSM_F32); k = 1 when q = 0.  More than 2^24 sweeps: LSM_ERR_ARG. */
+int32_t lsm_semi_implicit_sweeps(double courant, int32_t dtype, int64_t* sweeps_out);
 
 /* EikonalReinitializationTerm(phi0) constructor (levelsetterms.jl:217-221): dst = phi0/sqrt(phi0^2+min(h)^2). */
 int32_t lsm_eikonal_s0(lsm_field* dst, const lsm_field* phi0);

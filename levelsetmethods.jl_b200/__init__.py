@@ -10,7 +10,7 @@ from ._lib import LSMError, CFLError, TimeError, BCError, build
 from .api import (Context, MultiContext, integrate_multi, compute_cfl_multi, default_context, set_default_context, CartesianGrid, BoundaryCondition, PeriodicBC,
                   ExtrapolationBC, NeumannBC, LinearExtrapolationBC, SymmetryBC, MeshField, Upwind, WENO5,
                   TimeScaled, DeviceExpr, SeparableVelocity, LevelSetTerm, AdvectionTerm, CurvatureTerm, NormalMotionTerm,
-                  EikonalReinitializationTerm, update_term, compute_cfl, step_plan, TimeIntegrator, ForwardEuler, RK2, RK3,
+                  EikonalReinitializationTerm, update_term, compute_cfl, step_plan, TimeIntegrator, ForwardEuler, RK2, RK3, SemiImplicit, semi_implicit_sweeps,
                   LevelSetEquation, current_state, current_time, integrate, integrate_bang, volume, perimeter, eikonal_reinitialize, extend_along_normals,
                   InterfaceMesh, extract_interface, merge_interfaces, extract_interface_multi, redistance, extend_closest_point,
                   CubicInterpolation, interpolate, LevelSetIntegrals, level_set_integrals, level_set_integrals_multi,

@@ -22,7 +22,7 @@ UPWIND, WENO5 = 0, 1
 COEF_CONST, COEF_FIELD, COEF_SEPARABLE, COEF_NONE, COEF_EXPR = 0, 1, 2, 3, 4
 TS_NONE, TS_COS, TS_HOST = 0, 1, 2
 SHAPE_SPHERE, SHAPE_BOX, SHAPE_PLANE, SHAPE_CONST = 0, 1, 2, 3
-FORWARD_EULER, RK2, RK3 = 0, 1, 2
+FORWARD_EULER, RK2, RK3, SEMI_IMPLICIT = 0, 1, 2, 3
 OPT_KERNEL, OPT_TIME_STAGES, OPT_CFL_CACHE, OPT_OVERLAP, OPT_GRAPH, OPT_CFL_CANDIDATES, OPT_RESIDENT = 0, 1, 2, 3, 5, 6, 7
 MAX_TERMS = 4
 
@@ -40,7 +40,7 @@ class lsm_counters(C.Structure):
     _fields_ = [("kernel_launches", C.c_int64), ("stage_launches", C.c_int64), ("cfl_passes", C.c_int64),
                 ("h2d_bytes", C.c_int64), ("d2h_bytes", C.c_int64), ("halo_bytes_sent", C.c_int64),
                 ("last_stage_ms", C.c_double), ("sum_stage_ms", C.c_double), ("timed_stages", C.c_int64),
-                ("pair_launches", C.c_int64), ("resident_steps", C.c_int64)]
+                ("pair_launches", C.c_int64), ("resident_steps", C.c_int64), ("jacobi_sweeps", C.c_int64)]
 
 
 class LSMError(RuntimeError):
@@ -108,6 +108,7 @@ SYMBOLS = {
     "lsm_advance": (_i32, [_vp, _i32, _vp, C.POINTER(lsm_term), _i32, _dbl, _dbl]),
     "lsm_integrate": (_i32, [_vp, _i32, _dbl, _vp, C.POINTER(lsm_term), _i32, _dbl, _dbl, _dbl, _i64, _pdbl,
                              C.POINTER(_i64)]),
+    "lsm_semi_implicit_sweeps": (_i32, [_dbl, _i32, C.POINTER(_i64)]),
     "lsm_eikonal_s0": (_i32, [_vp, _vp]),
     "lsm_volume": (_i32, [_vp, _vp, _pdbl]),
     "lsm_perimeter": (_i32, [_vp, _vp, _pdbl]),

@@ -853,7 +853,27 @@ class RK3(TimeIntegrator):
     code, nstages = L.RK3, 3
 
 
+class SemiImplicit(TimeIntegrator):
+    """Inflow-implicit / outflow-explicit steps of ONE AdvectionTerm (``LSM_SEMI_IMPLICIT``, include/lsm_b200.h): second order and
+    stable above Courant number 1, so it takes ``cfl`` = 2 by default, four times RK3's steps of 0.5.  The idea of the reference's
+    ``SemiImplicitI2OE``, not its bits.  The velocity is taken at mid-step, the implicit half is solved with a fixed number of
+    Jacobi sweeps on the device (``semi_implicit_sweeps``)."""
+    code, nstages = L.SEMI_IMPLICIT, 1
+
+    def __init__(self, cfl: float = 2.0):
+        super().__init__(cfl)
+
+
+def semi_implicit_sweeps(courant: float, dtype=np.float64) -> int:
+    """Jacobi sweeps of a semi-implicit step at Courant number ``courant`` (``lsm_semi_implicit_sweeps``; no GPU needed)."""
+    k = C.c_int64()
+    L.check(L.lib().lsm_semi_implicit_sweeps(float(courant), L.F64 if np.dtype(dtype) == np.float64 else L.F32, C.byref(k)))
+    return k.value
+
+
 def _stage_times(integ: TimeIntegrator, tc: float, dt: float):
+    if isinstance(integ, SemiImplicit):
+        return [tc + 0.5 * dt]           # the velocity of a semi-implicit step is taken at mid-step
     if isinstance(integ, ForwardEuler):
         return [tc]
     if isinstance(integ, RK2):
@@ -863,7 +883,7 @@ def _stage_times(integ: TimeIntegrator, tc: float, dt: float):
 
 def _stage_inputs(integ: TimeIntegrator, phi: MeshField):
     """The field each stage differentiates (what ``update_term!`` receives, timestepping.jl:131,146,157,173,186,197)."""
-    if isinstance(integ, ForwardEuler):
+    if isinstance(integ, (ForwardEuler, SemiImplicit)):
         return [phi]
     h1, h2 = C.c_void_p(), C.c_void_p()
     L.check(L.lib().lsm_field_stage_buffer(phi.device(), 1, C.byref(h1)))

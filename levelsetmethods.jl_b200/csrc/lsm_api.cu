@@ -522,6 +522,9 @@ int32_t check_state(lsm_ctx* ctx, lsm_field* phi, const lsm_term* terms, int nte
     return LSM_OK;
 }
 
+// LSM_SEMI_IMPLICIT: one whole step (below, after the CFL code it uses)
+int32_t si_step(lsm_ctx* ctx, lsm_field* phi, const lsm_term* terms, int nterms, double tc, double dt, const double* gs);
+
 int32_t stage_impl(lsm_ctx* ctx, int integ, int stage, lsm_field* phi, const lsm_term* terms, int nterms, double tc, double dt, const double* gs) {
     switch (integ) {
         case LSM_FORWARD_EULER:      // timestepping.jl:128-137
@@ -541,11 +544,14 @@ int32_t stage_impl(lsm_ctx* ctx, int integ, int stage, lsm_field* phi, const lsm
             if (stage == 2) return run_stage(ctx, phi->buf1, phi, phi->buf2, nullptr, BASE_RK3_S2, 0.25 * dt, 0, terms, nterms, tc + dt, gs, true);
             if (stage == 3) return run_stage(ctx, phi->buf2, phi, phi, nullptr, BASE_RK3_S3, (2.0 / 3.0) * dt, 0, terms, nterms, tc + 0.5 * dt, gs, true);
             return fail(LSM_ERR_ARG, "RK3 has 3 stages");
+        case LSM_SEMI_IMPLICIT:
+            if (stage != 1) return fail(LSM_ERR_ARG, "the semi-implicit integrator has 1 stage (a whole step)");
+            return si_step(ctx, phi, terms, nterms, tc, dt, gs);
         default: return fail(LSM_ERR_ARG, "bad integrator %d", integ);
     }
 }
 
-int nstages(int integ) { return integ == LSM_FORWARD_EULER ? 1 : integ == LSM_RK2 ? 2 : 3; }
+int nstages(int integ) { return integ == LSM_FORWARD_EULER || integ == LSM_SEMI_IMPLICIT ? 1 : integ == LSM_RK2 ? 2 : 3; }
 
 // The step sizes of the time loop for a CONSTANT CFL step dt_cfl (static coefficients), replayed with the loop's own arithmetic
 // (timestepping.jl:104-118): while t <= tf - eps(t): dt = min(dt_max, cfl * dt_cfl, tf - t); t += dt.  Run-length encoded; stops
@@ -840,6 +846,66 @@ int32_t check_level_set(lsm_ctx* ctx, const lsm_field* phi, const char* what, in
     if (single_rank && ctx->nranks > 1)
         return fail(LSM_ERR_UNSUPPORTED, "%s: slab decomposition is not supported (nranks = %d)", what, ctx->nranks);
     return LSM_OK;
+}
+
+// ---- LSM_SEMI_IMPLICIT (lsm_semi_implicit.cu) ------------------------------------------------------------------------------
+// Jacobi sweeps for Courant number C: q = (C/2) / (1 + C/2) is the contraction of one sweep, k = ceil(log tol / log q)
+int32_t si_sweeps(double courant, int dtype, int64_t* k) {
+    if (!(courant >= 0.0 && std::isfinite(courant))) return fail(LSM_ERR_ARG, "semi-implicit step: the Courant number must be finite and >= 0 (got %g)", courant);
+    const double q = (courant / 2) / (1 + courant / 2);
+    const double tol = dtype == LSM_F64 ? 1e-15 : 1e-8;
+    const double n = q > 0.0 ? std::ceil(std::log(tol) / std::log(q)) : 1.0;
+    constexpr double cap = double(1 << 24);
+    if (!(n <= cap)) return fail(LSM_ERR_ARG, "semi-implicit step: Courant number %g needs more than %.0f Jacobi sweeps", courant, cap);
+    *k = std::max<int64_t>(1, (int64_t)n);
+    return LSM_OK;
+}
+
+int32_t si_check(lsm_ctx* ctx, const lsm_field* phi, const lsm_term* terms, int nterms) {
+    TRY(check_level_set(ctx, phi, "the semi-implicit integrator", 2, true));
+    if (nterms != 1 || terms[0].kind != LSM_TERM_ADVECTION)
+        return fail(LSM_ERR_ARG, "the semi-implicit integrator takes exactly one AdvectionTerm (got %d terms, the first of kind %d)", nterms, terms[0].kind);
+    for (int d = 0; d < phi->ndim; ++d)
+        for (int sd = 0; sd < 2; ++sd)
+            if (phi->bc[d][sd].kind == LSM_BC_EXTRAP && phi->bc[d][sd].P >= 1)
+                return fail(LSM_ERR_UNSUPPORTED, "the semi-implicit integrator does not support ExtrapolationBC{%d} (dimension %d, %s side): its "
+                            "ghost weights are negative, so the implicit system is not an M-matrix", phi->bc[d][sd].P, d + 1, sd ? "right" : "left");
+    return LSM_OK;
+}
+
+// One step: r = the explicit outflow half into buf1, then k Jacobi sweeps from x = r, alternating between buf2 and phi so that
+// the last one lands in phi (phi^n is not read after the right-hand side).
+template <class T>
+int32_t si_step_t(lsm_ctx* ctx, lsm_field* phi, const lsm_term& t, double tc, double dt, const double* gs) {
+    NvtxRange nvtx("lsm semi-implicit step");
+    const double ts = tc + 0.5 * dt;
+    double dt_cfl;
+    TRY(compute_cfl_impl(ctx, phi, &t, 1, ts, gs, &dt_cfl));     // also materialises an expression velocity at t*
+    int64_t k;
+    TRY(si_sweeps(dt / dt_cfl, phi->dtype, &k));
+    TRY(ensure_buffers(phi, 2));
+    SemiArgs<T> A{};
+    A.x = make_view<T>(phi);
+    A.phi = static_cast<const T*>(phi->p);
+    A.r = static_cast<const T*>(phi->buf1->p);
+    TRY(make_term_dev(phi, t, term_scale(t, ts, gs, 0), &A.u));
+    A.dt = dt;
+    for (int d = 0; d < 3; ++d) A.h[d] = phi->h[d];
+    cudaError_t e = launch_si_rhs<T>(phi->ndim, A, static_cast<T*>(phi->buf1->p), ctx->stream);
+    if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "semi-implicit right-hand side kernel launch failed: %s", cudaGetErrorString(e));
+    int launches = 0;
+    e = launch_si_sweeps<T>(phi->ndim, A, (int)k, ctx->opt_kernel == 2, static_cast<T*>(phi->p), static_cast<T*>(phi->buf2->p), ctx->stream, &launches);
+    ctx->cnt.kernel_launches += 1 + launches;
+    if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "semi-implicit sweep kernel launch failed: %s", cudaGetErrorString(e));
+    ctx->cnt.jacobi_sweeps += k;
+    for (lsm_field* f : {phi, phi->buf1, phi->buf2}) { f->version++; f->halo_valid = true; }
+    return LSM_OK;
+}
+
+int32_t si_step(lsm_ctx* ctx, lsm_field* phi, const lsm_term* terms, int nterms, double tc, double dt, const double* gs) {
+    TRY(si_check(ctx, phi, terms, nterms));
+    if (!(dt >= 0.0)) return fail(LSM_ERR_ARG, "semi-implicit step: dt must be >= 0 (got %g)", dt);
+    return phi->dtype == LSM_F64 ? si_step_t<double>(ctx, phi, terms[0], tc, dt, gs) : si_step_t<float>(ctx, phi, terms[0], tc, dt, gs);
 }
 
 // A second field F of an operation on phi (checked by check_level_set too) must lie on phi's grid: same node counts, same owned
@@ -1407,7 +1473,7 @@ int32_t lsm_stage(lsm_ctx* ctx, int32_t integrator, int32_t stage, lsm_field* ph
 int32_t lsm_advance(lsm_ctx* ctx, int32_t integrator, lsm_field* phi, const lsm_term* terms, int32_t nterms,
                     double tc, double dt) {
     TRY(check_state(ctx, phi, terms, nterms));
-    if (integrator < LSM_FORWARD_EULER || integrator > LSM_RK3) return fail(LSM_ERR_ARG, "bad integrator %d", integrator);
+    if (integrator < LSM_FORWARD_EULER || integrator > LSM_SEMI_IMPLICIT) return fail(LSM_ERR_ARG, "bad integrator %d", integrator);
     lsm_term tl[LSM_MAX_TERMS];
     TRY(prepare_terms(phi, terms, nterms, tl));
     for (int s = 1; s <= nstages(integrator); ++s) TRY(stage_impl(ctx, integrator, s, phi, tl, nterms, tc, dt, nullptr));
@@ -1419,12 +1485,13 @@ int32_t lsm_integrate(lsm_ctx* ctx, int32_t integrator, double cfl, lsm_field* p
                       double* t_out, int64_t* steps_out) {
     TRY(check_state(ctx, phi, terms, nterms));
     NvtxRange nvtx("lsm_integrate");
-    if (integrator < LSM_FORWARD_EULER || integrator > LSM_RK3) return fail(LSM_ERR_ARG, "bad integrator %d", integrator);
+    if (integrator < LSM_FORWARD_EULER || integrator > LSM_SEMI_IMPLICIT) return fail(LSM_ERR_ARG, "bad integrator %d", integrator);
     if (!(tf >= t0))     // levelsetequation.jl:196
         return fail(LSM_ERR_TIME, "final time %g must be >= initial time %g: the level-set equation cannot be solved back in time", tf, t0);
     lsm_term tl[LSM_MAX_TERMS];
     TRY(prepare_terms(phi, terms, nterms, tl));
     terms = tl;
+    if (integrator == LSM_SEMI_IMPLICIT) TRY(si_check(ctx, phi, terms, nterms));      // before any collective CFL reduction
     double tc = t0;
     int64_t steps = 0;
     bool finished = true;
@@ -1433,7 +1500,7 @@ int32_t lsm_integrate(lsm_ctx* ctx, int32_t integrator, double cfl, lsm_field* p
     // state changes from step to step — single rank, RK2/RK3 (whose buffers do not rotate), terms without a time factor, no
     // per-stage timing — the stage launches of one step are captured once into a CUDA graph and every later step with the same
     // dt replays it (one graph launch instead of 2-3 kernel launches plus their host-side setup).
-    bool graph_ok = ctx->opt_graph && ctx->nranks == 1 && integrator != LSM_FORWARD_EULER && !ctx->opt_time &&
+    bool graph_ok = ctx->opt_graph && ctx->nranks == 1 && integrator != LSM_FORWARD_EULER && integrator != LSM_SEMI_IMPLICIT && !ctx->opt_time &&
                     phi->owned <= (1L << 22);
     // (a time-dependent expression coefficient is materialised at each stage time: a captured fill would freeze t)
     for (int k = 0; k < nterms && graph_ok; ++k) if (terms[k].tscale_kind != LSM_TS_NONE || terms[k].coef_kind == LSM_COEF_EXPR) graph_ok = false;
@@ -1446,7 +1513,7 @@ int32_t lsm_integrate(lsm_ctx* ctx, int32_t integrator, double cfl, lsm_field* p
     // known in advance: dt = min(dt_max, cfl * dt_cfl, tf - tc) with a constant dt_cfl (timestepping.jl:104-118), so the host replays
     // the loop's arithmetic and hands the kernel the run-length encoded sequence.  Whatever is left (max_steps, more than
     // RES_STEP_CAP steps, a launch that is not possible) is done by the regular loop below.
-    if (resident_eligible(ctx, phi, terms, nterms) && tc <= tf - jl_eps(tc) && (max_steps < 0 || max_steps > 0)) {
+    if (integrator != LSM_SEMI_IMPLICIT && resident_eligible(ctx, phi, terms, nterms) && tc <= tf - jl_eps(tc) && (max_steps < 0 || max_steps > 0)) {
         double dt_cfl;
         rc = compute_cfl_impl(ctx, phi, terms, nterms, tc, nullptr, &dt_cfl);
         if (rc != LSM_OK) { if (t_out) *t_out = tc; if (steps_out) *steps_out = 0; return rc; }
@@ -1517,6 +1584,11 @@ int32_t lsm_integrate(lsm_ctx* ctx, int32_t integrator, double cfl, lsm_field* p
     if (rc != LSM_OK) return rc;
     if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "device error during integration: %s", cudaGetErrorString(e));
     return LSM_OK;
+}
+
+int32_t lsm_semi_implicit_sweeps(double courant, int32_t dtype, int64_t* sweeps_out) {
+    if (!sweeps_out || (dtype != LSM_F32 && dtype != LSM_F64)) return fail(LSM_ERR_ARG, "bad argument");
+    return si_sweeps(courant, dtype, sweeps_out);
 }
 
 int32_t lsm_eikonal_s0(lsm_field* dst, const lsm_field* phi0) {

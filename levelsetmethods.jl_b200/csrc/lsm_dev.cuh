@@ -67,6 +67,27 @@ struct StageParams {
     TermDev terms[4];
 };
 
+// component d of a term's coefficient at node (i0, i1, i2), linear index `node`, times its time factor
+template <class T>
+__device__ __forceinline__ double coef_comp(const TermDev& t, long node, int d, int i0, int i1, int i2, int N) {
+    double v;
+    if (t.coef_kind == COEF_CONST) {
+        v = t.cval[d];
+    } else if (t.coef_kind == COEF_FIELD) {
+        const long l = (long)d * t.cstride + node;
+        v = t.coef_f64 ? static_cast<const double*>(t.coef)[l] : double(static_cast<const T*>(t.coef)[l]);
+    } else if (t.coef_kind == COEF_SEPARABLE) {
+        v = t.cval[d];
+        v = v * t.tab[d][0][i0];
+        if (N > 1) v = v * t.tab[d][1][i1];
+        if (N > 2) v = v * t.tab[d][2][i2];
+    } else {
+        v = 0.0;
+    }
+    if (t.scaled) v = v * t.g;
+    return v;
+}
+
 // coefficient box without ghost planes: linear node index of (i0,i1,i2)
 struct CoefBox { int n0, n1; };
 

@@ -111,26 +111,6 @@ __device__ __forceinline__ double weno5_strict(double v1, double v2, double v3, 
     return w1 * d1 + w2 * d2 + w3 * d3;
 }
 
-template <class T>
-__device__ __forceinline__ double coef_comp(const TermDev& t, long node, int d, int i0, int i1, int i2, int N) {
-    double v;
-    if (t.coef_kind == COEF_CONST) {
-        v = t.cval[d];
-    } else if (t.coef_kind == COEF_FIELD) {
-        const long l = (long)d * t.cstride + node;
-        v = t.coef_f64 ? static_cast<const double*>(t.coef)[l] : double(static_cast<const T*>(t.coef)[l]);
-    } else if (t.coef_kind == COEF_SEPARABLE) {
-        v = t.cval[d];
-        v = v * t.tab[d][0][i0];
-        if (N > 1) v = v * t.tab[d][1][i1];
-        if (N > 2) v = v * t.tab[d][2][i2];
-    } else {
-        v = 0.0;
-    }
-    if (t.scaled) v = v * t.g;
-    return v;
-}
-
 // levelsetterms.jl:156-170 / 252-265 : second-order ENO one-sided pair along dim d
 template <int N, class T>
 __device__ __forceinline__ void eno2_pair(const Reader<N, T>& r, int d, double h, double& neg, double& pos) {

@@ -168,6 +168,21 @@ struct ResidentArgs {
 template <class T> bool resident2d_supported(int n0, int n1);
 template <class T> cudaError_t launch_resident2d(const ResidentArgs<T>& R, cudaStream_t s);
 
+// lsm_semi_implicit.cu (LSM_SEMI_IMPLICIT: one AdvectionTerm, inflow implicit / outflow explicit, Jacobi sweeps)
+template <class T>
+struct SemiArgs {
+    View<T> x;             // the state's box and boundary conditions (x.p unused; single rank, no ghost planes)
+    const T* phi;          // phi^n (read by the right-hand side kernel)
+    const T* r;            // right-hand side (read by the sweeps)
+    TermDev u;             // the velocity at t* = tc + dt/2, time factor included
+    double dt, h[3];
+};
+// r = phi^n - sum_d a_d (phi^n_{I + s_d e_d} - phi^n_I)
+template <class T> cudaError_t launch_si_rhs(int ndim, const SemiArgs<T>& A, T* r, cudaStream_t s);
+// k >= 1 Jacobi sweeps from x^0 = A.r, alternating between xa and xb so that the last one lands in xa; blocked: temporally blocked
+// launches of several sweeps each, else one sweep per launch (bit-identical; the default, measured faster).  *launches = kernels enqueued.
+template <class T> cudaError_t launch_si_sweeps(int ndim, const SemiArgs<T>& A, int k, bool blocked, T* xa, T* xb, cudaStream_t s, int* launches);
+
 // lsm_tiled.cu (performance kernels).  Returns cudaErrorNotSupported when the configuration is
 // not covered, in which case the caller uses the generic kernel.
 template <class T> cudaError_t launch_stage_tiled(int ndim, const StageParams<T>& P, int sm_count, cudaStream_t s, int pair_mode = 1, int* used_pair = nullptr);   // pair_mode: 0 never, 1 x-pair kernels (3-D: 20-bit eps max), 2 3-D x-pair kernel with the exact eps max, 3 x-pair kernels forced on small 2-D grids too

@@ -471,12 +471,52 @@ function LSM._advance!(integ::Explicit, ϕ::DeviceMeshField, _buffers, terms, tc
     return ϕ
 end
 
+# ---- InflowImplicit: the engine's semi-implicit advection integrator (LSM_SEMI_IMPLICIT) -------------------------------------------
+"""
+    InflowImplicit(; cfl = 2.0)
+
+Inflow-implicit / outflow-explicit steps of ONE `AdvectionTerm` on a `DeviceMeshField` (include/lsm_b200.h, "semi-implicit
+advection"): the velocity at mid-step, the implicit half solved on the device by a fixed number of Jacobi sweeps.  Stable above
+Courant number 1, hence `cfl = 2`.  The idea of `LevelSetMethods.SemiImplicitI2OE`, not its bits: this is a separate type until
+the two have been compared where Julia runs.
+"""
+Base.@kwdef struct InflowImplicit <: LSM.TimeIntegrator
+    cfl::Float64 = 2.0
+end
+LSM.cfl(integ::InflowImplicit) = integ.cfl
+_code(::InflowImplicit) = Int32(3)
+
+"`_alloc_buffers`: the right-hand side and the second Jacobi iterate live in the library's stage buffers of `ϕ`."
+LSM._alloc_buffers(::InflowImplicit, ϕ::DeviceMeshField) = ()
+
+"`_advance!`: one whole step (`lsm_stage` 1 of 1), `update_term!` first at the mid-step time the velocity is taken at."
+function LSM._advance!(integ::InflowImplicit, ϕ::DeviceMeshField, _buffers, terms, tc, Δt)
+    ts = tc + 0.5Δt
+    if any(term -> !_isdefault(_update_func(term)), terms)
+        for term in terms
+            LSM.update_term!(term, ϕ, ts)
+        end
+    end
+    low = lower(terms, ϕ, ts)
+    GC.@preserve low check(ccall((:lsm_stage, LIB), Int32, (Ptr{Cvoid}, Int32, Int32, Ptr{Cvoid}, Ptr{CTerm}, Int32, Float64, Float64, Ptr{Float64}),
+                                 ϕ.ctx.handle, _code(integ), 1, handle!(ϕ), low.terms, length(low.terms), tc, Δt, low.gscale))
+    _device_advanced!(ϕ)
+    return ϕ
+end
+
+"Jacobi sweeps of a semi-implicit step at Courant number `courant` (`lsm_semi_implicit_sweeps`; no GPU needed)."
+function semi_implicit_sweeps(courant::Real, ::Type{T} = Float64) where {T}
+    k = Ref{Int64}(0)
+    check(ccall((:lsm_semi_implicit_sweeps, LIB), Int32, (Float64, Int32, Ref{Int64}), courant, T === Float64 ? Int32(1) : Int32(0), k))
+    return k[]
+end
+
 """
 `_integrate!` — src/timestepping.jl:101-122.  Default hooks and device-resident coefficients: the whole loop is one
 `lsm_integrate` call (Δt = min(Δt_max, cfl·compute_cfl, tf − tc) while tc ≤ tf − eps(tc), landing on tf).  Otherwise the
 reference's generic method runs and its calls dispatch to the methods above.
 """
-function LSM._integrate!(ls, ϕ::DeviceMeshField, integ::Explicit, terms, tc, tf, Δt_max, prehook, posthook)
+function LSM._integrate!(ls, ϕ::DeviceMeshField, integ::Union{Explicit, InflowImplicit}, terms, tc, tf, Δt_max, prehook, posthook)
     low = lower(terms, ϕ, tc)
     if prehook === identity && posthook === identity && low.device_only
         t_out, steps = Ref{Float64}(tc), Ref{Int64}(0)

@@ -101,9 +101,7 @@ typedef struct {
 /* options for lsm_set_option */
 enum {
     LSM_OPT_KERNEL = 0,       /* 0 auto (x-pair / tiled where available), 1 force generic strict kernel, 2 force tiled / x-pair, 3 tiled without the x-pair kernel,
-                                 4 x-pair kernel with the exact WENO epsilon maximum (bit-identical to 3; default is a 20-bit maximum).
-                                 LSM_SEMI_IMPLICIT: 2 runs the temporally blocked Jacobi sweeps, every other value one sweep per launch
-                                 (the faster form on a B200, see DESIGN.md 4.6); the two are bit-identical */
+                                 4 x-pair kernel with the exact WENO epsilon maximum (bit-identical to 3; default is a 20-bit maximum) */
     LSM_OPT_TIME_STAGES = 1,  /* 1: bracket every stage launch with CUDA events, resolved at the next sync  */
     LSM_OPT_CFL_CACHE = 2,    /* 1 (default): reuse the CFL reduction while coefficient data/scale unchanged  */
     LSM_OPT_OVERLAP = 3,      /* 1 (default): overlap halo exchange with interior compute (multi-rank)        */

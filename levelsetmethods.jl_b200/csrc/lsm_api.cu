@@ -88,7 +88,6 @@ struct lsm_ctx {
     unsigned long long* h_scalar = nullptr;     // pinned
     lsm_counters cnt{};
     int opt_kernel = 0, opt_time = 0, opt_cfl_cache = 1, opt_overlap = 1;
-    int interior_first = 0;     // LSM_B200_INTERIOR_FIRST (experiments): round-2's original launch order of the overlapped stage
     std::vector<CflMemo> cfl_memo;
     int opt_cand = 1;           // LSM_OPT_CFL_CANDIDATES
     int opt_resident = 1;       // LSM_OPT_RESIDENT
@@ -160,7 +159,7 @@ int32_t ctx_common_init(lsm_ctx* c) {
     {   // the boundary-slab stream and the halo-exchange stream outrank the compute stream: their (small) grids are placed first
         int lo = 0, hi = 0;
         CU(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-        CU(cudaStreamCreateWithPriority(&c->comm, cudaStreamNonBlocking, getenv("LSM_B200_INTERIOR_FIRST") ? lo : hi));
+        CU(cudaStreamCreateWithPriority(&c->comm, cudaStreamNonBlocking, hi));
         CU(cudaStreamCreateWithPriority(&c->bstream, cudaStreamNonBlocking, hi));
     }
     CU(cudaEventCreateWithFlags(&c->ev_main, cudaEventDisableTiming));
@@ -169,8 +168,6 @@ int32_t ctx_common_init(lsm_ctx* c) {
     CU(cudaMalloc(&c->d_scalar, 64));
     CU(cudaMallocHost(&c->h_scalar, 64));
     if (getenv("LSM_B200_NO_OVERLAP")) c->opt_overlap = 0;
-    if (getenv("LSM_B200_INTERIOR_FIRST")) c->interior_first = 1;
-    if (getenv("LSM_B200_NO_GRAPH")) c->opt_graph = 0;
     return LSM_OK;
 }
 
@@ -433,9 +430,11 @@ int32_t launch_stage_range(lsm_ctx* c, int ndim, StageParams<T>& P, int r0, int 
     P.r0 = r0; P.r1 = r1;
     cudaError_t e = cudaErrorNotSupported;
     int used_pair = 0;
-    if (c->opt_kernel != 1 && stage_tiled_supported<T>(ndim, P)) e = launch_stage_tiled<T>(ndim, P, c->sm_count, st, c->opt_kernel == 3 ? 0 : (c->opt_kernel == 4 ? 2 : (c->opt_kernel == 2 ? 3 : 1)), &used_pair);
-    else if (c->opt_kernel == 2) return fail(LSM_ERR_UNSUPPORTED, "tiled kernel forced but this configuration is not covered");
-    if (e == cudaErrorNotSupported) e = launch_stage_generic<T>(ndim, P, st);
+    if (c->opt_kernel != 1) e = launch_stage_tiled<T>(ndim, P, c->opt_kernel, c->sm_count, st, &used_pair);
+    if (e == cudaErrorNotSupported) {
+        if (c->opt_kernel == 2) return fail(LSM_ERR_UNSUPPORTED, "tiled kernel forced but this configuration is not covered");
+        e = launch_stage_generic<T>(ndim, P, st);
+    }
     if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "stage kernel launch failed: %s", cudaGetErrorString(e));
     c->cnt.kernel_launches += 1; c->cnt.stage_launches += 1; c->cnt.pair_launches += used_pair;
     return LSM_OK;
@@ -486,7 +485,7 @@ int32_t run_stage_t(lsm_ctx* c, lsm_field* in, lsm_field* p0, lsm_field* out, ls
         // (a few blocks of NCCL's, more registers per block than an SM has left beside a resident interior block) then becomes
         // runnable TOGETHER with the interior grid and — on a higher-priority stream — is placed first; launched behind an
         // interior grid that already occupies every SM it would only run in that grid's tail, i.e. not overlapped at all.
-        if (!c->interior_first) CU(cudaStreamWaitEvent(c->stream, c->ev_boundary, 0));
+        CU(cudaStreamWaitEvent(c->stream, c->ev_boundary, 0));
         TRY(launch_stage_range<T>(c, in->ndim, P, sl, nl - sl));
         CU(cudaStreamWaitEvent(c->stream, c->ev_boundary, 0));
         CU(cudaStreamWaitEvent(c->stream, c->ev_halo, 0));
@@ -578,10 +577,8 @@ bool resident_eligible(const lsm_ctx* ctx, const lsm_field* phi, const lsm_term*
     if (!t.field || t.field->separable || t.field->dtype != phi->dtype || t.field->ncomp != 2 || t.field->ctx != ctx) return false;
     for (int d = 0; d < 2; ++d) {
         if (t.field->nglob[d] != phi->nglob[d]) return false;
-        for (int sd = 0; sd < 2; ++sd) {
-            const int k = phi->bc[d][sd].kind;
-            if (!(k == LSM_BC_PERIODIC || k == LSM_BC_SYMMETRY || (k == LSM_BC_EXTRAP && phi->bc[d][sd].P == 0))) return false;
-        }
+        for (int sd = 0; sd < 2; ++sd)
+            if (!bc_index_map(phi->bc[d][sd].kind, phi->bc[d][sd].P)) return false;
     }
     return phi->dtype == LSM_F64 ? resident2d_supported<double>(phi->n[0], phi->n[1]) : resident2d_supported<float>(phi->n[0], phi->n[1]);
 }
@@ -867,7 +864,7 @@ int32_t si_check(lsm_ctx* ctx, const lsm_field* phi, const lsm_term* terms, int 
         return fail(LSM_ERR_ARG, "the semi-implicit integrator takes exactly one AdvectionTerm (got %d terms, the first of kind %d)", nterms, terms[0].kind);
     for (int d = 0; d < phi->ndim; ++d)
         for (int sd = 0; sd < 2; ++sd)
-            if (phi->bc[d][sd].kind == LSM_BC_EXTRAP && phi->bc[d][sd].P >= 1)
+            if (!bc_index_map(phi->bc[d][sd].kind, phi->bc[d][sd].P))
                 return fail(LSM_ERR_UNSUPPORTED, "the semi-implicit integrator does not support ExtrapolationBC{%d} (dimension %d, %s side): its "
                             "ghost weights are negative, so the implicit system is not an M-matrix", phi->bc[d][sd].P, d + 1, sd ? "right" : "left");
     return LSM_OK;
@@ -894,7 +891,7 @@ int32_t si_step_t(lsm_ctx* ctx, lsm_field* phi, const lsm_term& t, double tc, do
     cudaError_t e = launch_si_rhs<T>(phi->ndim, A, static_cast<T*>(phi->buf1->p), ctx->stream);
     if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "semi-implicit right-hand side kernel launch failed: %s", cudaGetErrorString(e));
     int launches = 0;
-    e = launch_si_sweeps<T>(phi->ndim, A, (int)k, ctx->opt_kernel == 2, static_cast<T*>(phi->p), static_cast<T*>(phi->buf2->p), ctx->stream, &launches);
+    e = launch_si_sweeps<T>(phi->ndim, A, (int)k, static_cast<T*>(phi->p), static_cast<T*>(phi->buf2->p), ctx->stream, &launches);
     ctx->cnt.kernel_launches += 1 + launches;
     if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "semi-implicit sweep kernel launch failed: %s", cudaGetErrorString(e));
     ctx->cnt.jacobi_sweeps += k;

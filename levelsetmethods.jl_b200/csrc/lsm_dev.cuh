@@ -27,6 +27,13 @@ enum : int {
 
 struct BCDev { int kind, P; };
 
+// Is a boundary side (kind, extrapolation order P) a pure index map with weight 1: periodic, symmetry, ExtrapolationBC{0}, or
+// the stored ghost planes of the decomposed axis?  ExtrapolationBC{P >= 1} is a weighted stencil.  Takes the BC_* kinds of a
+// View and the LSM_BC_* kinds of a field alike (they share 0..2; BC_HALO appears only on the last axis, see make_view).
+__host__ __device__ inline bool bc_index_map(int kind, int P) {
+    return kind == BC_PERIODIC || kind == BC_SYMMETRY || kind == BC_HALO || (kind == BC_EXTRAP && P == 0);
+}
+
 template <class T>
 struct View {
     const T* p;          // first owned node

@@ -179,13 +179,13 @@ struct SemiArgs {
 };
 // r = phi^n - sum_d a_d (phi^n_{I + s_d e_d} - phi^n_I)
 template <class T> cudaError_t launch_si_rhs(int ndim, const SemiArgs<T>& A, T* r, cudaStream_t s);
-// k >= 1 Jacobi sweeps from x^0 = A.r, alternating between xa and xb so that the last one lands in xa; blocked: temporally blocked
-// launches of several sweeps each, else one sweep per launch (bit-identical; the default, measured faster).  *launches = kernels enqueued.
-template <class T> cudaError_t launch_si_sweeps(int ndim, const SemiArgs<T>& A, int k, bool blocked, T* xa, T* xb, cudaStream_t s, int* launches);
+// k >= 1 Jacobi sweeps from x^0 = A.r, one per launch, alternating between xa and xb so that the last one lands in xa.
+// *launches = kernels enqueued.
+template <class T> cudaError_t launch_si_sweeps(int ndim, const SemiArgs<T>& A, int k, T* xa, T* xb, cudaStream_t s, int* launches);
 
-// lsm_tiled.cu (performance kernels).  Returns cudaErrorNotSupported when the configuration is
-// not covered, in which case the caller uses the generic kernel.
-template <class T> cudaError_t launch_stage_tiled(int ndim, const StageParams<T>& P, int sm_count, cudaStream_t s, int pair_mode = 1, int* used_pair = nullptr);   // pair_mode: 0 never, 1 x-pair kernels (3-D: 20-bit eps max), 2 3-D x-pair kernel with the exact eps max, 3 x-pair kernels forced on small 2-D grids too
-template <class T> bool stage_tiled_supported(int ndim, const StageParams<T>& P);
+// lsm_tiled.cu (performance kernels), for LSM_OPT_KERNEL value `kernel` (not 1): 3 takes no x-pair kernel, 4 the 3-D x-pair kernel
+// with the exact eps maximum, 2 the 2-D x-pair kernel below its size threshold too.  *used_pair = 1 when an x-pair kernel ran.
+// Returns cudaErrorNotSupported when the configuration is not covered, in which case the caller uses the generic kernel.
+template <class T> cudaError_t launch_stage_tiled(int ndim, const StageParams<T>& P, int kernel, int sm_count, cudaStream_t s, int* used_pair);
 
 }  // namespace lsm

@@ -286,15 +286,7 @@ cudaError_t launch_pair2(const StageParams<T>& P, const AuxList& A, cudaStream_t
 
 template <class T, bool XMAX, bool CURV>
 cudaError_t launch_pair2_sb(const StageParams<T>& P, const AuxList& A, cudaStream_t s, int sm_count) {
-    if (A.p0 >= 0 && A.p0 != 2) return cudaErrorNotSupported;
-    if (P.base == BASE_IN && !P.p0) {
-        if (!P.out2) return launch_pair2<T, SB_IN, XMAX, CURV>(P, A, s, sm_count);
-        return launch_pair2<T, SB_IN_OUT2, XMAX, CURV>(P, A, s, sm_count);
-    }
-    if (P.base == BASE_RK3_S2 && P.p0 && !P.out2) return launch_pair2<T, SB_S2, XMAX, CURV>(P, A, s, sm_count);
-    if (P.base == BASE_RK3_S3 && P.p0 && !P.out2) return launch_pair2<T, SB_S3, XMAX, CURV>(P, A, s, sm_count);
-    if (P.base == BASE_P0 && P.p0 && !P.out2) return launch_pair2<T, SB_P0, XMAX, CURV>(P, A, s, sm_count);
-    return cudaErrorNotSupported;
+    return with_static_base(static_base(P, A, 2), [&](auto SB) { return launch_pair2<T, decltype(SB)::value, XMAX, CURV>(P, A, s, sm_count); });
 }
 
 }  // namespace
@@ -303,7 +295,7 @@ cudaError_t launch_pair2_sb(const StageParams<T>& P, const AuxList& A, cudaStrea
 // box; anything else reports cudaErrorNotSupported and the caller takes the general tiled kernel.
 template <class T>
 cudaError_t launch_stage_pair2d(const StageParams<T>& P, const AuxList& A, cudaStream_t s, bool force, int sm_count) {
-    if (pair_kernel_disabled() || tma_disabled() || !encode_tiled_fn()) return cudaErrorNotSupported;
+    if (tma_disabled() || !encode_tiled_fn()) return cudaErrorNotSupported;
     if (P.nterms != 1 && P.nterms != 2) return cudaErrorNotSupported;
     const TermDev& ta = P.terms[0];
     if (ta.kind != TERM_ADVECTION || ta.scheme != SCHEME_WENO5 || ta.coef_kind != COEF_FIELD || ta.coef_f64 || A.first[0] != 0) return cudaErrorNotSupported;
@@ -315,11 +307,8 @@ cudaError_t launch_stage_pair2d(const StageParams<T>& P, const AuxList& A, cudaS
     // (measured 29.7 vs 11.1 us per RK3 step at 128^2); LSM_OPT_KERNEL = 2 forces this kernel for tests
     if (!force && (long)v.n[0] * v.n[1] < (1L << 18)) return cudaErrorNotSupported;
     for (int d = 0; d < 2; ++d)
-        for (int sd = 0; sd < 2; ++sd) {
-            const BCDev& b = v.bc[d][sd];
-            const bool index_map = b.kind == BC_PERIODIC || b.kind == BC_SYMMETRY || (b.kind == BC_EXTRAP && b.P == 0) || (b.kind == BC_HALO && d == 1);
-            if (!index_map) return cudaErrorNotSupported;
-        }
+        for (int sd = 0; sd < 2; ++sd)
+            if (!bc_index_map(v.bc[d][sd].kind, v.bc[d][sd].P)) return cudaErrorNotSupported;
     // 2-D always evaluates eps from the EXACT maximum: with the curvature term on kinked data (C2) the 20-bit maximum of the 3-D
     // advection kernel is amplified past the 1e-10 bar at 512^2 (DESIGN.md §2)
     if (curv) return launch_pair2_sb<T, true, true>(P, A, s, sm_count);

@@ -490,8 +490,7 @@ cudaError_t launch_pair_x(const StageParams<T>& P, const AuxList& A, cudaStream_
     int nchunks = std::max(1, (nr + 32) / 64);
     const long want = (2L * 296 + tiles - 1) / tiles;                  // chunks needed for ~2 waves
     if (nchunks < want) nchunks = (int)std::min<long>(want, std::max(1, nr / 8));
-    static const int cz_env = [] { const char* e = getenv("LSM_B200_CZ"); return e ? atoi(e) : 0; }();     // experiments only
-    const int cz = cz_env > 0 ? std::min(cz_env, nr) : (nr + nchunks - 1) / nchunks;
+    const int cz = (nr + nchunks - 1) / nchunks;
     dim3 block(32, NT / 32), grid((v.n[0] + G::BX - 1) / G::BX, (v.n[1] + G::BY - 1) / G::BY, (nr + cz - 1) / cz);
     kern<<<grid, block, smem, s>>>(P, A, M, cz);
     return cudaGetLastError();
@@ -511,15 +510,7 @@ cudaError_t launch_pair(const StageParams<T>& P, const AuxList& A, cudaStream_t 
 template <class T, int CK, bool HASN = false>
 cudaError_t launch_pair_sb(const StageParams<T>& P, const AuxList& A, cudaStream_t s, bool exact_eps) {
     constexpr int SP0 = CK == PAIR_EIK ? 1 : (CK == COEF_FIELD ? 3 : 0) + (HASN ? 1 : 0);
-    if (A.p0 >= 0 && A.p0 != SP0) return cudaErrorNotSupported;
-    if (P.base == BASE_IN && !P.p0) {
-        if (!P.out2) return launch_pair<T, CK, SB_IN, HASN>(P, A, s, exact_eps);
-        return launch_pair<T, CK, SB_IN_OUT2, HASN>(P, A, s, exact_eps);
-    }
-    if (P.base == BASE_RK3_S2 && P.p0 && !P.out2) return launch_pair<T, CK, SB_S2, HASN>(P, A, s, exact_eps);
-    if (P.base == BASE_RK3_S3 && P.p0 && !P.out2) return launch_pair<T, CK, SB_S3, HASN>(P, A, s, exact_eps);
-    if (P.base == BASE_P0 && P.p0 && !P.out2) return launch_pair<T, CK, SB_P0, HASN>(P, A, s, exact_eps);
-    return cudaErrorNotSupported;
+    return with_static_base(static_base(P, A, SP0), [&](auto SB) { return launch_pair<T, CK, decltype(SB)::value, HASN>(P, A, s, exact_eps); });
 }
 
 }  // namespace
@@ -528,7 +519,7 @@ cudaError_t launch_pair_sb(const StageParams<T>& P, const AuxList& A, cudaStream
 // cudaErrorNotSupported and the caller takes the general tiled kernel.
 template <class T>
 cudaError_t launch_stage_pair3d(const StageParams<T>& P, const AuxList& A, cudaStream_t s, bool exact_eps) {
-    if (pair_kernel_disabled() || tma_disabled() || !encode_tiled_fn()) return cudaErrorNotSupported;
+    if (tma_disabled() || !encode_tiled_fn()) return cudaErrorNotSupported;
     if (P.nterms != 1 && P.nterms != 2) return cudaErrorNotSupported;
     const TermDev& ta = P.terms[P.nterms - 1];          // the advection term (last)
     const bool eik = P.nterms == 1 && ta.kind == TERM_EIKONAL && ta.coef_kind == COEF_FIELD && !ta.coef_f64 && A.first[0] == 0;
@@ -537,11 +528,8 @@ cudaError_t launch_stage_pair3d(const StageParams<T>& P, const AuxList& A, cudaS
     if ((v.n[0] * sizeof(T)) % 16 != 0 || v.n[0] < 8 || v.n[1] < 8 || v.n[2] < 4) return cudaErrorNotSupported;
     if ((long)v.n[0] * v.n[1] >= (1L << 31)) return cudaErrorNotSupported;
     for (int d = 0; d < 3; ++d)
-        for (int sd = 0; sd < 2; ++sd) {
-            const BCDev& b = v.bc[d][sd];
-            const bool index_map = b.kind == BC_PERIODIC || b.kind == BC_SYMMETRY || (b.kind == BC_EXTRAP && b.P == 0) || (b.kind == BC_HALO && d == 2);
-            if (!index_map) return cudaErrorNotSupported;
-        }
+        for (int sd = 0; sd < 2; ++sd)
+            if (!bc_index_map(v.bc[d][sd].kind, v.bc[d][sd].P)) return cudaErrorNotSupported;
     if (eik) return launch_pair_sb<T, PAIR_EIK>(P, A, s, exact_eps);
     if (P.nterms == 2) {
         // (NormalMotionTerm(stored speed), AdvectionTerm(stored velocity)) in this order, Float64

@@ -273,7 +273,6 @@ size_t resident_smem(int n0, int n1) {
 
 template <class T>
 bool resident2d_supported(int n0, int n1) {
-    if (env_flag("LSM_B200_NO_RESIDENT")) return false;
     // n1 >= 3 * CS: every strip holds at least the 3 rows its neighbours' halos need (and a row has at most RES_MAXD mirrors)
     // n0 >= 8 like the tiled kernels (tinier grids take the strict kernel, whose rounding differs)
     if (n0 < 8 || n0 > 0xFFFF || n1 < HAL * RES_CS || (long)n0 * n1 > RES_MAX_NODES) return false;

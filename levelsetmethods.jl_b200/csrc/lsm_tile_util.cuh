@@ -200,6 +200,30 @@ __host__ __device__ constexpr int sig_first(int TK, int COEFK, int k, int ndim) 
     return f;
 }
 
+// The static base mode of a launch whose kernel expects phi^n / corr (when staged) in aux slot p0_slot, or -1 when none fits.
+template <class T>
+int static_base(const StageParams<T>& P, const AuxList& A, int p0_slot) {
+    if (A.p0 >= 0 && A.p0 != p0_slot) return -1;
+    if (P.base == BASE_IN && !P.p0) return P.out2 ? SB_IN_OUT2 : SB_IN;
+    if (!P.p0 || P.out2) return -1;
+    if (P.base == BASE_RK3_S2) return SB_S2;
+    if (P.base == BASE_RK3_S3) return SB_S3;
+    if (P.base == BASE_P0) return SB_P0;
+    return -1;
+}
+// launch(std::integral_constant<int, SB>{}) for a static base mode sb >= 0; cudaErrorNotSupported for sb = -1
+template <class F>
+cudaError_t with_static_base(int sb, F launch) {
+    switch (sb) {
+        case SB_IN:      return launch(std::integral_constant<int, SB_IN>{});
+        case SB_S2:      return launch(std::integral_constant<int, SB_S2>{});
+        case SB_S3:      return launch(std::integral_constant<int, SB_S3>{});
+        case SB_IN_OUT2: return launch(std::integral_constant<int, SB_IN_OUT2>{});
+        case SB_P0:      return launch(std::integral_constant<int, SB_P0>{});
+        default:         return cudaErrorNotSupported;
+    }
+}
+
 // levelsetterms.jl:184-187
 // Same-sign test on the sign bits (LOP3 + ISETP instead of DMUL + DSETP): identical to `x*y > 0` except where the product
 // underflows (|x||y| < 5e-324), where the reference returns 0 and this returns min(|x|,|y|) < 1e-150 — far below any tolerance.
@@ -289,7 +313,6 @@ bool cached_map3(CUtensorMap* out, const void* base, long n0, long n1, long npla
 // environment switches are read once per process
 inline bool env_flag(const char* name) { const char* v = getenv(name); return v && *v && *v != '0'; }
 inline bool tma_disabled() { static const bool v = env_flag("LSM_B200_NO_TMA"); return v; }
-inline bool pair_kernel_disabled() { static const bool v = env_flag("LSM_B200_NO_PAIR"); return v; }
 
 // cudaFuncAttributeMaxDynamicSharedMemorySize is a per-device attribute: remember the opt-in per (kernel instantiation, device)
 template <class K>

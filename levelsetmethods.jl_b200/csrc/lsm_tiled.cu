@@ -492,18 +492,10 @@ cudaError_t launch_tiled(const StageParams<T>& P, const AuxList& A, cudaStream_t
 template <class T, int NDIM, int MASK, int NTS, int COEFK, bool REMAP, int TK>
 cudaError_t launch_static(const StageParams<T>& P, const AuxList& A, cudaStream_t s) {
     constexpr int SP0 = TK >= 0 ? sig_first(TK, COEFK, NTS, NDIM) : (COEFK == COEF_FIELD ? NDIM : 0);
-    const bool p0_ok = A.p0 < 0 || A.p0 == SP0;
-    if (p0_ok) {
-        if (P.base == BASE_IN && !P.p0) {
-            if (!P.out2) return launch_tiled<T, NDIM, MASK, NTS, COEFK, REMAP, TK, SB_IN>(P, A, s);
-            return launch_tiled<T, NDIM, MASK, NTS, COEFK, REMAP, TK, SB_IN_OUT2>(P, A, s);
-        }
-        if (P.base == BASE_RK3_S2 && P.p0 && !P.out2) return launch_tiled<T, NDIM, MASK, NTS, COEFK, REMAP, TK, SB_S2>(P, A, s);
-        if (P.base == BASE_RK3_S3 && P.p0 && !P.out2) return launch_tiled<T, NDIM, MASK, NTS, COEFK, REMAP, TK, SB_S3>(P, A, s);
-        if (P.base == BASE_P0 && P.p0 && !P.out2) return launch_tiled<T, NDIM, MASK, NTS, COEFK, REMAP, TK, SB_P0>(P, A, s);
-    }
+    const int sb = static_base(P, A, SP0);
     // (cannot happen with the aux list launch_stage_tiled builds; the all-terms kernel handles anything)
-    return launch_tiled<T, NDIM, M_ALL, 0, -1, REMAP>(P, A, s);
+    if (sb < 0) return launch_tiled<T, NDIM, M_ALL, 0, -1, REMAP>(P, A, s);
+    return with_static_base(sb, [&](auto SB) { return launch_tiled<T, NDIM, MASK, NTS, COEFK, REMAP, TK, decltype(SB)::value>(P, A, s); });
 }
 
 template <class T, int NDIM, bool REMAP>
@@ -559,8 +551,6 @@ int term_mask(const TermDev& t) {
     }
 }
 
-}  // namespace
-
 template <class T>
 bool stage_tiled_supported(int ndim, const StageParams<T>& P) {
     if (ndim != 2 && ndim != 3) return false;
@@ -575,8 +565,10 @@ bool stage_tiled_supported(int ndim, const StageParams<T>& P) {
     return naux <= 8;
 }
 
+}  // namespace
+
 template <class T>
-cudaError_t launch_stage_tiled(int ndim, const StageParams<T>& P, int sm_count, cudaStream_t s, int pair_mode, int* used_pair) {
+cudaError_t launch_stage_tiled(int ndim, const StageParams<T>& P, int kernel, int sm_count, cudaStream_t s, int* used_pair) {
     if (!stage_tiled_supported<T>(ndim, P)) return cudaErrorNotSupported;
     if (P.r1 <= P.r0) return cudaSuccess;
     AuxList A{};
@@ -593,18 +585,13 @@ cudaError_t launch_stage_tiled(int ndim, const StageParams<T>& P, int sm_count, 
         }
     }
     if (P.p0) { A.p0 = A.n; A.src[A.n++] = P.p0; }
-    if (pair_mode && ndim == 3 && (mask == M_ADV_WENO || (mask == (M_NORMAL | M_ADV_WENO) && P.nterms == 2) || (mask == M_EIK && P.nterms == 1))) {      // headline path: x-pair kernel (lsm_pair3d.cu); falls through when it does not apply
-        const cudaError_t e = launch_stage_pair3d<T>(P, A, s, pair_mode == 2);
-        if (e != cudaErrorNotSupported) { if (used_pair) *used_pair = 1; return e; }
+    if (kernel != 3) {     // the x-pair kernels (lsm_pair3d.cu, lsm_pair2d.cu) report cudaErrorNotSupported for what they do not cover
+        const cudaError_t e = ndim == 3 ? launch_stage_pair3d<T>(P, A, s, kernel == 4) : launch_stage_pair2d<T>(P, A, s, kernel == 2, sm_count);
+        if (e != cudaErrorNotSupported) { *used_pair = 1; return e; }
     }
-    if (pair_mode && ndim == 2 && (mask == M_ADV_WENO || (mask == (M_ADV_WENO | M_CURV) && P.nterms == 2))) {      // 2-D x-pair kernel (lsm_pair2d.cu)
-        const cudaError_t e = launch_stage_pair2d<T>(P, A, s, pair_mode == 3, sm_count);
-        if (e != cudaErrorNotSupported) { if (used_pair) *used_pair = 1; return e; }
-    }
-    bool remap = true;     // every BC an index map?  (ExtrapolationBC{P>=1} is a weighted stencil)
+    bool remap = true;     // every BC an index map?
     for (int d = 0; d < ndim; ++d)
-        for (int sd = 0; sd < 2; ++sd)
-            if (P.in.bc[d][sd].kind == BC_EXTRAP && P.in.bc[d][sd].P > 0) remap = false;
+        for (int sd = 0; sd < 2; ++sd) remap = remap && bc_index_map(P.in.bc[d][sd].kind, P.in.bc[d][sd].P);
     if (ndim == 3) return remap ? launch_by_mask<T, 3, true>(mask, P, A, s) : launch_by_mask<T, 3, false>(mask, P, A, s);
     return remap ? launch_by_mask<T, 2, true>(mask, P, A, s) : launch_by_mask<T, 2, false>(mask, P, A, s);
 }
@@ -612,12 +599,10 @@ cudaError_t launch_stage_tiled(int ndim, const StageParams<T>& P, int sm_count, 
 // The Makefile compiles this file twice (-DLSM_TILED_F32 / -DLSM_TILED_F64) so that the two halves of the ~160 kernel
 // instantiations build in parallel; without either macro both are instantiated here.
 #if !defined(LSM_TILED_F64)
-template bool stage_tiled_supported<float>(int, const StageParams<float>&);
-template cudaError_t launch_stage_tiled<float>(int, const StageParams<float>&, int, cudaStream_t, int, int*);
+template cudaError_t launch_stage_tiled<float>(int, const StageParams<float>&, int, int, cudaStream_t, int*);
 #endif
 #if !defined(LSM_TILED_F32)
-template bool stage_tiled_supported<double>(int, const StageParams<double>&);
-template cudaError_t launch_stage_tiled<double>(int, const StageParams<double>&, int, cudaStream_t, int, int*);
+template cudaError_t launch_stage_tiled<double>(int, const StageParams<double>&, int, int, cudaStream_t, int*);
 #endif
 
 }  // namespace lsm

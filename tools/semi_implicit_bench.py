@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""tools/semi_implicit_bench.py — the semi-implicit advection integrator (SemiImplicit, LSM_SEMI_IMPLICIT, cfl 2) in its one-sweep-per-launch
-(default) and temporally blocked forms, against TVD-RK3 (cfl 0.5) with WENO5 and with Upwind, Float64, on:
+"""tools/semi_implicit_bench.py — the semi-implicit advection integrator (SemiImplicit, LSM_SEMI_IMPLICIT, cfl 2, one Jacobi sweep per
+launch) against TVD-RK3 (cfl 0.5) with WENO5 and with Upwind, Float64, on:
 
   rot2048  a circle in the rigid rotation (-2 pi y, 2 pi x) on [-1, 1]^2, 2048^2 nodes, NeumannBC, stored velocity;
   c3_256, c3_512  bench.py's C3 (Enright sphere, stored velocity x cos(pi t / 3), NeumannBC) at 256^3 and 512^3.
@@ -9,7 +9,7 @@ For each case and integrator the same simulated time S = --steps semi-implicit s
 integrate() after one warm-up step, timed with CUDA events on the library's stream: time per step and per unit of simulated time.
 Bytes per step are the compulsory HBM traffic computed from shapes (8 bytes per node and value): RK3 3 stages x (phi, N velocity
 components, one more read for stages 2-3, one write); semi-implicit: the right-hand side (phi, N components, one write) and every
-sweep launch (r, x, N components, one write), times the number of launches (k / sweeps per launch).  The card's name and power limit
+sweep launch (r, x, N components, one write), times the number of sweeps k.  The card's name and power limit
 are read in the same run.  One JSON line per case.
 
     python tools/semi_implicit_bench.py [--steps 8] [--cases rot2048,c3_256,c3_512]
@@ -30,8 +30,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 for p in (ROOT, os.path.join(ROOT, "tests")):
     if p not in sys.path:
         sys.path.insert(0, p)
-
-SWEEPS_PER_LAUNCH = {1: 16, 2: 8, 3: 2}     # lsm_semi_implicit.cu: SiShape<N>::M
 
 
 def card():
@@ -100,14 +98,11 @@ def main():
         S = a.steps * 2.0 * m.compute_cfl(terms, phi, 0.0)
         res = {"case": name, "n": list(n), "card": info, "sim_time": S}
         for label, integ, scheme in (("semi_implicit", m.SemiImplicit(2.0), m.Upwind()),
-                                     ("semi_implicit_blocked", m.SemiImplicit(2.0), m.Upwind()),
                                      ("rk3_weno5", m.RK3(0.5), m.WENO5()), ("rk3_upwind", m.RK3(0.5), m.Upwind())):
-            # LSM_OPT_KERNEL = 2: the temporally blocked sweeps instead of the default one sweep per launch
-            m._lib.check(m._lib.lib().lsm_set_option(ctx.handle, m._lib.OPT_KERNEL, 2 if label.endswith("blocked") else 0))
             ms, steps, c = run(m, ctx, build, integ, scheme, S)
-            if label.startswith("semi_implicit"):
+            if label == "semi_implicit":
                 k = c["jacobi_sweeps"] / max(steps, 1)
-                launches = math.ceil(k / SWEEPS_PER_LAUNCH[N]) if label.endswith("blocked") else math.ceil(k)
+                launches = math.ceil(k)
                 bytes_step = 8 * nodes * ((N + 2) + launches * (N + 3))
                 extra = {"sweeps_per_step": k, "sweep_launches_per_step": launches}
             else:

@@ -507,7 +507,8 @@ int32_t lsm_multi_level_set_integrals(int32_t n, lsm_ctx* const* ctx, lsm_field*
                                       double level, double* out);
 
 /* ---- diagnostics (test harness; SURVEY.md §2.2 K6) -------------------------------------------- */
-/* max |a - b| over all owned nodes, all-reduced over ranks. */
+/* max |a - b| over all owned nodes, all-reduced over ranks.  a and b are scalar, non-separable fields of ctx of one dtype, with the
+ * same dimension and the same node counts; else LSM_ERR_ARG. */
 int32_t lsm_max_abs_diff(lsm_ctx* ctx, const lsm_field* a, const lsm_field* b, double* out);
 
 #ifdef __cplusplus

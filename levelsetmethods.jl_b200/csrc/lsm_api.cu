@@ -177,6 +177,23 @@ void slab_plan(int n_last, int nranks, int rank, int* first, int* count) {
     *first = rank * base + (rank < rem ? rank : rem);
 }
 
+// The grid of a new field (ctx and ndim set): n[d] >= 1 nodes from lc to hc, this rank's slab of the last dimension, no BCs
+int32_t grid_setup(lsm_field* f, const int32_t* n, const double* lc, const double* hc) {
+    const int ndim = f->ndim, last = ndim - 1;
+    for (int d = 0; d < 3; ++d) {
+        if (d < ndim && n[d] < 1) return fail(LSM_ERR_ARG, "n[%d] = %d", d, n[d]);
+        f->nglob[d] = f->n[d] = d < ndim ? n[d] : 1;
+        f->lc[d] = (d < ndim && lc) ? lc[d] : 0.0;
+        f->hc[d] = (d < ndim && hc) ? hc[d] : 1.0;
+        f->h[d] = d < ndim ? (f->hc[d] - f->lc[d]) / double(f->nglob[d] - 1) : 1.0;    // meshes.jl:109-110
+        f->bc[d][0] = {LSM_BC_NONE, 0}; f->bc[d][1] = {LSM_BC_NONE, 0};
+    }
+    if (f->ctx->nranks > 1) slab_plan(f->nglob[last], f->ctx->nranks, f->ctx->rank, &f->first_last, &f->n[last]);
+    f->plane = 1; for (int d = 0; d < last; ++d) f->plane *= f->n[d];
+    f->owned = f->plane * f->n[last];
+    return LSM_OK;
+}
+
 int32_t field_alloc(lsm_ctx* ctx, int ndim, const int32_t* n, int dtype, int ncomp, const double* lc, const double* hc,
                     bool with_halo, lsm_field** out) {
     if (!ctx || !n || !out) return fail(LSM_ERR_ARG, "null argument");
@@ -186,24 +203,8 @@ int32_t field_alloc(lsm_ctx* ctx, int ndim, const int32_t* n, int dtype, int nco
     lsm_field* f = new (std::nothrow) lsm_field();
     if (!f) return fail(LSM_ERR_OOM, "host allocation failed");
     f->ctx = ctx; f->ndim = ndim; f->dtype = dtype; f->ncomp = ncomp;
-    for (int d = 0; d < 3; ++d) {
-        f->nglob[d] = d < ndim ? n[d] : 1;
-        f->n[d] = f->nglob[d];
-        f->lc[d] = (d < ndim && lc) ? lc[d] : 0.0;
-        f->hc[d] = (d < ndim && hc) ? hc[d] : 1.0;
-        if (d < ndim && n[d] < 1) { delete f; return fail(LSM_ERR_ARG, "n[%d] = %d", d, n[d]); }
-        f->h[d] = d < ndim ? (f->hc[d] - f->lc[d]) / double(f->nglob[d] - 1) : 1.0;    // meshes.jl:109-110
-        f->bc[d][0] = {LSM_BC_NONE, 0}; f->bc[d][1] = {LSM_BC_NONE, 0};
-    }
-    const int last = ndim - 1;
-    int first = 0, count = f->nglob[last];
-    if (ctx->nranks > 1) {
-        slab_plan(f->nglob[last], ctx->nranks, ctx->rank, &first, &count);
-        if (count < HALO + 1) { delete f; return fail(LSM_ERR_ARG, "slab of %d planes is thinner than %d; use fewer ranks", count, HALO + 1); }
-    }
-    f->first_last = first; f->n[last] = count;
-    f->plane = 1; for (int d = 0; d < last; ++d) f->plane *= f->n[d];
-    f->owned = f->plane * f->n[last];
+    if (const int32_t rc = grid_setup(f, n, lc, hc); rc != LSM_OK) { delete f; return rc; }
+    if (const int count = f->n[ndim - 1]; ctx->nranks > 1 && count < HALO + 1) { delete f; return fail(LSM_ERR_ARG, "slab of %d planes is thinner than %d; use fewer ranks", count, HALO + 1); }
     f->halo = (with_halo && ctx->nranks > 1 && ncomp == 1) ? HALO : 0;
     const long per_comp = f->owned + 2L * f->halo * f->plane;
     f->cstride = per_comp;
@@ -245,14 +246,47 @@ int32_t ctx_scratch(lsm_ctx* c, size_t bytes, void** out) {
     return LSM_OK;
 }
 
+enum class Reduce { none, max_u64, sum_f64 };
+
+// The one way a device result reaches the host: n 8-byte words at d_ptr, all-reduced over ranks by op, into h_scalar[0 .. n-1]
+int32_t read_back(lsm_ctx* c, void* d_ptr, int n, Reduce op) {
+    const bool mx = op == Reduce::max_u64;
+    if (op != Reduce::none && c->nranks > 1) NC(nccl().AllReduce(d_ptr, d_ptr, n, mx ? ncclUint64 : ncclDouble, mx ? ncclMax : ncclSum, c->nccl_comm, c->stream));
+    CU(cudaMemcpyAsync(c->h_scalar, d_ptr, 8 * n, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    c->cnt.d2h_bytes += 8 * n;
+    return LSM_OK;
+}
+
+// The boundary conditions of f and of its stage buffers, which always carry f's.  The caller decides about stale halos.
+void write_bcs(lsm_field* f, const lsm_bc (&bc)[3][2], bool has_bc) {
+    for (lsm_field* g : {f, f->buf1, f->buf2})
+        if (g) { std::memcpy(g->bc, bc, sizeof g->bc); g->has_bc = has_bc; }
+}
+
+// Gives f other boundary conditions for the life of the guard; f's own come back on every exit path, also on new stage buffers.
+struct BcOverride {
+    lsm_field* f; lsm_bc saved[3][2]; bool had;
+    BcOverride(lsm_field* f, const lsm_bc (&bc)[3][2], bool has_bc) : f(f), had(f->has_bc) { std::memcpy(saved, f->bc, sizeof saved); write_bcs(f, bc, has_bc); }
+    ~BcOverride() { write_bcs(f, saved, had); }
+};
+
+// phi's boundary conditions, or LinearExtrapolationBC on every side when it has none
+void bcs_or_linear_extrap(const lsm_field* phi, lsm_bc (&bc)[3][2]) {
+    std::memcpy(bc, phi->bc, sizeof bc);
+    if (!phi->has_bc) for (int d = 0; d < phi->ndim; ++d) bc[d][0] = bc[d][1] = {LSM_BC_EXTRAP, 1};
+}
+
+// f's data has changed: memos keyed on its version are stale, and so are its ghost planes
+void mark_written(lsm_field* f) { f->version++; f->halo_valid = false; }
+
 int32_t ensure_buffers(lsm_field* phi, int nbuf) {
     lsm_field** slots[2] = {&phi->buf1, &phi->buf2};
     for (int b = 0; b < nbuf; ++b) {
         if (*slots[b]) continue;
         lsm_field* nb = nullptr;
         TRY(field_alloc(phi->ctx, phi->ndim, phi->nglob, phi->dtype, 1, phi->lc, phi->hc, true, &nb));
-        std::memcpy(nb->bc, phi->bc, sizeof phi->bc);
-        nb->has_bc = phi->has_bc;
+        write_bcs(nb, phi->bc, phi->has_bc);
         *slots[b] = nb;
     }
     return LSM_OK;
@@ -286,6 +320,21 @@ double term_scale(const lsm_term& t, double time, const double* gscale, int k) {
     }
 }
 
+// A field that `what` reads or writes node by node: not null, of this context, with dense storage (not separable), one component.
+int32_t check_dense(const lsm_ctx* ctx, const lsm_field* f, const char* what) {
+    if (!ctx || !f) return fail(LSM_ERR_ARG, "%s: null argument", what);
+    if (f->ctx != ctx) return fail(LSM_ERR_ARG, "%s: the field belongs to another context", what);
+    if (f->separable || f->ncomp != 1) return fail(LSM_ERR_ARG, "%s needs a scalar field with stored values (ncomp = %d%s)", what, f->ncomp, f->separable ? ", separable" : "");
+    return LSM_OK;
+}
+
+// Two fields of one operation `what` have the same dimension and the same global node counts.
+int32_t check_same_shape(const lsm_field* a, const lsm_field* b, const char* what) {
+    bool same = a->ndim == b->ndim;
+    for (int d = 0; same && d < a->ndim; ++d) same = a->nglob[d] == b->nglob[d];
+    return same ? LSM_OK : fail(LSM_ERR_ARG, "%s: the fields differ in dimension or shape", what);
+}
+
 int32_t make_term_dev(const lsm_field* phi, const lsm_term& t, double g, TermDev* out) {
     TermDev d{};
     if (t.kind < LSM_TERM_ADVECTION || t.kind > LSM_TERM_EIKONAL) return fail(LSM_ERR_ARG, "bad term kind %d", t.kind);
@@ -300,10 +349,9 @@ int32_t make_term_dev(const lsm_field* phi, const lsm_term& t, double g, TermDev
         const lsm_field* cf = t.field;
         if (!cf) return fail(LSM_ERR_ARG, "coefficient field is NULL");
         if (cf->ctx != phi->ctx) return fail(LSM_ERR_ARG, "coefficient field belongs to another context");
+        TRY(check_same_shape(cf, phi, "coefficient field and state"));
         const int want = t.kind == LSM_TERM_ADVECTION ? phi->ndim : 1;
-        if (cf->ndim != phi->ndim || cf->ncomp != want) return fail(LSM_ERR_ARG, "coefficient field has ndim=%d ncomp=%d, expected %d/%d", cf->ndim, cf->ncomp, phi->ndim, want);
-        for (int a = 0; a < phi->ndim; ++a)
-            if (cf->nglob[a] != phi->nglob[a]) return fail(LSM_ERR_ARG, "coefficient field shape mismatch along dim %d", a + 1);
+        if (cf->ncomp != want) return fail(LSM_ERR_ARG, "coefficient field has ncomp=%d, expected %d", cf->ncomp, want);
         if (t.coef_kind == LSM_COEF_SEPARABLE) {
             if (!cf->separable) return fail(LSM_ERR_ARG, "LSM_COEF_SEPARABLE needs a field from lsm_field_create_separable");
             for (int c = 0; c < 3; ++c) { d.cval[c] = cf->scale[c]; for (int a = 0; a < 3; ++a) d.tab[c][a] = cf->tab[c][a]; }
@@ -333,7 +381,7 @@ int32_t expr_fill(lsm_field* f, double t, int cfl_kind) {
     cudaError_t e = launch_expr_fill(f->expr, A, c->sm_count, c->stream);
     if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "expression kernel launch failed: %s", cudaGetErrorString(e));
     c->cnt.kernel_launches += 1;
-    f->version++; f->halo_valid = false;
+    mark_written(f);
     f->expr_filled = true; f->expr_t = t; f->expr_ver = f->version;
     f->expr_cfl_kind = cfl_kind; f->expr_cfl_read = false;
     return LSM_OK;
@@ -512,10 +560,8 @@ void swap_storage(lsm_field* a, lsm_field* b) {
 }
 
 int32_t check_state(lsm_ctx* ctx, lsm_field* phi, const lsm_term* terms, int nterms) {
-    if (!ctx || !phi || !terms) return fail(LSM_ERR_ARG, "null argument");
-    if (phi->ctx != ctx) return fail(LSM_ERR_ARG, "field belongs to another context");
-    if (nterms < 1 || nterms > LSM_MAX_TERMS) return fail(LSM_ERR_ARG, "nterms must be in 1..%d", LSM_MAX_TERMS);
-    if (phi->ncomp != 1 || phi->separable) return fail(LSM_ERR_ARG, "the state must be a scalar field");
+    TRY(check_dense(ctx, phi, "the state"));
+    if (!terms || nterms < 1 || nterms > LSM_MAX_TERMS) return fail(LSM_ERR_ARG, "terms is null or nterms is not in 1..%d", LSM_MAX_TERMS);
     if (!phi->has_bc) return fail(LSM_ERR_BC, "no boundary conditions: call lsm_field_set_bc on the state");   // levelsetequation.jl:69-70
     CU(cudaSetDevice(ctx->device));
     return LSM_OK;
@@ -612,10 +658,8 @@ int32_t run_resident(lsm_ctx* ctx, int integ, lsm_field* phi, const lsm_term& te
         ctx->cnt.kernel_launches += 1; ctx->cnt.resident_steps += here;
     }
     phi->version++; phi->halo_valid = true;
-    CU(cudaMemcpyAsync(ctx->h_scalar + 2, R.status, 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));                    // lsm_integrate returns synchronised anyway
-    ctx->cnt.d2h_bytes += 8;
-    if (ctx->h_scalar[2] != 0ULL) return fail(LSM_ERR_CUDA, "resident kernel: halo protocol failure (status %llu); the state is not valid", ctx->h_scalar[2]);
+    TRY(read_back(ctx, R.status, 1, Reduce::none));            // lsm_integrate returns synchronised anyway
+    if (ctx->h_scalar[0] != 0ULL) return fail(LSM_ERR_CUDA, "resident kernel: halo protocol failure (status %llu); the state is not valid", ctx->h_scalar[0]);
     return LSM_OK;
 }
 
@@ -670,11 +714,8 @@ int32_t full_cfl_pass(lsm_ctx* ctx, lsm_field* phi, const TermDev& td, unsigned 
     cudaError_t e = launch_cfl(phi->ndim, phi->dtype == LSM_F64, P, ctx->sm_count, ctx->stream);
     if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "CFL kernel launch failed: %s", cudaGetErrorString(e));
     ctx->cnt.kernel_launches += 1; ctx->cnt.cfl_passes += 1;
-    if (ctx->nranks > 1) NC(nccl().AllReduce(ctx->d_scalar, ctx->d_scalar, 1, ncclUint64, ncclMax, ctx->nccl_comm, ctx->stream));
-    CU(cudaMemcpyAsync(ctx->h_scalar, ctx->d_scalar, 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    ctx->cnt.d2h_bytes += 8;
-    *bits_out = *ctx->h_scalar;
+    TRY(read_back(ctx, ctx->d_scalar, 1, Reduce::max_u64));
+    *bits_out = ctx->h_scalar[0];
     return LSM_OK;
 }
 
@@ -777,11 +818,8 @@ double bits_to_double(unsigned long long b) { double d; std::memcpy(&d, &b, 8); 
 int32_t expr_cfl_bits(lsm_ctx* ctx, lsm_field* f, double t, int term_kind, unsigned long long* bits_out) {
     TRY(expr_ensure(f, t, term_kind, true));
     if (!f->expr_cfl_read) {
-        if (ctx->nranks > 1) NC(nccl().AllReduce(f->d_expr_cfl, f->d_expr_cfl, 1, ncclUint64, ncclMax, ctx->nccl_comm, ctx->stream));
-        CU(cudaMemcpyAsync(ctx->h_scalar + 3, f->d_expr_cfl, 8, cudaMemcpyDeviceToHost, ctx->stream));
-        CU(cudaStreamSynchronize(ctx->stream));
-        ctx->cnt.d2h_bytes += 8;
-        f->expr_cfl_bits = ctx->h_scalar[3];
+        TRY(read_back(ctx, f->d_expr_cfl, 1, Reduce::max_u64));
+        f->expr_cfl_bits = ctx->h_scalar[0];
         f->expr_cfl_read = true;
     }
     *bits_out = f->expr_cfl_bits;
@@ -835,8 +873,7 @@ int32_t compute_cfl_impl(lsm_ctx* ctx, lsm_field* phi, const lsm_term* terms, in
 // The checks every operation on a level set makes: a real-valued field of this context with at least min_n nodes along every
 // dimension and, for the operations that have no multi-rank form, a context of one rank.  `what` names the operation.
 int32_t check_level_set(lsm_ctx* ctx, const lsm_field* phi, const char* what, int min_n, bool single_rank) {
-    if (!ctx || !phi) return fail(LSM_ERR_ARG, "null argument");
-    if (phi->ctx != ctx || phi->ncomp != 1 || phi->separable) return fail(LSM_ERR_ARG, "%s needs a real-valued field of this context", what);
+    TRY(check_dense(ctx, phi, what));
     for (int d = 0; d < phi->ndim; ++d)
         if (phi->nglob[d] < min_n)
             return fail(LSM_ERR_ARG, "%s needs at least %d nodes along every dimension (n[%d] = %d)", what, min_n, d, phi->nglob[d]);
@@ -908,11 +945,10 @@ int32_t si_step(lsm_ctx* ctx, lsm_field* phi, const lsm_term* terms, int nterms,
 // A second field F of an operation on phi (checked by check_level_set too) must lie on phi's grid: same node counts, same owned
 // slab, same lower corner and spacing.
 int32_t check_same_grid(const lsm_field* F, const lsm_field* phi) {
-    bool same = F->ndim == phi->ndim;
+    bool same = check_same_shape(F, phi, "F and phi") == LSM_OK;
     for (int d = 0; same && d < phi->ndim; ++d)
-        same = F->nglob[d] == phi->nglob[d] && F->n[d] == phi->n[d] && F->lc[d] == phi->lc[d] && F->h[d] == phi->h[d];
-    if (!same) return fail(LSM_ERR_ARG, "F and phi must be on the same grid (n, lc and h)");
-    return LSM_OK;
+        same = F->n[d] == phi->n[d] && F->lc[d] == phi->lc[d] && F->h[d] == phi->h[d];
+    return same ? LSM_OK : fail(LSM_ERR_ARG, "F and phi must be on the same grid (n, lc and h)");
 }
 
 // The node box of phi for the kernels: this rank's owned nodes and, with `ghost`, the first plane of the next rank.  Level 0,
@@ -931,14 +967,6 @@ IfaceArgs field_box(const lsm_field* phi, bool ghost) {
     A.nodes = (long long)A.m[0] * A.m[1] * A.m[2];
     A.lin0 = (long long)phi->first_last * phi->plane;
     return A;
-}
-
-// one synchronisation and one copy of n adjacent 8-byte device counters into ctx->h_scalar[0 .. n-1]
-int32_t read_counts(lsm_ctx* ctx, const void* d_counts, int n) {
-    CU(cudaMemcpyAsync(ctx->h_scalar, d_counts, 8 * n, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    ctx->cnt.d2h_bytes += 8 * n;
-    return LSM_OK;
 }
 
 // The closest-point passes on phi (checked by the caller): the extension of F unless F is null, redistancing of phi when write_phi
@@ -969,10 +997,10 @@ int32_t closest_points(lsm_ctx* ctx, lsm_field* phi, int32_t band, lsm_field* F,
     int launches = 0;
     CU(launch_closest_points(R, ctx->sm_count, ctx->stream, &launches));
     ctx->cnt.kernel_launches += launches;
-    if (F) { F->version++; F->halo_valid = false; }
-    if (R.write_phi) { phi->version++; phi->halo_valid = false; }
+    if (F) mark_written(F);
+    if (R.write_phi) mark_written(phi);
     if (band_nodes_out || fallback_nodes_out) {
-        TRY(read_counts(ctx, R.count, cubic ? 2 : 1));
+        TRY(read_back(ctx, R.count, cubic ? 2 : 1, Reduce::none));
         if (band_nodes_out) *band_nodes_out = (int64_t)ctx->h_scalar[0];
         if (fallback_nodes_out) *fallback_nodes_out = (int64_t)ctx->h_scalar[1];
     }
@@ -1246,18 +1274,10 @@ int32_t lsm_field_create_separable(lsm_ctx* ctx, int32_t ndim, const int32_t* n,
     lsm_field* f = new (std::nothrow) lsm_field();
     if (!f) return fail(LSM_ERR_OOM, "host allocation failed");
     f->ctx = ctx; f->ndim = ndim; f->dtype = LSM_F64; f->ncomp = ndim; f->separable = true;
+    if (const int32_t rc = grid_setup(f, n, lc, hc); rc != LSM_OK) { delete f; return rc; }
     long tot = 0;
-    for (int d = 0; d < 3; ++d) {
-        f->nglob[d] = d < ndim ? n[d] : 1; f->n[d] = f->nglob[d];
-        f->lc[d] = (d < ndim && lc) ? lc[d] : 0; f->hc[d] = (d < ndim && hc) ? hc[d] : 1;
-        f->h[d] = d < ndim ? (f->hc[d] - f->lc[d]) / double(f->nglob[d] - 1) : 1.0;
-        f->scale[d] = d < ndim ? scale[d] : 0.0;
-        if (d < ndim) tot += n[d];
-    }
-    const int last = ndim - 1;
-    int first = 0, count = f->nglob[last];
-    if (ctx->nranks > 1) slab_plan(f->nglob[last], ctx->nranks, ctx->rank, &first, &count);
-    f->first_last = first; f->n[last] = count;
+    for (int d = 0; d < 3; ++d) { f->scale[d] = d < ndim ? scale[d] : 0.0; tot += d < ndim ? n[d] : 0; }
+    const int last = ndim - 1, first = f->first_last;
     const size_t bytes = (size_t)tot * ndim * sizeof(double);
     cudaError_t e = cudaMalloc(&f->d_tabs, bytes);
     if (e != cudaSuccess) { delete f; return fail(LSM_ERR_OOM, "cudaMalloc failed: %s", cudaGetErrorString(e)); }
@@ -1288,6 +1308,8 @@ int32_t lsm_field_destroy(lsm_field* f) {
 
 int32_t lsm_field_set_bc(lsm_field* f, const lsm_bc* bc) {
     if (!f || !bc) return fail(LSM_ERR_ARG, "null argument");
+    lsm_bc nb[3][2];
+    std::memcpy(nb, f->bc, sizeof nb);
     for (int d = 0; d < f->ndim; ++d) {
         const lsm_bc l = bc[2 * d], r = bc[2 * d + 1];
         for (const lsm_bc& b : {l, r}) {
@@ -1296,11 +1318,10 @@ int32_t lsm_field_set_bc(lsm_field* f, const lsm_bc* bc) {
         }
         if ((l.kind == LSM_BC_PERIODIC) != (r.kind == LSM_BC_PERIODIC))     // boundaryconditions.jl:184-186
             return fail(LSM_ERR_BC, "periodic boundary conditions cannot be mixed with others in dimension %d", d + 1);
+        nb[d][0] = l; nb[d][1] = r;
     }
-    for (int d = 0; d < f->ndim; ++d) { f->bc[d][0] = bc[2 * d]; f->bc[d][1] = bc[2 * d + 1]; }
-    f->has_bc = true;
-    f->halo_valid = false;
-    for (lsm_field* b : {f->buf1, f->buf2}) if (b) { std::memcpy(b->bc, f->bc, sizeof f->bc); b->has_bc = true; b->halo_valid = false; }
+    write_bcs(f, nb, true);
+    for (lsm_field* g : {f, f->buf1, f->buf2}) if (g) g->halo_valid = false;
     return LSM_OK;
 }
 
@@ -1319,8 +1340,8 @@ int32_t lsm_field_meshsize(const lsm_field* f, double* h_out) {
 
 int32_t lsm_field_getindex(lsm_field* f, const int32_t* I, int32_t count, double* out) {
     if (!f || !I || !out || count < 1) return fail(LSM_ERR_ARG, "bad argument");
-    if (f->separable || f->ncomp != 1) return fail(LSM_ERR_ARG, "getindex needs a scalar dense field");
     lsm_ctx* c = f->ctx;
+    TRY(check_dense(c, f, "lsm_field_getindex"));
     if (c->nranks > 1) return fail(LSM_ERR_UNSUPPORTED, "lsm_field_getindex is single-rank only");
     CU(cudaSetDevice(c->device));
     // in-grid reads need no BC; out-of-grid reads without BCs throw in the reference (meshfield.jl:222-232)
@@ -1344,7 +1365,7 @@ int32_t lsm_field_getindex(lsm_field* f, const int32_t* I, int32_t count, double
 
 int32_t lsm_field_stage_buffer(lsm_field* phi, int32_t which, lsm_field** out) {
     if (!phi || !out || (which != 1 && which != 2)) return fail(LSM_ERR_ARG, "bad argument");
-    if (phi->ncomp != 1 || phi->separable) return fail(LSM_ERR_ARG, "not a state field");
+    TRY(check_dense(phi->ctx, phi, "lsm_field_stage_buffer"));
     CU(cudaSetDevice(phi->ctx->device));
     TRY(ensure_buffers(phi, which));
     *out = which == 1 ? phi->buf1 : phi->buf2;
@@ -1410,7 +1431,7 @@ int32_t lsm_field_upload(lsm_field* f, const void* host) {
         TRY(staged_vector_transfer(f, const_cast<void*>(host), true));
     }
     c->cnt.h2d_bytes += (int64_t)bytes;
-    f->version++; f->halo_valid = false;
+    mark_written(f);
     return LSM_OK;
 }
 
@@ -1434,9 +1455,9 @@ int32_t lsm_field_download(lsm_field* f, void* host) {
 int32_t lsm_field_copy(lsm_field* dst, const lsm_field* src) {
     if (!dst || !src) return fail(LSM_ERR_ARG, "null argument");
     if (dst->separable || src->separable) return fail(LSM_ERR_ARG, "separable fields cannot be copied");
-    if (dst->ctx != src->ctx || dst->ndim != src->ndim || dst->dtype != src->dtype || dst->ncomp != src->ncomp)
+    if (dst->ctx != src->ctx || dst->dtype != src->dtype || dst->ncomp != src->ncomp)
         return fail(LSM_ERR_ARG, "copy between incompatible fields");
-    for (int d = 0; d < dst->ndim; ++d) if (dst->nglob[d] != src->nglob[d]) return fail(LSM_ERR_ARG, "copy between fields of different shape");
+    TRY(check_same_shape(dst, src, "lsm_field_copy"));
     lsm_ctx* c = dst->ctx;
     CU(cudaSetDevice(c->device));
     for (int k = 0; k < dst->ncomp; ++k) {
@@ -1444,7 +1465,7 @@ int32_t lsm_field_copy(lsm_field* dst, const lsm_field* src) {
         char* d = static_cast<char*>(dst->p) + (size_t)k * dst->cstride * esize(dst->dtype);
         CU(cudaMemcpyAsync(d, s, (size_t)dst->owned * esize(dst->dtype), cudaMemcpyDeviceToDevice, c->stream));
     }
-    dst->version++; dst->halo_valid = false;
+    mark_written(dst);
     return LSM_OK;
 }
 
@@ -1491,8 +1512,12 @@ int32_t lsm_integrate(lsm_ctx* ctx, int32_t integrator, double cfl, lsm_field* p
     if (integrator == LSM_SEMI_IMPLICIT) TRY(si_check(ctx, phi, terms, nterms));      // before any collective CFL reduction
     double tc = t0;
     int64_t steps = 0;
-    bool finished = true;
+    bool finished = true;           // false: stopped by max_steps
     int32_t rc = LSM_OK;
+    auto step = [&](double dt) -> int32_t {
+        for (int s = 1; s <= nstages(integrator); ++s) TRY(stage_impl(ctx, integrator, s, phi, terms, nterms, tc, dt, nullptr));
+        return LSM_OK;
+    };
     // Launch-bound regime (small grids: a stage kernel lasts a few microseconds, comparable to its launch): when nothing but the
     // state changes from step to step — single rank, RK2/RK3 (whose buffers do not rotate), terms without a time factor, no
     // per-stage timing — the stage launches of one step are captured once into a CUDA graph and every later step with the same
@@ -1511,11 +1536,10 @@ int32_t lsm_integrate(lsm_ctx* ctx, int32_t integrator, double cfl, lsm_field* p
     // the loop's arithmetic and hands the kernel the run-length encoded sequence.  Whatever is left (max_steps, more than
     // RES_STEP_CAP steps, a launch that is not possible) is done by the regular loop below.
     if (integrator != LSM_SEMI_IMPLICIT && resident_eligible(ctx, phi, terms, nterms) && tc <= tf - jl_eps(tc) && (max_steps < 0 || max_steps > 0)) {
-        double dt_cfl;
+        double dt_cfl = 0.0;
         rc = compute_cfl_impl(ctx, phi, terms, nterms, tc, nullptr, &dt_cfl);
-        if (rc != LSM_OK) { if (t_out) *t_out = tc; if (steps_out) *steps_out = 0; return rc; }
         const double D = jl_min(dt_max, cfl * dt_cfl);
-        if (std::isfinite(D) && D > 0.0) {
+        if (rc == LSM_OK && std::isfinite(D) && D > 0.0) {
             constexpr int64_t RES_STEP_CAP = 1 << 22;
             std::vector<std::pair<double, long>> runs;
             double t = tc; int64_t n = 0;
@@ -1523,18 +1547,18 @@ int32_t lsm_integrate(lsm_ctx* ctx, int32_t integrator, double cfl, lsm_field* p
             int32_t rr = phi->dtype == LSM_F64 ? run_resident<double>(ctx, integrator, phi, terms[0], runs)
                                                : run_resident<float>(ctx, integrator, phi, terms[0], runs);
             if (rr == LSM_OK) { tc = t; steps = n; }
-            else if (rr != LSM_ERR_UNSUPPORTED) { if (t_out) *t_out = tc; if (steps_out) *steps_out = 0; return rr; }
+            else if (rr != LSM_ERR_UNSUPPORTED) rc = rr;
         }
     }
-    while (tc <= tf - jl_eps(tc)) {                                   // timestepping.jl:104
+    while (rc == LSM_OK && tc <= tf - jl_eps(tc)) {                   // timestepping.jl:104
         if (max_steps >= 0 && steps >= max_steps) { finished = false; break; }
         double dt_cfl;
         rc = compute_cfl_impl(ctx, phi, terms, nterms, tc, nullptr, &dt_cfl);
-        if (rc != LSM_OK) { finished = false; break; }
+        if (rc != LSM_OK) break;
         const double dt = jl_min(jl_min(dt_max, cfl * dt_cfl), tf - tc);   // timestepping.jl:111
         if (gexec && dt == gdt) {
             cudaError_t ge = cudaGraphLaunch(gexec, ctx->stream);
-            if (ge != cudaSuccess) { rc = fail(LSM_ERR_CUDA, "cudaGraphLaunch failed: %s", cudaGetErrorString(ge)); finished = false; break; }
+            if (ge != cudaSuccess) { rc = fail(LSM_ERR_CUDA, "cudaGraphLaunch failed: %s", cudaGetErrorString(ge)); break; }
             ctx->cnt.kernel_launches += gdelta.kernel_launches; ctx->cnt.stage_launches += gdelta.stage_launches;
             phi->version += gver[0]; if (phi->buf1) phi->buf1->version += gver[1]; if (phi->buf2) phi->buf2->version += gver[2];
             tc += dt;
@@ -1547,7 +1571,7 @@ int32_t lsm_integrate(lsm_ctx* ctx, int32_t integrator, double cfl, lsm_field* p
         uint64_t vb[3] = {phi->version, phi->buf1 ? phi->buf1->version : 0, phi->buf2 ? phi->buf2->version : 0};
         if (capture && cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) { cudaGetLastError(); graph_ok = false; }
         const bool capturing = capture && graph_ok;
-        for (int s = 1; s <= nstages(integrator) && rc == LSM_OK; ++s) rc = stage_impl(ctx, integrator, s, phi, terms, nterms, tc, dt, nullptr);
+        rc = step(dt);
         if (capturing) {
             cudaGraph_t graph = nullptr;
             cudaError_t ge = cudaStreamEndCapture(ctx->stream, &graph);
@@ -1565,18 +1589,17 @@ int32_t lsm_integrate(lsm_ctx* ctx, int32_t integrator, double cfl, lsm_field* p
                 if (gexec) { cudaGraphExecDestroy(gexec); gexec = nullptr; }
                 graph_ok = false;
                 ctx->cnt = before;
-                rc = LSM_OK;
-                for (int s = 1; s <= nstages(integrator) && rc == LSM_OK; ++s) rc = stage_impl(ctx, integrator, s, phi, terms, nterms, tc, dt, nullptr);
+                rc = step(dt);
             }
         }
-        if (rc != LSM_OK) { finished = false; break; }
+        if (rc != LSM_OK) break;
         tc += dt;
         ++steps;
     }
     if (gexec) { cudaStreamSynchronize(ctx->stream); cudaGraphExecDestroy(gexec); }
     cudaStreamSynchronize(ctx->comm);
     cudaError_t e = cudaStreamSynchronize(ctx->stream);
-    if (t_out) *t_out = finished ? tf : tc;                           // timestepping.jl:120
+    if (t_out) *t_out = finished && rc == LSM_OK ? tf : tc;           // timestepping.jl:120
     if (steps_out) *steps_out = steps;
     if (rc != LSM_OK) return rc;
     if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "device error during integration: %s", cudaGetErrorString(e));
@@ -1589,51 +1612,40 @@ int32_t lsm_semi_implicit_sweeps(double courant, int32_t dtype, int64_t* sweeps_
 }
 
 int32_t lsm_eikonal_s0(lsm_field* dst, const lsm_field* phi0) {
-    if (!dst || !phi0) return fail(LSM_ERR_ARG, "null argument");
-    if (dst->ctx != phi0->ctx || dst->ndim != phi0->ndim || dst->ncomp != 1 || phi0->ncomp != 1 || dst->separable || phi0->separable)
-        return fail(LSM_ERR_ARG, "incompatible fields");
-    for (int d = 0; d < dst->ndim; ++d) if (dst->nglob[d] != phi0->nglob[d]) return fail(LSM_ERR_ARG, "shape mismatch");
-    lsm_ctx* c = dst->ctx;
+    lsm_ctx* c = dst ? dst->ctx : nullptr;
+    TRY(check_dense(c, dst, "lsm_eikonal_s0"));
+    TRY(check_dense(c, phi0, "lsm_eikonal_s0"));
+    TRY(check_same_shape(dst, phi0, "lsm_eikonal_s0"));
     CU(cudaSetDevice(c->device));
     double dx = phi0->h[0];
     for (int d = 1; d < phi0->ndim; ++d) dx = std::min(dx, phi0->h[d]);
     cudaError_t e = launch_eikonal_s0(phi0->dtype == LSM_F64, dst->dtype == LSM_F64, phi0->p, dst->p, phi0->owned, dx, c->stream);
     if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
     c->cnt.kernel_launches += 1;
-    dst->version++; dst->halo_valid = false;
+    mark_written(dst);
     return LSM_OK;
 }
 
 static int32_t measure_impl(lsm_ctx* ctx, lsm_field* phi, bool perimeter, double* out) {
-    if (!ctx || !phi || !out) return fail(LSM_ERR_ARG, "null argument");
-    if (phi->ctx != ctx || phi->ncomp != 1 || phi->separable) return fail(LSM_ERR_ARG, "volume/perimeter need a real-valued field of this context");
+    if (!out) return fail(LSM_ERR_ARG, "null argument");
+    TRY(check_dense(ctx, phi, perimeter ? "lsm_perimeter" : "lsm_volume"));
     CU(cudaSetDevice(ctx->device));
     CU(cudaStreamSynchronize(ctx->comm));
     const int nblocks = ctx->sm_count * 8;
     void* work = nullptr;
     TRY(ctx_scratch(ctx, sizeof(double) * (size_t)(nblocks + 1), &work));      // persistent: a posthook payload must not cudaMalloc per call
     double* d_part = static_cast<double*>(work);
-    cudaError_t e;
     // perimeter reaches off-grid at the border: a field without BCs gets LinearExtrapolationBC (levelsetops.jl:142)
-    lsm_bc saved[3][2];
-    std::memcpy(saved, phi->bc, sizeof saved);
-    const bool had_bc = phi->has_bc;
-    if (perimeter && !had_bc) for (int d = 0; d < phi->ndim; ++d) { phi->bc[d][0] = {LSM_BC_EXTRAP, 1}; phi->bc[d][1] = {LSM_BC_EXTRAP, 1}; }
-    if (perimeter && ctx->nranks > 1 && !phi->halo_valid) {
-        int32_t rc = exchange_halo(phi, ctx->stream);
-        if (rc != LSM_OK) return rc;
-    }
-    if (phi->dtype == LSM_F64) e = launch_measure<double>(phi->ndim, perimeter, make_view<double>(phi), phi->h, d_part, nblocks, d_part + nblocks, ctx->stream);
-    else e = launch_measure<float>(phi->ndim, perimeter, make_view<float>(phi), phi->h, d_part, nblocks, d_part + nblocks, ctx->stream);
-    std::memcpy(phi->bc, saved, sizeof saved);
-    if (e == cudaSuccess && ctx->nranks > 1) {
-        ncclResult_t r = nccl().AllReduce(d_part + nblocks, d_part + nblocks, 1, ncclDouble, ncclSum, ctx->nccl_comm, ctx->stream);
-        if (r != ncclSuccess) return fail(LSM_ERR_NCCL, "ncclAllReduce failed: %s", nccl().GetErrorString(r));
-    }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(out, d_part + nblocks, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    lsm_bc bc[3][2];
+    bcs_or_linear_extrap(phi, bc);
+    BcOverride keep(phi, bc, phi->has_bc);
+    if (perimeter && ctx->nranks > 1 && !phi->halo_valid) TRY(exchange_halo(phi, ctx->stream));
+    const cudaError_t e = phi->dtype == LSM_F64 ? launch_measure<double>(phi->ndim, perimeter, make_view<double>(phi), phi->h, d_part, nblocks, d_part + nblocks, ctx->stream)
+                                                : launch_measure<float>(phi->ndim, perimeter, make_view<float>(phi), phi->h, d_part, nblocks, d_part + nblocks, ctx->stream);
     if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "measure kernel failed: %s", cudaGetErrorString(e));
-    ctx->cnt.kernel_launches += 2; ctx->cnt.d2h_bytes += 8;
+    TRY(read_back(ctx, d_part + nblocks, 1, Reduce::sum_f64));
+    ctx->cnt.kernel_launches += 2;
+    *out = bits_to_double(ctx->h_scalar[0]);
     return LSM_OK;
 }
 int32_t lsm_volume(lsm_ctx* ctx, lsm_field* phi, double* out) { return measure_impl(ctx, phi, false, out); }
@@ -1641,31 +1653,22 @@ int32_t lsm_perimeter(lsm_ctx* ctx, lsm_field* phi, double* out) { return measur
 
 int32_t lsm_extend_along_normals(lsm_ctx* ctx, lsm_field* F, lsm_field* phi, int32_t nb_iters, double cfl, const uint8_t* frozen,
                                  double interface_band, double min_norm) {
-    if (!ctx || !F || !phi) return fail(LSM_ERR_ARG, "null argument");
-    if (F->ctx != ctx || phi->ctx != ctx || F == phi || F->ncomp != 1 || phi->ncomp != 1 || F->separable || phi->separable)
-        return fail(LSM_ERR_ARG, "F and phi must be distinct scalar fields of this context");
-    if (F->ndim != phi->ndim || F->dtype != phi->dtype) return fail(LSM_ERR_ARG, "F and phi must be defined on the same mesh with the same valtype");
-    for (int d = 0; d < F->ndim; ++d) if (F->nglob[d] != phi->nglob[d]) return fail(LSM_ERR_ARG, "F and phi must have the same size");
+    for (const lsm_field* f : {F, phi}) TRY(check_dense(ctx, f, "lsm_extend_along_normals"));
+    if (F == phi) return fail(LSM_ERR_ARG, "the extended field F must not be phi");
+    TRY(check_same_shape(F, phi, "lsm_extend_along_normals"));
+    if (F->dtype != phi->dtype) return fail(LSM_ERR_ARG, "F and phi must have the same valtype");
     if (nb_iters < 0) return fail(LSM_ERR_ARG, "nb_iters must be non-negative");
     if (!(cfl > 0)) return fail(LSM_ERR_ARG, "cfl must be strictly positive");
     if (interface_band < 0 || min_norm < 0) return fail(LSM_ERR_ARG, "interface_band and min_norm must be non-negative");
     CU(cudaSetDevice(ctx->device));
     // boundary conditions: phi's, or LinearExtrapolationBC everywhere (velocityextension.jl:38-43); F gets the same
-    lsm_bc savedP[3][2], savedF[3][2];
-    std::memcpy(savedP, phi->bc, sizeof savedP); std::memcpy(savedF, F->bc, sizeof savedF);
-    const bool hadP = phi->has_bc, hadF = F->has_bc;
-    if (!hadP) for (int d = 0; d < phi->ndim; ++d) { phi->bc[d][0] = {LSM_BC_EXTRAP, 1}; phi->bc[d][1] = {LSM_BC_EXTRAP, 1}; }
-    std::memcpy(F->bc, phi->bc, sizeof savedF);
-    F->has_bc = true; F->halo_valid = false;
-    for (lsm_field* b : {F->buf1, F->buf2}) if (b) { std::memcpy(b->bc, F->bc, sizeof savedF); b->has_bc = true; }
-    auto restore = [&]() {
-        std::memcpy(phi->bc, savedP, sizeof savedP);
-        std::memcpy(F->bc, savedF, sizeof savedF); F->has_bc = hadF; F->halo_valid = false;
-        for (lsm_field* b : {F->buf1, F->buf2}) if (b) { std::memcpy(b->bc, F->bc, sizeof savedF); b->has_bc = hadF; }
-    };
+    lsm_bc bc[3][2];
+    bcs_or_linear_extrap(phi, bc);
+    BcOverride keep_phi(phi, bc, phi->has_bc), keep_F(F, bc, true);
+    F->halo_valid = false;
     lsm_field* vel = nullptr;
     int32_t rc = field_alloc(ctx, phi->ndim, phi->nglob, phi->dtype, phi->ndim, phi->lc, phi->hc, false, &vel);
-    if (rc != LSM_OK) { restore(); return rc; }
+    if (rc != LSM_OK) return rc;
     unsigned char* d_frozen = nullptr;
     cudaError_t e = cudaSuccess;
     if (frozen) {
@@ -1696,7 +1699,7 @@ int32_t lsm_extend_along_normals(lsm_ctx* ctx, lsm_field* F, lsm_field* phi, int
     cudaError_t e2 = cudaStreamSynchronize(ctx->stream);
     if (d_frozen) cudaFree(d_frozen);
     field_free(vel);
-    restore();
+    F->halo_valid = false;          // its ghost planes follow the boundary conditions the guard is about to restore
     if (rc != LSM_OK) return rc;
     if (e != cudaSuccess || e2 != cudaSuccess) return fail(LSM_ERR_CUDA, "extend_along_normals failed: %s", cudaGetErrorString(e != cudaSuccess ? e : e2));
     F->version++;
@@ -1719,7 +1722,7 @@ int32_t lsm_interface_extract(lsm_ctx* ctx, lsm_field* phi, double level, int64_
     void* work = nullptr;
     TRY(ctx_scratch(ctx, iface_scratch_bytes(A.ntiles), &work));
     CU(launch_iface(A, 0, work, nullptr, nullptr, nullptr, ctx->stream));
-    TRY(read_counts(ctx, iface_totals(A, work), 2));
+    TRY(read_back(ctx, iface_totals(A, work), 2, Reduce::none));
     ctx->cnt.kernel_launches += 2;
     const int64_t nv = (int64_t)ctx->h_scalar[0], np = (int64_t)ctx->h_scalar[1];
     if (nv > (int64_t)std::numeric_limits<int32_t>::max())
@@ -1838,7 +1841,7 @@ int32_t lsm_level_set_integrals(lsm_ctx* ctx, lsm_field* phi, lsm_field* F, doub
     if (ctx->nranks > 1) NC(nccl().AllReduce(I.part, I.part, (size_t)(4 * nplanes), ncclDouble, ncclSum, ctx->nccl_comm, ctx->stream));
     CU(launch_integral_sum(I.part, nplanes, res, ctx->stream));
     ctx->cnt.kernel_launches += 2;
-    TRY(read_counts(ctx, res, 4));
+    TRY(read_back(ctx, res, 4, Reduce::none));
     std::memcpy(out, ctx->h_scalar, 4 * sizeof(double));
     if (!F) out[2] = out[3] = std::numeric_limits<double>::quiet_NaN();
     return LSM_OK;
@@ -1854,19 +1857,17 @@ int32_t lsm_multi_level_set_integrals(int32_t n, lsm_ctx* const* ctx, lsm_field*
 }
 
 int32_t lsm_field_csg(lsm_ctx* ctx, lsm_field* dst, const lsm_field* src, int32_t op) {
-    if (!ctx || !dst) return fail(LSM_ERR_ARG, "null argument");
+    TRY(check_dense(ctx, dst, "lsm_field_csg"));
     if (op < LSM_CSG_UNION || op > LSM_CSG_COMPLEMENT) return fail(LSM_ERR_ARG, "unknown set operation %d", op);
-    if (dst->ctx != ctx || dst->ncomp != 1 || dst->separable) return fail(LSM_ERR_ARG, "set operations need a real-valued field of this context");
     if (op != LSM_CSG_COMPLEMENT) {
-        if (!src) return fail(LSM_ERR_ARG, "null argument");
-        if (src->ctx != ctx || src->ncomp != 1 || src->separable || src->ndim != dst->ndim || src->dtype != dst->dtype)
-            return fail(LSM_ERR_ARG, "set operation between incompatible fields");
-        for (int d = 0; d < dst->ndim; ++d) if (dst->nglob[d] != src->nglob[d]) return fail(LSM_ERR_ARG, "set operation between fields of different shape");
+        TRY(check_dense(ctx, src, "lsm_field_csg"));
+        TRY(check_same_shape(dst, src, "lsm_field_csg"));
+        if (src->dtype != dst->dtype) return fail(LSM_ERR_ARG, "set operation between fields of different valtype");
     }
     CU(cudaSetDevice(ctx->device));
     CU(launch_csg(dst->dtype == LSM_F64, dst->p, op == LSM_CSG_COMPLEMENT ? nullptr : src->p, dst->owned, op, ctx->stream));
     ctx->cnt.kernel_launches += 1;
-    dst->version++; dst->halo_valid = false;
+    mark_written(dst);
     return LSM_OK;
 }
 
@@ -1886,21 +1887,21 @@ int32_t lsm_field_fill_shape(lsm_field* f, int32_t shape, const double* params, 
     cudaError_t e = launch_fill_shape(f->dtype == LSM_F64, f->p, P, ctx->stream);
     if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
     ctx->cnt.kernel_launches += 1;
-    f->version++; f->halo_valid = false;
+    mark_written(f);
     return LSM_OK;
 }
 
 int32_t lsm_field_fill_separable(lsm_field* dst, const lsm_field* sep) {
     if (!dst || !sep) return fail(LSM_ERR_ARG, "null argument");
     if (!sep->separable || dst->separable) return fail(LSM_ERR_ARG, "lsm_field_fill_separable(dst, sep): sep must come from lsm_field_create_separable, dst must be a stored field");
-    if (dst->ctx != sep->ctx || dst->ndim != sep->ndim || dst->ncomp != sep->ndim) return fail(LSM_ERR_ARG, "destination must be a vector field of the same context and dimension");
-    for (int d = 0; d < dst->ndim; ++d) if (dst->nglob[d] != sep->nglob[d]) return fail(LSM_ERR_ARG, "shape mismatch along dim %d", d + 1);
+    if (dst->ctx != sep->ctx || dst->ncomp != sep->ndim) return fail(LSM_ERR_ARG, "destination must be a vector field of the same context and dimension");
+    TRY(check_same_shape(dst, sep, "lsm_field_fill_separable"));
     lsm_ctx* ctx = dst->ctx;
     CU(cudaSetDevice(ctx->device));
     cudaError_t e = launch_fill_separable(dst->dtype == LSM_F64, dst->p, dst->cstride, dst->n, dst->ndim, sep->scale, sep->tab, ctx->stream);
     if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
     ctx->cnt.kernel_launches += 1;
-    dst->version++; dst->halo_valid = false;
+    mark_written(dst);
     return LSM_OK;
 }
 
@@ -1934,20 +1935,18 @@ int32_t lsm_field_fill_expr(lsm_field* f, double t) {
 }
 
 int32_t lsm_max_abs_diff(lsm_ctx* ctx, const lsm_field* a, const lsm_field* b, double* out) {
-    if (!ctx || !a || !b || !out) return fail(LSM_ERR_ARG, "null argument");
-    if (a->ctx != ctx || b->ctx != ctx || a->dtype != b->dtype || a->ncomp != 1 || b->ncomp != 1 || a->owned != b->owned)
-        return fail(LSM_ERR_ARG, "incompatible fields");
+    if (!out) return fail(LSM_ERR_ARG, "null argument");
+    for (const lsm_field* f : {a, b}) TRY(check_dense(ctx, f, "lsm_max_abs_diff"));
+    TRY(check_same_shape(a, b, "lsm_max_abs_diff"));
+    if (a->dtype != b->dtype) return fail(LSM_ERR_ARG, "lsm_max_abs_diff: the fields differ in valtype");
     CU(cudaSetDevice(ctx->device));
     CU(cudaStreamSynchronize(ctx->comm));
     CU(cudaMemsetAsync(ctx->d_scalar, 0, 8, ctx->stream));
     cudaError_t e = launch_max_abs_diff(a->dtype == LSM_F64, a->p, b->p, a->owned, ctx->d_scalar, ctx->stream);
     if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
     ctx->cnt.kernel_launches += 1;
-    if (ctx->nranks > 1) NC(nccl().AllReduce(ctx->d_scalar, ctx->d_scalar, 1, ncclUint64, ncclMax, ctx->nccl_comm, ctx->stream));
-    CU(cudaMemcpyAsync(ctx->h_scalar, ctx->d_scalar, 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    ctx->cnt.d2h_bytes += 8;
-    *out = bits_to_double(*ctx->h_scalar);
+    TRY(read_back(ctx, ctx->d_scalar, 1, Reduce::max_u64));
+    *out = bits_to_double(ctx->h_scalar[0]);
     return LSM_OK;
 }
 

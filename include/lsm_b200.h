@@ -96,6 +96,7 @@ typedef struct {
     int64_t pair_launches;    /* stage launches that took the x-pair kernel (3-D single-term WENO5 advection)  */
     int64_t resident_steps;   /* time steps taken inside the resident cluster kernel (small 2-D grids; one launch per lsm_integrate) */
     int64_t jacobi_sweeps;    /* Jacobi sweeps of LSM_SEMI_IMPLICIT steps (k per step, see lsm_semi_implicit_sweeps)          */
+    int64_t band_full_scans;  /* narrow-band rebuilds that scanned every brick (see lsm_field_set_band)                        */
 } lsm_counters;
 
 /* options for lsm_set_option */
@@ -244,6 +245,38 @@ int32_t lsm_integrate(lsm_ctx* ctx, int32_t integrator, double cfl, lsm_field* p
  * max(1, ceil(log(tol) / log(q))), q = (C/2) / (1 + C/2) the contraction factor of a sweep, tol = 1e-15 (LSM_F64) or 1e-8
  * (LSM_F32); k = 1 when q = 0.  More than 2^24 sweeps: LSM_ERR_ARG. */
 int32_t lsm_semi_implicit_sweeps(double courant, int32_t dtype, int64_t* sweeps_out);
+
+/* ---- narrow band: step only the bricks near the zero level set ---------------------------------------------------------------
+ * The idea of the reference's NarrowBandMeshField and update_band! (meshfield.jl:314-588), not its bits: storage stays dense and
+ * nodes off the band are frozen (the reference stores no values there and extrapolates off-band reads).
+ *  - Bricks: a 3-D field is cut into bricks of 32 x 16 x 16 nodes (x, y, z), a 2-D field into 32 x 16 - the tiled stage kernel's
+ *    x-y tile, so one CTA handles one brick.  Brick b (0-based) holds the nodes B_d b_d <= i_d < min(n_d, B_d (b_d + 1)); bricks are
+ *    numbered column-major, and partial bricks at the high faces are ordinary bricks.
+ *  - Band of phi with halfwidth w > 0: gamma = w * min_d |h_d|.  A CORE brick holds a node with !(|double(phi)| > gamma), i.e.
+ *    |phi| <= gamma or NaN.  The neighbourhood N(b) is every brick b' with b'_d in R_d(b_d) on each axis, R_d(b) = {b-1, b, b+1} in
+ *    range; on a PERIODIC axis (node n duplicates node 1, boundaryconditions.jl:107-119) R_d also wraps: a brick holding any of the
+ *    nodes 0..2 adds the brick(s) holding nodes n-4..n-2, and a brick holding any of the nodes n-3..n-1 adds the brick holding nodes
+ *    1..3.  ACTIVE = the bricks with a core brick in N(b); SHELL = the bricks in N(a) of an active brick a that are not active;
+ *    every other brick is FROZEN.  No stencil read (reach 3) of a brick's nodes leaves N(b).
+ *  - A step of a band field is the dense step, with the same dt and the same stage arithmetic, in which every node outside the
+ *    active bricks holds phi^n at every stage: the step copies phi into the stage buffers on the shell bricks (RK2, RK3), the stage
+ *    kernels write the active bricks only, and ForwardEuler copies the active bricks of its buffer back into phi.  A node that is
+ *    never active keeps its bits; values off the band are stale by design.  dt is the whole-grid CFL step, as for the dense field.
+ *  - The band is rebuilt from phi at stage 1 of a step and by lsm_field_band.  After a band step only the active bricks have
+ *    changed, so the rebuild rescans only them; any other write to phi (upload, copy, fill, CSG, redistance, a dense stage) forces
+ *    a scan of every brick (lsm_counters.band_full_scans).  Both give the same band.  Everything stays on the device: a band step
+ *    reads nothing back.
+ *  - The band applies to lsm_stage, lsm_advance and lsm_integrate with phi as the state.  Every other operation sees the dense
+ *    field (measures, integrals, extraction, redistancing, interpolation, CSG, and lsm_extend_along_normals, which also steps a
+ *    band field F densely).  lsm_integrate uses neither its CUDA-graph nor its resident 2-D path for a band field, and
+ *    LSM_SEMI_IMPLICIT refuses one (LSM_ERR_UNSUPPORTED).  Expression coefficients are still filled over the whole grid at each
+ *    stage time. */
+/* w > 0 and finite turns the band on (or changes w); w = 0 turns it off and frees its scratch (a few bytes per brick); anything else
+ * LSM_ERR_ARG.  nranks > 1, 1-D fields, separable and vector fields: LSM_ERR_UNSUPPORTED. */
+int32_t lsm_field_set_band(lsm_field* phi, double halfwidth);
+/* Rebuilds the band if phi has changed since, and returns counts3 = (core, active, shell) bricks and, when states is not NULL, one
+ * byte per brick: 0 frozen, 1 shell, 2 active, 3 active and core.  Blocking.  LSM_ERR_ARG when phi has no band. */
+int32_t lsm_field_band(lsm_field* phi, int64_t* counts3, uint8_t* states);
 
 /* EikonalReinitializationTerm(phi0) constructor (levelsetterms.jl:217-221): dst = phi0/sqrt(phi0^2+min(h)^2). */
 int32_t lsm_eikonal_s0(lsm_field* dst, const lsm_field* phi0);

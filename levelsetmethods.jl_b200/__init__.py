@@ -8,7 +8,7 @@ Julia API for this path), ``julia/`` (the ccall glue for the real package).
 from . import _lib
 from ._lib import LSMError, CFLError, TimeError, BCError, build
 from .api import (Context, MultiContext, integrate_multi, compute_cfl_multi, default_context, set_default_context, CartesianGrid, BoundaryCondition, PeriodicBC,
-                  ExtrapolationBC, NeumannBC, LinearExtrapolationBC, SymmetryBC, MeshField, Upwind, WENO5,
+                  ExtrapolationBC, NeumannBC, LinearExtrapolationBC, SymmetryBC, MeshField, NarrowBandMeshField, Upwind, WENO5,
                   TimeScaled, DeviceExpr, SeparableVelocity, LevelSetTerm, AdvectionTerm, CurvatureTerm, NormalMotionTerm,
                   EikonalReinitializationTerm, update_term, compute_cfl, step_plan, TimeIntegrator, ForwardEuler, RK2, RK3, SemiImplicit, semi_implicit_sweeps,
                   LevelSetEquation, current_state, current_time, integrate, integrate_bang, volume, perimeter, eikonal_reinitialize, extend_along_normals,

@@ -40,7 +40,8 @@ class lsm_counters(C.Structure):
     _fields_ = [("kernel_launches", C.c_int64), ("stage_launches", C.c_int64), ("cfl_passes", C.c_int64),
                 ("h2d_bytes", C.c_int64), ("d2h_bytes", C.c_int64), ("halo_bytes_sent", C.c_int64),
                 ("last_stage_ms", C.c_double), ("sum_stage_ms", C.c_double), ("timed_stages", C.c_int64),
-                ("pair_launches", C.c_int64), ("resident_steps", C.c_int64), ("jacobi_sweeps", C.c_int64)]
+                ("pair_launches", C.c_int64), ("resident_steps", C.c_int64), ("jacobi_sweeps", C.c_int64),
+                ("band_full_scans", C.c_int64)]
 
 
 class LSMError(RuntimeError):
@@ -102,6 +103,8 @@ SYMBOLS = {
     "lsm_field_meshsize": (_i32, [_vp, _pdbl]),
     "lsm_field_getindex": (_i32, [_vp, _pi32, _i32, _pdbl]),
     "lsm_field_stage_buffer": (_i32, [_vp, _i32, C.POINTER(_vp)]),
+    "lsm_field_set_band": (_i32, [_vp, _dbl]),
+    "lsm_field_band": (_i32, [_vp, C.POINTER(_i64), _vp]),
     "lsm_compute_cfl": (_i32, [_vp, _vp, C.POINTER(lsm_term), _i32, _dbl, _pdbl, _pdbl]),
     "lsm_nstages": (_i32, [_i32]),
     "lsm_stage": (_i32, [_vp, _i32, _i32, _vp, C.POINTER(lsm_term), _i32, _dbl, _dbl, _pdbl]),

@@ -553,6 +553,49 @@ class MeshField:
         return f"MeshField on {self.mesh!r}, valtype={self._dtype}, bc={self.bcs}"
 
 
+BRICK = (32, 16, 16)     # narrow-band brick extents (x, y, z), include/lsm_b200.h
+
+
+class NarrowBandMeshField(MeshField):
+    """``NarrowBandMeshField(phi; halfwidth = 3)`` (meshfield.jl:314-588): a copy of ``phi`` whose explicit steps update only the
+    bricks near its zero level set (``lsm_field_set_band``).  Storage stays dense and nodes off the band keep their values; every
+    other operation sees the whole field.  ``halfwidth`` is in cells of the smallest mesh size; bricks are 32 x 16 (x 16) nodes."""
+
+    def __init__(self, phi: MeshField, halfwidth: float = 3):
+        self._adopt(phi.copy(), halfwidth)
+
+    def _adopt(self, f: MeshField, halfwidth: float):
+        self.__dict__.update(f.__dict__)
+        f._dev = None            # the handle now belongs to self
+        self.halfwidth = float(halfwidth)
+        self._band_handle = None
+        self.device()            # refusals (1-D, vector field, bad halfwidth, nranks > 1) surface here
+
+    def device(self):
+        h = super().device()
+        if self._band_handle != h.value:
+            L.check(L.lib().lsm_field_set_band(h, self.halfwidth))
+            self._band_handle = h.value
+        return h
+
+    def copy(self) -> "NarrowBandMeshField":
+        out = NarrowBandMeshField.__new__(NarrowBandMeshField)
+        out._adopt(MeshField.copy(self), self.halfwidth)
+        return out
+
+    def band_info(self) -> dict:
+        """The band of the current values (``lsm_field_band``): counts of ``core``, ``active`` and ``shell`` bricks, and ``states``,
+        one byte per brick in an array of brick coordinates (0 frozen, 1 shell, 2 active, 3 active and core)."""
+        nb = tuple(-(-n // b) for n, b in zip(self.mesh.n, BRICK))
+        states = np.empty(nb, dtype=np.uint8, order="F")
+        counts = (C.c_int64 * 3)()
+        L.check(L.lib().lsm_field_band(self.device(), counts, states.ctypes.data))
+        return {"core": counts[0], "active": counts[1], "shell": counts[2], "states": states}
+
+    def __repr__(self):
+        return f"NarrowBandMeshField on {self.mesh!r}, valtype={self._dtype}, bc={self.bcs}, halfwidth={self.halfwidth}"
+
+
 def _add_boundary_conditions(phi: MeshField, bc) -> MeshField:
     """meshfield.jl:150-153 — same data, new BCs (the data is aliased)."""
     out = MeshField.__new__(MeshField)

@@ -143,6 +143,12 @@ struct lsm_field {
     bool expr_cfl_read = false;  // expr_cfl_bits holds that maximum, all-reduced over ranks
     unsigned long long expr_cfl_bits = 0;
     unsigned long long* d_expr_cfl = nullptr;
+    // narrow band (lsm_field_set_band): halfwidth (0: off), bricks, the device scratch of BandArgs, and the versions of this field
+    // that the band's states describe and that the last band step left (its active list is the one still in the scratch)
+    double band_w = 0;
+    int band_nb = 0;
+    void* d_band = nullptr;
+    uint64_t band_built_ver = 0, band_step_ver = 0;
 };
 
 namespace {
@@ -223,6 +229,7 @@ void field_free(lsm_field* f) {
     if (f->base) cudaFree(f->base);
     if (f->d_tabs) cudaFree(f->d_tabs);
     if (f->d_expr_cfl) cudaFree(f->d_expr_cfl);
+    if (f->d_band) cudaFree(f->d_band);
     delete f;
 }
 
@@ -492,7 +499,7 @@ int32_t launch_stage_range(lsm_ctx* c, int ndim, StageParams<T>& P, int r0, int 
 // order, with the output's halo exchange overlapped with the interior update.
 template <class T>
 int32_t run_stage_t(lsm_ctx* c, lsm_field* in, lsm_field* p0, lsm_field* out, lsm_field* out2, int base, double cc, double c2,
-                    const lsm_term* terms, int nterms, double tstage, const double* gscale, bool out_needs_halo) {
+                    const lsm_term* terms, int nterms, double tstage, const double* gscale, bool out_needs_halo, const int* bricks) {
     NvtxRange nvtx("lsm RK stage");
     StageParams<T> P{};
     P.in = make_view<T>(in);
@@ -507,6 +514,7 @@ int32_t run_stage_t(lsm_ctx* c, lsm_field* in, lsm_field* p0, lsm_field* out, ls
     for (int k = 0; k < nterms; ++k)
         if (terms[k].coef_kind == LSM_COEF_EXPR) TRY(expr_ensure(terms[k].field, tstage, terms[k].kind, false));
     P.skip_zero_u = c->stage_skip_zero_u;
+    P.bricks = bricks;
 
     const int last = in->ndim - 1, nl = in->n[last];
     if (c->nranks > 1 && !in->halo_valid) {        // e.g. right after an upload
@@ -547,10 +555,11 @@ int32_t run_stage_t(lsm_ctx* c, lsm_field* in, lsm_field* p0, lsm_field* out, ls
     return LSM_OK;
 }
 
+// bricks: the narrow band's active list (only those bricks of out and out2 are written), or nullptr for the whole field
 int32_t run_stage(lsm_ctx* c, lsm_field* in, lsm_field* p0, lsm_field* out, lsm_field* out2, int base, double cc, double c2,
-                  const lsm_term* terms, int nterms, double tstage, const double* gscale, bool out_needs_halo) {
-    if (in->dtype == LSM_F64) return run_stage_t<double>(c, in, p0, out, out2, base, cc, c2, terms, nterms, tstage, gscale, out_needs_halo);
-    return run_stage_t<float>(c, in, p0, out, out2, base, cc, c2, terms, nterms, tstage, gscale, out_needs_halo);
+                  const lsm_term* terms, int nterms, double tstage, const double* gscale, bool out_needs_halo, const int* bricks = nullptr) {
+    if (in->dtype == LSM_F64) return run_stage_t<double>(c, in, p0, out, out2, base, cc, c2, terms, nterms, tstage, gscale, out_needs_halo, bricks);
+    return run_stage_t<float>(c, in, p0, out, out2, base, cc, c2, terms, nterms, tstage, gscale, out_needs_halo, bricks);
 }
 
 void swap_storage(lsm_field* a, lsm_field* b) {
@@ -570,30 +579,105 @@ int32_t check_state(lsm_ctx* ctx, lsm_field* phi, const lsm_term* terms, int nte
 // LSM_SEMI_IMPLICIT: one whole step (below, after the CFL code it uses)
 int32_t si_step(lsm_ctx* ctx, lsm_field* phi, const lsm_term* terms, int nterms, double tc, double dt, const double* gs);
 
-int32_t stage_impl(lsm_ctx* ctx, int integ, int stage, lsm_field* phi, const lsm_term* terms, int nterms, double tc, double dt, const double* gs) {
+// ---- narrow band (lsm_field_set_band; kernels in lsm_narrow_band.cu) --------------------------------------------------------
+// d_band: the three counts (padded to 32 bytes), the active and shell lists (nb + 1 ints each), then core flags and states (nb bytes each)
+size_t band_bytes(int nb) { return 32 + 2 * ((size_t)nb + 1) * sizeof(int) + 2 * (size_t)nb; }
+
+BandArgs band_args(const lsm_field* f) {
+    BandArgs A{};
+    A.phi = f->p; A.f64 = f->dtype == LSM_F64; A.ndim = f->ndim;
+    double hmin = std::fabs(f->h[0]);
+    for (int d = 0; d < 3; ++d) {
+        A.n[d] = f->n[d];
+        A.periodic[d] = d < f->ndim && f->bc[d][0].kind == LSM_BC_PERIODIC;
+        if (d < f->ndim) hmin = std::min(hmin, std::fabs(f->h[d]));
+    }
+    A.nbricks = f->band_nb; A.gamma = f->band_w * hmin;
+    char* p = static_cast<char*>(f->d_band);
+    A.counts = reinterpret_cast<long long*>(p);
+    A.active = reinterpret_cast<int*>(p + 32);
+    A.shell = A.active + f->band_nb + 1;
+    A.core = reinterpret_cast<uint8_t*>(A.shell + f->band_nb + 1);
+    A.state = A.core + f->band_nb;
+    return A;
+}
+
+// The band of phi's current values.  After a band step only that step's active bricks have changed, so only their core flags are
+// recomputed; any other write to phi has changed its version and costs a full scan.  Both give the same band.
+int32_t band_rebuild(lsm_ctx* ctx, lsm_field* phi) {
+    if (phi->band_built_ver == phi->version) return LSM_OK;
+    const bool incremental = phi->band_step_ver == phi->version;
+    int launches = 0;
+    const cudaError_t e = launch_band_rebuild(band_args(phi), incremental, ctx->stream, &launches);
+    if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "narrow-band rebuild launch failed: %s", cudaGetErrorString(e));
+    ctx->cnt.kernel_launches += launches;
+    if (!incremental) ctx->cnt.band_full_scans += 1;
+    phi->band_built_ver = phi->version;
+    return LSM_OK;
+}
+
+// Before a band stage: stage 1 rebuilds the band and, for RK2 / RK3, copies phi^n into the stage buffers on the shell, where the
+// later stages read them.  *bricks = the active list.
+int32_t band_prepare(lsm_ctx* ctx, lsm_field* phi, int integ, int stage, const int** bricks) {
+    TRY(ensure_buffers(phi, integ == LSM_FORWARD_EULER ? 1 : 2));
+    if (stage == 1 || phi->band_built_ver == 0) TRY(band_rebuild(ctx, phi));
+    const BandArgs A = band_args(phi);
+    if (stage == 1 && integ != LSM_FORWARD_EULER) {
+        const cudaError_t e = launch_band_copy(A, A.shell, phi->p, phi->buf1->p, phi->buf2->p, ctx->stream);
+        if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "narrow-band shell copy launch failed: %s", cudaGetErrorString(e));
+        ctx->cnt.kernel_launches += 1;
+        mark_written(phi->buf1); mark_written(phi->buf2);
+    }
+    *bricks = A.active;
+    return LSM_OK;
+}
+
+// dense = true: phi's narrow band (if any) does not apply (lsm_extend_along_normals steps its F densely)
+int32_t stage_impl(lsm_ctx* ctx, int integ, int stage, lsm_field* phi, const lsm_term* terms, int nterms, double tc, double dt, const double* gs,
+                   bool dense = false) {
+    const int ns = integ == LSM_RK2 ? 2 : integ == LSM_RK3 ? 3 : 1;
+    const int* bk = nullptr;        // the narrow band's active bricks: the only ones a stage writes
+    bool clean = false;             // phi still holds the values the band was built from
+    if (phi->band_w > 0 && !dense && integ >= LSM_FORWARD_EULER && integ <= LSM_RK3 && stage >= 1 && stage <= ns) {
+        TRY(band_prepare(ctx, phi, integ, stage, &bk));
+        clean = phi->version == phi->band_built_ver;
+    }
     switch (integ) {
         case LSM_FORWARD_EULER:      // timestepping.jl:128-137
             if (stage != 1) return fail(LSM_ERR_ARG, "ForwardEuler has 1 stage");
             TRY(ensure_buffers(phi, 1));
-            TRY(run_stage(ctx, phi, nullptr, phi->buf1, nullptr, BASE_IN, dt, 0, terms, nterms, tc, gs, true));
-            swap_storage(phi, phi->buf1);          // copy!(phi, dst) without the copy
-            return LSM_OK;
+            TRY(run_stage(ctx, phi, nullptr, phi->buf1, nullptr, BASE_IN, dt, 0, terms, nterms, tc, gs, true, bk));
+            if (bk) {                // copy the active bricks back: a swap would expose stale buffer values off the band
+                const BandArgs A = band_args(phi);
+                const cudaError_t e = launch_band_copy(A, A.active, phi->buf1->p, phi->p, nullptr, ctx->stream);
+                if (e != cudaSuccess) return fail(LSM_ERR_CUDA, "narrow-band write-back launch failed: %s", cudaGetErrorString(e));
+                ctx->cnt.kernel_launches += 1;
+                mark_written(phi);
+            } else {
+                swap_storage(phi, phi->buf1);          // copy!(phi, dst) without the copy
+            }
+            break;
         case LSM_RK2:                // timestepping.jl:143-164
             TRY(ensure_buffers(phi, 2));
-            if (stage == 1) return run_stage(ctx, phi, nullptr, phi->buf1, phi->buf2, BASE_IN, dt, 0.5 * dt, terms, nterms, tc, gs, true);
-            if (stage == 2) return run_stage(ctx, phi->buf1, phi->buf2, phi, nullptr, BASE_P0, 0.5 * dt, 0, terms, nterms, tc + dt, gs, true);
-            return fail(LSM_ERR_ARG, "RK2 has 2 stages");
+            if (stage == 1) TRY(run_stage(ctx, phi, nullptr, phi->buf1, phi->buf2, BASE_IN, dt, 0.5 * dt, terms, nterms, tc, gs, true, bk));
+            else if (stage == 2) TRY(run_stage(ctx, phi->buf1, phi->buf2, phi, nullptr, BASE_P0, 0.5 * dt, 0, terms, nterms, tc + dt, gs, true, bk));
+            else return fail(LSM_ERR_ARG, "RK2 has 2 stages");
+            break;
         case LSM_RK3:                // timestepping.jl:170-202
             TRY(ensure_buffers(phi, 2));
-            if (stage == 1) return run_stage(ctx, phi, nullptr, phi->buf1, nullptr, BASE_IN, dt, 0, terms, nterms, tc, gs, true);
-            if (stage == 2) return run_stage(ctx, phi->buf1, phi, phi->buf2, nullptr, BASE_RK3_S2, 0.25 * dt, 0, terms, nterms, tc + dt, gs, true);
-            if (stage == 3) return run_stage(ctx, phi->buf2, phi, phi, nullptr, BASE_RK3_S3, (2.0 / 3.0) * dt, 0, terms, nterms, tc + 0.5 * dt, gs, true);
-            return fail(LSM_ERR_ARG, "RK3 has 3 stages");
+            if (stage == 1) TRY(run_stage(ctx, phi, nullptr, phi->buf1, nullptr, BASE_IN, dt, 0, terms, nterms, tc, gs, true, bk));
+            else if (stage == 2) TRY(run_stage(ctx, phi->buf1, phi, phi->buf2, nullptr, BASE_RK3_S2, 0.25 * dt, 0, terms, nterms, tc + dt, gs, true, bk));
+            else if (stage == 3) TRY(run_stage(ctx, phi->buf2, phi, phi, nullptr, BASE_RK3_S3, (2.0 / 3.0) * dt, 0, terms, nterms, tc + 0.5 * dt, gs, true, bk));
+            else return fail(LSM_ERR_ARG, "RK3 has 3 stages");
+            break;
         case LSM_SEMI_IMPLICIT:
             if (stage != 1) return fail(LSM_ERR_ARG, "the semi-implicit integrator has 1 stage (a whole step)");
             return si_step(ctx, phi, terms, nterms, tc, dt, gs);
         default: return fail(LSM_ERR_ARG, "bad integrator %d", integ);
     }
+    // the last stage of a band step: the next rebuild need only rescan this band's active bricks
+    if (bk && stage == ns) phi->band_step_ver = clean ? phi->version : 0;
+    return LSM_OK;
 }
 
 int nstages(int integ) { return integ == LSM_FORWARD_EULER || integ == LSM_SEMI_IMPLICIT ? 1 : integ == LSM_RK2 ? 2 : 3; }
@@ -616,7 +700,7 @@ void plan_steps(double t0, double tf, double dt_max, double cfl, double dt_cfl, 
 // lsm_resident2d.cu covers: single rank, 2-D, ONE AdvectionTerm(stored velocity of the state's dtype, WENO5) without a time factor,
 // index-map boundary conditions (periodic / Neumann / symmetry), automatic kernel selection, no per-stage timing
 bool resident_eligible(const lsm_ctx* ctx, const lsm_field* phi, const lsm_term* terms, int nterms) {
-    if (!ctx->opt_resident || ctx->nranks != 1 || ctx->opt_time || ctx->opt_kernel != 0) return false;
+    if (!ctx->opt_resident || ctx->nranks != 1 || ctx->opt_time || ctx->opt_kernel != 0 || phi->band_w > 0) return false;
     if (phi->ndim != 2 || nterms != 1) return false;
     const lsm_term& t = terms[0];
     if (t.kind != LSM_TERM_ADVECTION || t.scheme != LSM_WENO5 || t.coef_kind != LSM_COEF_FIELD || t.tscale_kind != LSM_TS_NONE) return false;
@@ -897,6 +981,7 @@ int32_t si_sweeps(double courant, int dtype, int64_t* k) {
 
 int32_t si_check(lsm_ctx* ctx, const lsm_field* phi, const lsm_term* terms, int nterms) {
     TRY(check_level_set(ctx, phi, "the semi-implicit integrator", 2, true));
+    if (phi->band_w > 0) return fail(LSM_ERR_UNSUPPORTED, "the semi-implicit integrator does not support narrow-band fields (lsm_field_set_band)");
     if (nterms != 1 || terms[0].kind != LSM_TERM_ADVECTION)
         return fail(LSM_ERR_ARG, "the semi-implicit integrator takes exactly one AdvectionTerm (got %d terms, the first of kind %d)", nterms, terms[0].kind);
     for (int d = 0; d < phi->ndim; ++d)
@@ -1322,6 +1407,7 @@ int32_t lsm_field_set_bc(lsm_field* f, const lsm_bc* bc) {
     }
     write_bcs(f, nb, true);
     for (lsm_field* g : {f, f->buf1, f->buf2}) if (g) g->halo_valid = false;
+    f->band_built_ver = 0;          // a periodic axis changes the neighbourhoods of the narrow band
     return LSM_OK;
 }
 
@@ -1369,6 +1455,47 @@ int32_t lsm_field_stage_buffer(lsm_field* phi, int32_t which, lsm_field** out) {
     CU(cudaSetDevice(phi->ctx->device));
     TRY(ensure_buffers(phi, which));
     *out = which == 1 ? phi->buf1 : phi->buf2;
+    return LSM_OK;
+}
+
+int32_t lsm_field_set_band(lsm_field* phi, double halfwidth) {
+    if (!phi) return fail(LSM_ERR_ARG, "lsm_field_set_band: null argument");
+    lsm_ctx* c = phi->ctx;
+    if (c->nranks > 1) return fail(LSM_ERR_UNSUPPORTED, "lsm_field_set_band: slab decomposition is not supported (nranks = %d)", c->nranks);
+    if (phi->ndim == 1) return fail(LSM_ERR_UNSUPPORTED, "lsm_field_set_band: 1-D fields have no narrow band");
+    if (phi->separable || phi->ncomp != 1) return fail(LSM_ERR_UNSUPPORTED, "lsm_field_set_band needs a scalar field with stored values");
+    if (!(halfwidth == 0.0 || (halfwidth > 0.0 && std::isfinite(halfwidth))))
+        return fail(LSM_ERR_ARG, "lsm_field_set_band: the halfwidth must be finite and > 0, or 0 to turn the band off (got %g)", halfwidth);
+    CU(cudaSetDevice(c->device));
+    if (halfwidth == 0.0) {
+        if (phi->d_band) { CU(cudaStreamSynchronize(c->stream)); cudaFree(phi->d_band); }
+        phi->d_band = nullptr; phi->band_nb = 0;
+    } else if (!phi->d_band) {
+        const int nb = band_bricks(phi->ndim, phi->n);
+        if (nb < 0) return fail(LSM_ERR_UNSUPPORTED, "lsm_field_set_band: more than 2^30 bricks");
+        cudaError_t e = cudaMalloc(&phi->d_band, band_bytes(nb));
+        if (e != cudaSuccess) { phi->d_band = nullptr; return fail(LSM_ERR_OOM, "lsm_field_set_band: cudaMalloc failed: %s", cudaGetErrorString(e)); }
+        phi->band_nb = nb;
+    }
+    phi->band_w = halfwidth;
+    phi->band_built_ver = phi->band_step_ver = 0;
+    return LSM_OK;
+}
+
+int32_t lsm_field_band(lsm_field* phi, int64_t* counts3, uint8_t* states) {
+    if (!phi || !counts3) return fail(LSM_ERR_ARG, "lsm_field_band: null argument");
+    if (!(phi->band_w > 0)) return fail(LSM_ERR_ARG, "lsm_field_band: the field has no narrow band (lsm_field_set_band)");
+    lsm_ctx* c = phi->ctx;
+    CU(cudaSetDevice(c->device));
+    TRY(band_rebuild(c, phi));
+    const BandArgs A = band_args(phi);
+    TRY(read_back(c, A.counts, 3, Reduce::none));
+    for (int k = 0; k < 3; ++k) counts3[k] = (int64_t)c->h_scalar[k];
+    if (states) {
+        CU(cudaMemcpyAsync(states, A.state, (size_t)A.nbricks, cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaStreamSynchronize(c->stream));
+        c->cnt.d2h_bytes += A.nbricks;
+    }
     return LSM_OK;
 }
 
@@ -1523,7 +1650,7 @@ int32_t lsm_integrate(lsm_ctx* ctx, int32_t integrator, double cfl, lsm_field* p
     // per-stage timing — the stage launches of one step are captured once into a CUDA graph and every later step with the same
     // dt replays it (one graph launch instead of 2-3 kernel launches plus their host-side setup).
     bool graph_ok = ctx->opt_graph && ctx->nranks == 1 && integrator != LSM_FORWARD_EULER && integrator != LSM_SEMI_IMPLICIT && !ctx->opt_time &&
-                    phi->owned <= (1L << 22);
+                    phi->owned <= (1L << 22) && !(phi->band_w > 0);     // a band step's launches depend on the band
     // (a time-dependent expression coefficient is materialised at each stage time: a captured fill would freeze t)
     for (int k = 0; k < nterms && graph_ok; ++k) if (terms[k].tscale_kind != LSM_TS_NONE || terms[k].coef_kind == LSM_COEF_EXPR) graph_ok = false;
     cudaGraphExec_t gexec = nullptr;
@@ -1692,7 +1819,7 @@ int32_t lsm_extend_along_normals(lsm_ctx* ctx, lsm_field* F, lsm_field* phi, int
         // frozen / degenerate nodes carry a zero velocity: with skip_zero_u they keep their value exactly even when a neighbour of
         // F is NaN / Inf (F is often undefined away from the interface) — the reference copies them untouched (velocityextension.jl:53-56)
         ctx->stage_skip_zero_u = 1;
-        for (int it = 0; it < nb_iters && rc == LSM_OK; ++it) rc = stage_impl(ctx, LSM_FORWARD_EULER, 1, F, &term, 1, 0.0, tau, nullptr);
+        for (int it = 0; it < nb_iters && rc == LSM_OK; ++it) rc = stage_impl(ctx, LSM_FORWARD_EULER, 1, F, &term, 1, 0.0, tau, nullptr, true);
         ctx->stage_skip_zero_u = 0;
     }
     cudaStreamSynchronize(ctx->comm);

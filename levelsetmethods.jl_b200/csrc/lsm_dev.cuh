@@ -27,6 +27,9 @@ enum : int {
 
 struct BCDev { int kind, P; };
 
+// Narrow-band bricks (lsm_narrow_band.cu): the tiled stage kernel's x-y tile times 16 planes; 2-D fields use BRICK_X x BRICK_Y
+enum : int { BRICK_X = 32, BRICK_Y = 16, BRICK_Z = 16 };
+
 // Is a boundary side (kind, extrapolation order P) a pure index map with weight 1: periodic, symmetry, ExtrapolationBC{0}, or
 // the stored ghost planes of the decomposed axis?  ExtrapolationBC{P >= 1} is a weighted stencil.  Takes the BC_* kinds of a
 // View and the LSM_BC_* kinds of a field alike (they share 0..2; BC_HALO appears only on the last axis, see make_view).
@@ -69,8 +72,10 @@ struct StageParams {
     int r0, r1;          // range [r0, r1) of the LAST dimension to update (interior/boundary split)
     int skip_zero_u;     // upwind advection: a component with u_d == 0 contributes exactly 0 even when its one-sided difference is
     int _pad1;           // NaN / Inf (extend_along_normals!: frozen nodes keep their value, velocityextension.jl:53-56)
-    double _pad2;        // keeps terms[] 8 bytes past a 16-byte boundary: that alignment decides which of its fields the stage
-                         // kernels fetch in pairs with 128-bit constant loads, and so the code they compile to
+    const int* bricks;   // narrow band: device list {count, brick, brick, ...} of the bricks to update (BRICK_X x BRICK_Y x BRICK_Z,
+                         // column-major numbering), or nullptr for the whole box.  Its 8 bytes keep terms[] 8 bytes past a 16-byte
+                         // boundary: that alignment decides which of its fields the stage kernels fetch in pairs with 128-bit
+                         // constant loads, and so the code they compile to
     TermDev terms[4];
 };
 

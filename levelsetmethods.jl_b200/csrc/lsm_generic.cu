@@ -232,14 +232,28 @@ template <int N, class T>
 __global__ void __launch_bounds__(256) stage_generic_kernel(const __grid_constant__ StageParams<T> P) {
     const View<T>& v = P.in;
     const int n0 = v.n[0], n1 = v.n[1];
-    const int nr = P.r1 - P.r0;
-    const long total = (N == 1) ? (long)nr : (N == 2) ? (long)n0 * nr : (long)n0 * n1 * nr;
-    const long idx = (long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx >= total) return;
     int i0, i1 = 0, i2 = 0;
-    if (N == 1) { i0 = P.r0 + (int)idx; }
-    else if (N == 2) { i0 = (int)(idx % n0); i1 = P.r0 + (int)(idx / n0); }
-    else { i0 = (int)(idx % n0); long q = idx / n0; i1 = (int)(q % n1); i2 = P.r0 + (int)(q / n1); }
+    if (N > 1 && P.bricks) {
+        // narrow band: the blocks of list entry e cover the nodes of brick P.bricks[1 + e] (x fastest); entries past the count exit
+        constexpr int BN = BRICK_X * BRICK_Y * (N == 3 ? BRICK_Z : 1);
+        const long local = (long)blockIdx.x * blockDim.x + threadIdx.x;
+        const int e = (int)(local / BN), q = (int)(local % BN);
+        if (e >= P.bricks[0]) return;
+        const int b = P.bricks[1 + e];
+        const int nbx = (n0 + BRICK_X - 1) / BRICK_X, nby = (n1 + BRICK_Y - 1) / BRICK_Y;
+        i0 = (b % nbx) * BRICK_X + q % BRICK_X;
+        i1 = ((b / nbx) % nby) * BRICK_Y + (q / BRICK_X) % BRICK_Y;
+        if (N == 3) i2 = (b / (nbx * nby)) * BRICK_Z + q / (BRICK_X * BRICK_Y);
+        if (i0 >= n0 || i1 >= n1 || (N == 3 && i2 >= v.n[2])) return;
+    } else {
+        const int nr = P.r1 - P.r0;
+        const long total = (N == 1) ? (long)nr : (N == 2) ? (long)n0 * nr : (long)n0 * n1 * nr;
+        const long idx = (long)blockIdx.x * blockDim.x + threadIdx.x;
+        if (idx >= total) return;
+        if (N == 1) { i0 = P.r0 + (int)idx; }
+        else if (N == 2) { i0 = (int)(idx % n0); i1 = P.r0 + (int)(idx / n0); }
+        else { i0 = (int)(idx % n0); long q = idx / n0; i1 = (int)(q % n1); i2 = P.r0 + (int)(q / n1); }
+    }
 
     const long lin = (long)i0 + (long)i1 * v.s1 + (long)i2 * v.s2;
     const long node = (long)i0 + (long)n0 * ((long)i1 + (long)n1 * i2);   // coefficient boxes carry no ghosts
@@ -279,7 +293,12 @@ cudaError_t launch_stage_generic(int ndim, const StageParams<T>& P, cudaStream_t
     const View<T>& v = P.in;
     const long nr = P.r1 - P.r0;
     if (nr <= 0) return cudaSuccess;
-    const long total = ndim == 1 ? nr : ndim == 2 ? (long)v.n[0] * nr : (long)v.n[0] * v.n[1] * nr;
+    long total = ndim == 1 ? nr : ndim == 2 ? (long)v.n[0] * nr : (long)v.n[0] * v.n[1] * nr;
+    if (P.bricks) {        // every brick of the box: the list's count stays on the device
+        if (ndim == 1) return cudaErrorNotSupported;
+        const long nb = (long)((v.n[0] + BRICK_X - 1) / BRICK_X) * ((v.n[1] + BRICK_Y - 1) / BRICK_Y) * (ndim == 3 ? (v.n[2] + BRICK_Z - 1) / BRICK_Z : 1);
+        total = nb * BRICK_X * BRICK_Y * (ndim == 3 ? BRICK_Z : 1);
+    }
     const int block = 256;
     const long grid = (total + block - 1) / block;
     if (grid > 2147483647L) return cudaErrorInvalidConfiguration;

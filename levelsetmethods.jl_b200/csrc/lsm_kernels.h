@@ -183,6 +183,28 @@ template <class T> cudaError_t launch_si_rhs(int ndim, const SemiArgs<T>& A, T* 
 // *launches = kernels enqueued.
 template <class T> cudaError_t launch_si_sweeps(int ndim, const SemiArgs<T>& A, int k, T* xa, T* xb, cudaStream_t s, int* launches);
 
+// lsm_narrow_band.cu (lsm_field_set_band): the brick band of a single-rank scalar field in 2-D or 3-D
+struct BandArgs {
+    const void* phi;           // the field (dense, no ghost planes)
+    int f64, ndim;
+    int n[3];                  // nodes per dim (1 for unused dims)
+    int periodic[3];           // axis d is periodic
+    int nbricks;               // band_bricks(ndim, n)
+    double gamma;              // halfwidth * min_d |h_d|
+    // device scratch: one core flag and one state byte per brick (0 frozen, 1 shell, 2 active, 3 active and core), the active and
+    // shell lists {count, brick, ...} (nbricks + 1 ints each) and the (core, active, shell) counts
+    uint8_t* core;
+    uint8_t* state;
+    int* active;
+    int* shell;
+    long long* counts;
+};
+int band_bricks(int ndim, const int* n);       // -1: more than 2^30 bricks
+// core flags (every brick, or from_active: the bricks of the current active list), the states, the two lists and the counts
+cudaError_t launch_band_rebuild(const BandArgs& A, bool from_active, cudaStream_t s, int* launches);
+// the listed bricks of src into d0 and, when not null, d1 (fields of A's box and dtype)
+cudaError_t launch_band_copy(const BandArgs& A, const int* list, const void* src, void* d0, void* d1, cudaStream_t s);
+
 // lsm_tiled.cu (performance kernels), for LSM_OPT_KERNEL value `kernel` (not 1): 3 takes no x-pair kernel, 4 the 3-D x-pair kernel
 // with the exact eps maximum, 2 the 2-D x-pair kernel below its size threshold too.  *used_pair = 1 when an x-pair kernel ran.
 // Returns cudaErrorNotSupported when the configuration is not covered, in which case the caller uses the generic kernel.

@@ -81,9 +81,17 @@ stage_tiled_kernel(const __grid_constant__ StageParams<T> P, const __grid_consta
     const T* __restrict__ const vp = P.in.p;
     const int tx = threadIdx.x, ty = threadIdx.y;
     const int lane = tx & 31, warp = (ty * TX + tx) >> 5;
-    const int x0 = blockIdx.x * TX, y0 = blockIdx.y * (TY * NY);
+    // block -> tile: the grid's own coordinates, or (narrow band) brick blockIdx.x of the list, a tile of cz = BRICK_Z planes
+    unsigned bx = blockIdx.x, by = blockIdx.y, bz = blockIdx.z;
+    if (P.bricks) {
+        if ((int)blockIdx.x >= P.bricks[0]) return;
+        const unsigned b = (unsigned)P.bricks[1 + blockIdx.x];
+        const unsigned nbx = (n0 + TX - 1) / TX, nby = (n1 + TY * NY - 1) / (TY * NY);
+        bx = b % nbx; by = (b / nbx) % nby; bz = b / (nbx * nby);
+    }
+    const int x0 = bx * TX, y0 = by * (TY * NY);
     // range of the LAST dimension to update: z planes in 3-D, rows in 2-D (slab decomposition splits it)
-    const int zbeg = NDIM == 3 ? P.r0 + blockIdx.z * cz : 0;
+    const int zbeg = NDIM == 3 ? P.r0 + bz * cz : 0;
     const int zend = NDIM == 3 ? min(P.r1, zbeg + cz) : 1;
     if (zbeg >= zend) return;
     const int ylo = NDIM == 2 ? P.r0 : 0, yhi = NDIM == 2 ? P.r1 : n1;
@@ -476,7 +484,13 @@ cudaError_t launch_tiled(const StageParams<T>& P, const AuxList& A, cudaStream_t
     }
     dim3 block(TX, TY), grid;
     int cz = 1;
-    if (NDIM == 3) {
+    if (P.bricks) {
+        // one block per brick of the whole box: blocks past the list's device-side count exit at once, so the host never reads it
+        static_assert(TX == BRICK_X && TY * NY == BRICK_Y, "a narrow-band brick is one x-y tile");
+        cz = BRICK_Z;
+        const long nb = (long)((v.n[0] + TX - 1) / TX) * ((v.n[1] + TY * NY - 1) / (TY * NY)) * (NDIM == 3 ? (v.n[2] + cz - 1) / cz : 1);
+        grid = dim3((unsigned)nb, 1, 1);
+    } else if (NDIM == 3) {
         const int nr = P.r1 - P.r0;
         cz = nr >= 128 ? 64 : (nr >= 32 ? 32 : nr);
         grid = dim3((v.n[0] + TX - 1) / TX, (v.n[1] + TY * NY - 1) / (TY * NY), (nr + cz - 1) / cz);
@@ -585,7 +599,9 @@ cudaError_t launch_stage_tiled(int ndim, const StageParams<T>& P, int kernel, in
         }
     }
     if (P.p0) { A.p0 = A.n; A.src[A.n++] = P.p0; }
-    if (kernel != 3) {     // the x-pair kernels (lsm_pair3d.cu, lsm_pair2d.cu) report cudaErrorNotSupported for what they do not cover
+    // the x-pair kernels (lsm_pair3d.cu, lsm_pair2d.cu) report cudaErrorNotSupported for what they do not cover; they have no
+    // brick-list mode
+    if (kernel != 3 && !P.bricks) {
         const cudaError_t e = ndim == 3 ? launch_stage_pair3d<T>(P, A, s, kernel == 4) : launch_stage_pair2d<T>(P, A, s, kernel == 2, sm_count);
         if (e != cudaErrorNotSupported) { *used_pair = 1; return e; }
     }

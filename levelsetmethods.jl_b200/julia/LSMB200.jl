@@ -642,6 +642,34 @@ function redistance!(ϕ::DeviceMeshField; band::Integer = 3, order::Integer = 1)
 end
 
 """
+    narrow_band!(ϕ::DeviceMeshField; halfwidth = 3) -> ϕ
+
+Make the explicit steps of ϕ update only the bricks near its zero level set (`lsm_field_set_band`), the idea of the reference's
+`NarrowBandMeshField` and `update_band!` (meshfield.jl:314-588) with dense storage: nodes off the band keep their values, and every
+other operation sees the whole field.  `halfwidth` is in cells of the smallest mesh size; `halfwidth = 0` turns the band off.
+Bricks are 32 × 16 (× 16) nodes; see include/lsm_b200.h for the band's rules.
+"""
+function narrow_band!(ϕ::DeviceMeshField; halfwidth::Real = 3)
+    check(ccall((:lsm_field_set_band, LIB), Int32, (Ptr{Cvoid}, Float64), handle!(ϕ), Float64(halfwidth)))
+    return ϕ
+end
+
+"""
+    band_info(ϕ::DeviceMeshField) -> (core, active, shell, states)
+
+The band of ϕ's current values (`lsm_field_band`): brick counts and one state per brick in an array of brick coordinates
+(0 frozen, 1 shell, 2 active, 3 active and core).
+"""
+function band_info(ϕ::DeviceMeshField{N}) where {N}
+    n = size(ϕ.vals)
+    nb = ntuple(d -> cld(n[d], (32, 16, 16)[d]), N)
+    states = Array{UInt8, N}(undef, nb)
+    counts = zeros(Int64, 3)
+    check(ccall((:lsm_field_band, LIB), Int32, (Ptr{Cvoid}, Ptr{Int64}, Ptr{UInt8}), handle!(ϕ), counts, states))
+    return (core = counts[1], active = counts[2], shell = counts[3], states = states)
+end
+
+"""
     interpolate_cubic(ϕ::DeviceMeshField, X::AbstractMatrix) -> (values, gradients, hessians)
 
 The tensor-product cubic interpolant of ϕ (`lsm_interpolate_cubic`) at the columns of X (N × npts): `values` (npts),
